@@ -4,7 +4,8 @@
 // srcnn_b200.h, implemented in srcnn_cpp_b200/cli/libsrcnn.cpp and exported by libsrcnn_b200.so.
 //
 //   refbuff   packed 8-bit pixels, `d` bytes per pixel: 3 = RGB, 4 = RGBA (alpha takes the path's plain
-//             bicubic resize -- srcnn_resize_plane_host, no CNN -- colour goes through the SRCNN path), 1 = grey, 2 = grey+alpha -- the inputs
+//             bicubic resize -- srcnn_resize_plane_host, no CNN -- colour goes through the SRCNN path), 1 = grey, 2 = grey+alpha (grey: the
+//             one-plane path, SRCNN_ORDER_GRAY) -- the inputs
 //             src/test.cpp:34-134 (convImage) can produce
 //   w, h, d   geometry
 //   muliply   scale ratio (sic, the reference's spelling)

@@ -14,9 +14,12 @@
  * (0 = OK, negative = error) and never throws.  There is NO CPU fallback: without a usable CUDA
  * device srcnn_create() fails with SRCNN_E_NODEVICE.
  *
- * Pixel format everywhere: 8-bit, 3 interleaved channels (HWC), row stride in BYTES.  `order` says
- * whether memory order is B,G,R (OpenCV / bin/srcnn, src/srcnn.cpp:462) or R,G,B (ProcessSRCNN,
- * src/test.cpp:334).  Output size is ow=(int)((float)w*scale), oh=(int)((float)h*scale) -- the
+ * Pixel formats: 8-bit, row stride in BYTES.  `order` says whether memory order is B,G,R (OpenCV /
+ * bin/srcnn, src/srcnn.cpp:462) or R,G,B (ProcessSRCNN, src/test.cpp:334) -- 3 interleaved channels (HWC)
+ * -- or SRCNN_ORDER_GRAY: one channel, 1 byte per pixel in and out (src_stride >= w, dst_stride >= ow).
+ * A grey call returns the CNN's Y' of resize(grey) and never computes chroma; it is bit-identical to any
+ * channel of the colour path on the grey image replicated to 3 channels (a grey pixel has Y = v and
+ * Cr = Cb = 128, which convert back to B = G = R = Y').  Output size is ow=(int)((float)w*scale), oh=(int)((float)h*scale) -- the
  * reference's truncation (src/srcnn.cpp:573-575, src/test.cpp:357-358).
  */
 #ifndef SRCNN_B200_H
@@ -43,7 +46,7 @@ enum {
     SRCNN_VARIANT_FP32 = 1  /* strict FP32 CUDA-core kernels in the reference's summation order (bit-exact) */
 };
 
-enum { SRCNN_ORDER_BGR = 0, SRCNN_ORDER_RGB = 1 };
+enum { SRCNN_ORDER_BGR = 0, SRCNN_ORDER_RGB = 1, SRCNN_ORDER_GRAY = 2 };
 
 /* Status codes.  -1 / -2 / -3 / -10 keep the reference CLI's meanings (src/srcnn.cpp:479,493,526,555,684). */
 enum {
@@ -194,20 +197,25 @@ int srcnn_jpeg_stream_process(srcnn_jpeg_stream* s, const uint8_t* const* jpegs,
 void srcnn_jpeg_free(uint8_t* p);
 
 /* ---- stages (device pointers; enqueued on the context stream) ------------------------------------ */
-/* cvtColor + split + 3x resize (src/srcnn.cpp:509,540,570-583): BGR8 -> three u8 planes of ow x oh. */
+/* cvtColor + split + 3x resize (src/srcnn.cpp:509,540,570-583): BGR8 -> three u8 planes of ow x oh.  Colour orders only
+ * (SRCNN_ORDER_GRAY: SRCNN_E_ARG; srcnn_stage_resize_plane_device is the one-plane stage). */
 int srcnn_stage_color_bicubic_device(srcnn_ctx* ctx, const uint8_t* d_src, int w, int h, size_t src_stride,
                                      int order, float scale, uint8_t* d_y, uint8_t* d_cr, uint8_t* d_cb,
                                      size_t plane_pitch);
 /* One 8-bit plane through resize(..., CV_INTER_CUBIC) (src/srcnn.cpp:577-582), host buffers (ProcessSRCNN's alpha). */
 int srcnn_resize_plane_host(srcnn_ctx* ctx, const uint8_t* src, int w, int h, size_t src_stride, float scale,
                             uint8_t* dst, size_t dst_stride);
+/* The same on device buffers, enqueued on the context stream: one u8 plane through resize(..., CV_INTER_CUBIC).  Any
+ * stride >= the row and any alignment (an unaligned destination costs one extra device copy). */
+int srcnn_stage_resize_plane_device(srcnn_ctx* ctx, const uint8_t* d_src, int w, int h, size_t src_stride, float scale,
+                                    uint8_t* d_dst, size_t dst_stride);
 /* Convolution99x11 + Convolution55 (src/srcnn.cpp:609,627): Y plane -> Y' plane, `variant` as above. */
 int srcnn_stage_cnn_device(srcnn_ctx* ctx, int variant, const uint8_t* d_y, int w, int h, size_t pitch,
                            uint8_t* d_out, size_t out_pitch);
 /* FP32 variant only: also returns conv2's activations, 32 planes of h*w float (src/srcnn.cpp:602-607). */
 int srcnn_stage_conv99x11_fp32_device(srcnn_ctx* ctx, const uint8_t* d_y, int w, int h, size_t pitch,
                                       float* d_act2);
-/* merge + cvtColor back (src/srcnn.cpp:637-639,657): three planes -> BGR8 HWC. */
+/* merge + cvtColor back (src/srcnn.cpp:637-639,657): three planes -> BGR8 HWC.  Colour orders only. */
 int srcnn_stage_merge_device(srcnn_ctx* ctx, const uint8_t* d_y, const uint8_t* d_cr, const uint8_t* d_cb,
                              int w, int h, size_t plane_pitch, int order, uint8_t* d_dst, size_t dst_stride);
 

@@ -20,6 +20,7 @@ VARIANT_TC = 0
 VARIANT_FP32 = 1
 ORDER_BGR = 0
 ORDER_RGB = 1
+ORDER_GRAY = 2   # one channel: HxW (NxHxW) arrays and tensors in and out; the result is the CNN's Y'
 
 OK = 0
 E_RATIO = -1
@@ -39,7 +40,7 @@ ABI_SYMBOLS = [
     "srcnn_stage_cnn_device", "srcnn_stage_conv99x11_fp32_device", "srcnn_stage_merge_device",
     "srcnn_fraw_scale_device",
     "srcnn_last_failed_stage", "srcnn_get_device", "srcnn_host_register", "srcnn_host_unregister",
-    "srcnn_process_band_host", "srcnn_resize_plane_host",
+    "srcnn_process_band_host", "srcnn_resize_plane_host", "srcnn_stage_resize_plane_device",
     "srcnn_mgpu_create", "srcnn_mgpu_destroy", "srcnn_mgpu_device_count", "srcnn_mgpu_context", "srcnn_mgpu_last_error",
     "srcnn_mgpu_band_plan", "srcnn_mgpu_process_batch_host", "srcnn_mgpu_process_banded_host",
     "srcnn_mgpu_process_batch_device", "srcnn_mgpu_process_banded_device", "srcnn_mgpu_last_timing",
@@ -106,6 +107,7 @@ def load_library():
     L.srcnn_host_unregister.argtypes = [vp]
     L.srcnn_process_band_host.argtypes = [vp, u8p, C.c_int, C.c_int, sz, C.c_int, C.c_float, C.c_int, C.c_int, u8p, sz]
     L.srcnn_resize_plane_host.argtypes = [vp, u8p, C.c_int, C.c_int, sz, C.c_float, u8p, sz]
+    L.srcnn_stage_resize_plane_device.argtypes = [vp, u8p, C.c_int, C.c_int, sz, C.c_float, u8p, sz]
     L.srcnn_mgpu_create.argtypes = [C.POINTER(vp), i32p, C.c_int, C.c_int]
     L.srcnn_mgpu_destroy.argtypes = [vp]
     L.srcnn_mgpu_device_count.argtypes = [vp]
@@ -176,6 +178,18 @@ class PinnedBuffer:
             pass
 
 
+def _pixel_shape(order):
+    """trailing shape of one pixel: () for ORDER_GRAY, (3,) for the colour orders"""
+    return () if order == ORDER_GRAY else (3,)
+
+
+def _check_host_image(a, order, lead):
+    """a: numpy uint8 array of `lead` leading dims (1: HxW[x3], 2: NxHxW[x3]) in the layout `order` implies"""
+    px = _pixel_shape(order)
+    if a.dtype != np.uint8 or a.ndim != lead + 1 + len(px) or tuple(a.shape[lead + 1:]) != px:
+        raise SrcnnError(E_ARG, "expected a %s uint8 array" % ("x".join(["N"] * (lead - 1) + ["H", "W"] + ["3"] * len(px))))
+
+
 def _dptr(t):
     """device pointer of a torch CUDA uint8/float tensor (must be contiguous in its last dim)"""
     return C.c_void_p(t.data_ptr())
@@ -244,27 +258,28 @@ class Engine:
 
     # -- whole path, host buffers (numpy) ----------------------------------------------------------
     def process(self, img, scale, order=ORDER_BGR, out=None):
-        """img: HxWx3 uint8 numpy array (BGR by default, like cv::imread).  Returns OHxOWx3 uint8."""
+        """img: HxWx3 uint8 numpy array (BGR by default, like cv::imread), or HxW with order=ORDER_GRAY.  Returns OHxOWx3
+        (OHxOW) uint8."""
         img = np.asarray(img)
-        if img.ndim != 3 or img.shape[2] != 3 or img.dtype != np.uint8:
-            raise SrcnnError(E_ARG, "expected an HxWx3 uint8 image")
+        _check_host_image(img, order, 1)
         if not img.flags.c_contiguous:
             img = np.ascontiguousarray(img)
-        h, w, _ = img.shape
+        h, w = img.shape[:2]
         ow, oh = out_dims(w, h, scale)
         if out is None:
-            out = np.empty((oh, ow, 3), np.uint8)
+            out = np.empty((oh, ow) + _pixel_shape(order), np.uint8)
         self._check(self.L.srcnn_process_host(self.ctx, img.ctypes.data, w, h, img.strides[0], order, C.c_float(scale),
                                               out.ctypes.data, out.strides[0]))
         return out
 
     def process_batch(self, frames, scale, order=ORDER_BGR, out=None):
-        """frames: NxHxWx3 uint8 numpy array -> NxOHxOWx3."""
+        """frames: NxHxWx3 (NxHxW with order=ORDER_GRAY) uint8 numpy array -> NxOHxOWx3 (NxOHxOW)."""
         frames = np.ascontiguousarray(frames)
-        n, h, w, _ = frames.shape
+        _check_host_image(frames, order, 2)
+        n, h, w = frames.shape[:3]
         ow, oh = out_dims(w, h, scale)
         if out is None:
-            out = np.empty((n, oh, ow, 3), np.uint8)
+            out = np.empty((n, oh, ow) + _pixel_shape(order), np.uint8)
         self._check(self.L.srcnn_process_batch_host(self.ctx, frames.ctypes.data, n, w, h, frames.strides[1],
                                                     frames.strides[0], order, C.c_float(scale), out.ctypes.data,
                                                     out.strides[1], out.strides[0]))
@@ -272,19 +287,20 @@ class Engine:
 
     # -- whole path, device buffers (torch CUDA tensors) -------------------------------------------
     def process_device(self, src, scale, dst, order=ORDER_BGR):
-        h, w, _ = src.shape
+        """src: HxWx3 (HxW with order=ORDER_GRAY) uint8 device tensor; dst: OHxOWx3 (OHxOW)."""
+        h, w = src.shape[:2]
         self._check(self.L.srcnn_process_device(self.ctx, _dptr(src), w, h, src.stride(0), order, C.c_float(scale),
                                                 _dptr(dst), dst.stride(0)))
         return dst
 
     def process_batch_device(self, src, scale, dst, order=ORDER_BGR):
-        n, h, w, _ = src.shape
+        n, h, w = src.shape[:3]
         self._check(self.L.srcnn_process_batch_device(self.ctx, _dptr(src), n, w, h, src.stride(1), src.stride(0), order,
                                                       C.c_float(scale), _dptr(dst), dst.stride(1), dst.stride(0)))
         return dst
 
     def process_band_device(self, src_rows, w, h, s0, s1, scale, r0, r1, dst_rows, order=ORDER_BGR):
-        """src_rows: (s1-s0)xWx3 device tensor holding source rows [s0,s1); dst_rows: (r1-r0)xOWx3."""
+        """src_rows: (s1-s0)xWx3 device tensor holding source rows [s0,s1); dst_rows: (r1-r0)xOWx3 (no x3 with ORDER_GRAY)."""
         self._check(self.L.srcnn_process_band_device(self.ctx, _dptr(src_rows), w, h, src_rows.stride(0), s0, s1, order,
                                                      C.c_float(scale), r0, r1, _dptr(dst_rows), dst_rows.stride(0)))
         return dst_rows
@@ -294,6 +310,13 @@ class Engine:
         h, w, _ = src.shape
         self._check(self.L.srcnn_stage_color_bicubic_device(self.ctx, _dptr(src), w, h, src.stride(0), order,
                                                             C.c_float(scale), _dptr(y), _dptr(cr), _dptr(cb), y.stride(0)))
+
+    def stage_resize_plane(self, src, scale, dst):
+        """One HxW uint8 device plane through the path's cubic resize (cv::resize INTER_CUBIC) into dst (OHxOW, any stride)."""
+        h, w = src.shape
+        self._check(self.L.srcnn_stage_resize_plane_device(self.ctx, _dptr(src), w, h, src.stride(0), C.c_float(scale),
+                                                           _dptr(dst), dst.stride(0)))
+        return dst
 
     def stage_cnn(self, y, out, variant=None):
         h, w = y.shape
@@ -307,12 +330,13 @@ class Engine:
         self._check(self.L.srcnn_debug_set_host_bands(self.ctx, int(bands)))
 
     def process_band_host(self, img, scale, r0, r1, out_rows=None, order=ORDER_BGR):
-        """img: the WHOLE HxWx3 source image; returns output rows [r0, r1) as an (r1-r0)xOWx3 array."""
+        """img: the WHOLE HxWx3 (HxW) source image; returns output rows [r0, r1) as an (r1-r0)xOWx3 ((r1-r0)xOW) array."""
         img = np.ascontiguousarray(img)
-        h, w, _ = img.shape
+        _check_host_image(img, order, 1)
+        h, w = img.shape[:2]
         ow, oh = out_dims(w, h, scale)
         if out_rows is None:
-            out_rows = np.empty((r1 - r0, ow, 3), np.uint8)
+            out_rows = np.empty((r1 - r0, ow) + _pixel_shape(order), np.uint8)
         self._check(self.L.srcnn_process_band_host(self.ctx, img.ctypes.data, w, h, img.strides[0], order, C.c_float(scale),
                                                    r0, r1, out_rows.ctypes.data, out_rows.strides[0]))
         return out_rows
@@ -420,29 +444,32 @@ class MultiEngine:
     # -- host buffers (numpy, or raw pointers for pinned memory) -------------------------------------
     def process_banded(self, img, scale, order=ORDER_BGR, out=None):
         img = np.ascontiguousarray(img)
-        h, w, _ = img.shape
+        _check_host_image(img, order, 1)
+        h, w = img.shape[:2]
         ow, oh = out_dims(w, h, scale)
         if out is None:
-            out = np.empty((oh, ow, 3), np.uint8)
+            out = np.empty((oh, ow) + _pixel_shape(order), np.uint8)
         self._check(self.L.srcnn_mgpu_process_banded_host(self.h, img.ctypes.data, w, h, img.strides[0], order, C.c_float(scale),
                                                           out.ctypes.data, out.strides[0]))
         return out
 
     def process_batch(self, frames, scale, order=ORDER_BGR, out=None):
         frames = np.ascontiguousarray(frames)
-        n, h, w, _ = frames.shape
+        _check_host_image(frames, order, 2)
+        n, h, w = frames.shape[:3]
         ow, oh = out_dims(w, h, scale)
         if out is None:
-            out = np.empty((n, oh, ow, 3), np.uint8)
+            out = np.empty((n, oh, ow) + _pixel_shape(order), np.uint8)
         self._check(self.L.srcnn_mgpu_process_batch_host(self.h, frames.ctypes.data, n, w, h, frames.strides[1], frames.strides[0],
                                                          order, C.c_float(scale), out.ctypes.data, out.strides[1], out.strides[0]))
         return out
 
     # -- device-resident shares (torch CUDA tensors, one per worker, each on that worker's device) -----
     def process_batch_device(self, srcs, scale, dsts, order=ORDER_BGR):
-        """srcs[i]: n_i x H x W x 3 on worker i's device (n_i may be 0 -> pass None); dsts[i]: n_i x OH x OW x 3."""
+        """srcs[i]: n_i x H x W x 3 (no x 3 with ORDER_GRAY) on worker i's device (n_i may be 0 -> pass None); dsts[i]:
+        n_i x OH x OW x 3."""
         ref = next(t for t in srcs if t is not None)
-        _, h, w, _ = ref.shape
+        h, w = ref.shape[1:3]
         dref = next(t for t in dsts if t is not None)
         ps = (C.c_void_p * self.n)(*[t.data_ptr() if t is not None else None for t in srcs])
         pd = (C.c_void_p * self.n)(*[t.data_ptr() if t is not None else None for t in dsts])

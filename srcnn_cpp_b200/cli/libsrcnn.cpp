@@ -29,31 +29,37 @@ int ProcessSRCNN(const unsigned char* refbuff, unsigned w, unsigned h, unsigned 
         if (rc) return rc;
     }
     const size_t npx = (size_t)w * h, onpx = (size_t)ow * oh;
-    std::vector<unsigned char> rgb(npx * 3), out_rgb(onpx * 3);
-    const bool has_alpha = (d == 2 || d == 4);
-    std::vector<unsigned char> alpha, alpha_out;
-    if (has_alpha) { alpha.resize(npx); alpha_out.resize(onpx); }
-    for (size_t i = 0; i < npx; i++) {
-        const unsigned char* p = refbuff + i * d;
-        if (d >= 3) { rgb[3 * i] = p[0]; rgb[3 * i + 1] = p[1]; rgb[3 * i + 2] = p[2]; }
-        else { rgb[3 * i] = rgb[3 * i + 1] = rgb[3 * i + 2] = p[0]; }
-        if (has_alpha) alpha[i] = p[d - 1];
-    }
-    rc = srcnn_process_host(g_ctx, rgb.data(), (int)w, (int)h, (size_t)w * 3, SRCNN_ORDER_RGB, muliply, out_rgb.data(), (size_t)ow * 3);
-    if (rc) return rc;
+    const bool has_alpha = (d == 2 || d == 4), gray = d <= 2;
     unsigned char* out = new (std::nothrow) unsigned char[onpx * d];
     if (!out) return SRCNN_E_NOMEM;
+    // grey (d = 1, 2): the one-plane path, straight into `out` when there is no alpha to interleave
+    std::vector<unsigned char> pix, pix_out, alpha, alpha_out;
+    const size_t ch = gray ? 1 : 3;
+    if (d == 1) {
+        rc = srcnn_process_host(g_ctx, refbuff, (int)w, (int)h, (size_t)w, SRCNN_ORDER_GRAY, muliply, out, (size_t)ow);
+    } else {
+        pix.resize(npx * ch); pix_out.resize(onpx * ch);
+        if (has_alpha) { alpha.resize(npx); alpha_out.resize(onpx); }
+        for (size_t i = 0; i < npx; i++) {
+            const unsigned char* p = refbuff + i * d;
+            for (size_t k = 0; k < ch; k++) pix[ch * i + k] = p[k];
+            if (has_alpha) alpha[i] = p[d - 1];
+        }
+        rc = srcnn_process_host(g_ctx, pix.data(), (int)w, (int)h, (size_t)w * ch, gray ? SRCNN_ORDER_GRAY : SRCNN_ORDER_RGB, muliply,
+                                pix_out.data(), (size_t)ow * ch);
+    }
+    if (rc) { delete[] out; return rc; }
     if (has_alpha) {
         // alpha: the plain bicubic resize of the path (resize(..., CV_INTER_CUBIC), src/srcnn.cpp:577-582), no CNN
         rc = srcnn_resize_plane_host(g_ctx, alpha.data(), (int)w, (int)h, (size_t)w, muliply, alpha_out.data(), (size_t)ow);
         if (rc) { delete[] out; return rc; }
     }
-    for (size_t i = 0; i < onpx; i++) {
-        unsigned char* q = out + i * d;
-        if (d >= 3) { q[0] = out_rgb[3 * i]; q[1] = out_rgb[3 * i + 1]; q[2] = out_rgb[3 * i + 2]; }
-        else { q[0] = out_rgb[3 * i + 1]; }
-        if (has_alpha) q[d - 1] = alpha_out[i];
-    }
+    if (d > 1)
+        for (size_t i = 0; i < onpx; i++) {
+            unsigned char* q = out + i * d;
+            for (size_t k = 0; k < ch; k++) q[k] = pix_out[ch * i + k];
+            if (has_alpha) q[d - 1] = alpha_out[i];
+        }
     outbuff = out;
     outbuffsz = (unsigned)(onpx * d);
     return 0;

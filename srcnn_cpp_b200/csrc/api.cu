@@ -66,19 +66,23 @@ static int scaled_dim(int n, float scale) {
     return (int)((float)n * scale);
 }
 
+static size_t bytes_per_pixel(int order) { return order == SRCNN_ORDER_GRAY ? 1 : 3; }
+
 static int check_image(Ctx* c, const void* src, int w, int h, size_t stride, int order, float scale, const void* dst,
                        size_t dst_stride, int* ow, int* oh) {
     if (!c) return SRCNN_E_ARG;
     if (!src || !dst) return fail(c, SRCNN_E_ARG, "null image pointer");
     if (w <= 0 || h <= 0) return fail(c, SRCNN_E_ARG, "non-positive image size %dx%d", w, h);
-    if (stride < (size_t)w * 3) return fail(c, SRCNN_E_ARG, "source stride %zu < 3*w", stride);
-    if (order != SRCNN_ORDER_BGR && order != SRCNN_ORDER_RGB) return fail(c, SRCNN_E_ARG, "unknown channel order %d", order);
+    if (order != SRCNN_ORDER_BGR && order != SRCNN_ORDER_RGB && order != SRCNN_ORDER_GRAY)
+        return fail(c, SRCNN_E_ARG, "unknown pixel order %d", order);
+    const size_t bpp = bytes_per_pixel(order);
+    if (stride < (size_t)w * bpp) return fail(c, SRCNN_E_ARG, "source stride %zu < %zu*w", stride, bpp);
     // src/srcnn.cpp:485-495 "ratio too small"
     if (!(((float)w * scale) > 0.f) || !(((float)h * scale) > 0.f)) return fail(c, SRCNN_E_RATIO, "scale %g gives an empty image", scale);
     *ow = scaled_dim(w, scale);
     *oh = scaled_dim(h, scale);
     if (*ow <= 0 || *oh <= 0) return fail(c, SRCNN_E_RATIO, "scale %g gives an empty image", scale);
-    if (dst_stride < (size_t)*ow * 3) return fail(c, SRCNN_E_ARG, "destination stride %zu < 3*ow", dst_stride);
+    if (dst_stride < (size_t)*ow * bpp) return fail(c, SRCNN_E_ARG, "destination stride %zu < %zu*ow", dst_stride, bpp);
     return SRCNN_OK;
 }
 
@@ -88,8 +92,9 @@ static int check_image(Ctx* c, const void* src, int w, int h, size_t stride, int
 // 4 GiB); Y, Y' and the FP16 Y plane are shared (the merge never reads Y / FP16 Y, and Y' is written by the next CNN launch, which
 // waits for everything before it).  c->plane_sel says which pair this call got.  Keeping the rest single also keeps the planes
 // L2-resident from step to step: two whole plane sets (116 MB at 4K) measured 3 us slower in the colour+bicubic kernel.
-// The host-buffer pipeline keeps to pair 0 (its sub-bands are separated by copies and events anyway).
-static int carve_planes(Ctx* c, int ow, int rows, int row0, Planes* pl, int nframes = 1) {
+// The host-buffer pipeline keeps to pair 0 (its sub-bands are separated by copies and events anyway).  A grey call has no Cr/Cb
+// planes: it leaves the pair selection alone (and ends the early-start chain, end_merge_chain).
+static int carve_planes(Ctx* c, int ow, int rows, int row0, Planes* pl, int nframes = 1, bool gray = false) {
     const size_t pitch = align_up((size_t)ow, 128);
     const size_t plane = pitch * (size_t)rows;
     const size_t pitch16 = y16_pitch_bytes(ow);
@@ -97,15 +102,15 @@ static int carve_planes(Ctx* c, int ow, int rows, int row0, Planes* pl, int nfra
     const size_t nf = (size_t)nframes;
     const size_t bytes = (plane * 4 + plane16) * nf + 512;   // slack: the last row's last strip copy may run past the row
     const bool two = c->overlap && !c->host_path && !c->capturing && plane * 2 * nf <= ((size_t)4 << 30);
-    c->plane_sel = two ? (c->plane_sel ^ 1) : 0;
+    if (!gray) c->plane_sel = two ? (c->plane_sel ^ 1) : 0;
     int rc = ensure(c, c->plane_buf, bytes);
     if (rc) return rc;
-    if (c->plane_sel && (rc = ensure(c, c->plane_buf2, plane * 2 * nf))) return rc;
+    if (!gray && c->plane_sel && (rc = ensure(c, c->plane_buf2, plane * 2 * nf))) return rc;
     c->plane_layout[0] = pitch; c->plane_layout[1] = (size_t)rows; c->plane_layout[2] = nf;
     uint8_t* base = (uint8_t*)c->plane_buf.p;
     pl->y = base;
-    pl->cr = c->plane_sel ? (uint8_t*)c->plane_buf2.p : base + plane * nf;
-    pl->cb = c->plane_sel ? (uint8_t*)c->plane_buf2.p + plane * nf : base + 2 * plane * nf;
+    pl->cr = gray ? nullptr : c->plane_sel ? (uint8_t*)c->plane_buf2.p : base + plane * nf;
+    pl->cb = gray ? nullptr : c->plane_sel ? (uint8_t*)c->plane_buf2.p + plane * nf : base + 2 * plane * nf;
     pl->yout = base + 3 * plane * nf;
     pl->y16 = base + 4 * plane * nf;
     pl->frame_stride = plane;
@@ -129,6 +134,13 @@ static Ctx* last_merge_on(cudaStream_t s) {
     std::lock_guard<std::mutex> lk(g_merge_mu);
     auto it = g_last_merge.find(s);
     return it == g_last_merge.end() ? nullptr : it->second;
+}
+// A grey call launches no merge: the kernel that ends up last on the stream does not release its dependents, so neither this
+// context's next colour call nor any other context's on this stream may start early.
+static void end_merge_chain(Ctx* c) {
+    c->merge_sel = -1;
+    std::lock_guard<std::mutex> lk(g_merge_mu);
+    g_last_merge.erase(c->stream);
 }
 static void forget_merges_of(Ctx* c) {
     std::lock_guard<std::mutex> lk(g_merge_mu);
@@ -173,9 +185,12 @@ static int process_rows_impl(Ctx* c, const uint8_t* d_src, int w, int h, size_t 
     rc = get_taps(c, h, oh, &ty);
     if (rc) return rc;
     const int p0 = std::max(r0 - 6, 0), p1 = std::min(r1 + 6, oh);  // 6-px halo: 4 (conv1) + 2 (conv3)
+    // grey: one-plane resize, then the CNN straight into the caller's rows; no chroma, no merge
+    const bool gray = order == SRCNN_ORDER_GRAY;
+    if (gray) end_merge_chain(c);
     Planes pl;
     c->fail_stage = SRCNN_STAGE_PLANES;
-    rc = carve_planes(c, ow, p1 - p0, p0, &pl);
+    rc = carve_planes(c, ow, p1 - p0, p0, &pl, 1, gray);
     if (rc) return rc;
     c->fail_stage = SRCNN_STAGE_COLOR_BICUBIC;
     // the band must bring every source row its taps touch
@@ -192,7 +207,7 @@ static int process_rows_impl(Ctx* c, const uint8_t* d_src, int w, int h, size_t 
     ra.row_begin = p0; ra.row_end = p1;
     ra.pl = pl; ra.tx = tx; ra.ty = ty;
     if (c->variant != SRCNN_VARIANT_TC) ra.pl.y16 = nullptr;      // the strict FP32 kernels read the u8 plane
-    ra.early = may_start_early(c, d_src, (size_t)(s1 - s0) * src_stride);
+    ra.early = !gray && may_start_early(c, d_src, (size_t)(s1 - s0) * src_stride);
     c->early_launches += ra.early;
     if ((rc = prof_mark(c, 0))) return rc;
     rc = launch_color_bicubic(c, ra);
@@ -206,10 +221,11 @@ static int process_rows_impl(Ctx* c, const uint8_t* d_src, int w, int h, size_t 
     ca.W = ow; ca.H = oh;
     ca.row0 = p0; ca.rows = p1 - p0;
     ca.out_begin = r0; ca.out_end = r1;
-    ca.out = pl.yout; ca.out_pitch = pl.pitch;
+    if (gray) { ca.out = d_dst; ca.out_pitch = dst_stride; ca.out_row0 = r0; }
+    else { ca.out = pl.yout; ca.out_pitch = pl.pitch; ca.out_row0 = p0; }
     // optionally the row-walking tcgen05 kernel merges Cr/Cb and converts back to BGR in its last epilogue (no Y' plane, no
     // K-C launch); measured slower than the separate launch (byte stores from one-thread-per-column lanes), so off by default
-    const bool fused = c->variant == SRCNN_VARIANT_TC && c->fuse_merge;
+    const bool fused = !gray && c->variant == SRCNN_VARIANT_TC && c->fuse_merge;
     if (fused) {
         ca.cr = pl.cr; ca.cb = pl.cb;
         ca.bgr = d_dst; ca.bgr_stride = dst_stride; ca.order = order;
@@ -217,7 +233,7 @@ static int process_rows_impl(Ctx* c, const uint8_t* d_src, int w, int h, size_t 
     rc = run_cnn(c, c->variant, ca);
     if (rc) return rc;
     if ((rc = prof_mark(c, 2))) return rc;
-    if (fused) return prof_mark(c, 3);
+    if (fused || gray) return prof_mark(c, 3);
 
     c->fail_stage = SRCNN_STAGE_MERGE;
     MergeArgs ma;
@@ -253,11 +269,13 @@ static int process_frames_impl(Ctx* c, const uint8_t* d_src, int n, int w, int h
     if ((rc = get_taps(c, h, oh, &ty))) return rc;
     const size_t per_frame = align_up((size_t)ow, 128) * (size_t)oh * 4 + y16_pitch_bytes(ow) * (size_t)oh;
     const int chunk = (int)std::max<size_t>(1, std::min<size_t>((size_t)n, ((size_t)1 << 30) / per_frame));
+    const bool gray = order == SRCNN_ORDER_GRAY;
+    if (gray) end_merge_chain(c);
     for (int f0 = 0; f0 < n; f0 += chunk) {
         const int m = std::min(chunk, n - f0);
         Planes pl;
         c->fail_stage = SRCNN_STAGE_PLANES;
-        if ((rc = carve_planes(c, ow, oh, 0, &pl, m))) return rc;
+        if ((rc = carve_planes(c, ow, oh, 0, &pl, m, gray))) return rc;
         c->fail_stage = SRCNN_STAGE_COLOR_BICUBIC;
         ResizeArgs ra;
         ra.src = d_src + (size_t)f0 * src_frame_stride; ra.src_stride = src_stride;
@@ -267,7 +285,7 @@ static int process_frames_impl(Ctx* c, const uint8_t* d_src, int n, int w, int h
         ra.row_begin = 0; ra.row_end = oh;
         ra.pl = pl; ra.tx = tx; ra.ty = ty;
         ra.nframes = m; ra.src_frame_stride = src_frame_stride;
-        ra.early = may_start_early(c, ra.src, (size_t)(m - 1) * src_frame_stride + (size_t)h * src_stride);
+        ra.early = !gray && may_start_early(c, ra.src, (size_t)(m - 1) * src_frame_stride + (size_t)h * src_stride);
         c->early_launches += ra.early;
         if ((rc = prof_mark(c, 0))) return rc;
         if ((rc = launch_color_bicubic(c, ra))) return rc;
@@ -281,14 +299,19 @@ static int process_frames_impl(Ctx* c, const uint8_t* d_src, int n, int w, int h
         ca.out_begin = 0; ca.out_end = oh;
         ca.out = pl.yout; ca.out_pitch = pl.pitch;
         ca.nframes = m; ca.y16_frame_stride = pl.frame_stride16; ca.out_frame_stride = pl.frame_stride;
+        uint8_t* dst0 = d_dst + (size_t)f0 * dst_frame_stride;
+        if (gray) { ca.out = dst0; ca.out_pitch = dst_stride; ca.out_frame_stride = dst_frame_stride; }
         if ((rc = launch_cnn_tc2(c, ca))) return rc;
         if ((rc = prof_mark(c, 2))) return rc;
+        if (gray) {
+            if ((rc = prof_mark(c, 3))) return rc;
+            continue;
+        }
         c->fail_stage = SRCNN_STAGE_MERGE;
         MergeArgs ma;
         ma.y = pl.yout; ma.cr = pl.cr; ma.cb = pl.cb;
         ma.pitch = pl.pitch; ma.w = ow;
         ma.order = order;
-        uint8_t* dst0 = d_dst + (size_t)f0 * dst_frame_stride;
         if (m == 1 || dst_frame_stride == dst_stride * (size_t)oh) {   // the chunk's results are one tall image too
             ma.rows = oh * m; ma.dst = dst0; ma.dst_stride = dst_stride;
             if ((rc = launch_merge(c, ma))) return rc;
@@ -308,7 +331,7 @@ static int process_frames_impl(Ctx* c, const uint8_t* d_src, int n, int w, int h
 static int process_frames(Ctx* c, const uint8_t* d_src, int n, int w, int h, size_t src_stride, size_t src_frame_stride, int order,
                           float scale, int ow, int oh, uint8_t* d_dst, size_t dst_stride, size_t dst_frame_stride) {
     // one launch per stage and chunk needs the row-walking kernel with a separate merge; everything else goes frame by frame
-    if (n == 1 || c->variant != SRCNN_VARIANT_TC || c->fuse_merge || !c->batch_launch) {
+    if (n == 1 || c->variant != SRCNN_VARIANT_TC || (c->fuse_merge && order != SRCNN_ORDER_GRAY) || !c->batch_launch) {
         for (int f = 0; f < n; f++) {
             int rc = process_rows(c, d_src + (size_t)f * src_frame_stride, w, h, src_stride, 0, h, order, scale, ow, oh, 0, oh,
                                   d_dst + (size_t)f * dst_frame_stride, dst_stride);
@@ -368,6 +391,7 @@ static int enqueue_chunk(Ctx* c, const uint8_t* src, int f0, int m, int w, int h
                          const TapTable* ty, int S0, int S1, const std::vector<int>& edges, int group, size_t s_row, size_t d_row, size_t s_frame,
                          size_t d_frame) {
     const int bands = (int)edges.size() - 1;
+    const size_t bpp = bytes_per_pixel(order), w_bytes = (size_t)w * bpp, ow_bytes = (size_t)ow * bpp;
     int rc;
     uint8_t* ds = (uint8_t*)c->src_buf.p;
     uint8_t* dd = (uint8_t*)c->dst_buf.p;
@@ -396,8 +420,8 @@ static int enqueue_chunk(Ctx* c, const uint8_t* src, int f0, int m, int w, int h
         // A batch of whole frames: groups of frames travel together -- one copy in, ONE launch per stage (process_frames: no
         // per-frame pipeline fill / drain in the fused kernel), one copy out -- sized so that a group's result is >= 64 MB:
         // large copies keep the PCIe link busy, and the next group's kernels still hide behind this group's D2H.
-        const bool rows_tight_in = src_stride == (size_t)w * 3 && s_row == (size_t)w * 3;      // a frame is one contiguous run of bytes
-        const bool rows_tight_out = dst_stride == (size_t)ow * 3 && d_row == (size_t)ow * 3;
+        const bool rows_tight_in = src_stride == w_bytes && s_row == w_bytes;      // a frame is one contiguous run of bytes
+        const bool rows_tight_out = dst_stride == ow_bytes && d_row == ow_bytes;
         for (int g0 = 0; g0 < m; g0 += group) {
             const int g = std::min(group, m - g0);
             const uint8_t* hsrc = src + (size_t)(f0 + g0) * src_frame_stride;
@@ -410,7 +434,7 @@ static int enqueue_chunk(Ctx* c, const uint8_t* src, int f0, int m, int w, int h
             } else {
                 for (int f = 0; f < g; f++)
                     SRCNN_CUDA(c, cudaMemcpy2DAsync(ds + (size_t)(g0 + f) * s_frame, s_row, hsrc + (size_t)f * src_frame_stride + (size_t)S0 * src_stride,
-                                                    src_stride, (size_t)w * 3, S1 - S0, cudaMemcpyHostToDevice, c->s_in));
+                                                    src_stride, w_bytes, S1 - S0, cudaMemcpyHostToDevice, c->s_in));
             }
             SRCNN_CUDA(c, cudaEventRecord(ev_in, c->s_in));
             SRCNN_CUDA(c, cudaStreamWaitEvent(c->stream, ev_in, 0));
@@ -431,7 +455,7 @@ static int enqueue_chunk(Ctx* c, const uint8_t* src, int f0, int m, int w, int h
                                                 cudaMemcpyDeviceToHost, c->s_out));
             } else {
                 for (int f = 0; f < g; f++)
-                    SRCNN_CUDA(c, cudaMemcpy2DAsync(hdst + (size_t)f * dst_frame_stride, dst_stride, dd + (size_t)(g0 + f) * d_frame, d_row, (size_t)ow * 3, rows,
+                    SRCNN_CUDA(c, cudaMemcpy2DAsync(hdst + (size_t)f * dst_frame_stride, dst_stride, dd + (size_t)(g0 + f) * d_frame, d_row, ow_bytes, rows,
                                                     cudaMemcpyDeviceToHost, c->s_out));
             }
         }
@@ -447,7 +471,7 @@ static int enqueue_chunk(Ctx* c, const uint8_t* src, int f0, int m, int w, int h
                 cudaEvent_t ev_in;
                 if ((rc = event_at(ei++, &ev_in))) return rc;
                 SRCNN_CUDA(c, cudaMemcpy2DAsync(ds + f * s_frame + (size_t)(copied - S0) * s_row, s_row, hsrc + (size_t)copied * src_stride,
-                                                src_stride, (size_t)w * 3, s_hi - copied, cudaMemcpyHostToDevice, c->s_in));
+                                                src_stride, w_bytes, s_hi - copied, cudaMemcpyHostToDevice, c->s_in));
                 SRCNN_CUDA(c, cudaEventRecord(ev_in, c->s_in));
                 SRCNN_CUDA(c, cudaStreamWaitEvent(c->stream, ev_in, 0));
                 copied = s_hi;
@@ -460,7 +484,7 @@ static int enqueue_chunk(Ctx* c, const uint8_t* src, int f0, int m, int w, int h
             SRCNN_CUDA(c, cudaEventRecord(ev_done, c->stream));
             SRCNN_CUDA(c, cudaStreamWaitEvent(c->s_out, ev_done, 0));
             SRCNN_CUDA(c, cudaMemcpy2DAsync(hdst + (size_t)(r0 - R0) * dst_stride, dst_stride,
-                                            dd + f * d_frame + (size_t)(r0 - R0) * d_row, d_row, (size_t)ow * 3, r1 - r0,
+                                            dd + f * d_frame + (size_t)(r0 - R0) * d_row, d_row, ow_bytes, r1 - r0,
                                             cudaMemcpyDeviceToHost, c->s_out));
         }
     }
@@ -492,7 +516,8 @@ int host_pipeline(Ctx* c, const uint8_t* src, int n, int w, int h, size_t src_st
     };
     const int S0 = std::min(std::max(ty->h_ofs[std::max(R0 - 6, 0)] - 1, 0), h - 1), S1 = src_hi(R1);
     // device staging: tight rows, 256-byte aligned frames; only the rows this call needs
-    const size_t s_row = align_up((size_t)w * 3, 4), d_row = align_up((size_t)ow * 3, 4);
+    const size_t bpp = bytes_per_pixel(order);
+    const size_t s_row = align_up((size_t)w * bpp, 4), d_row = align_up((size_t)ow * bpp, 4);
     const size_t s_frame = align_up(s_row * (size_t)(S1 - S0), 256), d_frame = align_up(d_row * (size_t)(R1 - R0), 256);
     // frames in flight are bounded so staging stays modest (<= 4 GiB of output; one frame may be larger).  Chunks are separated by
     // a full drain of the pipeline, so the bound is generous: 180 GB of HBM is not the scarce resource here.
@@ -533,10 +558,11 @@ int host_pipeline(Ctx* c, const uint8_t* src, int n, int w, int h, size_t src_st
     int tallest = 0;
     for (int bi = 0; bi < bands; bi++) tallest = std::max(tallest, edges[bi + 1] - edges[bi]);
     // frames of a batch travel in groups whose result is >= 64 MB (see enqueue_chunk)
-    const int group = (int)std::max<size_t>(1, std::min<size_t>(16, ((size_t)64 << 20) / std::max<size_t>(1, (size_t)ow * 3 * (size_t)rows) + 1));
+    const int group = (int)std::max<size_t>(1, std::min<size_t>(16, ((size_t)64 << 20) / std::max<size_t>(1, (size_t)ow * bpp * (size_t)rows) + 1));
     {   // the planes of the tallest sub-band / of a group of frames, allocated before anything is enqueued or captured
         Planes pl;
-        if ((rc = carve_planes(c, ow, std::min(tallest + 12, oh), 0, &pl, (bands == 1 && n > 1) ? std::min(group, n) : 1))) return rc;
+        if ((rc = carve_planes(c, ow, std::min(tallest + 12, oh), 0, &pl, (bands == 1 && n > 1) ? std::min(group, n) : 1,
+                               order == SRCNN_ORDER_GRAY))) return rc;
     }
 
     // ---- CUDA-graph replay.  A call that repeats an earlier one exactly (same buffers, same geometry: a stream of frames through
@@ -962,6 +988,7 @@ int srcnn_stage_color_bicubic_device(srcnn_ctx* c, const uint8_t* d_src, int w, 
                                      float scale, uint8_t* d_y, uint8_t* d_cr, uint8_t* d_cb, size_t plane_pitch) {
     ENTER(c);
     if (!d_src || !d_y || !d_cr || !d_cb) return fail(c, SRCNN_E_ARG, "null pointer");
+    if (order != SRCNN_ORDER_BGR && order != SRCNN_ORDER_RGB) return fail(c, SRCNN_E_ARG, "colour order expected, got %d", order);
     if (w <= 0 || h <= 0 || src_stride < (size_t)w * 3) return fail(c, SRCNN_E_ARG, "bad source geometry");
     if (!(((float)w * scale) > 0.f) || !(((float)h * scale) > 0.f)) return fail(c, SRCNN_E_RATIO, "ratio too small");
     const int ow = scaled_dim(w, scale), oh = scaled_dim(h, scale);
@@ -984,42 +1011,65 @@ int srcnn_stage_color_bicubic_device(srcnn_ctx* c, const uint8_t* d_src, int w, 
     return launch_color_bicubic(c, ra);
 }
 
-// One 8-bit plane through cv::resize(..., INTER_CUBIC) (src/srcnn.cpp:577-582), host buffers.  The colour+bicubic kernel
-// does it: a grey pixel (v,v,v) has Y = (16384 v + 8192) >> 14 = v, so its Y plane IS the resized plane.
-int srcnn_resize_plane_host(srcnn_ctx* c, const uint8_t* src, int w, int h, size_t src_stride, float scale, uint8_t* dst,
-                            size_t dst_stride) {
-    ENTER(c);
+// One 8-bit plane through cv::resize(..., INTER_CUBIC) (src/srcnn.cpp:577-582): the one-plane resize kernels.  Device buffers,
+// enqueued; d_dst must be 4-byte aligned with a pitch that is a multiple of 4 (the tiled kernel's word stores).
+static int resize_plane(Ctx* c, const uint8_t* d_src, int w, int h, size_t src_stride, int ow, int oh, uint8_t* d_dst,
+                        size_t dst_stride) {
+    TapTable *tx, *ty;
+    int rc = get_taps(c, w, ow, &tx);
+    if (rc) return rc;
+    if ((rc = get_taps(c, h, oh, &ty))) return rc;
+    ResizeArgs ra;
+    ra.src = d_src; ra.src_stride = src_stride;
+    ra.sw = w; ra.sh = h; ra.src_row0 = 0; ra.src_row1 = h;
+    ra.order = SRCNN_ORDER_GRAY; ra.ow = ow; ra.oh = oh;
+    ra.row_begin = 0; ra.row_end = oh;
+    ra.pl.y = d_dst; ra.pl.pitch = dst_stride; ra.pl.row0 = 0; ra.pl.rows = oh;
+    ra.tx = tx; ra.ty = ty;
+    return launch_color_bicubic(c, ra);
+}
+
+static int check_plane(Ctx* c, const void* src, int w, int h, size_t src_stride, float scale, const void* dst, size_t dst_stride,
+                       int* ow, int* oh) {
     if (!src || !dst) return fail(c, SRCNN_E_ARG, "null pointer");
     if (w <= 0 || h <= 0 || src_stride < (size_t)w) return fail(c, SRCNN_E_ARG, "bad source geometry");
     if (!(((float)w * scale) > 0.f) || !(((float)h * scale) > 0.f)) return fail(c, SRCNN_E_RATIO, "ratio too small");
-    const int ow = scaled_dim(w, scale), oh = scaled_dim(h, scale);
-    if (ow <= 0 || oh <= 0) return fail(c, SRCNN_E_RATIO, "ratio too small");
-    if (dst_stride < (size_t)ow) return fail(c, SRCNN_E_ARG, "destination stride %zu < ow", dst_stride);
-    std::vector<uint8_t> grey;
-    try { grey.resize((size_t)w * h * 3); } catch (...) { return fail(c, SRCNN_E_NOMEM, "host staging"); }
-    for (int y = 0; y < h; y++)
-        for (int x = 0; x < w; x++) {
-            const uint8_t v = src[(size_t)y * src_stride + x];
-            uint8_t* q = &grey[((size_t)y * w + x) * 3];
-            q[0] = q[1] = q[2] = v;
-        }
-    int rc = ensure(c, c->src_buf, grey.size());
+    *ow = scaled_dim(w, scale);
+    *oh = scaled_dim(h, scale);
+    if (*ow <= 0 || *oh <= 0) return fail(c, SRCNN_E_RATIO, "ratio too small");
+    if (dst_stride < (size_t)*ow) return fail(c, SRCNN_E_ARG, "destination stride %zu < ow", dst_stride);
+    return SRCNN_OK;
+}
+
+int srcnn_stage_resize_plane_device(srcnn_ctx* c, const uint8_t* d_src, int w, int h, size_t src_stride, float scale,
+                                    uint8_t* d_dst, size_t dst_stride) {
+    ENTER(c);
+    int ow, oh;
+    int rc = check_plane(c, d_src, w, h, src_stride, scale, d_dst, dst_stride, &ow, &oh);
     if (rc) return rc;
-    Planes pl;
-    if ((rc = carve_planes(c, ow, oh, 0, &pl))) return rc;
-    TapTable *tx, *ty;
-    if ((rc = get_taps(c, w, ow, &tx))) return rc;
-    if ((rc = get_taps(c, h, oh, &ty))) return rc;
-    SRCNN_CUDA(c, cudaMemcpyAsync(c->src_buf.p, grey.data(), grey.size(), cudaMemcpyHostToDevice, c->stream));
-    ResizeArgs ra;
-    ra.src = (const uint8_t*)c->src_buf.p; ra.src_stride = (size_t)w * 3;
-    ra.sw = w; ra.sh = h; ra.src_row0 = 0; ra.src_row1 = h;
-    ra.order = SRCNN_ORDER_BGR; ra.ow = ow; ra.oh = oh;
-    ra.row_begin = 0; ra.row_end = oh;
-    ra.pl = pl; ra.tx = tx; ra.ty = ty;
-    ra.pl.y16 = nullptr;
-    if ((rc = launch_color_bicubic(c, ra))) return rc;
-    SRCNN_CUDA(c, cudaMemcpy2DAsync(dst, dst_stride, pl.y, pl.pitch, (size_t)ow, oh, cudaMemcpyDeviceToHost, c->stream));
+    if ((((uintptr_t)d_dst | dst_stride) & 3) == 0) return resize_plane(c, d_src, w, h, src_stride, ow, oh, d_dst, dst_stride);
+    // a destination the word stores cannot take: resize into the staging buffer, then one device copy
+    const size_t pitch = align_up((size_t)ow, 128);
+    if ((rc = ensure(c, c->dst_buf, pitch * (size_t)oh))) return rc;
+    if ((rc = resize_plane(c, d_src, w, h, src_stride, ow, oh, (uint8_t*)c->dst_buf.p, pitch))) return rc;
+    SRCNN_CUDA(c, cudaMemcpy2DAsync(d_dst, dst_stride, c->dst_buf.p, pitch, (size_t)ow, oh, cudaMemcpyDeviceToDevice, c->stream));
+    return SRCNN_OK;
+}
+
+// Host buffers (ProcessSRCNN's alpha): copy the plane in, resize, copy the result out.
+int srcnn_resize_plane_host(srcnn_ctx* c, const uint8_t* src, int w, int h, size_t src_stride, float scale, uint8_t* dst,
+                            size_t dst_stride) {
+    ENTER(c);
+    int ow, oh;
+    int rc = check_plane(c, src, w, h, src_stride, scale, dst, dst_stride, &ow, &oh);
+    if (rc) return rc;
+    const size_t s_pitch = align_up((size_t)w, 4), d_pitch = align_up((size_t)ow, 128);
+    if ((rc = ensure(c, c->src_buf, s_pitch * (size_t)h))) return rc;
+    if ((rc = ensure(c, c->dst_buf, d_pitch * (size_t)oh))) return rc;
+    StreamDrain drain{c};   // no copy may still reference the caller's buffers when this returns
+    SRCNN_CUDA(c, cudaMemcpy2DAsync(c->src_buf.p, s_pitch, src, src_stride, (size_t)w, h, cudaMemcpyHostToDevice, c->stream));
+    if ((rc = resize_plane(c, (const uint8_t*)c->src_buf.p, w, h, s_pitch, ow, oh, (uint8_t*)c->dst_buf.p, d_pitch))) return rc;
+    SRCNN_CUDA(c, cudaMemcpy2DAsync(dst, dst_stride, c->dst_buf.p, d_pitch, (size_t)ow, oh, cudaMemcpyDeviceToHost, c->stream));
     SRCNN_CUDA(c, cudaStreamSynchronize(c->stream));
     return SRCNN_OK;
 }
@@ -1051,6 +1101,7 @@ int srcnn_stage_merge_device(srcnn_ctx* c, const uint8_t* d_y, const uint8_t* d_
                              size_t plane_pitch, int order, uint8_t* d_dst, size_t dst_stride) {
     ENTER(c);
     if (!d_y || !d_cr || !d_cb || !d_dst) return fail(c, SRCNN_E_ARG, "null pointer");
+    if (order != SRCNN_ORDER_BGR && order != SRCNN_ORDER_RGB) return fail(c, SRCNN_E_ARG, "colour order expected, got %d", order);
     if (w <= 0 || h <= 0 || dst_stride < (size_t)w * 3) return fail(c, SRCNN_E_ARG, "bad geometry");
     if (plane_pitch < align_up((size_t)w, 4) || (plane_pitch & 3) || (((uintptr_t)d_y | (uintptr_t)d_cr | (uintptr_t)d_cb) & 3))
         return fail(c, SRCNN_E_ARG, "planes must be 4-byte aligned with pitch a multiple of 4 and >= w rounded up to 4");

@@ -12,7 +12,10 @@
 // (hence __fmul_rn/__fadd_rn: no FMA contraction), round-half-even, and the integer form on the
 // last (ow mod 8) columns.  Results are bit-identical to the oracle (tests/test_stage_parity.py).
 //
-// Algorithmic HBM bytes per output pixel: 3/s^2 (BGR read) + 3 (planes written); K-C: 3 + 3.
+// A grey source (SRCNN_ORDER_GRAY) takes the same kernels with one plane and no colour conversion: the plain
+// resize(..., CV_INTER_CUBIC) of that plane.
+//
+// Algorithmic HBM bytes per output pixel: 3/s^2 (BGR read) + 3 (planes written); K-C: 3 + 3.  Grey: 1/s^2 + 1.
 #include <cuda_fp16.h>
 
 #include <cmath>
@@ -105,6 +108,7 @@ int get_taps(Ctx* c, int src, int dst, TapTable** out) {
 // geometry the tiled kernel's shared-memory footprint cannot hold (strong down-scales) and as the
 // in-library cross-check of the tiled kernel.
 // ------------------------------------------------------------------------------------------------
+template <int NP>   // planes: 3 = Y, Cr, Cb of a colour source, 1 = the one plane of a grey source (no colour conversion)
 __global__ void __launch_bounds__(256) k_color_bicubic_direct(ResizeDev p) {
     const int dx = blockIdx.x * 32 + (threadIdx.x & 31);
     const int dy = p.row_begin + blockIdx.y * 8 + (threadIdx.x >> 5);
@@ -121,6 +125,10 @@ __global__ void __launch_bounds__(256) k_color_bicubic_direct(ResizeDev p) {
 #pragma unroll
         for (int k = 0; k < 4; k++) {
             const int gx = clampi(sx - 1 + k, 0, p.sw - 1);
+            if (NP == 1) {
+                aY += (int)row[gx] * cxs[k];
+                continue;
+            }
             int c0 = row[3 * gx], c1 = row[3 * gx + 1], c2 = row[3 * gx + 2];
             int B = p.swapRB ? c2 : c0, R = p.swapRB ? c0 : c2;
             int Y, Cr, Cb;
@@ -134,25 +142,27 @@ __global__ void __launch_bounds__(256) k_color_bicubic_direct(ResizeDev p) {
     const bool fpath = dx < p.simd_w;
     const size_t o = (size_t)(dy - p.plane_row0) * p.pitch + dx;
     p.y[o] = (uint8_t)vertical_tap(hY[0], hY[1], hY[2], hY[3], cy, fpath);
+    if (NP == 1) return;
     p.cr[o] = (uint8_t)vertical_tap(hCr[0], hCr[1], hCr[2], hCr[3], cy, fpath);
     p.cb[o] = (uint8_t)vertical_tap(hCb[0], hCb[1], hCb[2], hCb[3], cy, fpath);
 }
 
 // ------------------------------------------------------------------------------------------------
-// K-A, tiled form (the fast path for up-scaling).  One CTA produces a TW x TH tile of all three
+// K-A, tiled form (the fast path for up-scaling).  One CTA produces a TW x TH tile of all NP
 // planes: (1) the source footprint is colour-converted ONCE into shared memory (three u8 planes,
-// replicate border applied at load), (2) the integer horizontal pass runs once per footprint row,
-// (3) the vertical pass reads four shared-memory sums per sample and writes 4 pixels per store.
+// replicate border applied at load; a grey source, NP = 1, is copied as it is), (2) the integer
+// horizontal pass runs once per footprint row, (3) the vertical pass reads four shared-memory sums
+// per sample and writes 4 pixels per store.
 // ------------------------------------------------------------------------------------------------
 constexpr int kTW = 64;                 // output tile width; the height is a template parameter (64 or 32 rows)
 constexpr int kMaxSC = 72, kMaxSR = 40; // footprint capacity (source cols / rows incl. the 3-tap apron)
 
-template <int kTH>
+template <int kTH, int NP>
 __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p) {   // 5 CTAs per SM: 48 registers (4 CTAs measured 6 % slower)
-    __shared__ __align__(16) uint8_t sP[3][kMaxSR][kMaxSC + 8];   // +8: the 3-word window read of the last quad may run past a row
+    __shared__ __align__(16) uint8_t sP[NP][kMaxSR][kMaxSC + 8];   // +8: the 3-word window read of the last quad may run past a row
     // horizontal sums kept as float: they are integers below 2^24, so the conversion is exact and is done
     // once per sum instead of once per use in the vertical pass
-    __shared__ __align__(16) float sH[3][kMaxSR][kTW];
+    __shared__ __align__(16) float sH[NP][kMaxSR][kTW];
     // per tile row: the four vertical taps as floats (b_k = coef_k * 2^-22, exact) and the first tap's row in sH -- computed once
     // per tile instead of once per (thread, row) in the vertical pass
     __shared__ __align__(16) float4 sB[kTH];
@@ -183,6 +193,10 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p) {  
         const int r = (int)(((unsigned)i * rcp20) >> 20), c = i - r * nsc;
         const int gy = clampi(sy_lo + r, 0, p.sh - 1) - p.src_row0;
         const int gx = clampi(sx_lo + c, 0, p.sw - 1);
+        if (NP == 1) {
+            sP[0][r][c] = fsrc[(size_t)gy * p.src_stride + gx];
+            continue;
+        }
         const uint8_t* px = fsrc + (size_t)gy * p.src_stride + 3 * (size_t)gx;
         const int B = px[oB], G = px[1], R = px[oR];
         const int Y = (1868 * B + 9617 * G + 4899 * R + 8192) >> 14;          // OpenCV RGB2YCrCb_i<uchar>, yuv_shift 14
@@ -190,8 +204,8 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p) {  
         asm("cvt.sat.u8.s32 %0, %1;" : "=r"(Cr) : "r"(((R - Y) * 11682 + (128 << 14) + 8192) >> 14));
         asm("cvt.sat.u8.s32 %0, %1;" : "=r"(Cb) : "r"(((B - Y) * 9241 + (128 << 14) + 8192) >> 14));
         sP[0][r][c] = (uint8_t)Y;
-        sP[1][r][c] = (uint8_t)Cr;
-        sP[2][r][c] = (uint8_t)Cb;
+        sP[NP > 1 ? 1 : 0][r][c] = (uint8_t)Cr;
+        sP[NP - 1][r][c] = (uint8_t)Cb;
     }
     __syncthreads();
 
@@ -215,7 +229,7 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p) {  
             const int wsh = 8 * (s0 & 3);
             for (int r = tid >> 4; r < nsr; r += 16) {
 #pragma unroll
-                for (int pl = 0; pl < 3; pl++) {
+                for (int pl = 0; pl < NP; pl++) {
                     const uint32_t* w = reinterpret_cast<const uint32_t*>(&sP[pl][r][s0 & ~3]);
                     const uint32_t w0 = w[0], w1 = w[1], w2 = w[2];
                     const uint32_t lo = __funnelshift_r(w0, w1, wsh), hi = __funnelshift_r(w1, w2, wsh);
@@ -241,7 +255,7 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p) {  
             const int k0 = cx.x, k1 = cx.y, k2 = cx.z, k3 = cx.w;
             for (int r = tid >> 6; r < nsr; r += 256 / kTW) {
 #pragma unroll
-                for (int pl = 0; pl < 3; pl++) {
+                for (int pl = 0; pl < NP; pl++) {
                     const uint8_t* q = &sP[pl][r][s];
                     sH[pl][r][col] = (float)((int)q[0] * k0 + (int)q[1] * k1 + (int)q[2] * k2 + (int)q[3] * k3);
                 }
@@ -259,8 +273,8 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p) {  
         const int col = (tid & 15) * 4, ty0 = tid >> 4;
         const unsigned long long nz = p.negzero2;
         const size_t o = fplane + (size_t)(dy0 + ty0 - p.plane_row0) * p.pitch + (size_t)(dx0 + col);
-        uint8_t* pcr = p.cr + o;
-        uint8_t* pcb = p.cb + o;
+        uint8_t* pcr = NP == 3 ? p.cr + o : nullptr;
+        uint8_t* pcb = NP == 3 ? p.cb + o : nullptr;
         uint8_t* py = p.y16 ? p.y16 + fy16 + (size_t)(dy0 + ty0 - p.plane_row0) * p.pitch16 + 2 * (size_t)(dx0 + col + kY16Pad) : p.y + o;
         const size_t step = 16 * p.pitch, ystep = p.y16 ? 16 * p.pitch16 : step;
         const bool y16 = p.y16 != nullptr;
@@ -271,7 +285,7 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p) {  
             const float* hrow = &sH[0][sSr[ty]][col];
             uint32_t packed[3];
 #pragma unroll
-            for (int pl = 0; pl < 3; pl++) {
+            for (int pl = 0; pl < NP; pl++) {
                 const float* h = hrow + pl * (kMaxSR * kTW);
                 const ulonglong2 g0 = *reinterpret_cast<const ulonglong2*>(h);
                 const ulonglong2 g1 = *reinterpret_cast<const ulonglong2*>(h + kTW);
@@ -299,9 +313,12 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p) {  
                 }
             }
             if (!y16) *reinterpret_cast<uint32_t*>(py) = packed[0];
-            *reinterpret_cast<uint32_t*>(pcr) = packed[1];
-            *reinterpret_cast<uint32_t*>(pcb) = packed[2];
-            py += ystep; pcr += step; pcb += step;
+            py += ystep;
+            if (NP == 3) {
+                *reinterpret_cast<uint32_t*>(pcr) = packed[1];
+                *reinterpret_cast<uint32_t*>(pcb) = packed[2];
+                pcr += step; pcb += step;
+            }
         }
         return;
     }
@@ -319,7 +336,7 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p) {  
                 const size_t o = fplane + (size_t)(dy - p.plane_row0) * p.pitch + dx;
                 const unsigned long long bb0 = f2_pack(b0, b0), bb1 = f2_pack(b1, b1), bb2 = f2_pack(b2, b2), bb3 = f2_pack(b3, b3);
 #pragma unroll
-                for (int pl = 0; pl < 3; pl++) {
+                for (int pl = 0; pl < NP; pl++) {
                     if (all_float) {   // two samples per instruction: v = H0*b0 + (H1*b1 + (H2*b2 + H3*b3)), each op rounded
                         const ulonglong2 g0 = *reinterpret_cast<const ulonglong2*>(&sH[pl][sr][col]);
                         const ulonglong2 g1 = *reinterpret_cast<const ulonglong2*>(&sH[pl][sr + 1][col]);
@@ -434,10 +451,11 @@ int launch_color_bicubic(Ctx* c, const ResizeArgs& a) {
         const int rc = launch_color_bicubic_int(c, p, a, &done);
         if (rc || done) return rc;
     }
+    const bool gray = a.order == SRCNN_ORDER_GRAY;
     if (th) {
         dim3 grid((a.ow + kTW - 1) / kTW, (rows + th - 1) / th, nframes);   // a batch of frames is one launch
-        if (th == 64) k_color_bicubic_tiled<64><<<grid, 256, 0, c->stream>>>(p);
-        else k_color_bicubic_tiled<32><<<grid, 256, 0, c->stream>>>(p);
+        if (th == 64) (gray ? k_color_bicubic_tiled<64, 1> : k_color_bicubic_tiled<64, 3>)<<<grid, 256, 0, c->stream>>>(p);
+        else (gray ? k_color_bicubic_tiled<32, 1> : k_color_bicubic_tiled<32, 3>)<<<grid, 256, 0, c->stream>>>(p);
         c->launches++;
         SRCNN_CUDA(c, cudaGetLastError());
         return SRCNN_OK;
@@ -446,9 +464,10 @@ int launch_color_bicubic(Ctx* c, const ResizeArgs& a) {
     for (int f = 0; f < nframes; f++) {
         ResizeDev q = p;
         q.src += (size_t)f * p.src_frame;
-        q.y += (size_t)f * p.plane_frame; q.cr += (size_t)f * p.plane_frame; q.cb += (size_t)f * p.plane_frame;
+        q.y += (size_t)f * p.plane_frame;
+        if (!gray) { q.cr += (size_t)f * p.plane_frame; q.cb += (size_t)f * p.plane_frame; }
         dim3 grid((a.ow + 31) / 32, (rows + 7) / 8);
-        k_color_bicubic_direct<<<grid, 256, 0, c->stream>>>(q);
+        (gray ? k_color_bicubic_direct<1> : k_color_bicubic_direct<3>)<<<grid, 256, 0, c->stream>>>(q);
         c->launches++;
         SRCNN_CUDA(c, cudaGetLastError());
         if (a.pl.y16) {

@@ -16,6 +16,7 @@
 //       v = H0*b0 + (H1*b1 + (H2*b2 + H3*b3)), every product and sum rounded on its own (f2_mul_rn / f2_add_rn), round-half-even,
 //       saturate, one 8- or 16-byte store per lane and row.  No shared-memory round trip of the sums, no per-sample addressing.
 // Y goes to the padded FP16 plane of the tcgen05 kernel when the context has one (color_bicubic.cu explains the layout).
+// A grey source (SRCNN_ORDER_GRAY) has its own kernel below, k_gray_bicubic_int: raw bytes staged, the same walk.
 // Measured and not kept (tools/experiments/color_bicubic_int_persistent_tma.cu.txt, DESIGN.md): fetching a tile's raw rows by TMA
 // (neutral), persistent CTAs with the next tile's rows prefetched by TMA -- as one block-wide pipeline, with a producer warp, or
 // as three per-warp pipelines (all slower: the kernel is bound by instruction issue while a wave of tiles computes, and every
@@ -112,9 +113,9 @@ __device__ __forceinline__ void clamped_group(const uint8_t* row, int gx, int sw
     }
 }
 
-// (2) the walk of one warp (one plane) down a tile's converted footprint `plane` (rows kIPitch bytes apart): lane's output columns
+// (2) the walk of one warp (one plane) down a tile's converted footprint `plane` (rows kPitch bytes apart): lane's output columns
 // x0 .. x0+7 read footprint bytes cb .. cb+7 of a row
-template <int S>
+template <int S, int kPitch = kIPitch>
 __device__ __forceinline__ void walk_tile(const ResizeDev& p, const IntTaps& t, const uint8_t* plane, int pl, int lane, int X0, int a,
                                           int nit, size_t fz) {
     const int x0 = X0 + 8 * lane;
@@ -128,7 +129,7 @@ __device__ __forceinline__ void walk_tile(const ResizeDev& p, const IntTaps& t, 
     const size_t ostep = y16 ? p.pitch16 : p.pitch;
 
                 auto hsum = [&](int r, unsigned long long (&h)[4]) {
-                    const uint32_t* w = reinterpret_cast<const uint32_t*>(srow + r * kIPitch);
+                    const uint32_t* w = reinterpret_cast<const uint32_t*>(srow + r * kPitch);
                     const uint32_t w0 = w[0], w1 = w[1], w2 = w[2];
                     uint32_t lo = 0, hi = 0;
                     if (S != 2) { lo = __funnelshift_r(w0, w1, wsh); hi = __funnelshift_r(w1, w2, wsh); }
@@ -294,15 +295,74 @@ __global__ void __launch_bounds__(96, S == 2 ? SRCNN_KA_MINB : SRCNN_KA_MINB4) k
     if (tile == t.ntiles - 1) asm volatile("griddepcontrol.wait;" ::: "memory");
 }
 
-inline int floordiv(int a, int b) { return a >= 0 ? a / b : -((-a + b - 1) / b); }
+// ------------------------------------------------------------------------------------------------
+// One-plane form (SRCNN_ORDER_GRAY): the footprint is the source bytes as they are, with the replicate border.  One CTA of
+// three warps takes three ADJACENT tiles: their footprints are one contiguous run of 3 * kITW / S + 8 source columns, staged
+// once, and warp w walks tile w from its own offset in it -- the same 96-thread CTA (and occupancy tuning) and the same
+// walk as the colour kernel.
+// ------------------------------------------------------------------------------------------------
+constexpr int kGPitch = 400;       // bytes per staged row: 3 * 128 + 8 columns at x2 (98 words) + the spare word of the window read
 
 template <int S>
+__global__ void __launch_bounds__(96, S == 2 ? SRCNN_KA_MINB : SRCNN_KA_MINB4) k_gray_bicubic_int(const ResizeDev p, const IntTaps t) {
+    constexpr int GG = 3 * kITW / S / 4 + 2;       // four-byte groups per staged row
+    static_assert(4 * GG + 4 <= kGPitch, "staged row too short");
+    __shared__ __align__(16) uint8_t sP[kIRows][kGPitch];
+    const int tid = threadIdx.x;
+    const int tile = blockIdx.x;
+    const int bx = tile % t.ntx, rest = tile / t.ntx;
+    const int by = rest % t.nty;
+    const size_t fz = (size_t)(rest / t.nty);
+    const int X0 = 3 * kITW * bx;                  // first column of warp 0's tile
+    const int a = t.a_first + by * t.isr;          // staged row r is source row a - 1 + r
+    const int F0 = X0 / S - 4;                     // first staged column (a multiple of 4)
+    const int nit = min(t.isr, t.i_last - a + 1);
+    const int nsr = nit + 3;
+    const uint8_t* const fsrc = p.src + fz * p.src_frame;
+
+    // (1) stage the footprint: all of a thread's loads go out before its first shared store
+    constexpr int NG = (kIRows * GG + 95) / 96;
+    uint32_t raw[NG];
+#pragma unroll
+    for (int it = 0; it < NG; it++) {
+        const int g = tid + 96 * it;
+        if (g < nsr * GG) {
+            const int r = g / GG, gx = F0 + 4 * (g - r * GG);
+            const uint8_t* row = fsrc + (size_t)(clampi(a - 1 + r, 0, p.sh - 1) - p.src_row0) * p.src_stride;
+            if (t.vec_ok && gx >= 0 && gx + 4 <= p.sw) {
+                raw[it] = *reinterpret_cast<const uint32_t*>(row + gx);
+            } else {
+                uint32_t v = 0;
+#pragma unroll
+                for (int j = 0; j < 4; j++) v |= (uint32_t)row[clampi(gx + j, 0, p.sw - 1)] << (8 * j);
+                raw[it] = v;
+            }
+        }
+    }
+#pragma unroll
+    for (int it = 0; it < NG; it++) {
+        const int g = tid + 96 * it;
+        if (g < nsr * GG) {
+            const int r = g / GG;
+            *reinterpret_cast<uint32_t*>(&sP[r][4 * (g - r * GG)]) = raw[it];
+        }
+    }
+    __syncthreads();
+    // (2) the walk: warp w's tile starts w * kITW / S staged columns further
+    const int w = tid >> 5;
+    walk_tile<S, kGPitch>(p, t, &sP[0][w * (kITW / S)], 0, tid & 31, X0 + w * kITW, a, nit, fz);
+}
+
+inline int floordiv(int a, int b) { return a >= 0 ? a / b : -((-a + b - 1) / b); }
+
+template <int S, bool GRAY>
 int launch_variant(Ctx* c, const ResizeDev& p, IntTaps& t, int nframes, bool early) {
+    void (*const kern)(const ResizeDev, const IntTaps) = GRAY ? k_gray_bicubic_int<S> : k_color_bicubic_int<S>;
     static int ctas_per_sm[64] = {0};              // per device; a benign race: every writer stores the same value
     int& per_sm = ctas_per_sm[c->device & 63];
     if (per_sm == 0) {
         int n = 0;
-        SRCNN_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_color_bicubic_int<S>, 96, 0));
+        SRCNN_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kern, 96, 0));
         per_sm = std::max(1, n);
     }
     // Tile height (same-box A/B, B200): a single 4K frame runs fastest as ~1.5 waves of 8-row tiles (23.6 us; 6 rows: 23.7,
@@ -329,9 +389,9 @@ int launch_variant(Ctx* c, const ResizeDev& p, IntTaps& t, int nframes, bool ear
         at[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = at;
         cfg.numAttrs = 1;
-        SRCNN_CUDA(c, cudaLaunchKernelEx(&cfg, k_color_bicubic_int<S>, p, t));
+        SRCNN_CUDA(c, cudaLaunchKernelEx(&cfg, kern, p, t));
     } else {
-        k_color_bicubic_int<S><<<t.ntiles, 96, 0, c->stream>>>(p, t);
+        kern<<<t.ntiles, 96, 0, c->stream>>>(p, t);
     }
     c->launches++;
     SRCNN_CUDA(c, cudaGetLastError());
@@ -368,9 +428,13 @@ int launch_color_bicubic_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bo
     t.i_last = floordiv(a.row_end - 1 - S / 2, S);
     t.vec_ok = (((uintptr_t)p.src | p.src_stride | p.src_frame) & 3) == 0;
     const int nframes = std::max(1, a.nframes);
+    const bool gray = a.order == SRCNN_ORDER_GRAY;
     t.ntx = (a.ow + kITW - 1) / kITW;
+    if (gray) t.ntx = (t.ntx + 2) / 3;             // a CTA per three adjacent tiles
     if ((long long)t.ntx * (t.i_last - t.a_first + 1) * nframes > 0x3fffffffLL) return SRCNN_OK;
-    const int rc = S == 2 ? launch_variant<2>(c, p, t, nframes, a.early) : launch_variant<4>(c, p, t, nframes, a.early);
+    int rc;
+    if (gray) rc = S == 2 ? launch_variant<2, true>(c, p, t, nframes, false) : launch_variant<4, true>(c, p, t, nframes, false);   // never early (api.cu)
+    else rc = S == 2 ? launch_variant<2, false>(c, p, t, nframes, a.early) : launch_variant<4, false>(c, p, t, nframes, a.early);
     if (rc) return rc;
     *done = true;
     return SRCNN_OK;

@@ -207,7 +207,7 @@ struct ResizeArgs {
     size_t src_frame_stride = 0;
     bool early = false;   // may start while the previous kernel of the stream (a merge kernel of ours) is still running
 };
-int launch_color_bicubic(Ctx* c, const ResizeArgs& a);
+int launch_color_bicubic(Ctx* c, const ResizeArgs& a);   // order SRCNN_ORDER_GRAY: the one plane, into pl.y / pl.y16
 
 struct MergeArgs {
     const uint8_t* y;
@@ -225,7 +225,7 @@ void note_merge(Ctx* c);   // api.cu: this context has just put a merge kernel (
 int launch_y8_to_y16(Ctx* c, const uint8_t* y, size_t pitch, int w, int rows, uint8_t* y16, size_t pitch16);
 
 // CNN on a plane band.  y points at plane row 0 which is image row `row0`; the plane holds image rows
-// [row0, row0+rows).  Produces image rows [out_begin, out_end) into `out` (same row0 convention).
+// [row0, row0+rows).  Produces image rows [out_begin, out_end) into `out`, whose row 0 is image row `out_row0`.
 // Border clamps use the FULL image height H / width W (true borders only; band seams read real halo).
 struct CnnArgs {
     const uint8_t* y;
@@ -237,6 +237,7 @@ struct CnnArgs {
     int out_begin, out_end;
     uint8_t* out;
     size_t out_pitch;
+    int out_row0 = 0;   // the planes' row0 for the Y' plane; r0 when a grey call writes straight into the caller's band
     // optional fused merge + YCrCb->BGR (row-walking tcgen05 kernel only): when `bgr` is set the kernel reads the Cr/Cb planes
     // (same pitch / row0 convention as y) and writes interleaved pixels for output rows [out_begin, out_end) to `bgr`
     // (which points at row out_begin) instead of the Y' plane

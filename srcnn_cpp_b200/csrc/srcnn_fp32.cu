@@ -147,7 +147,7 @@ int launch_cnn_fp32(Ctx* c, const CnnArgs& a, float* act2_out) {
         c->launches++;
         SRCNN_CUDA(c, cudaGetLastError());
         dim3 g2((W + 31) / 32, (ce - cb + 7) / 8);
-        k_conv55_strict<<<g2, 256, 0, c->stream>>>(act2, plane_stride, ab, W, H, cb, ce, a.out, a.out_pitch, a.row0);
+        k_conv55_strict<<<g2, 256, 0, c->stream>>>(act2, plane_stride, ab, W, H, cb, ce, a.out, a.out_pitch, a.out_row0);
         c->launches++;
         SRCNN_CUDA(c, cudaGetLastError());
     }

@@ -308,8 +308,9 @@ struct Params {
     int W, H;
     int row0, rows;
     int out_begin, out_end;  // image rows to produce
-    uint8_t* out;          // same row0 convention as y
+    uint8_t* out;          // Y' plane: row 0 is image row out_row0
     size_t out_pitch;
+    int out_row0;
     const uint8_t* cr;     // fused merge (optional, bgr != nullptr): chroma planes, same pitch / row0 as y
     const uint8_t* cb;
     uint8_t* bgr;          // interleaved result, row out_begin first
@@ -755,7 +756,7 @@ __device__ __forceinline__ void role_loop(const Params& p, uint8_t* smem, const 
                 for (int n = 0; n < 5; n++) acc[k][n] = 0.f;
             // rows are stored in order ra, ra+1, ...
             uint8_t* outp = FUSED ? p.bgr + (size_t)(ra - p.out_begin) * p.bgr_stride + (size_t)3 * (col_ok ? x : 0)
-                                  : p.out + (size_t)frame * p.out_frame + (size_t)(ra - p.row0) * p.out_pitch + x;
+                                  : p.out + (size_t)frame * p.out_frame + (size_t)(ra - p.out_row0) * p.out_pitch + x;
             const uint8_t* crp = FUSED ? p.cr + (size_t)(ra - p.row0) * p.pitch + (col_ok ? x : 0) : nullptr;
             const uint8_t* cbp = FUSED ? p.cb + (size_t)(ra - p.row0) * p.pitch + (col_ok ? x : 0) : nullptr;
             E3Ctx cx{p, hx_s + 4 * tp, ctr + 4 * (uint32_t)(tp >> 5), bars, tml, tp, pipe, ta, tb, ra, rb, col_ok, first_seg, warp0, leader};
@@ -986,7 +987,7 @@ int launch_cnn_tc2(Ctx* c, const CnnArgs& a0) {
     p.W = a.W; p.H = a.H;
     p.row0 = a.row0; p.rows = a.rows;
     p.out_begin = a.out_begin; p.out_end = a.out_end;
-    p.out = a.out; p.out_pitch = a.out_pitch;
+    p.out = a.out; p.out_pitch = a.out_pitch; p.out_row0 = a.out_row0;
     p.cr = a.cr; p.cb = a.cb;
     p.bgr = a.bgr; p.bgr_stride = a.bgr_stride;
     p.swap_rb = a.order == SRCNN_ORDER_RGB ? 1 : 0;
