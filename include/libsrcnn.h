@@ -3,9 +3,9 @@
 // from that call site).  C++ (reference-compatible references); a thin wrapper over the C ABI in
 // srcnn_b200.h, implemented in srcnn_cpp_b200/cli/libsrcnn.cpp and exported by libsrcnn_b200.so.
 //
-//   refbuff   packed 8-bit pixels, `d` bytes per pixel: 3 = RGB, 4 = RGBA (alpha takes the path's plain
-//             bicubic resize -- srcnn_resize_plane_host, no CNN -- colour goes through the SRCNN path), 1 = grey, 2 = grey+alpha (grey: the
-//             one-plane path, SRCNN_ORDER_GRAY) -- the inputs
+//   refbuff   packed 8-bit pixels, `d` bytes per pixel: 3 = RGB, 4 = RGBA (one SRCNN_ORDER_RGBA call: colour goes through the
+//             SRCNN path, straight alpha takes the path's plain bicubic resize, no CNN), 1 = grey, 2 = grey+alpha (grey: the
+//             one-plane path, SRCNN_ORDER_GRAY; its alpha through srcnn_resize_plane_host) -- the inputs
 //             src/test.cpp:34-134 (convImage) can produce
 //   w, h, d   geometry
 //   muliply   scale ratio (sic, the reference's spelling)

@@ -19,8 +19,16 @@
  * -- or SRCNN_ORDER_GRAY: one channel, 1 byte per pixel in and out (src_stride >= w, dst_stride >= ow).
  * A grey call returns the CNN's Y' of resize(grey) and never computes chroma; it is bit-identical to any
  * channel of the colour path on the grey image replicated to 3 channels (a grey pixel has Y = v and
- * Cr = Cb = 128, which convert back to B = G = R = Y').  Output size is ow=(int)((float)w*scale), oh=(int)((float)h*scale) -- the
- * reference's truncation (src/srcnn.cpp:573-575, src/test.cpp:357-358).
+ * Cr = Cb = 128, which convert back to B = G = R = Y').
+ * SRCNN_ORDER_BGRA / SRCNN_ORDER_RGBA: 4 interleaved bytes per pixel in and out (src_stride >= 4*w, dst_stride >= 4*ow), straight
+ * (not premultiplied) alpha in byte 3.  Bytes 0..2 of every output pixel equal, byte for byte, the 3-channel call with the
+ * matching order (BGRA -> BGR, RGBA -> RGB) on bytes 0..2 of the source; alpha has no influence on them.  Byte 3 is the alpha
+ * plane through the one-plane resize (srcnn_stage_resize_plane_device: resize(alpha, INTER_CUBIC), no CNN) -- what the
+ * reference does to its planes after `split` (src/srcnn.cpp:540,577-582) and what ProcessSRCNN returns for d = 4.  It is NOT
+ * always channel 3 of cv::resize on a CV_8UC4 image: with 4 channels OpenCV splits its float body and integer tail at another
+ * column, and the two differ by 1 LSB on some geometries.
+ * Output size is ow=(int)((float)w*scale), oh=(int)((float)h*scale) -- the reference's truncation (src/srcnn.cpp:573-575,
+ * src/test.cpp:357-358).
  */
 #ifndef SRCNN_B200_H
 #define SRCNN_B200_H
@@ -46,7 +54,7 @@ enum {
     SRCNN_VARIANT_FP32 = 1  /* strict FP32 CUDA-core kernels in the reference's summation order (bit-exact) */
 };
 
-enum { SRCNN_ORDER_BGR = 0, SRCNN_ORDER_RGB = 1, SRCNN_ORDER_GRAY = 2 };
+enum { SRCNN_ORDER_BGR = 0, SRCNN_ORDER_RGB = 1, SRCNN_ORDER_GRAY = 2, SRCNN_ORDER_BGRA = 3, SRCNN_ORDER_RGBA = 4 };
 
 /* Status codes.  -1 / -2 / -3 / -10 keep the reference CLI's meanings (src/srcnn.cpp:479,493,526,555,684). */
 enum {
@@ -198,7 +206,7 @@ void srcnn_jpeg_free(uint8_t* p);
 
 /* ---- stages (device pointers; enqueued on the context stream) ------------------------------------ */
 /* cvtColor + split + 3x resize (src/srcnn.cpp:509,540,570-583): BGR8 -> three u8 planes of ow x oh.  Colour orders only
- * (SRCNN_ORDER_GRAY: SRCNN_E_ARG; srcnn_stage_resize_plane_device is the one-plane stage). */
+ * (SRCNN_ORDER_GRAY, _BGRA, _RGBA: SRCNN_E_ARG; srcnn_stage_resize_plane_device is the one-plane stage). */
 int srcnn_stage_color_bicubic_device(srcnn_ctx* ctx, const uint8_t* d_src, int w, int h, size_t src_stride,
                                      int order, float scale, uint8_t* d_y, uint8_t* d_cr, uint8_t* d_cb,
                                      size_t plane_pitch);
@@ -215,7 +223,7 @@ int srcnn_stage_cnn_device(srcnn_ctx* ctx, int variant, const uint8_t* d_y, int 
 /* FP32 variant only: also returns conv2's activations, 32 planes of h*w float (src/srcnn.cpp:602-607). */
 int srcnn_stage_conv99x11_fp32_device(srcnn_ctx* ctx, const uint8_t* d_y, int w, int h, size_t pitch,
                                       float* d_act2);
-/* merge + cvtColor back (src/srcnn.cpp:637-639,657): three planes -> BGR8 HWC.  Colour orders only. */
+/* merge + cvtColor back (src/srcnn.cpp:637-639,657): three planes -> BGR8 HWC.  Colour orders only (BGR, RGB). */
 int srcnn_stage_merge_device(srcnn_ctx* ctx, const uint8_t* d_y, const uint8_t* d_cr, const uint8_t* d_cb,
                              int w, int h, size_t plane_pitch, int order, uint8_t* d_dst, size_t dst_stride);
 

@@ -21,6 +21,8 @@ VARIANT_FP32 = 1
 ORDER_BGR = 0
 ORDER_RGB = 1
 ORDER_GRAY = 2   # one channel: HxW (NxHxW) arrays and tensors in and out; the result is the CNN's Y'
+ORDER_BGRA = 3   # four channels, straight alpha in byte 3: HxWx4 (NxHxWx4) in and out; colour bytes = the BGR call's,
+ORDER_RGBA = 4   # alpha = the one-plane cubic resize of the alpha plane (no CNN)
 
 OK = 0
 E_RATIO = -1
@@ -179,15 +181,17 @@ class PinnedBuffer:
 
 
 def _pixel_shape(order):
-    """trailing shape of one pixel: () for ORDER_GRAY, (3,) for the colour orders"""
-    return () if order == ORDER_GRAY else (3,)
+    """trailing shape of one pixel: () for ORDER_GRAY, (4,) for ORDER_BGRA / ORDER_RGBA, (3,) for the colour orders"""
+    if order == ORDER_GRAY:
+        return ()
+    return (4,) if order in (ORDER_BGRA, ORDER_RGBA) else (3,)
 
 
 def _check_host_image(a, order, lead):
-    """a: numpy uint8 array of `lead` leading dims (1: HxW[x3], 2: NxHxW[x3]) in the layout `order` implies"""
+    """a: numpy uint8 array of `lead` leading dims (1: HxW[xC], 2: NxHxW[xC]) in the layout `order` implies"""
     px = _pixel_shape(order)
     if a.dtype != np.uint8 or a.ndim != lead + 1 + len(px) or tuple(a.shape[lead + 1:]) != px:
-        raise SrcnnError(E_ARG, "expected a %s uint8 array" % ("x".join(["N"] * (lead - 1) + ["H", "W"] + ["3"] * len(px))))
+        raise SrcnnError(E_ARG, "expected a %s uint8 array" % ("x".join(["N"] * (lead - 1) + ["H", "W"] + [str(c) for c in px])))
 
 
 def _dptr(t):
@@ -258,8 +262,8 @@ class Engine:
 
     # -- whole path, host buffers (numpy) ----------------------------------------------------------
     def process(self, img, scale, order=ORDER_BGR, out=None):
-        """img: HxWx3 uint8 numpy array (BGR by default, like cv::imread), or HxW with order=ORDER_GRAY.  Returns OHxOWx3
-        (OHxOW) uint8."""
+        """img: HxWx3 uint8 numpy array (BGR by default, like cv::imread), HxW with order=ORDER_GRAY, or HxWx4 with
+        order=ORDER_BGRA / ORDER_RGBA.  Returns OHxOWx3 (OHxOW, OHxOWx4) uint8."""
         img = np.asarray(img)
         _check_host_image(img, order, 1)
         if not img.flags.c_contiguous:
@@ -273,7 +277,8 @@ class Engine:
         return out
 
     def process_batch(self, frames, scale, order=ORDER_BGR, out=None):
-        """frames: NxHxWx3 (NxHxW with order=ORDER_GRAY) uint8 numpy array -> NxOHxOWx3 (NxOHxOW)."""
+        """frames: NxHxWx3 (NxHxW with order=ORDER_GRAY, NxHxWx4 with ORDER_BGRA / ORDER_RGBA) uint8 numpy array -> NxOHxOWx3
+        (NxOHxOW, NxOHxOWx4)."""
         frames = np.ascontiguousarray(frames)
         _check_host_image(frames, order, 2)
         n, h, w = frames.shape[:3]
@@ -287,7 +292,8 @@ class Engine:
 
     # -- whole path, device buffers (torch CUDA tensors) -------------------------------------------
     def process_device(self, src, scale, dst, order=ORDER_BGR):
-        """src: HxWx3 (HxW with order=ORDER_GRAY) uint8 device tensor; dst: OHxOWx3 (OHxOW)."""
+        """src: HxWx3 (HxW with order=ORDER_GRAY, HxWx4 with ORDER_BGRA / ORDER_RGBA) uint8 device tensor; dst: OHxOWx3
+        (OHxOW, OHxOWx4)."""
         h, w = src.shape[:2]
         self._check(self.L.srcnn_process_device(self.ctx, _dptr(src), w, h, src.stride(0), order, C.c_float(scale),
                                                 _dptr(dst), dst.stride(0)))
@@ -300,7 +306,8 @@ class Engine:
         return dst
 
     def process_band_device(self, src_rows, w, h, s0, s1, scale, r0, r1, dst_rows, order=ORDER_BGR):
-        """src_rows: (s1-s0)xWx3 device tensor holding source rows [s0,s1); dst_rows: (r1-r0)xOWx3 (no x3 with ORDER_GRAY)."""
+        """src_rows: (s1-s0)xWx3 device tensor holding source rows [s0,s1); dst_rows: (r1-r0)xOWx3 (no x3 with ORDER_GRAY, x4
+        with ORDER_BGRA / ORDER_RGBA)."""
         self._check(self.L.srcnn_process_band_device(self.ctx, _dptr(src_rows), w, h, src_rows.stride(0), s0, s1, order,
                                                      C.c_float(scale), r0, r1, _dptr(dst_rows), dst_rows.stride(0)))
         return dst_rows
@@ -330,7 +337,8 @@ class Engine:
         self._check(self.L.srcnn_debug_set_host_bands(self.ctx, int(bands)))
 
     def process_band_host(self, img, scale, r0, r1, out_rows=None, order=ORDER_BGR):
-        """img: the WHOLE HxWx3 (HxW) source image; returns output rows [r0, r1) as an (r1-r0)xOWx3 ((r1-r0)xOW) array."""
+        """img: the WHOLE HxWx3 (HxW, HxWx4) source image; returns output rows [r0, r1) as an (r1-r0)xOWx3 ((r1-r0)xOW,
+        (r1-r0)xOWx4) array."""
         img = np.ascontiguousarray(img)
         _check_host_image(img, order, 1)
         h, w = img.shape[:2]
@@ -466,8 +474,8 @@ class MultiEngine:
 
     # -- device-resident shares (torch CUDA tensors, one per worker, each on that worker's device) -----
     def process_batch_device(self, srcs, scale, dsts, order=ORDER_BGR):
-        """srcs[i]: n_i x H x W x 3 (no x 3 with ORDER_GRAY) on worker i's device (n_i may be 0 -> pass None); dsts[i]:
-        n_i x OH x OW x 3."""
+        """srcs[i]: n_i x H x W x 3 (no x 3 with ORDER_GRAY, x 4 with ORDER_BGRA / ORDER_RGBA) on worker i's device (n_i may be
+        0 -> pass None); dsts[i]: n_i x OH x OW x 3 (likewise)."""
         ref = next(t for t in srcs if t is not None)
         h, w = ref.shape[1:3]
         dref = next(t for t in dsts if t is not None)
@@ -478,7 +486,8 @@ class MultiEngine:
                                                            pd, dref.stride(1), dref.stride(0)))
 
     def process_banded_device(self, src_bands, w, h, scale, dst_bands, order=ORDER_BGR):
-        """src_bands[i]: (s1_i-s0_i) x W x 3 holding the source rows of band_plan()[i]; dst_bands[i]: (r1_i-r0_i) x OW x 3."""
+        """src_bands[i]: (s1_i-s0_i) x W x 3 (x 4, or no channel dim, per `order`) holding the source rows of band_plan()[i];
+        dst_bands[i]: (r1_i-r0_i) x OW x 3 (likewise)."""
         ps = (C.c_void_p * self.n)(*[t.data_ptr() if t is not None else None for t in src_bands])
         pd = (C.c_void_p * self.n)(*[t.data_ptr() if t is not None else None for t in dst_bands])
         sref = next(t for t in src_bands if t is not None)

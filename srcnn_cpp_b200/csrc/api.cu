@@ -66,14 +66,14 @@ static int scaled_dim(int n, float scale) {
     return (int)((float)n * scale);
 }
 
-static size_t bytes_per_pixel(int order) { return order == SRCNN_ORDER_GRAY ? 1 : 3; }
+static size_t bytes_per_pixel(int order) { return order == SRCNN_ORDER_GRAY ? 1 : (four_channel(order) ? 4 : 3); }
 
 static int check_image(Ctx* c, const void* src, int w, int h, size_t stride, int order, float scale, const void* dst,
                        size_t dst_stride, int* ow, int* oh) {
     if (!c) return SRCNN_E_ARG;
     if (!src || !dst) return fail(c, SRCNN_E_ARG, "null image pointer");
     if (w <= 0 || h <= 0) return fail(c, SRCNN_E_ARG, "non-positive image size %dx%d", w, h);
-    if (order != SRCNN_ORDER_BGR && order != SRCNN_ORDER_RGB && order != SRCNN_ORDER_GRAY)
+    if (order != SRCNN_ORDER_BGR && order != SRCNN_ORDER_RGB && order != SRCNN_ORDER_GRAY && !four_channel(order))
         return fail(c, SRCNN_E_ARG, "unknown pixel order %d", order);
     const size_t bpp = bytes_per_pixel(order);
     if (stride < (size_t)w * bpp) return fail(c, SRCNN_E_ARG, "source stride %zu < %zu*w", stride, bpp);
@@ -86,31 +86,37 @@ static int check_image(Ctx* c, const void* src, int w, int h, size_t stride, int
     return SRCNN_OK;
 }
 
-// planes of `nframes` same-sized frames: [Y frames][Cr frames][Cb frames][Y' frames][FP16 Y frames]
+// planes of `nframes` same-sized frames: [Y frames][Cr frames][Cb frames][Y' frames][FP16 Y frames], and for a four-channel
+// call [A frames] after them (so the colour and grey layouts do not depend on it)
 // Cross-call overlap: the only planes the colour+bicubic kernel of call i+1 writes AND the merge kernel of call i reads are Cr and
-// Cb, so device-resident whole-path calls alternate between two Cr/Cb pairs (the second in plane_buf2, when a pair is at most
-// 4 GiB); Y, Y' and the FP16 Y plane are shared (the merge never reads Y / FP16 Y, and Y' is written by the next CNN launch, which
-// waits for everything before it).  c->plane_sel says which pair this call got.  Keeping the rest single also keeps the planes
-// L2-resident from step to step: two whole plane sets (116 MB at 4K) measured 3 us slower in the colour+bicubic kernel.
-// The host-buffer pipeline keeps to pair 0 (its sub-bands are separated by copies and events anyway).  A grey call has no Cr/Cb
-// planes: it leaves the pair selection alone (and ends the early-start chain, end_merge_chain).
-static int carve_planes(Ctx* c, int ow, int rows, int row0, Planes* pl, int nframes = 1, bool gray = false) {
+// Cb (and A, for four-channel calls), so device-resident whole-path calls alternate between two sets of them (the second in
+// plane_buf2, when a set is at most 4 GiB: Cr, Cb and A of a four-channel call); Y, Y' and the FP16 Y plane are shared (the merge
+// never reads Y / FP16 Y, and Y' is written by the next CNN launch, which waits for everything before it).  c->plane_sel says which
+// set this call got.  Keeping the rest single also keeps the planes L2-resident from step to step: two whole plane sets (116 MB
+// at 4K) measured 3 us slower in the colour+bicubic kernel.
+// The host-buffer pipeline keeps to set 0 (its sub-bands are separated by copies and events anyway).  A grey call has no Cr/Cb
+// planes: it leaves the set selection alone (and ends the early-start chain, end_merge_chain).
+static int carve_planes(Ctx* c, int ow, int rows, int row0, Planes* pl, int nframes = 1, int order = SRCNN_ORDER_BGR) {
+    const bool gray = order == SRCNN_ORDER_GRAY, four = four_channel(order);
     const size_t pitch = align_up((size_t)ow, 128);
     const size_t plane = pitch * (size_t)rows;
     const size_t pitch16 = y16_pitch_bytes(ow);
     const size_t plane16 = align_up(pitch16 * (size_t)rows, 256);
     const size_t nf = (size_t)nframes;
-    const size_t bytes = (plane * 4 + plane16) * nf + 512;   // slack: the last row's last strip copy may run past the row
-    const bool two = c->overlap && !c->host_path && !c->capturing && plane * 2 * nf <= ((size_t)4 << 30);
+    const size_t nalt = four ? 3 : 2;                         // planes of the alternating set: Cr, Cb (, A)
+    // slack: the last row's last strip copy may run past the row
+    const size_t bytes = (plane * 4 + plane16) * nf + (four ? plane * nf : 0) + 512;
+    const bool two = c->overlap && !c->host_path && !c->capturing && plane * nalt * nf <= ((size_t)4 << 30);
     if (!gray) c->plane_sel = two ? (c->plane_sel ^ 1) : 0;
     int rc = ensure(c, c->plane_buf, bytes);
     if (rc) return rc;
-    if (!gray && c->plane_sel && (rc = ensure(c, c->plane_buf2, plane * 2 * nf))) return rc;
+    if (!gray && c->plane_sel && (rc = ensure(c, c->plane_buf2, plane * nalt * nf))) return rc;
     c->plane_layout[0] = pitch; c->plane_layout[1] = (size_t)rows; c->plane_layout[2] = nf;
     uint8_t* base = (uint8_t*)c->plane_buf.p;
     pl->y = base;
     pl->cr = gray ? nullptr : c->plane_sel ? (uint8_t*)c->plane_buf2.p : base + plane * nf;
     pl->cb = gray ? nullptr : c->plane_sel ? (uint8_t*)c->plane_buf2.p + plane * nf : base + 2 * plane * nf;
+    pl->a = !four ? nullptr : c->plane_sel ? (uint8_t*)c->plane_buf2.p + 2 * plane * nf : base + (4 * plane + plane16) * nf;
     pl->yout = base + 3 * plane * nf;
     pl->y16 = base + 4 * plane * nf;
     pl->frame_stride = plane;
@@ -190,7 +196,7 @@ static int process_rows_impl(Ctx* c, const uint8_t* d_src, int w, int h, size_t 
     if (gray) end_merge_chain(c);
     Planes pl;
     c->fail_stage = SRCNN_STAGE_PLANES;
-    rc = carve_planes(c, ow, p1 - p0, p0, &pl, 1, gray);
+    rc = carve_planes(c, ow, p1 - p0, p0, &pl, 1, order);
     if (rc) return rc;
     c->fail_stage = SRCNN_STAGE_COLOR_BICUBIC;
     // the band must bring every source row its taps touch
@@ -225,7 +231,8 @@ static int process_rows_impl(Ctx* c, const uint8_t* d_src, int w, int h, size_t 
     else { ca.out = pl.yout; ca.out_pitch = pl.pitch; ca.out_row0 = p0; }
     // optionally the row-walking tcgen05 kernel merges Cr/Cb and converts back to BGR in its last epilogue (no Y' plane, no
     // K-C launch); measured slower than the separate launch (byte stores from one-thread-per-column lanes), so off by default
-    const bool fused = !gray && c->variant == SRCNN_VARIANT_TC && c->fuse_merge;
+    // (colour orders only: a four-channel call takes the separate merge, which writes alpha too)
+    const bool fused = !gray && !four_channel(order) && c->variant == SRCNN_VARIANT_TC && c->fuse_merge;
     if (fused) {
         ca.cr = pl.cr; ca.cb = pl.cb;
         ca.bgr = d_dst; ca.bgr_stride = dst_stride; ca.order = order;
@@ -239,6 +246,7 @@ static int process_rows_impl(Ctx* c, const uint8_t* d_src, int w, int h, size_t 
     MergeArgs ma;
     const size_t off = (size_t)(r0 - p0) * pl.pitch;
     ma.y = pl.yout + off; ma.cr = pl.cr + off; ma.cb = pl.cb + off;
+    if (pl.a) ma.a = pl.a + off;
     ma.pitch = pl.pitch; ma.w = ow; ma.rows = r1 - r0;
     ma.order = order;
     ma.dst = d_dst; ma.dst_stride = dst_stride;
@@ -267,7 +275,7 @@ static int process_frames_impl(Ctx* c, const uint8_t* d_src, int n, int w, int h
     int rc = get_taps(c, w, ow, &tx);
     if (rc) return rc;
     if ((rc = get_taps(c, h, oh, &ty))) return rc;
-    const size_t per_frame = align_up((size_t)ow, 128) * (size_t)oh * 4 + y16_pitch_bytes(ow) * (size_t)oh;
+    const size_t per_frame = align_up((size_t)ow, 128) * (size_t)oh * (four_channel(order) ? 5 : 4) + y16_pitch_bytes(ow) * (size_t)oh;
     const int chunk = (int)std::max<size_t>(1, std::min<size_t>((size_t)n, ((size_t)1 << 30) / per_frame));
     const bool gray = order == SRCNN_ORDER_GRAY;
     if (gray) end_merge_chain(c);
@@ -275,7 +283,7 @@ static int process_frames_impl(Ctx* c, const uint8_t* d_src, int n, int w, int h
         const int m = std::min(chunk, n - f0);
         Planes pl;
         c->fail_stage = SRCNN_STAGE_PLANES;
-        if ((rc = carve_planes(c, ow, oh, 0, &pl, m, gray))) return rc;
+        if ((rc = carve_planes(c, ow, oh, 0, &pl, m, order))) return rc;
         c->fail_stage = SRCNN_STAGE_COLOR_BICUBIC;
         ResizeArgs ra;
         ra.src = d_src + (size_t)f0 * src_frame_stride; ra.src_stride = src_stride;
@@ -309,7 +317,7 @@ static int process_frames_impl(Ctx* c, const uint8_t* d_src, int n, int w, int h
         }
         c->fail_stage = SRCNN_STAGE_MERGE;
         MergeArgs ma;
-        ma.y = pl.yout; ma.cr = pl.cr; ma.cb = pl.cb;
+        ma.y = pl.yout; ma.cr = pl.cr; ma.cb = pl.cb; ma.a = pl.a;
         ma.pitch = pl.pitch; ma.w = ow;
         ma.order = order;
         if (m == 1 || dst_frame_stride == dst_stride * (size_t)oh) {   // the chunk's results are one tall image too
@@ -318,6 +326,7 @@ static int process_frames_impl(Ctx* c, const uint8_t* d_src, int n, int w, int h
         } else {
             for (int f = 0; f < m; f++) {
                 ma.y = pl.yout + (size_t)f * pl.frame_stride; ma.cr = pl.cr + (size_t)f * pl.frame_stride; ma.cb = pl.cb + (size_t)f * pl.frame_stride;
+                if (pl.a) ma.a = pl.a + (size_t)f * pl.frame_stride;
                 ma.rows = oh; ma.dst = dst0 + (size_t)f * dst_frame_stride; ma.dst_stride = dst_stride;
                 if ((rc = launch_merge(c, ma))) return rc;
             }
@@ -331,7 +340,9 @@ static int process_frames_impl(Ctx* c, const uint8_t* d_src, int n, int w, int h
 static int process_frames(Ctx* c, const uint8_t* d_src, int n, int w, int h, size_t src_stride, size_t src_frame_stride, int order,
                           float scale, int ow, int oh, uint8_t* d_dst, size_t dst_stride, size_t dst_frame_stride) {
     // one launch per stage and chunk needs the row-walking kernel with a separate merge; everything else goes frame by frame
-    if (n == 1 || c->variant != SRCNN_VARIANT_TC || (c->fuse_merge && order != SRCNN_ORDER_GRAY) || !c->batch_launch) {
+    // (the fused merge only takes the colour orders: grey and four-channel batches stay batched with it switched on)
+    const bool fuses = c->fuse_merge && (order == SRCNN_ORDER_BGR || order == SRCNN_ORDER_RGB);
+    if (n == 1 || c->variant != SRCNN_VARIANT_TC || fuses || !c->batch_launch) {
         for (int f = 0; f < n; f++) {
             int rc = process_rows(c, d_src + (size_t)f * src_frame_stride, w, h, src_stride, 0, h, order, scale, ow, oh, 0, oh,
                                   d_dst + (size_t)f * dst_frame_stride, dst_stride);
@@ -537,7 +548,7 @@ int host_pipeline(Ctx* c, const uint8_t* src, int n, int w, int h, size_t src_st
     const int rows = R1 - R0;
     std::vector<int> edges{R0};
     if (n == 1 && rows >= 1024) {
-        const long long by_mem = ((long long)rows * (long long)ow * 4 + (256ll << 20) - 1) / (256ll << 20);
+        const long long by_mem = ((long long)rows * (long long)ow * (four_channel(order) ? 5 : 4) + (256ll << 20) - 1) / (256ll << 20);
         if (by_mem > c->host_bands) {
             const int nb = (int)std::min<long long>(by_mem, rows / 64);
             for (int bi = 1; bi < nb; bi++) edges.push_back(R0 + (int)((long long)rows * bi / nb));
@@ -561,8 +572,8 @@ int host_pipeline(Ctx* c, const uint8_t* src, int n, int w, int h, size_t src_st
     const int group = (int)std::max<size_t>(1, std::min<size_t>(16, ((size_t)64 << 20) / std::max<size_t>(1, (size_t)ow * bpp * (size_t)rows) + 1));
     {   // the planes of the tallest sub-band / of a group of frames, allocated before anything is enqueued or captured
         Planes pl;
-        if ((rc = carve_planes(c, ow, std::min(tallest + 12, oh), 0, &pl, (bands == 1 && n > 1) ? std::min(group, n) : 1,
-                               order == SRCNN_ORDER_GRAY))) return rc;
+        if ((rc = carve_planes(c, ow, std::min(tallest + 12, oh), 0, &pl, (bands == 1 && n > 1) ? std::min(group, n) : 1, order)))
+            return rc;
     }
 
     // ---- CUDA-graph replay.  A call that repeats an earlier one exactly (same buffers, same geometry: a stream of frames through

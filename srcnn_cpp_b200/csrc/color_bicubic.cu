@@ -15,7 +15,11 @@
 // A grey source (SRCNN_ORDER_GRAY) takes the same kernels with one plane and no colour conversion: the plain
 // resize(..., CV_INTER_CUBIC) of that plane.
 //
-// Algorithmic HBM bytes per output pixel: 3/s^2 (BGR read) + 3 (planes written); K-C: 3 + 3.  Grey: 1/s^2 + 1.
+// A four-channel source (SRCNN_ORDER_BGRA / _RGBA) takes them with a fourth plane: the raw alpha byte, resized like the others
+// (not colour-converted), and K-C writes it back as byte 3 of every pixel.
+//
+// Algorithmic HBM bytes per output pixel: 3/s^2 (BGR read) + 3 (planes written); K-C: 3 + 3.  Grey: 1/s^2 + 1.  Four-channel:
+// 4/s^2 + 4; K-C: 4 + 4.
 #include <cuda_fp16.h>
 
 #include <cmath>
@@ -108,20 +112,23 @@ int get_taps(Ctx* c, int src, int dst, TapTable** out) {
 // geometry the tiled kernel's shared-memory footprint cannot hold (strong down-scales) and as the
 // in-library cross-check of the tiled kernel.
 // ------------------------------------------------------------------------------------------------
-template <int NP>   // planes: 3 = Y, Cr, Cb of a colour source, 1 = the one plane of a grey source (no colour conversion)
-__global__ void __launch_bounds__(256) k_color_bicubic_direct(ResizeDev p) {
+// planes: 3 = Y, Cr, Cb of a colour source, 1 = the one plane of a grey source (no colour conversion), 4 = Y, Cr, Cb and the raw
+// alpha byte of a four-channel source (into pa)
+template <int NP>
+__global__ void __launch_bounds__(256) k_color_bicubic_direct(ResizeDev p, uint8_t* pa) {
     const int dx = blockIdx.x * 32 + (threadIdx.x & 31);
     const int dy = p.row_begin + blockIdx.y * 8 + (threadIdx.x >> 5);
     if (dx >= p.ow || dy >= p.row_end) return;
     const int sx = p.xofs[dx], sy = p.yofs[dy];
     const short4 cx = p.xcoef[dx], cy = p.ycoef[dy];
     const int cxs[4] = {cx.x, cx.y, cx.z, cx.w};
-    int hY[4], hCr[4], hCb[4];
+    constexpr int NC = NP == 4 ? 4 : 3;   // bytes per colour pixel
+    int hY[4], hCr[4], hCb[4], hA[4];
 #pragma unroll
     for (int r = 0; r < 4; r++) {
         const int gy = clampi(sy - 1 + r, 0, p.sh - 1) - p.src_row0;
         const uint8_t* row = p.src + (size_t)gy * p.src_stride;
-        int aY = 0, aCr = 0, aCb = 0;
+        int aY = 0, aCr = 0, aCb = 0, aA = 0;
 #pragma unroll
         for (int k = 0; k < 4; k++) {
             const int gx = clampi(sx - 1 + k, 0, p.sw - 1);
@@ -129,7 +136,8 @@ __global__ void __launch_bounds__(256) k_color_bicubic_direct(ResizeDev p) {
                 aY += (int)row[gx] * cxs[k];
                 continue;
             }
-            int c0 = row[3 * gx], c1 = row[3 * gx + 1], c2 = row[3 * gx + 2];
+            int c0 = row[NC * gx], c1 = row[NC * gx + 1], c2 = row[NC * gx + 2];
+            if (NP == 4) aA += (int)row[NC * gx + 3] * cxs[k];
             int B = p.swapRB ? c2 : c0, R = p.swapRB ? c0 : c2;
             int Y, Cr, Cb;
             bgr_to_ycc(B, c1, R, Y, Cr, Cb);
@@ -137,7 +145,7 @@ __global__ void __launch_bounds__(256) k_color_bicubic_direct(ResizeDev p) {
             aCr += Cr * cxs[k];
             aCb += Cb * cxs[k];
         }
-        hY[r] = aY; hCr[r] = aCr; hCb[r] = aCb;
+        hY[r] = aY; hCr[r] = aCr; hCb[r] = aCb; hA[r] = aA;
     }
     const bool fpath = dx < p.simd_w;
     const size_t o = (size_t)(dy - p.plane_row0) * p.pitch + dx;
@@ -145,6 +153,7 @@ __global__ void __launch_bounds__(256) k_color_bicubic_direct(ResizeDev p) {
     if (NP == 1) return;
     p.cr[o] = (uint8_t)vertical_tap(hCr[0], hCr[1], hCr[2], hCr[3], cy, fpath);
     p.cb[o] = (uint8_t)vertical_tap(hCb[0], hCb[1], hCb[2], hCb[3], cy, fpath);
+    if (NP == 4) pa[o] = (uint8_t)vertical_tap(hA[0], hA[1], hA[2], hA[3], cy, fpath);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -156,13 +165,17 @@ __global__ void __launch_bounds__(256) k_color_bicubic_direct(ResizeDev p) {
 // ------------------------------------------------------------------------------------------------
 constexpr int kTW = 64;                 // output tile width; the height is a template parameter (64 or 32 rows)
 constexpr int kMaxSC = 72, kMaxSR = 40; // footprint capacity (source cols / rows incl. the 3-tap apron)
+constexpr int kMaxSR4 = 35;             // ... rows with four planes (the static shared memory of one CTA stays within 48 KB)
+__host__ __device__ constexpr int tiled_max_rows(int np) { return np == 4 ? kMaxSR4 : kMaxSR; }
 
+// NP = 4: the planes of a four-channel source, plane 3 (alpha, the raw byte 3 of each pixel) into pa
 template <int kTH, int NP>
-__global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p) {   // 5 CTAs per SM: 48 registers (4 CTAs measured 6 % slower)
-    __shared__ __align__(16) uint8_t sP[NP][kMaxSR][kMaxSC + 8];   // +8: the 3-word window read of the last quad may run past a row
+__global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p, uint8_t* pa) {   // 5 CTAs per SM: 48 registers (4 CTAs measured 6 % slower)
+    constexpr int SR = tiled_max_rows(NP);
+    __shared__ __align__(16) uint8_t sP[NP][SR][kMaxSC + 8];   // +8: the 3-word window read of the last quad may run past a row
     // horizontal sums kept as float: they are integers below 2^24, so the conversion is exact and is done
     // once per sum instead of once per use in the vertical pass
-    __shared__ __align__(16) float sH[NP][kMaxSR][kTW];
+    __shared__ __align__(16) float sH[NP][SR][kTW];
     // per tile row: the four vertical taps as floats (b_k = coef_k * 2^-22, exact) and the first tap's row in sH -- computed once
     // per tile instead of once per (thread, row) in the vertical pass
     __shared__ __align__(16) float4 sB[kTH];
@@ -197,15 +210,16 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p) {  
             sP[0][r][c] = fsrc[(size_t)gy * p.src_stride + gx];
             continue;
         }
-        const uint8_t* px = fsrc + (size_t)gy * p.src_stride + 3 * (size_t)gx;
+        const uint8_t* px = fsrc + (size_t)gy * p.src_stride + (NP == 4 ? 4 : 3) * (size_t)gx;
         const int B = px[oB], G = px[1], R = px[oR];
+        if (NP == 4) sP[NP - 1][r][c] = px[3];
         const int Y = (1868 * B + 9617 * G + 4899 * R + 8192) >> 14;          // OpenCV RGB2YCrCb_i<uchar>, yuv_shift 14
         uint32_t Cr, Cb;
         asm("cvt.sat.u8.s32 %0, %1;" : "=r"(Cr) : "r"(((R - Y) * 11682 + (128 << 14) + 8192) >> 14));
         asm("cvt.sat.u8.s32 %0, %1;" : "=r"(Cb) : "r"(((B - Y) * 9241 + (128 << 14) + 8192) >> 14));
         sP[0][r][c] = (uint8_t)Y;
         sP[NP > 1 ? 1 : 0][r][c] = (uint8_t)Cr;
-        sP[NP - 1][r][c] = (uint8_t)Cb;
+        sP[NP > 1 ? 2 : 0][r][c] = (uint8_t)Cb;
     }
     __syncthreads();
 
@@ -273,8 +287,9 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p) {  
         const int col = (tid & 15) * 4, ty0 = tid >> 4;
         const unsigned long long nz = p.negzero2;
         const size_t o = fplane + (size_t)(dy0 + ty0 - p.plane_row0) * p.pitch + (size_t)(dx0 + col);
-        uint8_t* pcr = NP == 3 ? p.cr + o : nullptr;
-        uint8_t* pcb = NP == 3 ? p.cb + o : nullptr;
+        uint8_t* pcr = NP >= 3 ? p.cr + o : nullptr;
+        uint8_t* pcb = NP >= 3 ? p.cb + o : nullptr;
+        uint8_t* ppa = NP == 4 ? pa + o : nullptr;
         uint8_t* py = p.y16 ? p.y16 + fy16 + (size_t)(dy0 + ty0 - p.plane_row0) * p.pitch16 + 2 * (size_t)(dx0 + col + kY16Pad) : p.y + o;
         const size_t step = 16 * p.pitch, ystep = p.y16 ? 16 * p.pitch16 : step;
         const bool y16 = p.y16 != nullptr;
@@ -283,10 +298,10 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p) {  
             const int ty = ty0 + 16 * k;
             const float4 bq = sB[ty];
             const float* hrow = &sH[0][sSr[ty]][col];
-            uint32_t packed[3];
+            uint32_t packed[NP > 3 ? NP : 3];
 #pragma unroll
             for (int pl = 0; pl < NP; pl++) {
-                const float* h = hrow + pl * (kMaxSR * kTW);
+                const float* h = hrow + pl * (SR * kTW);
                 const ulonglong2 g0 = *reinterpret_cast<const ulonglong2*>(h);
                 const ulonglong2 g1 = *reinterpret_cast<const ulonglong2*>(h + kTW);
                 const ulonglong2 g2 = *reinterpret_cast<const ulonglong2*>(h + 2 * kTW);
@@ -314,10 +329,14 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p) {  
             }
             if (!y16) *reinterpret_cast<uint32_t*>(py) = packed[0];
             py += ystep;
-            if (NP == 3) {
+            if (NP >= 3) {
                 *reinterpret_cast<uint32_t*>(pcr) = packed[1];
                 *reinterpret_cast<uint32_t*>(pcb) = packed[2];
                 pcr += step; pcb += step;
+            }
+            if (NP == 4) {
+                *reinterpret_cast<uint32_t*>(ppa) = packed[NP - 1];
+                ppa += step;
             }
         }
         return;
@@ -372,7 +391,7 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p) {  
                             }
                             continue;
                         }
-                        uint8_t* outp = (pl == 0 ? p.y : (pl == 1 ? p.cr : p.cb)) + o;
+                        uint8_t* outp = (pl == 0 ? p.y : (pl == 1 ? p.cr : (NP == 4 && pl == 3 ? pa : p.cb))) + o;
                         *reinterpret_cast<uint32_t*>(outp) = r0 | (r1 << 8) | (r2 << 16) | (r3 << 24);
                         continue;
                     }
@@ -380,7 +399,7 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p) {  
                     const float4 h1 = *reinterpret_cast<const float4*>(&sH[pl][sr + 1][col]);
                     const float4 h2 = *reinterpret_cast<const float4*>(&sH[pl][sr + 2][col]);
                     const float4 h3 = *reinterpret_cast<const float4*>(&sH[pl][sr + 3][col]);
-                    uint8_t* out = (pl == 0 ? p.y : (pl == 1 ? p.cr : p.cb)) + o;
+                    uint8_t* out = (pl == 0 ? p.y : (pl == 1 ? p.cr : (NP == 4 && pl == 3 ? pa : p.cb))) + o;
                     {  // tile edge and/or cv::resize's integer scalar tail (last ow mod 8 columns)
                         const float hh[4][4] = {{h0.x, h0.y, h0.z, h0.w}, {h1.x, h1.y, h1.z, h1.w}, {h2.x, h2.y, h2.z, h2.w}, {h3.x, h3.y, h3.z, h3.w}};
                         for (int j = 0; j < 4 && dx + j < dx1; j++) {
@@ -411,7 +430,7 @@ int launch_color_bicubic(Ctx* c, const ResizeArgs& a) {
     p.src = a.src;
     p.src_stride = a.src_stride;
     p.sw = a.sw; p.sh = a.sh; p.src_row0 = a.src_row0;
-    p.swapRB = a.order == SRCNN_ORDER_RGB;
+    p.swapRB = a.order == SRCNN_ORDER_RGB || a.order == SRCNN_ORDER_RGBA;
     p.ow = a.ow; p.oh = a.oh;
     p.row_begin = a.row_begin; p.row_end = a.row_end;
     p.y = a.pl.y; p.cr = a.pl.cr; p.cb = a.pl.cb;
@@ -434,10 +453,13 @@ int launch_color_bicubic(Ctx* c, const ResizeArgs& a) {
         int dx1 = std::min(dx0 + kTW, a.ow);
         if (a.tx->h_ofs[dx1 - 1] - a.tx->h_ofs[dx0] + 4 > kMaxSC) fits_x = false;
     }
+    const bool gray = a.order == SRCNN_ORDER_GRAY, four = four_channel(a.order);
+    uint8_t* const pa = four ? a.pl.a : nullptr;
+    const int max_rows = tiled_max_rows(four ? 4 : 3);
     auto fits_rows = [&](int th) {
         for (int dy0 = a.row_begin; dy0 < a.row_end; dy0 += th) {
             int dy1 = std::min(dy0 + th, a.row_end);
-            if (a.ty->h_ofs[dy1 - 1] - a.ty->h_ofs[dy0] + 4 > kMaxSR) return false;
+            if (a.ty->h_ofs[dy1 - 1] - a.ty->h_ofs[dy0] + 4 > max_rows) return false;
         }
         return true;
     };
@@ -451,11 +473,10 @@ int launch_color_bicubic(Ctx* c, const ResizeArgs& a) {
         const int rc = launch_color_bicubic_int(c, p, a, &done);
         if (rc || done) return rc;
     }
-    const bool gray = a.order == SRCNN_ORDER_GRAY;
     if (th) {
         dim3 grid((a.ow + kTW - 1) / kTW, (rows + th - 1) / th, nframes);   // a batch of frames is one launch
-        if (th == 64) (gray ? k_color_bicubic_tiled<64, 1> : k_color_bicubic_tiled<64, 3>)<<<grid, 256, 0, c->stream>>>(p);
-        else (gray ? k_color_bicubic_tiled<32, 1> : k_color_bicubic_tiled<32, 3>)<<<grid, 256, 0, c->stream>>>(p);
+        if (th == 64) (gray ? k_color_bicubic_tiled<64, 1> : four ? k_color_bicubic_tiled<64, 4> : k_color_bicubic_tiled<64, 3>)<<<grid, 256, 0, c->stream>>>(p, pa);
+        else (gray ? k_color_bicubic_tiled<32, 1> : four ? k_color_bicubic_tiled<32, 4> : k_color_bicubic_tiled<32, 3>)<<<grid, 256, 0, c->stream>>>(p, pa);
         c->launches++;
         SRCNN_CUDA(c, cudaGetLastError());
         return SRCNN_OK;
@@ -466,8 +487,9 @@ int launch_color_bicubic(Ctx* c, const ResizeArgs& a) {
         q.src += (size_t)f * p.src_frame;
         q.y += (size_t)f * p.plane_frame;
         if (!gray) { q.cr += (size_t)f * p.plane_frame; q.cb += (size_t)f * p.plane_frame; }
+        uint8_t* const qa = four ? pa + (size_t)f * p.plane_frame : nullptr;
         dim3 grid((a.ow + 31) / 32, (rows + 7) / 8);
-        (gray ? k_color_bicubic_direct<1> : k_color_bicubic_direct<3>)<<<grid, 256, 0, c->stream>>>(q);
+        (gray ? k_color_bicubic_direct<1> : four ? k_color_bicubic_direct<4> : k_color_bicubic_direct<3>)<<<grid, 256, 0, c->stream>>>(q, qa);
         c->launches++;
         SRCNN_CUDA(c, cudaGetLastError());
         if (a.pl.y16) {
@@ -513,7 +535,8 @@ int launch_y8_to_y16(Ctx* c, const uint8_t* y, size_t pitch, int w, int rows, ui
 // tiled/direct agreement is covered by running geometries on both sides of the footprint limit)
 
 // ------------------------------------------------------------------------------------------------
-// K-C: merge + YCrCb -> BGR.  4 pixels per thread: three aligned 32-bit plane loads, 12 output bytes.
+// K-C: merge + YCrCb -> BGR.  4 pixels per thread: three aligned 32-bit plane loads, 12 output bytes.  NC = 4 (BGRA / RGBA):
+// a fourth plane `a` becomes byte 3 of every pixel, 16 output bytes.
 // ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ void ycc_to_bgr(int Y, int Cr, int Cb, int& B, int& G, int& R) {
     const int cr = Cr - 128, cb = Cb - 128;
@@ -522,10 +545,11 @@ __device__ __forceinline__ void ycc_to_bgr(int Y, int Cr, int Cb, int& B, int& G
     R = clampi(Y + ((cr * 22987 + 8192) >> 14), 0, 255);
 }
 
+template <int NC>
 __global__ void __launch_bounds__(256) k_merge_ycc2bgr(const uint8_t* __restrict__ y, const uint8_t* __restrict__ cr,
                                                        const uint8_t* __restrict__ cb, size_t pitch, int w, int rows,
                                                        int swapRB, uint8_t* __restrict__ dst, size_t dst_stride,
-                                                       int dst_aligned, int blocks_per_row) {
+                                                       int dst_aligned, int blocks_per_row, const uint8_t* __restrict__ a) {
     // 1-D grid (rows can exceed the 65535 limit of gridDim.y): blocks_per_row blocks per image row
     const int row = blockIdx.x / blocks_per_row;
     const int q = (blockIdx.x - row * blocks_per_row) * blockDim.x + threadIdx.x;  // 4-pixel group
@@ -535,23 +559,25 @@ __global__ void __launch_bounds__(256) k_merge_ycc2bgr(const uint8_t* __restrict
     const uint32_t vy = *reinterpret_cast<const uint32_t*>(y + o);
     const uint32_t vr = *reinterpret_cast<const uint32_t*>(cr + o);
     const uint32_t vb = *reinterpret_cast<const uint32_t*>(cb + o);
-    uint8_t px[12];
+    const uint32_t va = NC == 4 ? *reinterpret_cast<const uint32_t*>(a + o) : 0u;
+    uint8_t px[4 * NC];
 #pragma unroll
     for (int j = 0; j < 4; j++) {
         int B, G, R;
         ycc_to_bgr((vy >> (8 * j)) & 255, (vr >> (8 * j)) & 255, (vb >> (8 * j)) & 255, B, G, R);
-        px[3 * j] = (uint8_t)(swapRB ? R : B);
-        px[3 * j + 1] = (uint8_t)G;
-        px[3 * j + 2] = (uint8_t)(swapRB ? B : R);
+        px[NC * j] = (uint8_t)(swapRB ? R : B);
+        px[NC * j + 1] = (uint8_t)G;
+        px[NC * j + 2] = (uint8_t)(swapRB ? B : R);
+        if (NC == 4) px[NC * j + 3] = (uint8_t)(va >> (8 * j));
     }
-    uint8_t* d = dst + (size_t)row * dst_stride + 3 * (size_t)x;
+    uint8_t* d = dst + (size_t)row * dst_stride + NC * (size_t)x;
     if (dst_aligned && x + 3 < w) {
         uint32_t* d32 = reinterpret_cast<uint32_t*>(d);
-        d32[0] = px[0] | (px[1] << 8) | (px[2] << 16) | ((uint32_t)px[3] << 24);
-        d32[1] = px[4] | (px[5] << 8) | (px[6] << 16) | ((uint32_t)px[7] << 24);
-        d32[2] = px[8] | (px[9] << 8) | (px[10] << 16) | ((uint32_t)px[11] << 24);
+#pragma unroll
+        for (int k = 0; k < NC; k++)
+            d32[k] = px[4 * k] | (px[4 * k + 1] << 8) | (px[4 * k + 2] << 16) | ((uint32_t)px[4 * k + 3] << 24);
     } else {
-        const int n = min(4, w - x) * 3;
+        const int n = min(4, w - x) * NC;
         for (int j = 0; j < n; j++) d[j] = px[j];
     }
 }
@@ -582,11 +608,13 @@ __device__ __forceinline__ uint32_t pack_sat_u8(int lo, int hi, uint32_t upper) 
 // colour+bicubic kernel of the NEXT whole-path call -- when api.cu launched it with programmatic stream serialisation -- fills the
 // SMs' free warp slots while this kernel, which is bound by L2 / HBM and leaves the issue slots idle, is still running.  A kernel
 // launched the ordinary way waits for this one to finish as always.  Threads walk the 16-pixel groups row-major with a grid stride
-// (one group per thread unless the grid is capped).
+// (one group per thread unless the grid is capped).  NC = 4: a fourth 128-bit load of the alpha plane `a`, whose bytes join the
+// colour bytes with one byte permutation per pixel, and four 128-bit stores (64 bytes per 16 pixels).
+template <int NC>
 __global__ void __launch_bounds__(256) k_merge_ycc2bgr_v16(const uint8_t* __restrict__ y, const uint8_t* __restrict__ cr,
                                                            const uint8_t* __restrict__ cb, size_t pitch, int w, int rows,
                                                            int swapRB, uint8_t* __restrict__ dst, size_t dst_stride,
-                                                           int groups_per_row) {
+                                                           int groups_per_row, const uint8_t* __restrict__ a) {
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
     // 16-bit coefficient pairs (low half x Cb-128, high half x Cr-128): B = 29049 cb, G = -5636 cb - 11698 cr, R = 22987 cr
     const uint32_t kB = 29049u, kG = (uint32_t)(unsigned short)(-5636) | ((uint32_t)(unsigned short)(-11698) << 16), kR = 22987u << 16;
@@ -599,16 +627,19 @@ __global__ void __launch_bounds__(256) k_merge_ycc2bgr_v16(const uint8_t* __rest
     const int srow = (int)(stride / (unsigned)groups_per_row), sgrp = (int)(stride % (unsigned)groups_per_row);
     int row = (int)(first / (unsigned)groups_per_row), grp = (int)(first % (unsigned)groups_per_row);
     if (row >= rows) return;
-    uint4 vy, vr, vb;
+    uint4 vy, vr, vb, va;
     {
         const size_t o = (size_t)row * pitch + grp * 16;
         vy = *reinterpret_cast<const uint4*>(y + o);
         vr = *reinterpret_cast<const uint4*>(cr + o);
         vb = *reinterpret_cast<const uint4*>(cb + o);
+        if (NC == 4) va = *reinterpret_cast<const uint4*>(a + o);
     }
     for (;;) {
         const int x = grp * 16, crow = row;
         const uint32_t wy[4] = {vy.x, vy.y, vy.z, vy.w}, wr[4] = {vr.x, vr.y, vr.z, vr.w}, wb[4] = {vb.x, vb.y, vb.z, vb.w};
+        uint32_t wa[4];
+        if (NC == 4) { wa[0] = va.x; wa[1] = va.y; wa[2] = va.z; wa[3] = va.w; }
         row += srow; grp += sgrp;
         if (grp >= groups_per_row) { grp -= groups_per_row; row++; }
         const bool more = row < rows;
@@ -617,8 +648,9 @@ __global__ void __launch_bounds__(256) k_merge_ycc2bgr_v16(const uint8_t* __rest
             vy = *reinterpret_cast<const uint4*>(y + o);
             vr = *reinterpret_cast<const uint4*>(cr + o);
             vb = *reinterpret_cast<const uint4*>(cb + o);
+            if (NC == 4) va = *reinterpret_cast<const uint4*>(a + o);
         }
-        uint32_t outw[12];
+        uint32_t outw[4 * NC];
 #pragma unroll
         for (int k = 0; k < 4; k++) {   // 4 pixels -> 12 bytes -> 3 words
             const uint32_t sb = wb[k] ^ 0x80808080u, sr = wr[k] ^ 0x80808080u;     // Cb-128, Cr-128 as signed bytes
@@ -638,19 +670,29 @@ __global__ void __launch_bounds__(256) k_merge_ycc2bgr_v16(const uint8_t* __rest
                     v[j][2] = dp2a_lo_ss(k2, cc, t) >> 14;
                 }
             }
+            if (NC == 4) {
+                // pixel j: c0 c1 c2 from the conversion, byte 3 = byte j of the alpha word
+#pragma unroll
+                for (int j = 0; j < 4; j++)
+                    outw[4 * k + j] = __byte_perm(pack_sat_u8(v[j][0], v[j][1], pack_sat_u8(v[j][2], 0, 0u)), wa[k], 0x0210 | ((4 + j) << 12));
+                continue;
+            }
             // bytes: p0c0 p0c1 p0c2 p1c0 | p1c1 p1c2 p2c0 p2c1 | p2c2 p3c0 p3c1 p3c2
             outw[3 * k] = pack_sat_u8(v[0][0], v[0][1], pack_sat_u8(v[0][2], v[1][0], 0u));
             outw[3 * k + 1] = pack_sat_u8(v[1][1], v[1][2], pack_sat_u8(v[2][0], v[2][1], 0u));
             outw[3 * k + 2] = pack_sat_u8(v[2][2], v[3][0], pack_sat_u8(v[3][1], v[3][2], 0u));
         }
-        uint8_t* d = dst + (size_t)crow * dst_stride + 3 * (size_t)x;
+        uint8_t* d = dst + (size_t)crow * dst_stride + NC * (size_t)x;
         if (x + 15 < w) {
             uint4* d4 = reinterpret_cast<uint4*>(d);
-            d4[0] = make_uint4(outw[0], outw[1], outw[2], outw[3]);
-            d4[1] = make_uint4(outw[4], outw[5], outw[6], outw[7]);
-            d4[2] = make_uint4(outw[8], outw[9], outw[10], outw[11]);
+#pragma unroll
+            for (int k = 0; k < NC; k++) d4[k] = make_uint4(outw[4 * k], outw[4 * k + 1], outw[4 * k + 2], outw[4 * k + 3]);
+        } else if (NC == 4) {   // a pixel is one aligned word (static indices keep outw in registers)
+#pragma unroll
+            for (int j = 0; j < 16; j++)
+                if (x + j < w) reinterpret_cast<uint32_t*>(d)[j] = outw[j];
         } else {
-            const int n = (w - x) * 3;
+            const int n = (w - x) * NC;
             for (int j = 0; j < n; j++) d[j] = (uint8_t)(outw[j >> 2] >> (8 * (j & 3)));
         }
         if (!more) break;
@@ -659,7 +701,8 @@ __global__ void __launch_bounds__(256) k_merge_ycc2bgr_v16(const uint8_t* __rest
 
 int launch_merge(Ctx* c, const MergeArgs& a) {
     if (a.rows <= 0 || a.w <= 0) return SRCNN_OK;
-    const bool wide = ((((uintptr_t)a.dst) | a.dst_stride | (uintptr_t)a.y | (uintptr_t)a.cr | (uintptr_t)a.cb | a.pitch) & 15) == 0 &&
+    const bool four = four_channel(a.order), swap = a.order == SRCNN_ORDER_RGB || a.order == SRCNN_ORDER_RGBA;
+    const bool wide = ((((uintptr_t)a.dst) | a.dst_stride | (uintptr_t)a.y | (uintptr_t)a.cr | (uintptr_t)a.cb | (uintptr_t)a.a | a.pitch) & 15) == 0 &&
                       a.pitch >= align_up((size_t)a.w, 16);
     c->merge_sel = -1;   // a whole-path caller says afterwards which Cr/Cb pair this launch reads (api.cu, merged_into)
     note_merge(c);
@@ -671,8 +714,8 @@ int launch_merge(Ctx* c, const MergeArgs& a) {
         const long long want = (ngroups + 255) / 256, cap = c->merge_ctas_per_sm > 0 ? (long long)c->merge_ctas_per_sm * std::max(1, c->sm_count) : want;
         const long long k = (want + cap - 1) / cap;
         const int grid = (int)((want + k - 1) / k);
-        k_merge_ycc2bgr_v16<<<grid, 256, 0, c->stream>>>(a.y, a.cr, a.cb, a.pitch, a.w, a.rows, a.order == SRCNN_ORDER_RGB, a.dst,
-                                                        a.dst_stride, groups16);
+        (four ? k_merge_ycc2bgr_v16<4> : k_merge_ycc2bgr_v16<3>)<<<grid, 256, 0, c->stream>>>(a.y, a.cr, a.cb, a.pitch, a.w, a.rows, swap, a.dst,
+                                                                                           a.dst_stride, groups16, a.a);
         c->launches++;
         SRCNN_CUDA(c, cudaGetLastError());
         return SRCNN_OK;
@@ -681,8 +724,8 @@ int launch_merge(Ctx* c, const MergeArgs& a) {
     const int bpr = (groups + 255) / 256;
     const unsigned grid = (unsigned)bpr * (unsigned)a.rows;
     const int aligned = (((uintptr_t)a.dst & 3) == 0) && ((a.dst_stride & 3) == 0);
-    k_merge_ycc2bgr<<<grid, 256, 0, c->stream>>>(a.y, a.cr, a.cb, a.pitch, a.w, a.rows,
-                                                 a.order == SRCNN_ORDER_RGB, a.dst, a.dst_stride, aligned, bpr);
+    (four ? k_merge_ycc2bgr<4> : k_merge_ycc2bgr<3>)<<<grid, 256, 0, c->stream>>>(a.y, a.cr, a.cb, a.pitch, a.w, a.rows, swap, a.dst,
+                                                                               a.dst_stride, aligned, bpr, a.a);
     c->launches++;
     SRCNN_CUDA(c, cudaGetLastError());
     return SRCNN_OK;

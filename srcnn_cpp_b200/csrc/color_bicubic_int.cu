@@ -16,7 +16,8 @@
 //       v = H0*b0 + (H1*b1 + (H2*b2 + H3*b3)), every product and sum rounded on its own (f2_mul_rn / f2_add_rn), round-half-even,
 //       saturate, one 8- or 16-byte store per lane and row.  No shared-memory round trip of the sums, no per-sample addressing.
 // Y goes to the padded FP16 plane of the tcgen05 kernel when the context has one (color_bicubic.cu explains the layout).
-// A grey source (SRCNN_ORDER_GRAY) has its own kernel below, k_gray_bicubic_int: raw bytes staged, the same walk.
+// A grey source (SRCNN_ORDER_GRAY) has its own kernel below, k_gray_bicubic_int: raw bytes staged, the same walk.  A four-channel
+// source (SRCNN_ORDER_BGRA / _RGBA) has k_color4_bicubic_int: a fourth warp walks the alpha plane.
 // Measured and not kept (tools/experiments/color_bicubic_int_persistent_tma.cu.txt, DESIGN.md): fetching a tile's raw rows by TMA
 // (neutral), persistent CTAs with the next tile's rows prefetched by TMA -- as one block-wide pipeline, with a producer warp, or
 // as three per-warp pipelines (all slower: the kernel is bound by instruction issue while a wave of tiles computes, and every
@@ -48,6 +49,7 @@ struct IntTaps {
     uint32_t sel[4];                    // byte selectors that turn three source words into four (B, G, R, x) pixel words
     int a_first, i_last;                // first / last source row index i whose output rows S*i + S/2 .. + S-1 are wanted
     int vec_ok;                         // source rows are 4-byte aligned: footprint groups inside the image take 32-bit loads
+                                        // (2: 16-byte aligned, four-channel groups take one 128-bit load)
     int isr;                            // source rows a tile advances by (4 .. kISRMax)
     int ntx, nty, ntiles;               // tiles per row of tiles, rows of tiles per frame, tiles in the launch (frames included)
 };
@@ -82,15 +84,12 @@ struct Geo {
     static constexpr int G = kITW / S / 4 + 2;             // four-pixel groups per footprint row (the first starts 4 columns left of the tile)
 };
 
-// (1) twelve source bytes = four pixels -> one 32-bit word per plane of the converted footprint.  OpenCV RGB2YCrCb_i<uchar>, yuv_shift 14.
-__device__ __forceinline__ void convert_group(const IntTaps& t, uint32_t w0, uint32_t w1, uint32_t w2, uint8_t* y4, uint8_t* cr4, uint8_t* cb4) {
+// (1) four (B, G, R, x) pixel words -> one 32-bit word per plane of the converted footprint.  OpenCV RGB2YCrCb_i<uchar>, yuv_shift 14.
+// Byte 3 of a pixel word never counts: only the two dp2a.hi read it, against the upper 16-bit halves of kYhi and kR, and both
+// halves are zero -- so the x byte may be anything, the alpha byte of a four-channel pixel included.
+__device__ __forceinline__ void convert_px4(const uint32_t (&pw)[4], uint8_t* y4, uint8_t* cr4, uint8_t* cb4) {
     const uint32_t kYlo = 1868u | (9617u << 16), kYhi = 4899u, kR = 11682u, kB = 9241u;
     const int cadd = (128 << 14) + 8192;
-    uint32_t pw[4];     // (B, G, R, x) per pixel
-    pw[0] = __byte_perm(w0, w0, t.sel[0]);
-    pw[1] = __byte_perm(w0, w1, t.sel[1]);
-    pw[2] = __byte_perm(w1, w2, t.sel[2]);
-    pw[3] = __byte_perm(w2, w2, t.sel[3]);
     int Y[4], Cr[4], Cb[4];
 #pragma unroll
     for (int j = 0; j < 4; j++) {
@@ -101,6 +100,15 @@ __device__ __forceinline__ void convert_group(const IntTaps& t, uint32_t w0, uin
     *reinterpret_cast<uint32_t*>(y4) = __byte_perm(__byte_perm(Y[0], Y[1], 0x0040), __byte_perm(Y[2], Y[3], 0x0040), 0x5410);
     *reinterpret_cast<uint32_t*>(cr4) = pack2_sat_u8(Cr[0], Cr[1], pack2_sat_u8(Cr[2], Cr[3], 0u));
     *reinterpret_cast<uint32_t*>(cb4) = pack2_sat_u8(Cb[0], Cb[1], pack2_sat_u8(Cb[2], Cb[3], 0u));
+}
+// twelve source bytes = four three-byte pixels
+__device__ __forceinline__ void convert_group(const IntTaps& t, uint32_t w0, uint32_t w1, uint32_t w2, uint8_t* y4, uint8_t* cr4, uint8_t* cb4) {
+    uint32_t pw[4];     // (B, G, R, x) per pixel
+    pw[0] = __byte_perm(w0, w0, t.sel[0]);
+    pw[1] = __byte_perm(w0, w1, t.sel[1]);
+    pw[2] = __byte_perm(w1, w2, t.sel[2]);
+    pw[3] = __byte_perm(w2, w2, t.sel[3]);
+    convert_px4(pw, y4, cr4, cb4);
 }
 // the same twelve bytes for a group that crosses the left / right image edge: from clamped pixels of a row that starts at `row`
 // (the byte of pixel 0, channel 0)
@@ -114,10 +122,10 @@ __device__ __forceinline__ void clamped_group(const uint8_t* row, int gx, int sw
 }
 
 // (2) the walk of one warp (one plane) down a tile's converted footprint `plane` (rows kPitch bytes apart): lane's output columns
-// x0 .. x0+7 read footprint bytes cb .. cb+7 of a row
-template <int S, int kPitch = kIPitch>
+// x0 .. x0+7 read footprint bytes cb .. cb+7 of a row.  NPL = 4: plane 3 is the alpha plane `pa` (same pitch and frame stride).
+template <int S, int kPitch = kIPitch, int NPL = 3>
 __device__ __forceinline__ void walk_tile(const ResizeDev& p, const IntTaps& t, const uint8_t* plane, int pl, int lane, int X0, int a,
-                                          int nit, size_t fz) {
+                                          int nit, size_t fz, uint8_t* pa = nullptr) {
     const int x0 = X0 + 8 * lane;
     if (x0 >= p.ow) return;                        // ow is a multiple of 8 (launch condition)
     const int cb = (8 * lane) / S + 2;
@@ -155,7 +163,7 @@ __device__ __forceinline__ void walk_tile(const ResizeDev& p, const IntTaps& t, 
                 int dy = S * a + S / 2;
                 uint8_t* outp;
                 if (y16) outp = p.y16 + fz * p.y16_frame + ((long long)dy - p.plane_row0) * (long long)p.pitch16 + 2 * (size_t)(x0 + kY16Pad);
-                else outp = (pl == 0 ? p.y : (pl == 1 ? p.cr : p.cb)) + fz * p.plane_frame + ((long long)dy - p.plane_row0) * (long long)p.pitch + x0;
+                else outp = (pl == 0 ? p.y : (pl == 1 ? p.cr : (NPL == 4 && pl == 3 ? pa : p.cb))) + fz * p.plane_frame + ((long long)dy - p.plane_row0) * (long long)p.pitch + x0;
                 uint8_t* const outp0 = outp;
 
                 auto emit = [&](const unsigned long long (&h0)[4], const unsigned long long (&h1)[4], const unsigned long long (&h2)[4],
@@ -296,6 +304,100 @@ __global__ void __launch_bounds__(96, S == 2 ? SRCNN_KA_MINB : SRCNN_KA_MINB4) k
 }
 
 // ------------------------------------------------------------------------------------------------
+// Four-channel form (SRCNN_ORDER_BGRA / _RGBA): one CTA of FOUR warps per tile, warp w walks plane w (Y, Cr, Cb, A) with the
+// same walk.  A footprint group is 16 source bytes = four pixel words: one 128-bit load when the source is 16-byte aligned, four
+// 32-bit loads when it is 4-byte aligned, clamped bytes at the image edges.  A BGRA word already is the (B, G, R, x) word
+// convert_px4 takes (the alpha byte drops out of every dp2a); an RGBA word takes one byte permutation.  The alpha plane is byte 3
+// of the four words, gathered into one 32-bit shared store.  128 threads: the 96-thread budgets (80 / 126 registers at 8 / 5
+// CTAs per SM) would not fit the register file, so the same threads per SM are kept with 6 / 4 CTAs.
+// ------------------------------------------------------------------------------------------------
+#ifndef SRCNN_KA4_MINB
+#define SRCNN_KA4_MINB 6
+#endif
+#ifndef SRCNN_KA4_MINB4
+#define SRCNN_KA4_MINB4 4
+#endif
+
+__device__ __forceinline__ void convert_group4(uint32_t w0, uint32_t w1, uint32_t w2, uint32_t w3, bool swap, uint8_t* y4, uint8_t* cr4,
+                                               uint8_t* cb4, uint8_t* a4) {
+    uint32_t pw[4] = {w0, w1, w2, w3};
+    if (swap) {   // (R, G, B, A) -> (B, G, R, A)
+#pragma unroll
+        for (int j = 0; j < 4; j++) pw[j] = __byte_perm(pw[j], 0, 0x3012);
+    }
+    convert_px4(pw, y4, cr4, cb4);
+    *reinterpret_cast<uint32_t*>(a4) = __byte_perm(__byte_perm(w0, w1, 0x0073), __byte_perm(w2, w3, 0x0073), 0x5410);
+}
+
+template <int S>
+__global__ void __launch_bounds__(128, S == 2 ? SRCNN_KA4_MINB : SRCNN_KA4_MINB4) k_color4_bicubic_int(const ResizeDev p, const IntTaps t,
+                                                                                                      uint8_t* const pa) {
+    constexpr int G = Geo<S>::G;
+    __shared__ __align__(16) uint8_t sP[4][kIRows][kIPitch];
+    const int tid = threadIdx.x;
+    const int tile = blockIdx.x;
+    const int bx = tile % t.ntx, rest = tile / t.ntx;
+    const int by = rest % t.nty;
+    const size_t fz = (size_t)(rest / t.nty);
+    const int X0 = bx * kITW;
+    const int a = t.a_first + by * t.isr;          // footprint row r is source row a - 1 + r
+    const int F0 = X0 / S - 4;                     // first footprint column (a multiple of 4: 16-byte aligned groups)
+    const int nit = min(t.isr, t.i_last - a + 1);
+    const int nsr = nit + 3;
+    const uint8_t* const fsrc = p.src + fz * p.src_frame;
+    const bool swap = p.swapRB;
+
+    // (1) colour-convert the footprint; replicate border applied here
+    if (t.vec_ok && F0 >= 0 && F0 + 4 * G <= p.sw) {
+        constexpr int NG = (kIRows * G + 127) / 128;
+        uint32_t raw[NG][4];
+#pragma unroll
+        for (int it = 0; it < NG; it++) {
+            const int g = tid + 128 * it;
+            if (g < nsr * G) {
+                const int r = g / G, q = g - r * G;
+                const int gy = clampi(a - 1 + r, 0, p.sh - 1) - p.src_row0;
+                const uint8_t* px = fsrc + (size_t)gy * p.src_stride + 4 * (size_t)(F0 + 4 * q);
+                if (t.vec_ok == 2) {
+                    const uint4 v = *reinterpret_cast<const uint4*>(px);
+                    raw[it][0] = v.x; raw[it][1] = v.y; raw[it][2] = v.z; raw[it][3] = v.w;
+                } else {
+                    const uint32_t* w = reinterpret_cast<const uint32_t*>(px);
+                    raw[it][0] = w[0]; raw[it][1] = w[1]; raw[it][2] = w[2]; raw[it][3] = w[3];
+                }
+            }
+        }
+#pragma unroll
+        for (int it = 0; it < NG; it++) {
+            const int g = tid + 128 * it;
+            if (g < nsr * G) {
+                const int r = g / G, q = g - r * G;
+                convert_group4(raw[it][0], raw[it][1], raw[it][2], raw[it][3], swap, &sP[0][r][4 * q], &sP[1][r][4 * q], &sP[2][r][4 * q],
+                               &sP[3][r][4 * q]);
+            }
+        }
+    } else {
+        for (int g = tid; g < nsr * G; g += 128) {
+            const int r = g / G, q = g - r * G;
+            const int gy = clampi(a - 1 + r, 0, p.sh - 1) - p.src_row0;
+            const uint8_t* row = fsrc + (size_t)gy * p.src_stride;
+            uint32_t w[4] = {0u, 0u, 0u, 0u};
+#pragma unroll
+            for (int j = 0; j < 16; j++) {
+                const int x = clampi(F0 + 4 * q + j / 4, 0, p.sw - 1);
+                w[j >> 2] |= (uint32_t)row[4 * (size_t)x + (j & 3)] << (8 * (j & 3));
+            }
+            convert_group4(w[0], w[1], w[2], w[3], swap, &sP[0][r][4 * q], &sP[1][r][4 * q], &sP[2][r][4 * q], &sP[3][r][4 * q]);
+        }
+    }
+    __syncthreads();
+    // (2) the walk
+    walk_tile<S, kIPitch, 4>(p, t, &sP[tid >> 5][0][0], tid >> 5, tid & 31, X0, a, nit, fz, pa);
+    // may have started beside the previous call's merge kernel: see k_color_bicubic_int
+    if (tile == t.ntiles - 1) asm volatile("griddepcontrol.wait;" ::: "memory");
+}
+
+// ------------------------------------------------------------------------------------------------
 // One-plane form (SRCNN_ORDER_GRAY): the footprint is the source bytes as they are, with the replicate border.  One CTA of
 // three warps takes three ADJACENT tiles: their footprints are one contiguous run of 3 * kITW / S + 8 source columns, staged
 // once, and warp w walks tile w from its own offset in it -- the same 96-thread CTA (and occupancy tuning) and the same
@@ -355,14 +457,39 @@ __global__ void __launch_bounds__(96, S == 2 ? SRCNN_KA_MINB : SRCNN_KA_MINB4) k
 
 inline int floordiv(int a, int b) { return a >= 0 ? a / b : -((-a + b - 1) / b); }
 
-template <int S, bool GRAY>
-int launch_variant(Ctx* c, const ResizeDev& p, IntTaps& t, int nframes, bool early) {
-    void (*const kern)(const ResizeDev, const IntTaps) = GRAY ? k_gray_bicubic_int<S> : k_color_bicubic_int<S>;
+// one launch of an integer-scale kernel, ordinary or with programmatic stream serialisation
+template <typename K, typename... A>
+int launch_ka(Ctx* c, K kern, int grid, int threads, bool early, const A&... args) {
+    if (early) {   // programmatic dependent launch: may begin before the stream's previous kernel (a merge of ours) has finished
+        cudaLaunchConfig_t cfg = {};
+        cfg.gridDim = dim3((unsigned)grid);
+        cfg.blockDim = dim3(threads);
+        cfg.dynamicSmemBytes = 0;
+        cfg.stream = c->stream;
+        cudaLaunchAttribute at[1];
+        at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+        at[0].val.programmaticStreamSerializationAllowed = 1;
+        cfg.attrs = at;
+        cfg.numAttrs = 1;
+        SRCNN_CUDA(c, cudaLaunchKernelEx(&cfg, kern, args...));
+    } else {
+        kern<<<grid, threads, 0, c->stream>>>(args...);
+    }
+    c->launches++;
+    SRCNN_CUDA(c, cudaGetLastError());
+    return SRCNN_OK;
+}
+
+// NP = planes: 1 grey, 3 colour, 4 colour + alpha (pa)
+template <int S, int NP>
+int launch_variant(Ctx* c, const ResizeDev& p, IntTaps& t, uint8_t* pa, int nframes, bool early) {
+    constexpr int kThreads = NP == 4 ? 128 : 96;
     static int ctas_per_sm[64] = {0};              // per device; a benign race: every writer stores the same value
     int& per_sm = ctas_per_sm[c->device & 63];
     if (per_sm == 0) {
         int n = 0;
-        SRCNN_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kern, 96, 0));
+        if (NP == 4) SRCNN_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_color4_bicubic_int<S>, kThreads, 0));
+        else SRCNN_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, NP == 1 ? k_gray_bicubic_int<S> : k_color_bicubic_int<S>, kThreads, 0));
         per_sm = std::max(1, n);
     }
     // Tile height (same-box A/B, B200): a single 4K frame runs fastest as ~1.5 waves of 8-row tiles (23.6 us; 6 rows: 23.7,
@@ -378,24 +505,8 @@ int launch_variant(Ctx* c, const ResizeDev& p, IntTaps& t, int nframes, bool ear
     if (ntiles > 0x3fffffffLL) return SRCNN_E_ARG;
     t.nty = (nrows + t.isr - 1) / t.isr;
     t.ntiles = (int)ntiles;
-    if (early) {   // programmatic dependent launch: may begin before the stream's previous kernel (a merge of ours) has finished
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((unsigned)t.ntiles);
-        cfg.blockDim = dim3(96);
-        cfg.dynamicSmemBytes = 0;
-        cfg.stream = c->stream;
-        cudaLaunchAttribute at[1];
-        at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        at[0].val.programmaticStreamSerializationAllowed = 1;
-        cfg.attrs = at;
-        cfg.numAttrs = 1;
-        SRCNN_CUDA(c, cudaLaunchKernelEx(&cfg, kern, p, t));
-    } else {
-        kern<<<t.ntiles, 96, 0, c->stream>>>(p, t);
-    }
-    c->launches++;
-    SRCNN_CUDA(c, cudaGetLastError());
-    return SRCNN_OK;
+    if (NP == 4) return launch_ka(c, k_color4_bicubic_int<S>, t.ntiles, kThreads, early, p, t, pa);
+    return launch_ka(c, NP == 1 ? k_gray_bicubic_int<S> : k_color_bicubic_int<S>, t.ntiles, kThreads, early, p, t);
 }
 
 }  // namespace
@@ -405,7 +516,9 @@ int launch_color_bicubic_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bo
     const int S = a.tx->int_scale;
     if (S == 0 || a.ty->int_scale != S || (a.ow & 7) || a.row_end <= a.row_begin) return SRCNN_OK;
     // stores: 8 bytes per lane and row into the u8 planes, 16 into the FP16 plane
-    if ((((uintptr_t)p.y | (uintptr_t)p.cr | (uintptr_t)p.cb | p.pitch | p.plane_frame) & 7) != 0) return SRCNN_OK;
+    const bool four = a.order == SRCNN_ORDER_BGRA || a.order == SRCNN_ORDER_RGBA;
+    uint8_t* const pa = four ? a.pl.a : nullptr;
+    if ((((uintptr_t)p.y | (uintptr_t)p.cr | (uintptr_t)p.cb | (uintptr_t)pa | p.pitch | p.plane_frame) & 7) != 0) return SRCNN_OK;
     if (p.y16 && (((uintptr_t)p.y16 | p.pitch16 | p.y16_frame) & 15) != 0) return SRCNN_OK;
 
     IntTaps t;
@@ -427,14 +540,16 @@ int launch_color_bicubic_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bo
     t.a_first = floordiv(a.row_begin - S / 2, S);
     t.i_last = floordiv(a.row_end - 1 - S / 2, S);
     t.vec_ok = (((uintptr_t)p.src | p.src_stride | p.src_frame) & 3) == 0;
+    if (four && t.vec_ok && (((uintptr_t)p.src | p.src_stride | p.src_frame) & 15) == 0) t.vec_ok = 2;   // 128-bit group loads
     const int nframes = std::max(1, a.nframes);
     const bool gray = a.order == SRCNN_ORDER_GRAY;
     t.ntx = (a.ow + kITW - 1) / kITW;
     if (gray) t.ntx = (t.ntx + 2) / 3;             // a CTA per three adjacent tiles
     if ((long long)t.ntx * (t.i_last - t.a_first + 1) * nframes > 0x3fffffffLL) return SRCNN_OK;
     int rc;
-    if (gray) rc = S == 2 ? launch_variant<2, true>(c, p, t, nframes, false) : launch_variant<4, true>(c, p, t, nframes, false);   // never early (api.cu)
-    else rc = S == 2 ? launch_variant<2, false>(c, p, t, nframes, a.early) : launch_variant<4, false>(c, p, t, nframes, a.early);
+    if (gray) rc = S == 2 ? launch_variant<2, 1>(c, p, t, pa, nframes, false) : launch_variant<4, 1>(c, p, t, pa, nframes, false);   // never early (api.cu)
+    else if (four) rc = S == 2 ? launch_variant<2, 4>(c, p, t, pa, nframes, a.early) : launch_variant<4, 4>(c, p, t, pa, nframes, a.early);
+    else rc = S == 2 ? launch_variant<2, 3>(c, p, t, pa, nframes, a.early) : launch_variant<4, 3>(c, p, t, pa, nframes, a.early);
     if (rc) return rc;
     *done = true;
     return SRCNN_OK;

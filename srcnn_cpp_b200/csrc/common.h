@@ -67,6 +67,7 @@ struct Planes {
     size_t pitch16 = 0;
     uint8_t* cr = nullptr;
     uint8_t* cb = nullptr;
+    uint8_t* a = nullptr;       // alpha plane of a four-channel call (SRCNN_ORDER_BGRA / _RGBA), same pitch / frame stride as cr
     uint8_t* yout = nullptr;
     size_t pitch = 0;
     int row0 = 0, rows = 0;
@@ -207,7 +208,9 @@ struct ResizeArgs {
     size_t src_frame_stride = 0;
     bool early = false;   // may start while the previous kernel of the stream (a merge kernel of ours) is still running
 };
-int launch_color_bicubic(Ctx* c, const ResizeArgs& a);   // order SRCNN_ORDER_GRAY: the one plane, into pl.y / pl.y16
+int launch_color_bicubic(Ctx* c, const ResizeArgs& a);   // order SRCNN_ORDER_GRAY: the one plane, into pl.y / pl.y16;
+                                                         // SRCNN_ORDER_BGRA / _RGBA: pl.a as well
+inline bool four_channel(int order) { return order == SRCNN_ORDER_BGRA || order == SRCNN_ORDER_RGBA; }
 
 struct MergeArgs {
     const uint8_t* y;
@@ -218,6 +221,7 @@ struct MergeArgs {
     int order;
     uint8_t* dst;
     size_t dst_stride;
+    const uint8_t* a = nullptr;   // four-channel orders: the alpha plane (same pitch), written as byte 3 of every pixel
 };
 int launch_merge(Ctx* c, const MergeArgs& a);
 void note_merge(Ctx* c);   // api.cu: this context has just put a merge kernel (which releases its dependents early) on its stream
