@@ -27,6 +27,20 @@
  * reference does to its planes after `split` (src/srcnn.cpp:540,577-582) and what ProcessSRCNN returns for d = 4.  It is NOT
  * always channel 3 of cv::resize on a CV_8UC4 image: with 4 channels OpenCV splits its float body and integer tail at another
  * column, and the two differ by 1 LSB on some geometries.
+ * SRCNN_ORDER_NV12 / SRCNN_ORDER_I420: a packed 4:2:0 video frame in one buffer -- what (h*3/2) x w arrays are to FFmpeg raw
+ * video and OpenCV's COLOR_YUV2BGR_NV12 / _I420.  `stride` is in bytes.  NV12: rows 0 .. h-1 are Y (w bytes each, `stride`
+ * apart), rows h .. h + h/2 - 1 the interleaved chroma pairs (w bytes = w/2 pairs each, also `stride` apart).  I420: Y as in
+ * NV12; U at base + h*stride, h/2 rows of w/2 bytes, stride/2 apart; V follows at U + (h/2)*(stride/2) with the same geometry.
+ * The output has the same layout with ow, oh, dst_stride.  w, h, ow and oh must all be even (ow / oh are still the truncation
+ * below, so a scale may give an odd size: SRCNN_E_ARG), stride >= w, dst_stride >= ow, I420 strides even, and batch frame
+ * strides >= stride*h*3/2 (dst_stride*oh*3/2).  The chroma planes are treated independently, so NV21 (pairs V, U) and YV12
+ * (V plane first) are the same two orders.  Byte for byte: the output's Y plane is the SRCNN_ORDER_GRAY call on the source's
+ * Y plane; each output chroma plane is resize(plane, Size(ow/2, oh/2), INTER_CUBIC) of the matching source plane -- exactly
+ * srcnn_stage_resize_plane_device on it, no CNN.  NV12's interleaved plane is resized as two planes, not as one CV_8UC2 image
+ * (whose float body / integer tail split differs, as for alpha above).  No colour matrix is applied anywhere: the network sees
+ * the Y plane as it is (limited or full range), and chroma takes cv::resize's centre-aligned grid, so left-sited (MPEG-2 /
+ * H.264) chroma gets the quarter-pixel horizontal shift any centre-aligned resize gives -- not compensated.  Whole-frame calls
+ * only: the band calls (srcnn_process_band_*, srcnn_mgpu_process_banded_*) return SRCNN_E_ARG for these orders.
  * Output size is ow=(int)((float)w*scale), oh=(int)((float)h*scale) -- the reference's truncation (src/srcnn.cpp:573-575,
  * src/test.cpp:357-358).
  */
@@ -54,7 +68,9 @@ enum {
     SRCNN_VARIANT_FP32 = 1  /* strict FP32 CUDA-core kernels in the reference's summation order (bit-exact) */
 };
 
-enum { SRCNN_ORDER_BGR = 0, SRCNN_ORDER_RGB = 1, SRCNN_ORDER_GRAY = 2, SRCNN_ORDER_BGRA = 3, SRCNN_ORDER_RGBA = 4 };
+/* 5 is not assigned: it has been rejected as an unknown order since the four-channel orders were added, and stays so. */
+enum { SRCNN_ORDER_BGR = 0, SRCNN_ORDER_RGB = 1, SRCNN_ORDER_GRAY = 2, SRCNN_ORDER_BGRA = 3, SRCNN_ORDER_RGBA = 4,
+       SRCNN_ORDER_NV12 = 6, SRCNN_ORDER_I420 = 7 };
 
 /* Status codes.  -1 / -2 / -3 / -10 keep the reference CLI's meanings (src/srcnn.cpp:479,493,526,555,684). */
 enum {

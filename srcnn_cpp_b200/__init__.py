@@ -23,6 +23,8 @@ ORDER_RGB = 1
 ORDER_GRAY = 2   # one channel: HxW (NxHxW) arrays and tensors in and out; the result is the CNN's Y'
 ORDER_BGRA = 3   # four channels, straight alpha in byte 3: HxWx4 (NxHxWx4) in and out; colour bytes = the BGR call's,
 ORDER_RGBA = 4   # alpha = the one-plane cubic resize of the alpha plane (no CNN)
+ORDER_NV12 = 6   # packed 4:2:0 video frames: (H*3/2)xW ((N)x(H*3/2)xW) arrays and tensors in and out; Y plane = the grey call's,
+ORDER_I420 = 7   # chroma planes = the one-plane cubic resize of the source's (no CNN).  yuv420_planes() splits a frame
 
 OK = 0
 E_RATIO = -1
@@ -181,10 +183,52 @@ class PinnedBuffer:
 
 
 def _pixel_shape(order):
-    """trailing shape of one pixel: () for ORDER_GRAY, (4,) for ORDER_BGRA / ORDER_RGBA, (3,) for the colour orders"""
-    if order == ORDER_GRAY:
+    """trailing shape of one pixel: () for ORDER_GRAY and the 4:2:0 orders, (4,) for ORDER_BGRA / ORDER_RGBA, (3,) for the colour
+    orders"""
+    if order in (ORDER_GRAY, ORDER_NV12, ORDER_I420):
         return ()
     return (4,) if order in (ORDER_BGRA, ORDER_RGBA) else (3,)
+
+
+def _is_yuv420(order):
+    return order in (ORDER_NV12, ORDER_I420)
+
+
+def _frame_h(order, rows):
+    """image height of a frame of `rows` rows in memory: rows*2/3 for a 4:2:0 frame (Y rows, then h/2 chroma rows)"""
+    if not _is_yuv420(order):
+        return rows
+    if rows % 3:
+        raise SrcnnError(E_ARG, "a 4:2:0 frame has H*3/2 rows; %d is not a multiple of 3" % rows)
+    return rows * 2 // 3
+
+
+def _out_rows(order, oh):
+    return oh * 3 // 2 if _is_yuv420(order) else oh
+
+
+def yuv420_planes(frame, order):
+    """(Y, U, V) views of one packed 4:2:0 frame: an (H*3/2)xW uint8 numpy array or torch tensor whose rows may be padded
+    (row stride >= W; I420: even).  NV12: U and V are the even / odd bytes of the interleaved chroma rows.  I420: H/2 x W/2 planes
+    whose rows are stride/2 apart, V after U."""
+    if order not in (ORDER_NV12, ORDER_I420) or len(frame.shape) != 2:
+        raise SrcnnError(E_ARG, "expected one (H*3/2)xW frame and ORDER_NV12 / ORDER_I420")
+    rows, w = frame.shape
+    h = _frame_h(order, rows)
+    y, c = frame[:h], frame[h:]
+    if order == ORDER_NV12:
+        return y, c[:, 0::2], c[:, 1::2]
+    torch_like = hasattr(frame, "storage_offset")
+    s = frame.stride(0) if torch_like else frame.strides[0]
+    if s % 2:
+        raise SrcnnError(E_ARG, "I420 rows must be an even number of bytes apart")
+    shape, first, second = (h // 2, w // 2), h * s, h * s + (h // 2) * (s // 2)
+    if torch_like:
+        o = frame.storage_offset()
+        return y, frame.as_strided(shape, (s // 2, 1), o + first), frame.as_strided(shape, (s // 2, 1), o + second)
+    flat = np.lib.stride_tricks.as_strided(frame, shape=(second + (h // 2) * (s // 2),), strides=(1,))
+    as_plane = lambda k: np.lib.stride_tricks.as_strided(flat[k:], shape=shape, strides=(s // 2, 1))
+    return y, as_plane(first), as_plane(second)
 
 
 def _check_host_image(a, order, lead):
@@ -262,16 +306,17 @@ class Engine:
 
     # -- whole path, host buffers (numpy) ----------------------------------------------------------
     def process(self, img, scale, order=ORDER_BGR, out=None):
-        """img: HxWx3 uint8 numpy array (BGR by default, like cv::imread), HxW with order=ORDER_GRAY, or HxWx4 with
-        order=ORDER_BGRA / ORDER_RGBA.  Returns OHxOWx3 (OHxOW, OHxOWx4) uint8."""
+        """img: HxWx3 uint8 numpy array (BGR by default, like cv::imread), HxW with order=ORDER_GRAY, HxWx4 with
+        order=ORDER_BGRA / ORDER_RGBA, or an (H*3/2)xW frame with ORDER_NV12 / ORDER_I420.  Returns OHxOWx3 (OHxOW, OHxOWx4,
+        (OH*3/2)xOW) uint8."""
         img = np.asarray(img)
         _check_host_image(img, order, 1)
         if not img.flags.c_contiguous:
             img = np.ascontiguousarray(img)
-        h, w = img.shape[:2]
+        h, w = _frame_h(order, img.shape[0]), img.shape[1]
         ow, oh = out_dims(w, h, scale)
         if out is None:
-            out = np.empty((oh, ow) + _pixel_shape(order), np.uint8)
+            out = np.empty((_out_rows(order, oh), ow) + _pixel_shape(order), np.uint8)
         self._check(self.L.srcnn_process_host(self.ctx, img.ctypes.data, w, h, img.strides[0], order, C.c_float(scale),
                                               out.ctypes.data, out.strides[0]))
         return out
@@ -281,10 +326,10 @@ class Engine:
         (NxOHxOW, NxOHxOWx4)."""
         frames = np.ascontiguousarray(frames)
         _check_host_image(frames, order, 2)
-        n, h, w = frames.shape[:3]
+        n, h, w = frames.shape[0], _frame_h(order, frames.shape[1]), frames.shape[2]
         ow, oh = out_dims(w, h, scale)
         if out is None:
-            out = np.empty((n, oh, ow) + _pixel_shape(order), np.uint8)
+            out = np.empty((n, _out_rows(order, oh), ow) + _pixel_shape(order), np.uint8)
         self._check(self.L.srcnn_process_batch_host(self.ctx, frames.ctypes.data, n, w, h, frames.strides[1],
                                                     frames.strides[0], order, C.c_float(scale), out.ctypes.data,
                                                     out.strides[1], out.strides[0]))
@@ -293,14 +338,14 @@ class Engine:
     # -- whole path, device buffers (torch CUDA tensors) -------------------------------------------
     def process_device(self, src, scale, dst, order=ORDER_BGR):
         """src: HxWx3 (HxW with order=ORDER_GRAY, HxWx4 with ORDER_BGRA / ORDER_RGBA) uint8 device tensor; dst: OHxOWx3
-        (OHxOW, OHxOWx4)."""
-        h, w = src.shape[:2]
+        (OHxOW, OHxOWx4); (H*3/2)xW and (OH*3/2)xOW frames with ORDER_NV12 / ORDER_I420."""
+        h, w = _frame_h(order, src.shape[0]), src.shape[1]
         self._check(self.L.srcnn_process_device(self.ctx, _dptr(src), w, h, src.stride(0), order, C.c_float(scale),
                                                 _dptr(dst), dst.stride(0)))
         return dst
 
     def process_batch_device(self, src, scale, dst, order=ORDER_BGR):
-        n, h, w = src.shape[:3]
+        n, h, w = src.shape[0], _frame_h(order, src.shape[1]), src.shape[2]
         self._check(self.L.srcnn_process_batch_device(self.ctx, _dptr(src), n, w, h, src.stride(1), src.stride(0), order,
                                                       C.c_float(scale), _dptr(dst), dst.stride(1), dst.stride(0)))
         return dst
@@ -464,10 +509,10 @@ class MultiEngine:
     def process_batch(self, frames, scale, order=ORDER_BGR, out=None):
         frames = np.ascontiguousarray(frames)
         _check_host_image(frames, order, 2)
-        n, h, w = frames.shape[:3]
+        n, h, w = frames.shape[0], _frame_h(order, frames.shape[1]), frames.shape[2]
         ow, oh = out_dims(w, h, scale)
         if out is None:
-            out = np.empty((n, oh, ow) + _pixel_shape(order), np.uint8)
+            out = np.empty((n, _out_rows(order, oh), ow) + _pixel_shape(order), np.uint8)
         self._check(self.L.srcnn_mgpu_process_batch_host(self.h, frames.ctypes.data, n, w, h, frames.strides[1], frames.strides[0],
                                                          order, C.c_float(scale), out.ctypes.data, out.strides[1], out.strides[0]))
         return out
@@ -477,7 +522,7 @@ class MultiEngine:
         """srcs[i]: n_i x H x W x 3 (no x 3 with ORDER_GRAY, x 4 with ORDER_BGRA / ORDER_RGBA) on worker i's device (n_i may be
         0 -> pass None); dsts[i]: n_i x OH x OW x 3 (likewise)."""
         ref = next(t for t in srcs if t is not None)
-        h, w = ref.shape[1:3]
+        h, w = _frame_h(order, ref.shape[1]), ref.shape[2]
         dref = next(t for t in dsts if t is not None)
         ps = (C.c_void_p * self.n)(*[t.data_ptr() if t is not None else None for t in srcs])
         pd = (C.c_void_p * self.n)(*[t.data_ptr() if t is not None else None for t in dsts])

@@ -66,23 +66,53 @@ static int scaled_dim(int n, float scale) {
     return (int)((float)n * scale);
 }
 
-static size_t bytes_per_pixel(int order) { return order == SRCNN_ORDER_GRAY ? 1 : (four_channel(order) ? 4 : 3); }
+// bytes per pixel of a row (4:2:0: of a Y row; a chroma row of NV12 has as many, an I420 chroma row half as many)
+static size_t bytes_per_pixel(int order) { return order == SRCNN_ORDER_GRAY || yuv420(order) ? 1 : (four_channel(order) ? 4 : 3); }
+// rows of one frame in memory (4:2:0: h rows of Y, then h/2 rows of NV12 pairs or of I420 U and V)
+static size_t frame_rows(int order, int h) { return yuv420(order) ? (size_t)h / 2 * 3 : (size_t)h; }
 
 static int check_image(Ctx* c, const void* src, int w, int h, size_t stride, int order, float scale, const void* dst,
                        size_t dst_stride, int* ow, int* oh) {
     if (!c) return SRCNN_E_ARG;
     if (!src || !dst) return fail(c, SRCNN_E_ARG, "null image pointer");
     if (w <= 0 || h <= 0) return fail(c, SRCNN_E_ARG, "non-positive image size %dx%d", w, h);
-    if (order != SRCNN_ORDER_BGR && order != SRCNN_ORDER_RGB && order != SRCNN_ORDER_GRAY && !four_channel(order))
+    if (order != SRCNN_ORDER_BGR && order != SRCNN_ORDER_RGB && order != SRCNN_ORDER_GRAY && !four_channel(order) && !yuv420(order))
         return fail(c, SRCNN_E_ARG, "unknown pixel order %d", order);
     const size_t bpp = bytes_per_pixel(order);
     if (stride < (size_t)w * bpp) return fail(c, SRCNN_E_ARG, "source stride %zu < %zu*w", stride, bpp);
+    if (yuv420(order) && ((w | h) & 1)) return fail(c, SRCNN_E_ARG, "4:2:0 frames need an even width and height, got %dx%d", w, h);
+    if (order == SRCNN_ORDER_I420 && ((stride | dst_stride) & 1))
+        return fail(c, SRCNN_E_ARG, "I420 strides must be even (chroma rows are stride/2 apart), got %zu / %zu", stride, dst_stride);
     // src/srcnn.cpp:485-495 "ratio too small"
     if (!(((float)w * scale) > 0.f) || !(((float)h * scale) > 0.f)) return fail(c, SRCNN_E_RATIO, "scale %g gives an empty image", scale);
     *ow = scaled_dim(w, scale);
     *oh = scaled_dim(h, scale);
     if (*ow <= 0 || *oh <= 0) return fail(c, SRCNN_E_RATIO, "scale %g gives an empty image", scale);
+    if (yuv420(order) && ((*ow | *oh) & 1))
+        return fail(c, SRCNN_E_ARG, "scale %g gives an odd 4:2:0 output size %dx%d (width and height must be even)", scale, *ow, *oh);
     if (dst_stride < (size_t)*ow * bpp) return fail(c, SRCNN_E_ARG, "destination stride %zu < %zu*ow", dst_stride, bpp);
+    return SRCNN_OK;
+}
+
+// The chroma planes of 4:2:0 frames whose Y rows start at `src` / `dst` (frame 0), for the luma output rows [r0, r1): chroma output
+// rows [r0/2, r1/2).  A chroma row is resized without the CNN, so it needs no halo.
+static int chroma_planes(Ctx* c, int order, const uint8_t* src, int w, int h, size_t src_stride, uint8_t* dst, int ow, int oh,
+                         size_t dst_stride, size_t dst_frame_stride, int r0, int r1, Chroma420* ch) {
+    TapTable *tx, *ty;
+    int rc = get_taps(c, w / 2, ow / 2, &tx);
+    if (rc) return rc;
+    if ((rc = get_taps(c, h / 2, oh / 2, &ty))) return rc;
+    const bool i420 = order == SRCNN_ORDER_I420;
+    ch->src = src + (size_t)h * src_stride;
+    ch->src_pitch = i420 ? src_stride / 2 : src_stride;
+    ch->src_v = i420 ? (size_t)(h / 2) * (src_stride / 2) : 0;
+    ch->dst = dst + (size_t)oh * dst_stride;
+    ch->dst_pitch = i420 ? dst_stride / 2 : dst_stride;
+    ch->dst_v = i420 ? (size_t)(oh / 2) * (dst_stride / 2) : 0;
+    ch->dst_frame = dst_frame_stride;
+    ch->sw = w / 2; ch->sh = h / 2; ch->ow = ow / 2; ch->oh = oh / 2;
+    ch->row_begin = r0 / 2; ch->row_end = r1 / 2;
+    ch->tx = tx; ch->ty = ty;
     return SRCNN_OK;
 }
 
@@ -94,10 +124,10 @@ static int check_image(Ctx* c, const void* src, int w, int h, size_t stride, int
 // never reads Y / FP16 Y, and Y' is written by the next CNN launch, which waits for everything before it).  c->plane_sel says which
 // set this call got.  Keeping the rest single also keeps the planes L2-resident from step to step: two whole plane sets (116 MB
 // at 4K) measured 3 us slower in the colour+bicubic kernel.
-// The host-buffer pipeline keeps to set 0 (its sub-bands are separated by copies and events anyway).  A grey call has no Cr/Cb
-// planes: it leaves the set selection alone (and ends the early-start chain, end_merge_chain).
+// The host-buffer pipeline keeps to set 0 (its sub-bands are separated by copies and events anyway).  A grey or 4:2:0 call has no
+// Cr/Cb planes: it leaves the set selection alone (and ends the early-start chain, end_merge_chain).
 static int carve_planes(Ctx* c, int ow, int rows, int row0, Planes* pl, int nframes = 1, int order = SRCNN_ORDER_BGR) {
-    const bool gray = order == SRCNN_ORDER_GRAY, four = four_channel(order);
+    const bool gray = order == SRCNN_ORDER_GRAY || yuv420(order), four = four_channel(order);
     const size_t pitch = align_up((size_t)ow, 128);
     const size_t plane = pitch * (size_t)rows;
     const size_t pitch16 = y16_pitch_bytes(ow);
@@ -141,7 +171,7 @@ static Ctx* last_merge_on(cudaStream_t s) {
     auto it = g_last_merge.find(s);
     return it == g_last_merge.end() ? nullptr : it->second;
 }
-// A grey call launches no merge: the kernel that ends up last on the stream does not release its dependents, so neither this
+// A grey or 4:2:0 call launches no merge: the kernel that ends up last on the stream does not release its dependents, so neither this
 // context's next colour call nor any other context's on this stream may start early.
 static void end_merge_chain(Ctx* c) {
     c->merge_sel = -1;
@@ -191,8 +221,9 @@ static int process_rows_impl(Ctx* c, const uint8_t* d_src, int w, int h, size_t 
     rc = get_taps(c, h, oh, &ty);
     if (rc) return rc;
     const int p0 = std::max(r0 - 6, 0), p1 = std::min(r1 + 6, oh);  // 6-px halo: 4 (conv1) + 2 (conv3)
-    // grey: one-plane resize, then the CNN straight into the caller's rows; no chroma, no merge
-    const bool gray = order == SRCNN_ORDER_GRAY;
+    // grey: one-plane resize, then the CNN straight into the caller's rows; no chroma, no merge.  4:2:0: the same for Y, and the
+    // resize launch also writes the chroma rows [r0/2, r1/2) straight into the caller's frame (d_dst is its row r0)
+    const bool gray = order == SRCNN_ORDER_GRAY || yuv420(order);
     if (gray) end_merge_chain(c);
     Planes pl;
     c->fail_stage = SRCNN_STAGE_PLANES;
@@ -212,6 +243,9 @@ static int process_rows_impl(Ctx* c, const uint8_t* d_src, int w, int h, size_t 
     ra.ow = ow; ra.oh = oh;
     ra.row_begin = p0; ra.row_end = p1;
     ra.pl = pl; ra.tx = tx; ra.ty = ty;
+    if (yuv420(order) && (rc = chroma_planes(c, order, d_src - (size_t)s0 * src_stride, w, h, src_stride, d_dst - (size_t)r0 * dst_stride,
+                                             ow, oh, dst_stride, 0, r0, r1, &ra.ch)))
+        return rc;
     if (c->variant != SRCNN_VARIANT_TC) ra.pl.y16 = nullptr;      // the strict FP32 kernels read the u8 plane
     ra.early = !gray && may_start_early(c, d_src, (size_t)(s1 - s0) * src_stride);
     c->early_launches += ra.early;
@@ -277,7 +311,7 @@ static int process_frames_impl(Ctx* c, const uint8_t* d_src, int n, int w, int h
     if ((rc = get_taps(c, h, oh, &ty))) return rc;
     const size_t per_frame = align_up((size_t)ow, 128) * (size_t)oh * (four_channel(order) ? 5 : 4) + y16_pitch_bytes(ow) * (size_t)oh;
     const int chunk = (int)std::max<size_t>(1, std::min<size_t>((size_t)n, ((size_t)1 << 30) / per_frame));
-    const bool gray = order == SRCNN_ORDER_GRAY;
+    const bool gray = order == SRCNN_ORDER_GRAY || yuv420(order);   // the CNN writes into the caller's frames, no merge
     if (gray) end_merge_chain(c);
     for (int f0 = 0; f0 < n; f0 += chunk) {
         const int m = std::min(chunk, n - f0);
@@ -293,6 +327,9 @@ static int process_frames_impl(Ctx* c, const uint8_t* d_src, int n, int w, int h
         ra.row_begin = 0; ra.row_end = oh;
         ra.pl = pl; ra.tx = tx; ra.ty = ty;
         ra.nframes = m; ra.src_frame_stride = src_frame_stride;
+        if (yuv420(order) && (rc = chroma_planes(c, order, ra.src, w, h, src_stride, d_dst + (size_t)f0 * dst_frame_stride, ow, oh, dst_stride,
+                                                 dst_frame_stride, 0, oh, &ra.ch)))
+            return rc;
         ra.early = !gray && may_start_early(c, ra.src, (size_t)(m - 1) * src_frame_stride + (size_t)h * src_stride);
         c->early_launches += ra.early;
         if ((rc = prof_mark(c, 0))) return rc;
@@ -395,14 +432,40 @@ void drop_graphs(Ctx* c) {
     c->graphs.clear();
 }
 
+// Luma rows [y0, y1) and chroma rows [c0, c1) of one 4:2:0 frame between two buffers whose Y rows are `ds` / `ss` bytes apart
+// (w x h: the frame's size).  NV12's chroma rows follow the Y rows with the same stride; I420's U and V rows are half as long.
+static int copy_420(Ctx* c, bool i420, uint8_t* dst, size_t ds, const uint8_t* src, size_t ss, int w, int h, int y0, int y1, int c0,
+                    int c1, cudaMemcpyKind kind, cudaStream_t st) {
+    if (y1 > y0)
+        SRCNN_CUDA(c, cudaMemcpy2DAsync(dst + (size_t)y0 * ds, ds, src + (size_t)y0 * ss, ss, (size_t)w, y1 - y0, kind, st));
+    if (c1 <= c0) return SRCNN_OK;
+    dst += (size_t)h * ds;
+    src += (size_t)h * ss;
+    if (!i420) {
+        SRCNN_CUDA(c, cudaMemcpy2DAsync(dst + (size_t)c0 * ds, ds, src + (size_t)c0 * ss, ss, (size_t)w, c1 - c0, kind, st));
+        return SRCNN_OK;
+    }
+    ds /= 2;
+    ss /= 2;
+    for (int pl = 0; pl < 2; pl++) {   // U, then V h/2 rows further
+        const size_t r = (size_t)(pl * (h / 2) + c0);
+        SRCNN_CUDA(c, cudaMemcpy2DAsync(dst + r * ds, ds, src + r * ss, ss, (size_t)w / 2, c1 - c0, kind, st));
+    }
+    return SRCNN_OK;
+}
+
 // Enqueues the whole pipeline of one chunk of frames (f0 .. f0+m) on the three streams and joins the copy streams back
 // into the compute stream; does not wait.  Identical whether the streams are live or being captured into a CUDA graph.
 static int enqueue_chunk(Ctx* c, const uint8_t* src, int f0, int m, int w, int h, size_t src_stride, size_t src_frame_stride, int order,
                          float scale, int ow, int oh, int R0, int R1, uint8_t* dst, size_t dst_stride, size_t dst_frame_stride,
-                         const TapTable* ty, int S0, int S1, const std::vector<int>& edges, int group, size_t s_row, size_t d_row, size_t s_frame,
+                         const TapTable* ty, const TapTable* cty, int S0, int S1, const std::vector<int>& edges, int group, size_t s_row, size_t d_row, size_t s_frame,
                          size_t d_frame) {
     const int bands = (int)edges.size() - 1;
     const size_t bpp = bytes_per_pixel(order), w_bytes = (size_t)w * bpp, ow_bytes = (size_t)ow * bpp;
+    // 4:2:0: frames are staged whole (S0 = 0, R0 = 0), every row at its place in the frame; a sub-band copies the chroma rows its
+    // chroma output rows [r0/2, r1/2) read (chroma tap table cty) along with its Y rows
+    const bool yuv = yuv420(order), i420 = order == SRCNN_ORDER_I420;
+    const size_t in_rows = yuv ? frame_rows(order, h) : (size_t)(S1 - S0), out_rows = yuv ? frame_rows(order, oh) : (size_t)(R1 - R0);
     int rc;
     uint8_t* ds = (uint8_t*)c->src_buf.p;
     uint8_t* dd = (uint8_t*)c->dst_buf.p;
@@ -441,7 +504,12 @@ static int enqueue_chunk(Ctx* c, const uint8_t* src, int f0, int m, int w, int h
             if ((rc = event_at(ei++, &ev_in))) return rc;
             if (rows_tight_in) {   // frames are the "rows" of one 2-D copy
                 SRCNN_CUDA(c, cudaMemcpy2DAsync(ds + (size_t)g0 * s_frame, s_frame, hsrc + (size_t)S0 * src_stride, src_frame_stride,
-                                                (size_t)(S1 - S0) * s_row, g, cudaMemcpyHostToDevice, c->s_in));
+                                                in_rows * s_row, g, cudaMemcpyHostToDevice, c->s_in));
+            } else if (yuv) {
+                for (int f = 0; f < g; f++)
+                    if ((rc = copy_420(c, i420, ds + (size_t)(g0 + f) * s_frame, s_row, hsrc + (size_t)f * src_frame_stride, src_stride, w, h,
+                                       0, h, 0, h / 2, cudaMemcpyHostToDevice, c->s_in)))
+                        return rc;
             } else {
                 for (int f = 0; f < g; f++)
                     SRCNN_CUDA(c, cudaMemcpy2DAsync(ds + (size_t)(g0 + f) * s_frame, s_row, hsrc + (size_t)f * src_frame_stride + (size_t)S0 * src_stride,
@@ -462,8 +530,13 @@ static int enqueue_chunk(Ctx* c, const uint8_t* src, int f0, int m, int w, int h
             SRCNN_CUDA(c, cudaEventRecord(ev_done, c->stream));
             SRCNN_CUDA(c, cudaStreamWaitEvent(c->s_out, ev_done, 0));
             if (rows_tight_out) {
-                SRCNN_CUDA(c, cudaMemcpy2DAsync(hdst, dst_frame_stride, dd + (size_t)g0 * d_frame, d_frame, (size_t)rows * d_row, g,
+                SRCNN_CUDA(c, cudaMemcpy2DAsync(hdst, dst_frame_stride, dd + (size_t)g0 * d_frame, d_frame, out_rows * d_row, g,
                                                 cudaMemcpyDeviceToHost, c->s_out));
+            } else if (yuv) {
+                for (int f = 0; f < g; f++)
+                    if ((rc = copy_420(c, i420, hdst + (size_t)f * dst_frame_stride, dst_stride, dd + (size_t)(g0 + f) * d_frame, d_row, ow, oh,
+                                       0, oh, 0, oh / 2, cudaMemcpyDeviceToHost, c->s_out)))
+                        return rc;
             } else {
                 for (int f = 0; f < g; f++)
                     SRCNN_CUDA(c, cudaMemcpy2DAsync(hdst + (size_t)f * dst_frame_stride, dst_stride, dd + (size_t)(g0 + f) * d_frame, d_row, ow_bytes, rows,
@@ -475,17 +548,26 @@ static int enqueue_chunk(Ctx* c, const uint8_t* src, int f0, int m, int w, int h
         const uint8_t* hsrc = src + (size_t)(f0 + f) * src_frame_stride;
         uint8_t* hdst = dst + (size_t)(f0 + f) * dst_frame_stride;
         int copied = S0;   // source rows [S0, copied) of this frame are on their way to the device
+        int c_copied = 0;  // 4:2:0: chroma source rows [0, c_copied) likewise
         for (int bi = 0; bi < bands; bi++) {
             const int r0 = edges[bi], r1 = edges[bi + 1];
             const int s_hi = bi + 1 < bands ? src_hi(r1) : S1;
-            if (s_hi > copied) {
+            const int c_hi = !yuv ? 0 : bi + 1 < bands ? std::min(std::max(cty->h_ofs[r1 / 2 - 1] + 2, 0), h / 2 - 1) + 1 : h / 2;
+            if (s_hi > copied || c_hi > c_copied) {
                 cudaEvent_t ev_in;
                 if ((rc = event_at(ei++, &ev_in))) return rc;
-                SRCNN_CUDA(c, cudaMemcpy2DAsync(ds + f * s_frame + (size_t)(copied - S0) * s_row, s_row, hsrc + (size_t)copied * src_stride,
-                                                src_stride, w_bytes, s_hi - copied, cudaMemcpyHostToDevice, c->s_in));
+                if (yuv) {
+                    if ((rc = copy_420(c, i420, ds + f * s_frame, s_row, hsrc, src_stride, w, h, copied, s_hi, c_copied, c_hi,
+                                       cudaMemcpyHostToDevice, c->s_in)))
+                        return rc;
+                } else {
+                    SRCNN_CUDA(c, cudaMemcpy2DAsync(ds + f * s_frame + (size_t)(copied - S0) * s_row, s_row, hsrc + (size_t)copied * src_stride,
+                                                    src_stride, w_bytes, s_hi - copied, cudaMemcpyHostToDevice, c->s_in));
+                }
                 SRCNN_CUDA(c, cudaEventRecord(ev_in, c->s_in));
                 SRCNN_CUDA(c, cudaStreamWaitEvent(c->stream, ev_in, 0));
-                copied = s_hi;
+                copied = std::max(copied, s_hi);
+                c_copied = std::max(c_copied, c_hi);
             }
             rc = process_rows(c, ds + f * s_frame, w, h, s_row, S0, S1, order, scale, ow, oh, r0, r1,
                               dd + f * d_frame + (size_t)(r0 - R0) * d_row, d_row);
@@ -494,6 +576,12 @@ static int enqueue_chunk(Ctx* c, const uint8_t* src, int f0, int m, int w, int h
             if ((rc = event_at(ei++, &ev_done))) return rc;
             SRCNN_CUDA(c, cudaEventRecord(ev_done, c->stream));
             SRCNN_CUDA(c, cudaStreamWaitEvent(c->s_out, ev_done, 0));
+            if (yuv) {
+                if ((rc = copy_420(c, i420, hdst, dst_stride, dd + f * d_frame, d_row, ow, oh, r0, r1, r0 / 2, r1 / 2, cudaMemcpyDeviceToHost,
+                                   c->s_out)))
+                    return rc;
+                continue;
+            }
             SRCNN_CUDA(c, cudaMemcpy2DAsync(hdst + (size_t)(r0 - R0) * dst_stride, dst_stride,
                                             dd + f * d_frame + (size_t)(r0 - R0) * d_row, d_row, ow_bytes, r1 - r0,
                                             cudaMemcpyDeviceToHost, c->s_out));
@@ -518,18 +606,23 @@ int host_pipeline(Ctx* c, const uint8_t* src, int n, int w, int h, size_t src_st
         explicit HostPath(Ctx* c_) : c(c_) { c->host_path = true; c->merge_sel = -1; }
         ~HostPath() { c->host_path = false; c->merge_sel = -1; }
     } host_path{c};
-    TapTable *ty = nullptr, *tx = nullptr;
+    TapTable *ty = nullptr, *tx = nullptr, *cty = nullptr, *ctx_ = nullptr;
     if ((rc = get_taps(c, h, oh, &ty))) return rc;
     if ((rc = get_taps(c, w, ow, &tx))) return rc;      // uploaded here, not inside a graph capture
+    const bool yuv = yuv420(order);
+    if (yuv && ((rc = get_taps(c, h / 2, oh / 2, &cty)) || (rc = get_taps(c, w / 2, ow / 2, &ctx_)))) return rc;   // chroma
     auto src_hi = [&](int r1) {
         const int p1 = std::min(r1 + 6, oh);
         return std::min(std::max(ty->h_ofs[p1 - 1] + 2, 0), h - 1) + 1;
     };
-    const int S0 = std::min(std::max(ty->h_ofs[std::max(R0 - 6, 0)] - 1, 0), h - 1), S1 = src_hi(R1);
-    // device staging: tight rows, 256-byte aligned frames; only the rows this call needs
-    const size_t bpp = bytes_per_pixel(order);
-    const size_t s_row = align_up((size_t)w * bpp, 4), d_row = align_up((size_t)ow * bpp, 4);
-    const size_t s_frame = align_up(s_row * (size_t)(S1 - S0), 256), d_frame = align_up(d_row * (size_t)(R1 - R0), 256);
+    // 4:2:0 frames are staged whole (whole-frame calls only: R0 = 0, R1 = oh), every row at its place in the frame
+    const int S0 = yuv ? 0 : std::min(std::max(ty->h_ofs[std::max(R0 - 6, 0)] - 1, 0), h - 1), S1 = yuv ? h : src_hi(R1);
+    // device staging: tight rows (4:2:0: 16-byte multiples, so that I420's half-length chroma rows stay 8-byte aligned), 256-byte
+    // aligned frames; only the rows this call needs
+    const size_t bpp = bytes_per_pixel(order), row_align = yuv ? 16 : 4;
+    const size_t s_row = align_up((size_t)w * bpp, row_align), d_row = align_up((size_t)ow * bpp, row_align);
+    const size_t s_frame = align_up(s_row * (yuv ? frame_rows(order, h) : (size_t)(S1 - S0)), 256);
+    const size_t d_frame = align_up(d_row * (yuv ? frame_rows(order, oh) : (size_t)(R1 - R0)), 256);
     // frames in flight are bounded so staging stays modest (<= 4 GiB of output; one frame may be larger).  Chunks are separated by
     // a full drain of the pipeline, so the bound is generous: 180 GB of HBM is not the scarce resource here.
     const int chunk = (int)std::max<size_t>(1, std::min<size_t>((size_t)n, ((size_t)4 << 30) / d_frame));
@@ -551,12 +644,12 @@ int host_pipeline(Ctx* c, const uint8_t* src, int n, int w, int h, size_t src_st
         const long long by_mem = ((long long)rows * (long long)ow * (four_channel(order) ? 5 : 4) + (256ll << 20) - 1) / (256ll << 20);
         if (by_mem > c->host_bands) {
             const int nb = (int)std::min<long long>(by_mem, rows / 64);
-            for (int bi = 1; bi < nb; bi++) edges.push_back(R0 + (int)((long long)rows * bi / nb));
+            for (int bi = 1; bi < nb; bi++) edges.push_back((R0 + (int)((long long)rows * bi / nb)) & (yuv ? ~1 : ~0));   // 4:2:0: even
         } else if (c->host_bands > 1) {
             double len = c->band_first > 0 ? (double)c->band_first : std::max(256.0, (double)rows / c->host_bands);
             int pos = R0;
             while ((int)edges.size() < c->host_bands) {
-                const int take = (int)len;
+                const int take = (int)len & (yuv ? ~1 : ~0);
                 if (R1 - (pos + take) < take / 2) break;      // the rest joins the last band
                 pos += take;
                 edges.push_back(pos);
@@ -610,7 +703,7 @@ int host_pipeline(Ctx* c, const uint8_t* src, int n, int w, int h, size_t src_st
         if (e == cudaSuccess) {
             c->capturing = true;
             rc = enqueue_chunk(c, src, 0, n, w, h, src_stride, src_frame_stride, order, scale, ow, oh, R0, R1, dst, dst_stride,
-                               dst_frame_stride, ty, S0, S1, edges, group, s_row, d_row, s_frame, d_frame);
+                               dst_frame_stride, ty, cty, S0, S1, edges, group, s_row, d_row, s_frame, d_frame);
             e = cudaStreamEndCapture(c->stream, &graph);
             c->capturing = false;
             if (rc == SRCNN_OK && e == cudaSuccess && graph && cudaGraphInstantiate(&hit->exec, graph, 0) != cudaSuccess) hit->exec = nullptr;
@@ -631,7 +724,7 @@ int host_pipeline(Ctx* c, const uint8_t* src, int n, int w, int h, size_t src_st
         const int m = std::min(chunk, n - f0);
         const long long l0 = c->launches;
         rc = enqueue_chunk(c, src, f0, m, w, h, src_stride, src_frame_stride, order, scale, ow, oh, R0, R1, dst, dst_stride,
-                           dst_frame_stride, ty, S0, S1, edges, group, s_row, d_row, s_frame, d_frame);
+                           dst_frame_stride, ty, cty, S0, S1, edges, group, s_row, d_row, s_frame, d_frame);
         if (rc) return rc;
         if (graphable && f0 == 0)
             for (auto& g : c->graphs)
@@ -935,7 +1028,7 @@ int srcnn_process_batch_device(srcnn_ctx* c, const uint8_t* d_src, int n, int w,
     int ow, oh;
     int rc = check_image(c, d_src, w, h, src_stride, order, scale, d_dst, dst_stride, &ow, &oh);
     if (rc) return rc;
-    if (n > 1 && (src_frame_stride < src_stride * (size_t)h || dst_frame_stride < dst_stride * (size_t)oh))
+    if (n > 1 && (src_frame_stride < src_stride * frame_rows(order, h) || dst_frame_stride < dst_stride * frame_rows(order, oh)))
         return fail(c, SRCNN_E_ARG, "frame stride smaller than one frame");
     return process_frames(c, d_src, n, w, h, src_stride, src_frame_stride, order, scale, ow, oh, d_dst, dst_stride, dst_frame_stride);
 }
@@ -949,7 +1042,7 @@ int srcnn_process_batch_host(srcnn_ctx* c, const uint8_t* src, int n, int w, int
     int ow, oh;
     int rc = check_image(c, src, w, h, src_stride, order, scale, dst, dst_stride, &ow, &oh);
     if (rc) return rc;
-    if (n > 1 && (src_frame_stride < src_stride * (size_t)h || dst_frame_stride < dst_stride * (size_t)oh))
+    if (n > 1 && (src_frame_stride < src_stride * frame_rows(order, h) || dst_frame_stride < dst_stride * frame_rows(order, oh)))
         return fail(c, SRCNN_E_ARG, "frame stride smaller than one frame");
     return host_pipeline(c, src, n, w, h, src_stride, src_frame_stride, order, scale, ow, oh, 0, oh, dst, dst_stride, dst_frame_stride);
 }
@@ -980,6 +1073,7 @@ int srcnn_process_band_device(srcnn_ctx* c, const uint8_t* d_src, int w, int h, 
     int ow, oh;
     int rc = check_image(c, d_src, w, h, src_stride, order, scale, d_dst, dst_stride, &ow, &oh);
     if (rc) return rc;
+    if (yuv420(order)) return fail(c, SRCNN_E_ARG, "4:2:0 frames are whole-frame calls only (no band calls)");
     if (r0 < 0 || r1 > oh || r0 >= r1) return fail(c, SRCNN_E_ARG, "bad output band [%d,%d) of %d rows", r0, r1, oh);
     if (s0 < 0 || s1 > h || s0 >= s1) return fail(c, SRCNN_E_ARG, "bad source band [%d,%d) of %d rows", s0, s1, h);
     return process_rows(c, d_src, w, h, src_stride, s0, s1, order, scale, ow, oh, r0, r1, d_dst, dst_stride);
@@ -991,6 +1085,7 @@ int srcnn_process_band_host(srcnn_ctx* c, const uint8_t* src, int w, int h, size
     int ow, oh;
     int rc = check_image(c, src, w, h, src_stride, order, scale, dst_rows, dst_stride, &ow, &oh);
     if (rc) return rc;
+    if (yuv420(order)) return fail(c, SRCNN_E_ARG, "4:2:0 frames are whole-frame calls only (no band calls)");
     if (r0 < 0 || r1 > oh || r0 >= r1) return fail(c, SRCNN_E_ARG, "bad output band [%d,%d) of %d rows", r0, r1, oh);
     return host_pipeline(c, src, 1, w, h, src_stride, 0, order, scale, ow, oh, r0, r1, dst_rows, dst_stride, 0);
 }

@@ -156,6 +156,36 @@ __global__ void __launch_bounds__(256) k_color_bicubic_direct(ResizeDev p, uint8
     if (NP == 4) pa[o] = (uint8_t)vertical_tap(hA[0], hA[1], hA[2], hA[3], cy, fpath);
 }
 
+// The two chroma planes of a 4:2:0 frame in one launch of the direct form (byte loads and stores: any alignment).  Plane k's
+// sample x of a row is byte k * vs + x * step past the row's start in the source (k * vd + x * step in the output): NV12's pairs
+// are vs = vd = 1, step = 2; I420's planes are vs / vd = the V plane's distance from U, step = 1.
+__global__ void __launch_bounds__(256) k_chroma420_direct(ResizeDev p, size_t vs, size_t vd, int step) {
+    const int dx = blockIdx.x * 32 + (threadIdx.x & 31);
+    const int dy = p.row_begin + blockIdx.y * 8 + (threadIdx.x >> 5);
+    if (dx >= p.ow || dy >= p.row_end) return;
+    const int sx = p.xofs[dx], sy = p.yofs[dy];
+    const short4 cx = p.xcoef[dx], cy = p.ycoef[dy];
+    const int cxs[4] = {cx.x, cx.y, cx.z, cx.w};
+    int h[2][4];
+#pragma unroll
+    for (int r = 0; r < 4; r++) {
+        const uint8_t* row = p.src + (size_t)clampi(sy - 1 + r, 0, p.sh - 1) * p.src_stride;
+        int a0 = 0, a1 = 0;
+#pragma unroll
+        for (int k = 0; k < 4; k++) {
+            const size_t x = (size_t)clampi(sx - 1 + k, 0, p.sw - 1) * step;
+            a0 += (int)row[x] * cxs[k];
+            a1 += (int)row[vs + x] * cxs[k];
+        }
+        h[0][r] = a0;
+        h[1][r] = a1;
+    }
+    const bool fpath = dx < p.simd_w;
+    uint8_t* d = p.y + (size_t)(dy - p.plane_row0) * p.pitch + (size_t)dx * step;
+    d[0] = (uint8_t)vertical_tap(h[0][0], h[0][1], h[0][2], h[0][3], cy, fpath);
+    d[vd] = (uint8_t)vertical_tap(h[1][0], h[1][1], h[1][2], h[1][3], cy, fpath);
+}
+
 // ------------------------------------------------------------------------------------------------
 // K-A, tiled form (the fast path for up-scaling).  One CTA produces a TW x TH tile of all NP
 // planes: (1) the source footprint is colour-converted ONCE into shared memory (three u8 planes,
@@ -168,7 +198,8 @@ constexpr int kMaxSC = 72, kMaxSR = 40; // footprint capacity (source cols / row
 constexpr int kMaxSR4 = 35;             // ... rows with four planes (the static shared memory of one CTA stays within 48 KB)
 __host__ __device__ constexpr int tiled_max_rows(int np) { return np == 4 ? kMaxSR4 : kMaxSR; }
 
-// NP = 4: the planes of a four-channel source, plane 3 (alpha, the raw byte 3 of each pixel) into pa
+// NP = 4: the planes of a four-channel source, plane 3 (alpha, the raw byte 3 of each pixel) into pa.  NP = 2: the two bytes of an
+// interleaved pair (NV12 chroma) as two planes, written back interleaved into p.y (4-byte aligned rows)
 template <int kTH, int NP>
 __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p, uint8_t* pa) {   // 5 CTAs per SM: 48 registers (4 CTAs measured 6 % slower)
     constexpr int SR = tiled_max_rows(NP);
@@ -208,6 +239,12 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p, uin
         const int gx = clampi(sx_lo + c, 0, p.sw - 1);
         if (NP == 1) {
             sP[0][r][c] = fsrc[(size_t)gy * p.src_stride + gx];
+            continue;
+        }
+        if (NP == 2) {
+            const uint8_t* px = fsrc + (size_t)gy * p.src_stride + 2 * (size_t)gx;
+            sP[0][r][c] = px[0];
+            sP[NP - 1][r][c] = px[1];
             continue;
         }
         const uint8_t* px = fsrc + (size_t)gy * p.src_stride + (NP == 4 ? 4 : 3) * (size_t)gx;
@@ -286,7 +323,7 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p, uin
     if (dx0 > 0 && dx0 + kTW < p.ow && dx0 + kTW <= p.simd_w && dy0 + kTH <= p.row_end) {
         const int col = (tid & 15) * 4, ty0 = tid >> 4;
         const unsigned long long nz = p.negzero2;
-        const size_t o = fplane + (size_t)(dy0 + ty0 - p.plane_row0) * p.pitch + (size_t)(dx0 + col);
+        const size_t o = fplane + (size_t)(dy0 + ty0 - p.plane_row0) * p.pitch + (size_t)(dx0 + col) * (NP == 2 ? 2 : 1);
         uint8_t* pcr = NP >= 3 ? p.cr + o : nullptr;
         uint8_t* pcb = NP >= 3 ? p.cb + o : nullptr;
         uint8_t* ppa = NP == 4 ? pa + o : nullptr;
@@ -327,7 +364,12 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p, uin
                     packed[pl] = r0 | (r1 << 8) | (r2 << 16) | (r3 << 24);
                 }
             }
-            if (!y16) *reinterpret_cast<uint32_t*>(py) = packed[0];
+            if (NP == 2) {   // U0 V0 U1 V1 | U2 V2 U3 V3
+                reinterpret_cast<uint32_t*>(py)[0] = __byte_perm(packed[0], packed[1], 0x5140);
+                reinterpret_cast<uint32_t*>(py)[1] = __byte_perm(packed[0], packed[1], 0x7362);
+            } else if (!y16) {
+                *reinterpret_cast<uint32_t*>(py) = packed[0];
+            }
             py += ystep;
             if (NP >= 3) {
                 *reinterpret_cast<uint32_t*>(pcr) = packed[1];
@@ -391,6 +433,11 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p, uin
                             }
                             continue;
                         }
+                        if (NP == 2) {
+                            uint8_t* d = p.y + o + dx + pl;
+                            d[0] = (uint8_t)r0; d[2] = (uint8_t)r1; d[4] = (uint8_t)r2; d[6] = (uint8_t)r3;
+                            continue;
+                        }
                         uint8_t* outp = (pl == 0 ? p.y : (pl == 1 ? p.cr : (NP == 4 && pl == 3 ? pa : p.cb))) + o;
                         *reinterpret_cast<uint32_t*>(outp) = r0 | (r1 << 8) | (r2 << 16) | (r3 << 24);
                         continue;
@@ -413,6 +460,8 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p, uin
                                     for (int k = 1; k <= kY16Pad; k++) q16[-k] = e;
                                 if (dx + j == p.ow - 1)
                                     for (int k = 1; k <= 8; k++) q16[k] = e;
+                            } else if (NP == 2) {
+                                p.y[o + dx + 2 * j + pl] = (uint8_t)r;
                             } else {
                                 out[j] = (uint8_t)r;
                             }
@@ -425,7 +474,7 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p, uin
 }
 
 
-int launch_color_bicubic(Ctx* c, const ResizeArgs& a) {
+static ResizeDev resize_dev(const ResizeArgs& a) {
     ResizeDev p;
     p.src = a.src;
     p.src_stride = a.src_stride;
@@ -435,14 +484,23 @@ int launch_color_bicubic(Ctx* c, const ResizeArgs& a) {
     p.row_begin = a.row_begin; p.row_end = a.row_end;
     p.y = a.pl.y; p.cr = a.pl.cr; p.cb = a.pl.cb;
     p.pitch = a.pl.pitch;
-    p.y16 = nullptr; p.pitch16 = 0;
+    p.y16 = a.pl.y16; p.pitch16 = a.pl.pitch16;       // tiled kernel: the tcgen05 path's Y goes straight to the padded FP16 plane
     p.src_frame = a.src_frame_stride; p.plane_frame = a.pl.frame_stride; p.y16_frame = a.pl.frame_stride16;
-    const int nframes = std::max(1, a.nframes);
     p.plane_row0 = a.pl.row0;
     p.xofs = a.tx->d_ofs; p.xcoef = a.tx->d_coef;
     p.yofs = a.ty->d_ofs; p.ycoef = a.ty->d_coef;
     p.simd_w = (a.ow / 8) * 8;
     p.negzero2 = 0x8000000080000000ull;
+    p.quad_ok = 1;
+    return p;
+}
+
+static int launch_yuv420(Ctx* c, const ResizeArgs& a);
+
+int launch_color_bicubic(Ctx* c, const ResizeArgs& a) {
+    if (yuv420(a.order)) return launch_yuv420(c, a);
+    ResizeDev p = resize_dev(a);
+    const int nframes = std::max(1, a.nframes);
     const int rows = a.row_end - a.row_begin;
     if (rows <= 0) return SRCNN_OK;
 
@@ -453,7 +511,7 @@ int launch_color_bicubic(Ctx* c, const ResizeArgs& a) {
         int dx1 = std::min(dx0 + kTW, a.ow);
         if (a.tx->h_ofs[dx1 - 1] - a.tx->h_ofs[dx0] + 4 > kMaxSC) fits_x = false;
     }
-    const bool gray = a.order == SRCNN_ORDER_GRAY, four = four_channel(a.order);
+    const bool gray = a.order == SRCNN_ORDER_GRAY, four = four_channel(a.order), uv = a.order == kOrderUV;
     uint8_t* const pa = four ? a.pl.a : nullptr;
     const int max_rows = tiled_max_rows(four ? 4 : 3);
     auto fits_rows = [&](int th) {
@@ -464,19 +522,17 @@ int launch_color_bicubic(Ctx* c, const ResizeArgs& a) {
         return true;
     };
     const int th = !fits_x ? 0 : (fits_rows(64) ? 64 : (fits_rows(32) ? 32 : 0));
-    p.quad_ok = 1;
     for (int dx = 0; dx + 3 < a.ow && p.quad_ok; dx += 4)
         if (a.tx->h_ofs[dx + 3] - a.tx->h_ofs[dx] > 4) p.quad_ok = 0;
-    p.y16 = a.pl.y16; p.pitch16 = a.pl.pitch16;       // tiled kernel: the tcgen05 path's Y goes straight to the padded FP16 plane
-    if (c->ka_int) {                                  // x2 / x4: the integer-scale kernel (constant tap phases, no tables)
+    if (c->ka_int && !uv) {                           // x2 / x4: the integer-scale kernel (constant tap phases, no tables)
         bool done = false;
         const int rc = launch_color_bicubic_int(c, p, a, &done);
         if (rc || done) return rc;
     }
     if (th) {
         dim3 grid((a.ow + kTW - 1) / kTW, (rows + th - 1) / th, nframes);   // a batch of frames is one launch
-        if (th == 64) (gray ? k_color_bicubic_tiled<64, 1> : four ? k_color_bicubic_tiled<64, 4> : k_color_bicubic_tiled<64, 3>)<<<grid, 256, 0, c->stream>>>(p, pa);
-        else (gray ? k_color_bicubic_tiled<32, 1> : four ? k_color_bicubic_tiled<32, 4> : k_color_bicubic_tiled<32, 3>)<<<grid, 256, 0, c->stream>>>(p, pa);
+        if (th == 64) (gray ? k_color_bicubic_tiled<64, 1> : uv ? k_color_bicubic_tiled<64, 2> : four ? k_color_bicubic_tiled<64, 4> : k_color_bicubic_tiled<64, 3>)<<<grid, 256, 0, c->stream>>>(p, pa);
+        else (gray ? k_color_bicubic_tiled<32, 1> : uv ? k_color_bicubic_tiled<32, 2> : four ? k_color_bicubic_tiled<32, 4> : k_color_bicubic_tiled<32, 3>)<<<grid, 256, 0, c->stream>>>(p, pa);
         c->launches++;
         SRCNN_CUDA(c, cudaGetLastError());
         return SRCNN_OK;
@@ -486,10 +542,11 @@ int launch_color_bicubic(Ctx* c, const ResizeArgs& a) {
         ResizeDev q = p;
         q.src += (size_t)f * p.src_frame;
         q.y += (size_t)f * p.plane_frame;
-        if (!gray) { q.cr += (size_t)f * p.plane_frame; q.cb += (size_t)f * p.plane_frame; }
+        if (!gray && !uv) { q.cr += (size_t)f * p.plane_frame; q.cb += (size_t)f * p.plane_frame; }
         uint8_t* const qa = four ? pa + (size_t)f * p.plane_frame : nullptr;
         dim3 grid((a.ow + 31) / 32, (rows + 7) / 8);
-        (gray ? k_color_bicubic_direct<1> : four ? k_color_bicubic_direct<4> : k_color_bicubic_direct<3>)<<<grid, 256, 0, c->stream>>>(q, qa);
+        if (uv) k_chroma420_direct<<<grid, 256, 0, c->stream>>>(q, 1, 1, 2);
+        else (gray ? k_color_bicubic_direct<1> : four ? k_color_bicubic_direct<4> : k_color_bicubic_direct<3>)<<<grid, 256, 0, c->stream>>>(q, qa);
         c->launches++;
         SRCNN_CUDA(c, cudaGetLastError());
         if (a.pl.y16) {
@@ -498,6 +555,60 @@ int launch_color_bicubic(Ctx* c, const ResizeArgs& a) {
         }
     }
     return SRCNN_OK;
+}
+
+// A 4:2:0 frame (SRCNN_ORDER_NV12 / _I420).  x2 / x4 with ow/2 % 8 == 0 and 8-byte aligned chroma rows: one launch for luma and
+// chroma (color_bicubic_int.cu).  Otherwise the Y plane takes the grey instances and the chroma planes the generic ones, resized as
+// an image of their own straight into the caller's output: NV12's pairs as two interleaved planes (NP = 2), I420's U and V planes
+// as two frames of a one-plane launch (one launch for a single frame, one per plane for a batch).  Chroma rows of the output that
+// are not 4-byte aligned (the tiled kernel stores words) take k_chroma420_direct, one launch per frame for both planes.
+static int launch_yuv420(Ctx* c, const ResizeArgs& a) {
+    ResizeArgs y = a;
+    y.order = SRCNN_ORDER_GRAY;
+    if (c->ka_int) {
+        bool done = false;
+        const int rc = launch_yuv420_int(c, resize_dev(y), a, &done);
+        if (rc || done) return rc;
+    }
+    int rc = launch_color_bicubic(c, y);
+    if (rc) return rc;
+    const Chroma420& ch = a.ch;
+    const bool words = (((uintptr_t)ch.dst | ch.dst_pitch | ch.dst_v | ch.dst_frame) & 3) == 0;
+    ResizeArgs u;
+    u.src = ch.src; u.src_stride = ch.src_pitch;
+    u.sw = ch.sw; u.sh = ch.sh; u.src_row0 = 0; u.src_row1 = ch.sh;
+    u.ow = ch.ow; u.oh = ch.oh;
+    u.row_begin = ch.row_begin; u.row_end = ch.row_end;
+    u.pl.y = ch.dst; u.pl.pitch = ch.dst_pitch; u.pl.row0 = 0; u.pl.rows = ch.oh; u.pl.frame_stride = ch.dst_frame;
+    u.tx = ch.tx; u.ty = ch.ty;
+    u.nframes = a.nframes; u.src_frame_stride = a.src_frame_stride;
+    if (!words) {
+        if (ch.row_end <= ch.row_begin) return SRCNN_OK;
+        const bool nv12 = a.order == SRCNN_ORDER_NV12;
+        u.order = SRCNN_ORDER_GRAY;
+        for (int f = 0; f < std::max(1, a.nframes); f++) {
+            ResizeDev q = resize_dev(u);
+            q.src += (size_t)f * a.src_frame_stride;
+            q.y += (size_t)f * ch.dst_frame;
+            dim3 grid((ch.ow + 31) / 32, (ch.row_end - ch.row_begin + 7) / 8);
+            k_chroma420_direct<<<grid, 256, 0, c->stream>>>(q, nv12 ? 1 : ch.src_v, nv12 ? 1 : ch.dst_v, nv12 ? 2 : 1);
+            c->launches++;
+            SRCNN_CUDA(c, cudaGetLastError());
+        }
+        return SRCNN_OK;
+    }
+    if (a.order == SRCNN_ORDER_NV12) {
+        u.order = kOrderUV;
+        return launch_color_bicubic(c, u);
+    }
+    u.order = SRCNN_ORDER_GRAY;
+    if (std::max(1, a.nframes) == 1) {   // V is U's second frame
+        u.nframes = 2; u.src_frame_stride = ch.src_v; u.pl.frame_stride = ch.dst_v;
+        return launch_color_bicubic(c, u);
+    }
+    if ((rc = launch_color_bicubic(c, u))) return rc;
+    u.src += ch.src_v; u.pl.y += ch.dst_v;
+    return launch_color_bicubic(c, u);
 }
 
 // u8 Y plane -> padded FP16 plane (Planes::y16): 8 pixels per thread; the first / last group of a row also writes the

@@ -455,6 +455,245 @@ __global__ void __launch_bounds__(96, S == 2 ? SRCNN_KA_MINB : SRCNN_KA_MINB4) k
     walk_tile<S, kGPitch>(p, t, &sP[0][w * (kITW / S)], 0, tid & 31, X0 + w * kITW, a, nit, fz);
 }
 
+// The grey kernel's tile as a device function, for k_yuv420_bicubic_int below.  k_gray_bicubic_int keeps its own copy of these
+// lines: calling this function from it compiles to different SASS.
+template <int S>
+__device__ __forceinline__ void gray_tile(const ResizeDev& p, const IntTaps& t, int tile, uint8_t (&sP)[kIRows][kGPitch]) {
+    constexpr int GG = 3 * kITW / S / 4 + 2;       // four-byte groups per staged row
+    static_assert(4 * GG + 4 <= kGPitch, "staged row too short");
+    const int tid = threadIdx.x;
+    const int bx = tile % t.ntx, rest = tile / t.ntx;
+    const int by = rest % t.nty;
+    const size_t fz = (size_t)(rest / t.nty);
+    const int X0 = 3 * kITW * bx;                  // first column of warp 0's tile
+    const int a = t.a_first + by * t.isr;          // staged row r is source row a - 1 + r
+    const int F0 = X0 / S - 4;                     // first staged column (a multiple of 4)
+    const int nit = min(t.isr, t.i_last - a + 1);
+    const int nsr = nit + 3;
+    const uint8_t* const fsrc = p.src + fz * p.src_frame;
+
+    // (1) stage the footprint: all of a thread's loads go out before its first shared store
+    constexpr int NG = (kIRows * GG + 95) / 96;
+    uint32_t raw[NG];
+#pragma unroll
+    for (int it = 0; it < NG; it++) {
+        const int g = tid + 96 * it;
+        if (g < nsr * GG) {
+            const int r = g / GG, gx = F0 + 4 * (g - r * GG);
+            const uint8_t* row = fsrc + (size_t)(clampi(a - 1 + r, 0, p.sh - 1) - p.src_row0) * p.src_stride;
+            if (t.vec_ok && gx >= 0 && gx + 4 <= p.sw) {
+                raw[it] = *reinterpret_cast<const uint32_t*>(row + gx);
+            } else {
+                uint32_t v = 0;
+#pragma unroll
+                for (int j = 0; j < 4; j++) v |= (uint32_t)row[clampi(gx + j, 0, p.sw - 1)] << (8 * j);
+                raw[it] = v;
+            }
+        }
+    }
+#pragma unroll
+    for (int it = 0; it < NG; it++) {
+        const int g = tid + 96 * it;
+        if (g < nsr * GG) {
+            const int r = g / GG;
+            *reinterpret_cast<uint32_t*>(&sP[r][4 * (g - r * GG)]) = raw[it];
+        }
+    }
+    __syncthreads();
+    // (2) the walk: warp w's tile starts w * kITW / S staged columns further
+    const int w = tid >> 5;
+    walk_tile<S, kGPitch>(p, t, &sP[0][w * (kITW / S)], 0, tid & 31, X0 + w * kITW, a, nit, fz);
+}
+
+// ------------------------------------------------------------------------------------------------
+// 4:2:0 frames (SRCNN_ORDER_NV12 / _I420): ONE launch for luma and chroma.  CTAs [0, t.ntiles) are k_gray_bicubic_int's tiles
+// of the Y plane (into the workspace plane the CNN reads); the rest are chroma tiles, written straight into the caller's output
+// (no chroma workspace, no CNN).  A chroma CTA is three warps on three adjacent 128-column tiles whose footprints are staged
+// once, like the grey kernel's, as two shared-memory planes U and V: NV12's pairs are split with two byte permutations per
+// four columns, I420's planes are staged as they are.  A lane owns the SAME 4 columns of both planes, so the 8 horizontal
+// sums per footprint row, the four-row register window and the vertical pass are those of walk_tile (which gives a lane 8
+// columns of one plane); per output row it stores U0 V0 U1 V1 U2 V2 U3 V3 (NV12, one 8-byte store) or four bytes into each
+// plane (I420).  Launch conditions: ow/2 a multiple of 8, chroma rows of the output 8-byte aligned.
+// ------------------------------------------------------------------------------------------------
+#ifndef SRCNN_KA420_MINB
+#define SRCNN_KA420_MINB SRCNN_KA_MINB
+#endif
+#ifndef SRCNN_KA420_MINB4
+#define SRCNN_KA420_MINB4 SRCNN_KA_MINB4
+#endif
+
+struct ChromaDev {
+    const uint8_t* src;               // chroma row 0 of frame 0 (NV12: pairs; I420: U)
+    size_t src_pitch, src_v, src_frame;
+    uint8_t* dst;
+    size_t dst_pitch, dst_v, dst_frame;
+    int sw, sh, ow, row_begin, row_end;   // chroma plane sizes, chroma output rows wanted
+};
+constexpr int kCW = 128;           // chroma columns per warp: 4 per lane, of both planes
+template <int S>
+struct CGeo {
+    static constexpr int G = 3 * kCW / S / 4 + 2;                  // four-column groups per staged row
+    static constexpr int kPitch = (4 * G + 4 + 15) / 16 * 16;      // + the spare word of the window read
+};
+
+template <int S, bool kNV12>
+__device__ __forceinline__ void walk_pair(const ChromaDev& q, const IntTaps& t, unsigned long long nz, const uint8_t* su,
+                                          const uint8_t* sv, int lane, int X0, int a, int nit, size_t fz) {
+    constexpr int kPitch = CGeo<S>::kPitch;
+    const int x0 = X0 + 4 * lane;
+    if (x0 >= q.ow) return;                        // ow/2 is a multiple of 8 (launch condition)
+    const int cb = (4 * lane) / S + 2;             // footprint byte of the lane's first tap (x0 % S == 0)
+    const uint8_t* const ru = su + (cb & ~3);
+    const uint8_t* const rv = sv + (cb & ~3);
+    const int wsh = (cb & 3) * 8;
+    const unsigned long long mm = f2_pack(-kMagic, -kMagic);
+
+    auto hsum = [&](int r, unsigned long long (&h)[4]) {   // h[0], h[1]: U columns 0..3; h[2], h[3]: V columns 0..3
+        float f[8];
+#pragma unroll
+        for (int pl = 0; pl < 2; pl++) {
+            const uint32_t* w = reinterpret_cast<const uint32_t*>((pl ? rv : ru) + r * kPitch);
+            const uint32_t w0 = w[0], w1 = w[1], w2 = w[2];
+            const uint32_t lo = __funnelshift_r(w0, w1, wsh), hi = __funnelshift_r(w1, w2, wsh);
+#pragma unroll
+            for (int c = 0; c < 4; c++) {
+                const int o = win_ofs<S>(c);       // 0 .. 2
+                const uint32_t px4 = o == 0 ? lo : __funnelshift_r(lo, hi, 8 * o);
+                f[4 * pl + c] = __int_as_float(dp2a_hi_su(t.hk23[c % S], px4, dp2a_lo_su(t.hk01[c % S], px4, 0x4B400000)));
+            }
+        }
+#pragma unroll
+        for (int k = 0; k < 4; k++) h[k] = f2_add_rn(f2_pack(f[2 * k], f[2 * k + 1]), mm);
+    };
+
+    int dy = S * a + S / 2;
+    uint8_t* outp = q.dst + fz * q.dst_frame + (long long)dy * (long long)q.dst_pitch + (kNV12 ? 2 : 1) * (size_t)x0;
+    auto emit = [&](const unsigned long long (&h0)[4], const unsigned long long (&h1)[4], const unsigned long long (&h2)[4],
+                    const unsigned long long (&h3)[4]) {
+#pragma unroll
+        for (int m = 0; m < S; m++) {
+            const int ph = (S / 2 + m) % S;
+            const bool wanted = dy >= q.row_begin && dy < q.row_end;
+            uint32_t r[8];
+#pragma unroll
+            for (int k = 0; k < 4; k++) {
+                unsigned long long v = f2_mul_rn(h3[k], t.vb[ph][3], nz);
+                v = f2_add_rn(f2_mul_rn(h2[k], t.vb[ph][2], nz), v);
+                v = f2_add_rn(f2_mul_rn(h1[k], t.vb[ph][1], nz), v);
+                v = f2_add_rn(f2_mul_rn(h0[k], t.vb[ph][0], nz), v);
+                float va, vb;
+                f2_unpack(v, va, vb);
+                r[2 * k] = sat_u8_rn(va);
+                r[2 * k + 1] = sat_u8_rn(vb);
+            }
+            if (kNV12) {   // U0 V0 U1 V1 | U2 V2 U3 V3
+                const uint32_t lo = __byte_perm(__byte_perm(r[0], r[4], 0x0040), __byte_perm(r[1], r[5], 0x0040), 0x5410);
+                const uint32_t hi = __byte_perm(__byte_perm(r[2], r[6], 0x0040), __byte_perm(r[3], r[7], 0x0040), 0x5410);
+                if (wanted) *reinterpret_cast<uint2*>(outp) = make_uint2(lo, hi);
+            } else {
+                const uint32_t u = __byte_perm(__byte_perm(r[0], r[1], 0x0040), __byte_perm(r[2], r[3], 0x0040), 0x5410);
+                const uint32_t v = __byte_perm(__byte_perm(r[4], r[5], 0x0040), __byte_perm(r[6], r[7], 0x0040), 0x5410);
+                if (wanted) {
+                    *reinterpret_cast<uint32_t*>(outp) = u;
+                    *reinterpret_cast<uint32_t*>(outp + q.dst_v) = v;
+                }
+            }
+            dy++;
+            outp += q.dst_pitch;
+        }
+    };
+
+    unsigned long long hA[4], hB[4], hC[4], hD[4];
+    hsum(0, hA);
+    hsum(1, hB);
+    hsum(2, hC);
+    for (int tt = 0; tt < nit; tt += 4) {
+        hsum(tt + 3, hD);
+        emit(hA, hB, hC, hD);
+        if (tt + 1 >= nit) break;
+        hsum(tt + 4, hA);
+        emit(hB, hC, hD, hA);
+        if (tt + 2 >= nit) break;
+        hsum(tt + 5, hB);
+        emit(hC, hD, hA, hB);
+        if (tt + 3 >= nit) break;
+        hsum(tt + 6, hC);
+        emit(hD, hA, hB, hC);
+    }
+}
+
+template <int S, bool kNV12>
+__device__ __forceinline__ void chroma_tile(const ChromaDev& q, const IntTaps& t, unsigned long long nz, int tile, uint8_t* smem) {
+    constexpr int G = CGeo<S>::G, kPitch = CGeo<S>::kPitch;
+    uint8_t (*sU)[kPitch] = reinterpret_cast<uint8_t (*)[kPitch]>(smem);
+    uint8_t (*sV)[kPitch] = sU + kIRows;
+    const int tid = threadIdx.x;
+    const int bx = tile % t.ntx, rest = tile / t.ntx;
+    const int by = rest % t.nty;
+    const size_t fz = (size_t)(rest / t.nty);
+    const int X0 = 3 * kCW * bx;                   // first chroma column of warp 0's tile
+    const int a = t.a_first + by * t.isr;          // staged row r is chroma source row a - 1 + r
+    const int F0 = X0 / S - 4;                     // first staged column (a multiple of 4)
+    const int nit = min(t.isr, t.i_last - a + 1);
+    const int nsr = nit + 3;
+    const uint8_t* const fsrc = q.src + fz * q.src_frame;
+
+    // (1) stage both footprints: all of a thread's loads go out before its first shared store
+    constexpr int NG = (kIRows * G + 95) / 96;
+    uint32_t ru[NG], rv[NG];
+#pragma unroll
+    for (int it = 0; it < NG; it++) {
+        const int g = tid + 96 * it;
+        if (g < nsr * G) {
+            const int r = g / G, gx = F0 + 4 * (g - r * G);
+            const uint8_t* row = fsrc + (size_t)clampi(a - 1 + r, 0, q.sh - 1) * q.src_pitch;
+            if (t.vec_ok && gx >= 0 && gx + 4 <= q.sw) {
+                if (kNV12) {
+                    const uint32_t* w = reinterpret_cast<const uint32_t*>(row + 2 * gx);
+                    const uint32_t w0 = w[0], w1 = w[1];
+                    ru[it] = __byte_perm(w0, w1, 0x6420);
+                    rv[it] = __byte_perm(w0, w1, 0x7531);
+                } else {
+                    ru[it] = *reinterpret_cast<const uint32_t*>(row + gx);
+                    rv[it] = *reinterpret_cast<const uint32_t*>(row + q.src_v + gx);
+                }
+            } else {
+                uint32_t u = 0, v = 0;
+#pragma unroll
+                for (int j = 0; j < 4; j++) {
+                    const int x = clampi(gx + j, 0, q.sw - 1);
+                    u |= (uint32_t)(kNV12 ? row[2 * x] : row[x]) << (8 * j);
+                    v |= (uint32_t)(kNV12 ? row[2 * x + 1] : row[q.src_v + x]) << (8 * j);
+                }
+                ru[it] = u;
+                rv[it] = v;
+            }
+        }
+    }
+#pragma unroll
+    for (int it = 0; it < NG; it++) {
+        const int g = tid + 96 * it;
+        if (g < nsr * G) {
+            const int r = g / G, o = 4 * (g - r * G);
+            *reinterpret_cast<uint32_t*>(&sU[r][o]) = ru[it];
+            *reinterpret_cast<uint32_t*>(&sV[r][o]) = rv[it];
+        }
+    }
+    __syncthreads();
+    // (2) the walk: warp w's tile starts w * kCW / S staged columns further
+    const int w = tid >> 5;
+    walk_pair<S, kNV12>(q, t, nz, &sU[0][w * (kCW / S)], &sV[0][w * (kCW / S)], tid & 31, X0 + w * kCW, a, nit, fz);
+}
+
+template <int S, bool kNV12>
+__global__ void __launch_bounds__(96, S == 2 ? SRCNN_KA420_MINB : SRCNN_KA420_MINB4) k_yuv420_bicubic_int(const ResizeDev p, const IntTaps t,
+                                                                                                        const ChromaDev q, const IntTaps tc) {
+    constexpr int kLuma = kIRows * kGPitch, kChroma = 2 * kIRows * CGeo<S>::kPitch;
+    __shared__ __align__(16) uint8_t sm[kLuma > kChroma ? kLuma : kChroma];
+    if ((int)blockIdx.x < t.ntiles) gray_tile<S>(p, t, blockIdx.x, *reinterpret_cast<uint8_t (*)[kIRows][kGPitch]>(sm));
+    else chroma_tile<S, kNV12>(q, tc, p.negzero2, (int)blockIdx.x - t.ntiles, sm);
+}
+
 inline int floordiv(int a, int b) { return a >= 0 ? a / b : -((-a + b - 1) / b); }
 
 // one launch of an integer-scale kernel, ordinary or with programmatic stream serialisation
@@ -509,7 +748,79 @@ int launch_variant(Ctx* c, const ResizeDev& p, IntTaps& t, uint8_t* pa, int nfra
     return launch_ka(c, NP == 1 ? k_gray_bicubic_int<S> : k_color_bicubic_int<S>, t.ntiles, kThreads, early, p, t);
 }
 
+// the constant tap phases of an integer scale S and the source rows whose output rows [row_begin, row_end) are wanted
+void int_taps(const TapTable* tx, const TapTable* ty, int S, int row_begin, int row_end, IntTaps& t) {
+    const float sc = 1.0f / 4194304.0f;   // 2^-22, exact
+    for (int k = 0; k < 4; k++) {
+        const short4 cx = tx->h_coef[k % S], cy = ty->h_coef[k % S];
+        t.hk01[k] = (uint32_t)(unsigned short)cx.x | ((uint32_t)(unsigned short)cx.y << 16);
+        t.hk23[k] = (uint32_t)(unsigned short)cx.z | ((uint32_t)(unsigned short)cx.w << 16);
+        const float b[4] = {(float)cy.x * sc, (float)cy.y * sc, (float)cy.z * sc, (float)cy.w * sc};
+        for (int j = 0; j < 4; j++) {
+            uint32_t u;
+            memcpy(&u, &b[j], 4);
+            t.vb[k][j] = (unsigned long long)u | ((unsigned long long)u << 32);
+        }
+    }
+    t.a_first = floordiv(row_begin - S / 2, S);
+    t.i_last = floordiv(row_end - 1 - S / 2, S);
+}
+
 }  // namespace
+
+int launch_yuv420_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bool* done) {
+    *done = false;
+    const Chroma420& ch = a.ch;
+    const int S = a.tx->int_scale;
+    if (S == 0 || a.ty->int_scale != S || ch.tx->int_scale != S || ch.ty->int_scale != S) return SRCNN_OK;
+    if ((a.ow & 7) || (ch.ow & 7) || a.row_end <= a.row_begin || ch.row_end <= ch.row_begin) return SRCNN_OK;
+    // stores: luma as in a grey call; chroma 8 bytes (NV12) or 2 x 4 bytes (I420) per lane and row, 8-byte aligned chroma rows
+    if ((((uintptr_t)p.y | p.pitch | p.plane_frame) & 7) != 0) return SRCNN_OK;
+    if (p.y16 && (((uintptr_t)p.y16 | p.pitch16 | p.y16_frame) & 15) != 0) return SRCNN_OK;
+    if ((((uintptr_t)ch.dst | ch.dst_pitch | ch.dst_v | ch.dst_frame) & 7) != 0) return SRCNN_OK;
+    const bool nv12 = a.order == SRCNN_ORDER_NV12;
+    const int nframes = std::max(1, a.nframes);
+
+    IntTaps t = {}, tc = {};
+    int_taps(a.tx, a.ty, S, a.row_begin, a.row_end, t);
+    int_taps(ch.tx, ch.ty, S, ch.row_begin, ch.row_end, tc);
+    t.vec_ok = (((uintptr_t)p.src | p.src_stride | p.src_frame) & 3) == 0;
+    tc.vec_ok = (((uintptr_t)ch.src | ch.src_pitch | ch.src_v | p.src_frame) & 3) == 0;
+    t.ntx = ((a.ow + kITW - 1) / kITW + 2) / 3;    // a CTA per three adjacent tiles, as in a grey call
+    tc.ntx = (ch.ow + 3 * kCW - 1) / (3 * kCW);
+    auto kern = S == 2 ? (nv12 ? k_yuv420_bicubic_int<2, true> : k_yuv420_bicubic_int<2, false>)
+                       : (nv12 ? k_yuv420_bicubic_int<4, true> : k_yuv420_bicubic_int<4, false>);
+    static int ctas_per_sm[4][64] = {};            // per instance and device; a benign race: every writer stores the same value
+    int& per_sm = ctas_per_sm[(S == 4) * 2 + nv12][c->device & 63];
+    if (per_sm == 0) {
+        int n = 0;
+        SRCNN_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kern, 96, 0));
+        per_sm = std::max(1, n);
+    }
+    // tile height: the rule of launch_variant over the launch's luma and chroma tiles together
+    const int resident = per_sm * std::max(1, c->sm_count);
+    const int nrows = t.i_last - t.a_first + 1, crows = tc.i_last - tc.a_first + 1;
+    auto tiles_for = [&](int isr) {
+        return ((long long)t.ntx * ((nrows + isr - 1) / isr) + (long long)tc.ntx * ((crows + isr - 1) / isr)) * nframes;
+    };
+    t.isr = tiles_for(kISRMax) > 2LL * resident ? kISRMax : 8;
+    if (c->ka_int_isr >= 4 && c->ka_int_isr <= kISRMax) t.isr = c->ka_int_isr;
+    tc.isr = t.isr;
+    if (tiles_for(t.isr) > 0x3fffffffLL) return SRCNN_OK;
+    t.nty = (nrows + t.isr - 1) / t.isr;
+    tc.nty = (crows + tc.isr - 1) / tc.isr;
+    t.ntiles = t.ntx * t.nty * nframes;
+    tc.ntiles = tc.ntx * tc.nty * nframes;
+    ChromaDev q;
+    q.src = ch.src; q.src_pitch = ch.src_pitch; q.src_v = ch.src_v; q.src_frame = p.src_frame;
+    q.dst = ch.dst; q.dst_pitch = ch.dst_pitch; q.dst_v = ch.dst_v; q.dst_frame = ch.dst_frame;
+    q.sw = ch.sw; q.sh = ch.sh; q.ow = ch.ow; q.row_begin = ch.row_begin; q.row_end = ch.row_end;
+    // never early: a 4:2:0 call launches no merge (api.cu)
+    const int rc = launch_ka(c, kern, t.ntiles + tc.ntiles, 96, false, p, t, q, tc);
+    if (rc) return rc;
+    *done = true;
+    return SRCNN_OK;
+}
 
 int launch_color_bicubic_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bool* done) {
     *done = false;
@@ -522,23 +833,10 @@ int launch_color_bicubic_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bo
     if (p.y16 && (((uintptr_t)p.y16 | p.pitch16 | p.y16_frame) & 15) != 0) return SRCNN_OK;
 
     IntTaps t;
-    const float sc = 1.0f / 4194304.0f;   // 2^-22, exact
-    for (int k = 0; k < 4; k++) {
-        const short4 cx = a.tx->h_coef[k % S], cy = a.ty->h_coef[k % S];
-        t.hk01[k] = (uint32_t)(unsigned short)cx.x | ((uint32_t)(unsigned short)cx.y << 16);
-        t.hk23[k] = (uint32_t)(unsigned short)cx.z | ((uint32_t)(unsigned short)cx.w << 16);
-        const float b[4] = {(float)cy.x * sc, (float)cy.y * sc, (float)cy.z * sc, (float)cy.w * sc};
-        for (int j = 0; j < 4; j++) {
-            uint32_t u;
-            memcpy(&u, &b[j], 4);
-            t.vb[k][j] = (unsigned long long)u | ((unsigned long long)u << 32);
-        }
-    }
+    int_taps(a.tx, a.ty, S, a.row_begin, a.row_end, t);
     // three words = bytes c0 c1 c2 of pixels 0..3; pixel word = (B, G, R, x): B is c0 for BGR input, c2 for RGB input
     if (p.swapRB) { t.sel[0] = 0x3012; t.sel[1] = 0x6345; t.sel[2] = 0x5234; t.sel[3] = 0x0123; }
     else          { t.sel[0] = 0x3210; t.sel[1] = 0x6543; t.sel[2] = 0x5432; t.sel[3] = 0x0321; }
-    t.a_first = floordiv(a.row_begin - S / 2, S);
-    t.i_last = floordiv(a.row_end - 1 - S / 2, S);
     t.vec_ok = (((uintptr_t)p.src | p.src_stride | p.src_frame) & 3) == 0;
     if (four && t.vec_ok && (((uintptr_t)p.src | p.src_stride | p.src_frame) & 15) == 0) t.vec_ok = 2;   // 128-bit group loads
     const int nframes = std::max(1, a.nframes);

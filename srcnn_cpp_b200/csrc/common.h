@@ -193,6 +193,25 @@ void build_cubic_taps(int src, int dst, int* ofs, short4* coef);
 inline size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 // ---- kernel launchers (each enqueues on c->stream and bumps c->launches) ---------------------------
+inline bool yuv420(int order) { return order == SRCNN_ORDER_NV12 || order == SRCNN_ORDER_I420; }
+// internal order of the resize kernels: two interleaved one-byte planes (NV12's chroma pairs), resized plane by plane into pl.y,
+// written interleaved
+constexpr int kOrderUV = 100;
+
+// The chroma planes of 4:2:0 frames (SRCNN_ORDER_NV12 / _I420): resized, no CNN, straight into the caller's output.
+struct Chroma420 {
+    const uint8_t* src = nullptr;   // chroma row 0 of frame 0 (NV12: the interleaved pairs, I420: the U plane)
+    size_t src_pitch = 0;           // bytes between chroma rows
+    size_t src_v = 0;               // I420: V plane - U plane
+    uint8_t* dst = nullptr;         // the same in the output
+    size_t dst_pitch = 0, dst_v = 0;
+    size_t dst_frame = 0;           // output frame stride (the source's is ResizeArgs::src_frame_stride)
+    int sw = 0, sh = 0, ow = 0, oh = 0;   // chroma plane sizes: w/2, h/2, ow/2, oh/2
+    int row_begin = 0, row_end = 0;       // chroma output rows to produce: [r0/2, r1/2) of the luma rows [r0, r1)
+    const TapTable* tx = nullptr;
+    const TapTable* ty = nullptr;
+};
+
 struct ResizeArgs {
     const uint8_t* src;   // points at source row `src_row0`
     size_t src_stride;
@@ -207,9 +226,11 @@ struct ResizeArgs {
     int nframes = 1;      // same-sized frames in one launch, src_frame_stride / pl.frame_stride apart
     size_t src_frame_stride = 0;
     bool early = false;   // may start while the previous kernel of the stream (a merge kernel of ours) is still running
+    Chroma420 ch;         // SRCNN_ORDER_NV12 / _I420: the chroma planes (the Y plane is `src`, as for a grey call)
 };
 int launch_color_bicubic(Ctx* c, const ResizeArgs& a);   // order SRCNN_ORDER_GRAY: the one plane, into pl.y / pl.y16;
-                                                         // SRCNN_ORDER_BGRA / _RGBA: pl.a as well
+                                                         // SRCNN_ORDER_BGRA / _RGBA: pl.a as well;
+                                                         // SRCNN_ORDER_NV12 / _I420: Y into pl.y / pl.y16, chroma per `ch`
 inline bool four_channel(int order) { return order == SRCNN_ORDER_BGRA || order == SRCNN_ORDER_RGBA; }
 
 struct MergeArgs {
