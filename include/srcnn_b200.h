@@ -41,6 +41,18 @@
  * the Y plane as it is (limited or full range), and chroma takes cv::resize's centre-aligned grid, so left-sited (MPEG-2 /
  * H.264) chroma gets the quarter-pixel horizontal shift any centre-aligned resize gives -- not compensated.  Whole-frame calls
  * only: the band calls (srcnn_process_band_*, srcnn_mgpu_process_banded_*) return SRCNN_E_ARG for these orders.
+ * SRCNN_ORDER_YUY2 / SRCNN_ORDER_UYVY: packed 4:2:2 -- what V4L2 (YUYV), DeckLink (2vuy), Media Foundation (YUY2 / UYVY),
+ * FFmpeg (yuyv422 / uyvy422) and OpenCV's CV_8UC2 frames for COLOR_YUV2BGR_YUY2 / _UYVY hold.  A frame of w x h pixels is h rows
+ * of 2*w bytes, `stride` bytes apart: w/2 four-byte macropixels Y0 U Y1 V (YUY2) or U Y0 V Y1 (UYVY) per row.  The output has
+ * the same layout with ow, oh, dst_stride.  w and ow must be even (h and oh need not be), stride >= 2*w, dst_stride >= 2*ow,
+ * batch frame strides >= stride*h (dst_stride*oh); any alignment (unaligned buffers may take slower kernels).  Byte for byte:
+ * the output's Y plane is the SRCNN_ORDER_GRAY call on the source's Y plane; each output chroma plane (ow/2 x oh) is
+ * resize(plane, Size(ow/2, oh), INTER_CUBIC) of the matching source plane (w/2 x h) -- exactly srcnn_stage_resize_plane_device
+ * on it, no CNN.  U and V are resized as two planes, not as one CV_8UC2 image (see NV12 above).  No colour matrix is applied: the
+ * network sees Y as it is (limited or full range).  Chroma takes cv::resize's centre-aligned grid; 4:2:2 chroma is co-sited
+ * with the even luma samples, so it gets the quarter-pixel horizontal shift any centre-aligned resize gives -- not compensated.
+ * The planes are treated independently, so YVYU and VYUY (V before U) are the same two orders.  Chroma has the full vertical
+ * resolution, so every whole-path call takes these orders, the band calls and srcnn_mgpu_process_banded_* included.
  * Output size is ow=(int)((float)w*scale), oh=(int)((float)h*scale) -- the reference's truncation (src/srcnn.cpp:573-575,
  * src/test.cpp:357-358).
  */
@@ -70,7 +82,7 @@ enum {
 
 /* 5 is not assigned: it has been rejected as an unknown order since the four-channel orders were added, and stays so. */
 enum { SRCNN_ORDER_BGR = 0, SRCNN_ORDER_RGB = 1, SRCNN_ORDER_GRAY = 2, SRCNN_ORDER_BGRA = 3, SRCNN_ORDER_RGBA = 4,
-       SRCNN_ORDER_NV12 = 6, SRCNN_ORDER_I420 = 7 };
+       SRCNN_ORDER_NV12 = 6, SRCNN_ORDER_I420 = 7, SRCNN_ORDER_YUY2 = 8, SRCNN_ORDER_UYVY = 9 };
 
 /* Status codes.  -1 / -2 / -3 / -10 keep the reference CLI's meanings (src/srcnn.cpp:479,493,526,555,684). */
 enum {
@@ -222,7 +234,7 @@ void srcnn_jpeg_free(uint8_t* p);
 
 /* ---- stages (device pointers; enqueued on the context stream) ------------------------------------ */
 /* cvtColor + split + 3x resize (src/srcnn.cpp:509,540,570-583): BGR8 -> three u8 planes of ow x oh.  Colour orders only
- * (SRCNN_ORDER_GRAY, _BGRA, _RGBA: SRCNN_E_ARG; srcnn_stage_resize_plane_device is the one-plane stage). */
+ * (SRCNN_ORDER_GRAY, _BGRA, _RGBA, the 4:2:0 and 4:2:2 orders: SRCNN_E_ARG; srcnn_stage_resize_plane_device is the one-plane stage). */
 int srcnn_stage_color_bicubic_device(srcnn_ctx* ctx, const uint8_t* d_src, int w, int h, size_t src_stride,
                                      int order, float scale, uint8_t* d_y, uint8_t* d_cr, uint8_t* d_cb,
                                      size_t plane_pitch);

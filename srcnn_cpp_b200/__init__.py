@@ -25,6 +25,8 @@ ORDER_BGRA = 3   # four channels, straight alpha in byte 3: HxWx4 (NxHxWx4) in a
 ORDER_RGBA = 4   # alpha = the one-plane cubic resize of the alpha plane (no CNN)
 ORDER_NV12 = 6   # packed 4:2:0 video frames: (H*3/2)xW ((N)x(H*3/2)xW) arrays and tensors in and out; Y plane = the grey call's,
 ORDER_I420 = 7   # chroma planes = the one-plane cubic resize of the source's (no CNN).  yuv420_planes() splits a frame
+ORDER_YUY2 = 8   # packed 4:2:2 (bytes Y0 U Y1 V / U Y0 V Y1): HxWx2 (NxHxWx2) arrays and tensors in and out, OpenCV's CV_8UC2 shape;
+ORDER_UYVY = 9   # Y plane = the grey call's, U / V = the one-plane cubic resize of the source's.  yuv422_planes() splits a frame
 
 OK = 0
 E_RATIO = -1
@@ -183,10 +185,12 @@ class PinnedBuffer:
 
 
 def _pixel_shape(order):
-    """trailing shape of one pixel: () for ORDER_GRAY and the 4:2:0 orders, (4,) for ORDER_BGRA / ORDER_RGBA, (3,) for the colour
-    orders"""
+    """trailing shape of one pixel: () for ORDER_GRAY and the 4:2:0 orders, (4,) for ORDER_BGRA / ORDER_RGBA, (2,) for the 4:2:2
+    orders, (3,) for the colour orders"""
     if order in (ORDER_GRAY, ORDER_NV12, ORDER_I420):
         return ()
+    if order in (ORDER_YUY2, ORDER_UYVY):
+        return (2,)
     return (4,) if order in (ORDER_BGRA, ORDER_RGBA) else (3,)
 
 
@@ -229,6 +233,18 @@ def yuv420_planes(frame, order):
     flat = np.lib.stride_tricks.as_strided(frame, shape=(second + (h // 2) * (s // 2),), strides=(1,))
     as_plane = lambda k: np.lib.stride_tricks.as_strided(flat[k:], shape=shape, strides=(s // 2, 1))
     return y, as_plane(first), as_plane(second)
+
+
+def yuv422_planes(frame, order):
+    """(Y, U, V) views of one packed 4:2:2 frame: an HxWx2 uint8 numpy array or torch tensor (W even; rows may be padded).  Y is
+    HxW (byte 0 of each pixel with ORDER_YUY2, byte 1 with ORDER_UYVY), U and V are HxW/2 (bytes 1 / 3 of each 4-byte macropixel
+    with ORDER_YUY2, bytes 0 / 2 with ORDER_UYVY).  Strided views of the frame's memory, not copies."""
+    if order not in (ORDER_YUY2, ORDER_UYVY) or len(frame.shape) != 3 or frame.shape[2] != 2 or frame.shape[1] % 2:
+        raise SrcnnError(E_ARG, "expected one HxWx2 frame with an even W and ORDER_YUY2 / ORDER_UYVY")
+    y_byte, u_byte = (0, 1) if order == ORDER_YUY2 else (1, 0)
+    mp = frame[:, 0::2, :]                       # H x W/2 x 2: the first two bytes of each macropixel
+    mq = frame[:, 1::2, :]                       # ... and the last two
+    return frame[:, :, y_byte], mp[:, :, u_byte], mq[:, :, u_byte]
 
 
 def _check_host_image(a, order, lead):
@@ -307,8 +323,8 @@ class Engine:
     # -- whole path, host buffers (numpy) ----------------------------------------------------------
     def process(self, img, scale, order=ORDER_BGR, out=None):
         """img: HxWx3 uint8 numpy array (BGR by default, like cv::imread), HxW with order=ORDER_GRAY, HxWx4 with
-        order=ORDER_BGRA / ORDER_RGBA, or an (H*3/2)xW frame with ORDER_NV12 / ORDER_I420.  Returns OHxOWx3 (OHxOW, OHxOWx4,
-        (OH*3/2)xOW) uint8."""
+        order=ORDER_BGRA / ORDER_RGBA, an (H*3/2)xW frame with ORDER_NV12 / ORDER_I420, or HxWx2 with ORDER_YUY2 / ORDER_UYVY.
+        Returns OHxOWx3 (OHxOW, OHxOWx4, (OH*3/2)xOW, OHxOWx2) uint8."""
         img = np.asarray(img)
         _check_host_image(img, order, 1)
         if not img.flags.c_contiguous:
@@ -338,7 +354,8 @@ class Engine:
     # -- whole path, device buffers (torch CUDA tensors) -------------------------------------------
     def process_device(self, src, scale, dst, order=ORDER_BGR):
         """src: HxWx3 (HxW with order=ORDER_GRAY, HxWx4 with ORDER_BGRA / ORDER_RGBA) uint8 device tensor; dst: OHxOWx3
-        (OHxOW, OHxOWx4); (H*3/2)xW and (OH*3/2)xOW frames with ORDER_NV12 / ORDER_I420."""
+        (OHxOW, OHxOWx4); (H*3/2)xW and (OH*3/2)xOW frames with ORDER_NV12 / ORDER_I420; HxWx2 and OHxOWx2 with ORDER_YUY2 /
+        ORDER_UYVY."""
         h, w = _frame_h(order, src.shape[0]), src.shape[1]
         self._check(self.L.srcnn_process_device(self.ctx, _dptr(src), w, h, src.stride(0), order, C.c_float(scale),
                                                 _dptr(dst), dst.stride(0)))

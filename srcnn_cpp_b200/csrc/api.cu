@@ -66,8 +66,10 @@ static int scaled_dim(int n, float scale) {
     return (int)((float)n * scale);
 }
 
-// bytes per pixel of a row (4:2:0: of a Y row; a chroma row of NV12 has as many, an I420 chroma row half as many)
-static size_t bytes_per_pixel(int order) { return order == SRCNN_ORDER_GRAY || yuv420(order) ? 1 : (four_channel(order) ? 4 : 3); }
+// bytes per pixel of a row (4:2:0: of a Y row; a chroma row of NV12 has as many, an I420 chroma row half as many; packed 4:2:2: 2)
+static size_t bytes_per_pixel(int order) {
+    return order == SRCNN_ORDER_GRAY || yuv420(order) ? 1 : (yuv422(order) ? 2 : (four_channel(order) ? 4 : 3));
+}
 // rows of one frame in memory (4:2:0: h rows of Y, then h/2 rows of NV12 pairs or of I420 U and V)
 static size_t frame_rows(int order, int h) { return yuv420(order) ? (size_t)h / 2 * 3 : (size_t)h; }
 
@@ -76,11 +78,13 @@ static int check_image(Ctx* c, const void* src, int w, int h, size_t stride, int
     if (!c) return SRCNN_E_ARG;
     if (!src || !dst) return fail(c, SRCNN_E_ARG, "null image pointer");
     if (w <= 0 || h <= 0) return fail(c, SRCNN_E_ARG, "non-positive image size %dx%d", w, h);
-    if (order != SRCNN_ORDER_BGR && order != SRCNN_ORDER_RGB && order != SRCNN_ORDER_GRAY && !four_channel(order) && !yuv420(order))
+    if (order != SRCNN_ORDER_BGR && order != SRCNN_ORDER_RGB && order != SRCNN_ORDER_GRAY && !four_channel(order) && !yuv420(order) &&
+        !yuv422(order))
         return fail(c, SRCNN_E_ARG, "unknown pixel order %d", order);
     const size_t bpp = bytes_per_pixel(order);
     if (stride < (size_t)w * bpp) return fail(c, SRCNN_E_ARG, "source stride %zu < %zu*w", stride, bpp);
     if (yuv420(order) && ((w | h) & 1)) return fail(c, SRCNN_E_ARG, "4:2:0 frames need an even width and height, got %dx%d", w, h);
+    if (yuv422(order) && (w & 1)) return fail(c, SRCNN_E_ARG, "4:2:2 frames need an even width (whole macropixels), got %d", w);
     if (order == SRCNN_ORDER_I420 && ((stride | dst_stride) & 1))
         return fail(c, SRCNN_E_ARG, "I420 strides must be even (chroma rows are stride/2 apart), got %zu / %zu", stride, dst_stride);
     // src/srcnn.cpp:485-495 "ratio too small"
@@ -90,6 +94,8 @@ static int check_image(Ctx* c, const void* src, int w, int h, size_t stride, int
     if (*ow <= 0 || *oh <= 0) return fail(c, SRCNN_E_RATIO, "scale %g gives an empty image", scale);
     if (yuv420(order) && ((*ow | *oh) & 1))
         return fail(c, SRCNN_E_ARG, "scale %g gives an odd 4:2:0 output size %dx%d (width and height must be even)", scale, *ow, *oh);
+    if (yuv422(order) && (*ow & 1))
+        return fail(c, SRCNN_E_ARG, "scale %g gives an odd 4:2:2 output width %d (whole macropixels: it must be even)", scale, *ow);
     if (dst_stride < (size_t)*ow * bpp) return fail(c, SRCNN_E_ARG, "destination stride %zu < %zu*ow", dst_stride, bpp);
     return SRCNN_OK;
 }
@@ -116,6 +122,25 @@ static int chroma_planes(Ctx* c, int order, const uint8_t* src, int w, int h, si
     return SRCNN_OK;
 }
 
+// The chroma planes of packed 4:2:2 frames whose row 0 is at `src` (frame 0), for the output rows [r0, r1): U' and V' go into the
+// Cr / Cb planes of `pl` (its first ow/2 columns), which the pack kernel reads for the same rows.  No halo: chroma has no CNN.
+static int chroma_planes422(Ctx* c, const uint8_t* src, int w, int h, size_t src_stride, const Planes& pl, int ow, int oh, int r0,
+                            int r1, Chroma420* ch) {
+    TapTable *tx, *ty;
+    int rc = get_taps(c, w / 2, ow / 2, &tx);
+    if (rc) return rc;
+    if ((rc = get_taps(c, h, oh, &ty))) return rc;
+    ch->src = src; ch->src_pitch = src_stride; ch->src_v = 0;
+    ch->dst = pl.cr - (ptrdiff_t)pl.row0 * (ptrdiff_t)pl.pitch;   // chroma output row r at dst + r * pitch
+    ch->dst_pitch = pl.pitch;
+    ch->dst_v = (size_t)(pl.cb - pl.cr);
+    ch->dst_frame = pl.frame_stride;
+    ch->sw = w / 2; ch->sh = h; ch->ow = ow / 2; ch->oh = oh;
+    ch->row_begin = r0; ch->row_end = r1;
+    ch->tx = tx; ch->ty = ty;
+    return SRCNN_OK;
+}
+
 // planes of `nframes` same-sized frames: [Y frames][Cr frames][Cb frames][Y' frames][FP16 Y frames], and for a four-channel
 // call [A frames] after them (so the colour and grey layouts do not depend on it)
 // Cross-call overlap: the only planes the colour+bicubic kernel of call i+1 writes AND the merge kernel of call i reads are Cr and
@@ -125,7 +150,8 @@ static int chroma_planes(Ctx* c, int order, const uint8_t* src, int w, int h, si
 // set this call got.  Keeping the rest single also keeps the planes L2-resident from step to step: two whole plane sets (116 MB
 // at 4K) measured 3 us slower in the colour+bicubic kernel.
 // The host-buffer pipeline keeps to set 0 (its sub-bands are separated by copies and events anyway).  A grey or 4:2:0 call has no
-// Cr/Cb planes: it leaves the set selection alone (and ends the early-start chain, end_merge_chain).
+// Cr/Cb planes: it leaves the set selection alone (and ends the early-start chain, end_merge_chain).  A packed 4:2:2 call keeps its
+// U' / V' planes in the Cr / Cb slots and so takes part like a colour call.
 static int carve_planes(Ctx* c, int ow, int rows, int row0, Planes* pl, int nframes = 1, int order = SRCNN_ORDER_BGR) {
     const bool gray = order == SRCNN_ORDER_GRAY || yuv420(order), four = four_channel(order);
     const size_t pitch = align_up((size_t)ow, 128);
@@ -246,6 +272,9 @@ static int process_rows_impl(Ctx* c, const uint8_t* d_src, int w, int h, size_t 
     if (yuv420(order) && (rc = chroma_planes(c, order, d_src - (size_t)s0 * src_stride, w, h, src_stride, d_dst - (size_t)r0 * dst_stride,
                                              ow, oh, dst_stride, 0, r0, r1, &ra.ch)))
         return rc;
+    // 4:2:2: chroma rows [r0, r1) only (the pack kernel's); the luma halo rows [p0, r0) and [r1, p1) are the CNN's
+    if (yuv422(order) && (rc = chroma_planes422(c, d_src - (size_t)s0 * src_stride, w, h, src_stride, pl, ow, oh, r0, r1, &ra.ch)))
+        return rc;
     if (c->variant != SRCNN_VARIANT_TC) ra.pl.y16 = nullptr;      // the strict FP32 kernels read the u8 plane
     ra.early = !gray && may_start_early(c, d_src, (size_t)(s1 - s0) * src_stride);
     c->early_launches += ra.early;
@@ -265,8 +294,8 @@ static int process_rows_impl(Ctx* c, const uint8_t* d_src, int w, int h, size_t 
     else { ca.out = pl.yout; ca.out_pitch = pl.pitch; ca.out_row0 = p0; }
     // optionally the row-walking tcgen05 kernel merges Cr/Cb and converts back to BGR in its last epilogue (no Y' plane, no
     // K-C launch); measured slower than the separate launch (byte stores from one-thread-per-column lanes), so off by default
-    // (colour orders only: a four-channel call takes the separate merge, which writes alpha too)
-    const bool fused = !gray && !four_channel(order) && c->variant == SRCNN_VARIANT_TC && c->fuse_merge;
+    // (colour orders only: a four-channel call takes the separate merge, which writes alpha too; a 4:2:2 call its pack kernel)
+    const bool fused = (order == SRCNN_ORDER_BGR || order == SRCNN_ORDER_RGB) && c->variant == SRCNN_VARIANT_TC && c->fuse_merge;
     if (fused) {
         ca.cr = pl.cr; ca.cb = pl.cb;
         ca.bgr = d_dst; ca.bgr_stride = dst_stride; ca.order = order;
@@ -284,7 +313,7 @@ static int process_rows_impl(Ctx* c, const uint8_t* d_src, int w, int h, size_t 
     ma.pitch = pl.pitch; ma.w = ow; ma.rows = r1 - r0;
     ma.order = order;
     ma.dst = d_dst; ma.dst_stride = dst_stride;
-    rc = launch_merge(c, ma);
+    rc = yuv422(order) ? launch_pack422(c, ma) : launch_merge(c, ma);
     if (rc) return rc;
     merged_into(c, d_dst, (size_t)(r1 - r0) * dst_stride);
     return prof_mark(c, 3);
@@ -330,6 +359,7 @@ static int process_frames_impl(Ctx* c, const uint8_t* d_src, int n, int w, int h
         if (yuv420(order) && (rc = chroma_planes(c, order, ra.src, w, h, src_stride, d_dst + (size_t)f0 * dst_frame_stride, ow, oh, dst_stride,
                                                  dst_frame_stride, 0, oh, &ra.ch)))
             return rc;
+        if (yuv422(order) && (rc = chroma_planes422(c, ra.src, w, h, src_stride, pl, ow, oh, 0, oh, &ra.ch))) return rc;
         ra.early = !gray && may_start_early(c, ra.src, (size_t)(m - 1) * src_frame_stride + (size_t)h * src_stride);
         c->early_launches += ra.early;
         if ((rc = prof_mark(c, 0))) return rc;
@@ -357,15 +387,16 @@ static int process_frames_impl(Ctx* c, const uint8_t* d_src, int n, int w, int h
         ma.y = pl.yout; ma.cr = pl.cr; ma.cb = pl.cb; ma.a = pl.a;
         ma.pitch = pl.pitch; ma.w = ow;
         ma.order = order;
+        auto merge = [&]() { return yuv422(order) ? launch_pack422(c, ma) : launch_merge(c, ma); };   // 4:2:2: the pack kernel
         if (m == 1 || dst_frame_stride == dst_stride * (size_t)oh) {   // the chunk's results are one tall image too
             ma.rows = oh * m; ma.dst = dst0; ma.dst_stride = dst_stride;
-            if ((rc = launch_merge(c, ma))) return rc;
+            if ((rc = merge())) return rc;
         } else {
             for (int f = 0; f < m; f++) {
                 ma.y = pl.yout + (size_t)f * pl.frame_stride; ma.cr = pl.cr + (size_t)f * pl.frame_stride; ma.cb = pl.cb + (size_t)f * pl.frame_stride;
                 if (pl.a) ma.a = pl.a + (size_t)f * pl.frame_stride;
                 ma.rows = oh; ma.dst = dst0 + (size_t)f * dst_frame_stride; ma.dst_stride = dst_stride;
-                if ((rc = launch_merge(c, ma))) return rc;
+                if ((rc = merge())) return rc;
             }
         }
         merged_into(c, dst0, (size_t)(m - 1) * dst_frame_stride + (size_t)oh * dst_stride);
@@ -611,6 +642,7 @@ int host_pipeline(Ctx* c, const uint8_t* src, int n, int w, int h, size_t src_st
     if ((rc = get_taps(c, w, ow, &tx))) return rc;      // uploaded here, not inside a graph capture
     const bool yuv = yuv420(order);
     if (yuv && ((rc = get_taps(c, h / 2, oh / 2, &cty)) || (rc = get_taps(c, w / 2, ow / 2, &ctx_)))) return rc;   // chroma
+    if (yuv422(order) && (rc = get_taps(c, w / 2, ow / 2, &ctx_))) return rc;   // 4:2:2 chroma (its vertical table is ty)
     auto src_hi = [&](int r1) {
         const int p1 = std::min(r1 + 6, oh);
         return std::min(std::max(ty->h_ofs[p1 - 1] + 2, 0), h - 1) + 1;

@@ -113,7 +113,8 @@ int get_taps(Ctx* c, int src, int dst, TapTable** out) {
 // in-library cross-check of the tiled kernel.
 // ------------------------------------------------------------------------------------------------
 // planes: 3 = Y, Cr, Cb of a colour source, 1 = the one plane of a grey source (no colour conversion), 4 = Y, Cr, Cb and the raw
-// alpha byte of a four-channel source (into pa)
+// alpha byte of a four-channel source (into pa); packed 4:2:2 rows: 5 = one plane of every second byte (Y, kOrderY422), 6 = two
+// planes at bytes 0 and 2 of each 4-byte macropixel (U, V, kOrderUV422) into p.y and p.cr
 template <int NP>
 __global__ void __launch_bounds__(256) k_color_bicubic_direct(ResizeDev p, uint8_t* pa) {
     const int dx = blockIdx.x * 32 + (threadIdx.x & 31);
@@ -136,6 +137,15 @@ __global__ void __launch_bounds__(256) k_color_bicubic_direct(ResizeDev p, uint8
                 aY += (int)row[gx] * cxs[k];
                 continue;
             }
+            if (NP == 5) {
+                aY += (int)row[2 * gx] * cxs[k];
+                continue;
+            }
+            if (NP == 6) {
+                aY += (int)row[4 * gx] * cxs[k];
+                aCr += (int)row[4 * gx + 2] * cxs[k];
+                continue;
+            }
             int c0 = row[NC * gx], c1 = row[NC * gx + 1], c2 = row[NC * gx + 2];
             if (NP == 4) aA += (int)row[NC * gx + 3] * cxs[k];
             int B = p.swapRB ? c2 : c0, R = p.swapRB ? c0 : c2;
@@ -150,8 +160,9 @@ __global__ void __launch_bounds__(256) k_color_bicubic_direct(ResizeDev p, uint8
     const bool fpath = dx < p.simd_w;
     const size_t o = (size_t)(dy - p.plane_row0) * p.pitch + dx;
     p.y[o] = (uint8_t)vertical_tap(hY[0], hY[1], hY[2], hY[3], cy, fpath);
-    if (NP == 1) return;
+    if (NP == 1 || NP == 5) return;
     p.cr[o] = (uint8_t)vertical_tap(hCr[0], hCr[1], hCr[2], hCr[3], cy, fpath);
+    if (NP == 6) return;
     p.cb[o] = (uint8_t)vertical_tap(hCb[0], hCb[1], hCb[2], hCb[3], cy, fpath);
     if (NP == 4) pa[o] = (uint8_t)vertical_tap(hA[0], hA[1], hA[2], hA[3], cy, fpath);
 }
@@ -199,14 +210,16 @@ constexpr int kMaxSR4 = 35;             // ... rows with four planes (the static
 __host__ __device__ constexpr int tiled_max_rows(int np) { return np == 4 ? kMaxSR4 : kMaxSR; }
 
 // NP = 4: the planes of a four-channel source, plane 3 (alpha, the raw byte 3 of each pixel) into pa.  NP = 2: the two bytes of an
-// interleaved pair (NV12 chroma) as two planes, written back interleaved into p.y (4-byte aligned rows)
+// interleaved pair (NV12 chroma) as two planes, written back interleaved into p.y (4-byte aligned rows).  NP = 5 / 6: packed 4:2:2
+// rows as in k_color_bicubic_direct (one / two planes, NPL below), written like a grey call's plane / into p.y and p.cr.
 template <int kTH, int NP>
 __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p, uint8_t* pa) {   // 5 CTAs per SM: 48 registers (4 CTAs measured 6 % slower)
     constexpr int SR = tiled_max_rows(NP);
-    __shared__ __align__(16) uint8_t sP[NP][SR][kMaxSC + 8];   // +8: the 3-word window read of the last quad may run past a row
+    constexpr int NPL = NP == 5 ? 1 : (NP == 6 ? 2 : NP);    // planes
+    __shared__ __align__(16) uint8_t sP[NPL][SR][kMaxSC + 8];   // +8: the 3-word window read of the last quad may run past a row
     // horizontal sums kept as float: they are integers below 2^24, so the conversion is exact and is done
     // once per sum instead of once per use in the vertical pass
-    __shared__ __align__(16) float sH[NP][SR][kTW];
+    __shared__ __align__(16) float sH[NPL][SR][kTW];
     // per tile row: the four vertical taps as floats (b_k = coef_k * 2^-22, exact) and the first tap's row in sH -- computed once
     // per tile instead of once per (thread, row) in the vertical pass
     __shared__ __align__(16) float4 sB[kTH];
@@ -239,6 +252,16 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p, uin
         const int gx = clampi(sx_lo + c, 0, p.sw - 1);
         if (NP == 1) {
             sP[0][r][c] = fsrc[(size_t)gy * p.src_stride + gx];
+            continue;
+        }
+        if (NP == 5) {
+            sP[0][r][c] = fsrc[(size_t)gy * p.src_stride + 2 * (size_t)gx];
+            continue;
+        }
+        if (NP == 6) {
+            const uint8_t* px = fsrc + (size_t)gy * p.src_stride + 4 * (size_t)gx;
+            sP[0][r][c] = px[0];
+            sP[NPL - 1][r][c] = px[2];
             continue;
         }
         if (NP == 2) {
@@ -280,7 +303,7 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p, uin
             const int wsh = 8 * (s0 & 3);
             for (int r = tid >> 4; r < nsr; r += 16) {
 #pragma unroll
-                for (int pl = 0; pl < NP; pl++) {
+                for (int pl = 0; pl < NPL; pl++) {
                     const uint32_t* w = reinterpret_cast<const uint32_t*>(&sP[pl][r][s0 & ~3]);
                     const uint32_t w0 = w[0], w1 = w[1], w2 = w[2];
                     const uint32_t lo = __funnelshift_r(w0, w1, wsh), hi = __funnelshift_r(w1, w2, wsh);
@@ -306,7 +329,7 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p, uin
             const int k0 = cx.x, k1 = cx.y, k2 = cx.z, k3 = cx.w;
             for (int r = tid >> 6; r < nsr; r += 256 / kTW) {
 #pragma unroll
-                for (int pl = 0; pl < NP; pl++) {
+                for (int pl = 0; pl < NPL; pl++) {
                     const uint8_t* q = &sP[pl][r][s];
                     sH[pl][r][col] = (float)((int)q[0] * k0 + (int)q[1] * k1 + (int)q[2] * k2 + (int)q[3] * k3);
                 }
@@ -324,8 +347,8 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p, uin
         const int col = (tid & 15) * 4, ty0 = tid >> 4;
         const unsigned long long nz = p.negzero2;
         const size_t o = fplane + (size_t)(dy0 + ty0 - p.plane_row0) * p.pitch + (size_t)(dx0 + col) * (NP == 2 ? 2 : 1);
-        uint8_t* pcr = NP >= 3 ? p.cr + o : nullptr;
-        uint8_t* pcb = NP >= 3 ? p.cb + o : nullptr;
+        uint8_t* pcr = NP == 3 || NP == 4 || NP == 6 ? p.cr + o : nullptr;
+        uint8_t* pcb = NP == 3 || NP == 4 ? p.cb + o : nullptr;
         uint8_t* ppa = NP == 4 ? pa + o : nullptr;
         uint8_t* py = p.y16 ? p.y16 + fy16 + (size_t)(dy0 + ty0 - p.plane_row0) * p.pitch16 + 2 * (size_t)(dx0 + col + kY16Pad) : p.y + o;
         const size_t step = 16 * p.pitch, ystep = p.y16 ? 16 * p.pitch16 : step;
@@ -335,9 +358,9 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p, uin
             const int ty = ty0 + 16 * k;
             const float4 bq = sB[ty];
             const float* hrow = &sH[0][sSr[ty]][col];
-            uint32_t packed[NP > 3 ? NP : 3];
+            uint32_t packed[NPL > 3 ? NPL : 3];
 #pragma unroll
-            for (int pl = 0; pl < NP; pl++) {
+            for (int pl = 0; pl < NPL; pl++) {
                 const float* h = hrow + pl * (SR * kTW);
                 const ulonglong2 g0 = *reinterpret_cast<const ulonglong2*>(h);
                 const ulonglong2 g1 = *reinterpret_cast<const ulonglong2*>(h + kTW);
@@ -371,7 +394,11 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p, uin
                 *reinterpret_cast<uint32_t*>(py) = packed[0];
             }
             py += ystep;
-            if (NP >= 3) {
+            if (NP == 6) {
+                *reinterpret_cast<uint32_t*>(pcr) = packed[1];
+                pcr += step;
+            }
+            if (NP == 3 || NP == 4) {
                 *reinterpret_cast<uint32_t*>(pcr) = packed[1];
                 *reinterpret_cast<uint32_t*>(pcb) = packed[2];
                 pcr += step; pcb += step;
@@ -397,7 +424,7 @@ __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p, uin
                 const size_t o = fplane + (size_t)(dy - p.plane_row0) * p.pitch + dx;
                 const unsigned long long bb0 = f2_pack(b0, b0), bb1 = f2_pack(b1, b1), bb2 = f2_pack(b2, b2), bb3 = f2_pack(b3, b3);
 #pragma unroll
-                for (int pl = 0; pl < NP; pl++) {
+                for (int pl = 0; pl < NPL; pl++) {
                     if (all_float) {   // two samples per instruction: v = H0*b0 + (H1*b1 + (H2*b2 + H3*b3)), each op rounded
                         const ulonglong2 g0 = *reinterpret_cast<const ulonglong2*>(&sH[pl][sr][col]);
                         const ulonglong2 g1 = *reinterpret_cast<const ulonglong2*>(&sH[pl][sr + 1][col]);
@@ -496,9 +523,11 @@ static ResizeDev resize_dev(const ResizeArgs& a) {
 }
 
 static int launch_yuv420(Ctx* c, const ResizeArgs& a);
+static int launch_yuv422(Ctx* c, const ResizeArgs& a);
 
 int launch_color_bicubic(Ctx* c, const ResizeArgs& a) {
     if (yuv420(a.order)) return launch_yuv420(c, a);
+    if (yuv422(a.order)) return launch_yuv422(c, a);
     ResizeDev p = resize_dev(a);
     const int nframes = std::max(1, a.nframes);
     const int rows = a.row_end - a.row_begin;
@@ -512,6 +541,7 @@ int launch_color_bicubic(Ctx* c, const ResizeArgs& a) {
         if (a.tx->h_ofs[dx1 - 1] - a.tx->h_ofs[dx0] + 4 > kMaxSC) fits_x = false;
     }
     const bool gray = a.order == SRCNN_ORDER_GRAY, four = four_channel(a.order), uv = a.order == kOrderUV;
+    const bool y422 = a.order == kOrderY422, uv422 = a.order == kOrderUV422;
     uint8_t* const pa = four ? a.pl.a : nullptr;
     const int max_rows = tiled_max_rows(four ? 4 : 3);
     auto fits_rows = [&](int th) {
@@ -524,15 +554,17 @@ int launch_color_bicubic(Ctx* c, const ResizeArgs& a) {
     const int th = !fits_x ? 0 : (fits_rows(64) ? 64 : (fits_rows(32) ? 32 : 0));
     for (int dx = 0; dx + 3 < a.ow && p.quad_ok; dx += 4)
         if (a.tx->h_ofs[dx + 3] - a.tx->h_ofs[dx] > 4) p.quad_ok = 0;
-    if (c->ka_int && !uv) {                           // x2 / x4: the integer-scale kernel (constant tap phases, no tables)
+    if (c->ka_int && !uv && !y422 && !uv422) {                           // x2 / x4: the integer-scale kernel (constant tap phases, no tables)
         bool done = false;
         const int rc = launch_color_bicubic_int(c, p, a, &done);
         if (rc || done) return rc;
     }
     if (th) {
         dim3 grid((a.ow + kTW - 1) / kTW, (rows + th - 1) / th, nframes);   // a batch of frames is one launch
-        if (th == 64) (gray ? k_color_bicubic_tiled<64, 1> : uv ? k_color_bicubic_tiled<64, 2> : four ? k_color_bicubic_tiled<64, 4> : k_color_bicubic_tiled<64, 3>)<<<grid, 256, 0, c->stream>>>(p, pa);
-        else (gray ? k_color_bicubic_tiled<32, 1> : uv ? k_color_bicubic_tiled<32, 2> : four ? k_color_bicubic_tiled<32, 4> : k_color_bicubic_tiled<32, 3>)<<<grid, 256, 0, c->stream>>>(p, pa);
+        if (th == 64) (gray ? k_color_bicubic_tiled<64, 1> : uv ? k_color_bicubic_tiled<64, 2> : four ? k_color_bicubic_tiled<64, 4> : y422 ? k_color_bicubic_tiled<64, 5>
+                       : uv422 ? k_color_bicubic_tiled<64, 6> : k_color_bicubic_tiled<64, 3>)<<<grid, 256, 0, c->stream>>>(p, pa);
+        else (gray ? k_color_bicubic_tiled<32, 1> : uv ? k_color_bicubic_tiled<32, 2> : four ? k_color_bicubic_tiled<32, 4> : y422 ? k_color_bicubic_tiled<32, 5>
+              : uv422 ? k_color_bicubic_tiled<32, 6> : k_color_bicubic_tiled<32, 3>)<<<grid, 256, 0, c->stream>>>(p, pa);
         c->launches++;
         SRCNN_CUDA(c, cudaGetLastError());
         return SRCNN_OK;
@@ -542,11 +574,13 @@ int launch_color_bicubic(Ctx* c, const ResizeArgs& a) {
         ResizeDev q = p;
         q.src += (size_t)f * p.src_frame;
         q.y += (size_t)f * p.plane_frame;
-        if (!gray && !uv) { q.cr += (size_t)f * p.plane_frame; q.cb += (size_t)f * p.plane_frame; }
+        if (!gray && !uv && !y422) q.cr += (size_t)f * p.plane_frame;
+        if (!gray && !uv && !y422 && !uv422) q.cb += (size_t)f * p.plane_frame;
         uint8_t* const qa = four ? pa + (size_t)f * p.plane_frame : nullptr;
         dim3 grid((a.ow + 31) / 32, (rows + 7) / 8);
         if (uv) k_chroma420_direct<<<grid, 256, 0, c->stream>>>(q, 1, 1, 2);
-        else (gray ? k_color_bicubic_direct<1> : four ? k_color_bicubic_direct<4> : k_color_bicubic_direct<3>)<<<grid, 256, 0, c->stream>>>(q, qa);
+        else (gray ? k_color_bicubic_direct<1> : four ? k_color_bicubic_direct<4> : y422 ? k_color_bicubic_direct<5> : uv422 ? k_color_bicubic_direct<6>
+              : k_color_bicubic_direct<3>)<<<grid, 256, 0, c->stream>>>(q, qa);
         c->launches++;
         SRCNN_CUDA(c, cudaGetLastError());
         if (a.pl.y16) {
@@ -608,6 +642,37 @@ static int launch_yuv420(Ctx* c, const ResizeArgs& a) {
     }
     if ((rc = launch_color_bicubic(c, u))) return rc;
     u.src += ch.src_v; u.pl.y += ch.dst_v;
+    return launch_color_bicubic(c, u);
+}
+
+// A packed 4:2:2 frame (SRCNN_ORDER_YUY2 / _UYVY).  x2 / x4 with ow % 16 == 0: one launch for luma and chroma (color_bicubic_int.cu).
+// Otherwise two launches of the generic kernels: the Y plane as every second byte of the rows (kOrderY422, into pl.y / pl.y16 as a
+// grey call's), then U and V as bytes 0 and 2 of each macropixel (kOrderUV422) into the workspace's Cr / Cb planes.  The two
+// variants differ only in where the first Y / U byte of a row is.  (The direct kernels, for strong down-scales, go frame by frame.)
+static int launch_yuv422(Ctx* c, const ResizeArgs& a) {
+    const bool uyvy = a.order == SRCNN_ORDER_UYVY;
+    ResizeArgs y = a;
+    y.order = SRCNN_ORDER_GRAY;
+    if (c->ka_int) {
+        bool done = false;
+        const int rc = launch_yuv422_int(c, resize_dev(y), a, &done);
+        if (rc || done) return rc;
+    }
+    y.order = kOrderY422;
+    y.src = a.src + (uyvy ? 1 : 0);
+    int rc = launch_color_bicubic(c, y);
+    if (rc) return rc;
+    const Chroma420& ch = a.ch;
+    ResizeArgs u;
+    u.order = kOrderUV422;
+    u.src = ch.src + (uyvy ? 0 : 1); u.src_stride = ch.src_pitch;
+    u.sw = ch.sw; u.sh = ch.sh; u.src_row0 = 0; u.src_row1 = ch.sh;
+    u.ow = ch.ow; u.oh = ch.oh;
+    u.row_begin = ch.row_begin; u.row_end = ch.row_end;
+    u.pl.y = ch.dst; u.pl.cr = ch.dst + ch.dst_v; u.pl.pitch = ch.dst_pitch; u.pl.row0 = 0; u.pl.rows = ch.oh;
+    u.pl.frame_stride = ch.dst_frame;
+    u.tx = ch.tx; u.ty = ch.ty;
+    u.nframes = a.nframes; u.src_frame_stride = a.src_frame_stride;
     return launch_color_bicubic(c, u);
 }
 
@@ -808,6 +873,84 @@ __global__ void __launch_bounds__(256) k_merge_ycc2bgr_v16(const uint8_t* __rest
         }
         if (!more) break;
     }
+}
+
+// ------------------------------------------------------------------------------------------------
+// K-C for packed 4:2:2 (SRCNN_ORDER_YUY2 / _UYVY): Y' and the resized U', V' planes interleaved into macropixels -- no colour
+// conversion, so none of the merge's arithmetic.  16 pixels per thread: one 128-bit load of Y', 64 bits each of U' and V', four
+// byte permutations for the (U V U V) words and eight for the output, two 128-bit stores (needs 16-byte aligned rows).  Releases
+// its dependents on entry like k_merge_ycc2bgr_v16, so the next call's K-A may fill the SMs beside it.
+// ------------------------------------------------------------------------------------------------
+template <bool kUYVY>
+__global__ void __launch_bounds__(256) k_pack_yuv422_v16(const uint8_t* __restrict__ y, const uint8_t* __restrict__ u,
+                                                         const uint8_t* __restrict__ v, size_t pitch, int w, int rows,
+                                                         uint8_t* __restrict__ dst, size_t dst_stride, int groups_per_row) {
+    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+    const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const int row = (int)(gid / groups_per_row), x = 16 * (int)(gid - (long long)row * groups_per_row);
+    if (row >= rows) return;
+    const size_t o = (size_t)row * pitch;
+    const uint4 vy = *reinterpret_cast<const uint4*>(y + o + x);
+    const uint2 vu = *reinterpret_cast<const uint2*>(u + o + x / 2), vv = *reinterpret_cast<const uint2*>(v + o + x / 2);
+    const uint32_t wy[4] = {vy.x, vy.y, vy.z, vy.w};
+    // (U0 V0 U1 V1) for the first four Y, (U2 V2 U3 V3) for the next four, ...
+    const uint32_t wuv[4] = {__byte_perm(vu.x, vv.x, 0x5140), __byte_perm(vu.x, vv.x, 0x7362), __byte_perm(vu.y, vv.y, 0x5140),
+                             __byte_perm(vu.y, vv.y, 0x7362)};
+    uint32_t out[8];
+#pragma unroll
+    for (int k = 0; k < 4; k++) {   // Y0 U0 Y1 V0 | Y2 U1 Y3 V1  or  U0 Y0 V0 Y1 | U1 Y2 V1 Y3
+        out[2 * k] = __byte_perm(wy[k], wuv[k], kUYVY ? 0x1504 : 0x5140);
+        out[2 * k + 1] = __byte_perm(wy[k], wuv[k], kUYVY ? 0x3726 : 0x7362);
+    }
+    uint8_t* d = dst + (size_t)row * dst_stride + 2 * (size_t)x;
+    if (x + 15 < w) {
+        reinterpret_cast<uint4*>(d)[0] = make_uint4(out[0], out[1], out[2], out[3]);
+        reinterpret_cast<uint4*>(d)[1] = make_uint4(out[4], out[5], out[6], out[7]);
+    } else {   // the row's last, partial group: one aligned word per macropixel (w is even; static indices keep out in registers)
+#pragma unroll
+        for (int j = 0; j < 8; j++)
+            if (x + 2 * j < w) reinterpret_cast<uint32_t*>(d)[j] = out[j];
+    }
+}
+
+// The same for destinations the 128-bit stores cannot take: one macropixel (two pixels) per thread, byte stores.
+template <bool kUYVY>
+__global__ void __launch_bounds__(256) k_pack_yuv422(const uint8_t* __restrict__ y, const uint8_t* __restrict__ u,
+                                                     const uint8_t* __restrict__ v, size_t pitch, int w, int rows,
+                                                     uint8_t* __restrict__ dst, size_t dst_stride) {
+    const int mpr = w / 2;
+    const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const int row = (int)(gid / mpr), m = (int)(gid - (long long)row * mpr);
+    if (row >= rows) return;
+    const size_t o = (size_t)row * pitch;
+    const uint8_t y0 = y[o + 2 * m], y1 = y[o + 2 * m + 1], cu = u[o + m], cv = v[o + m];
+    uint8_t* d = dst + (size_t)row * dst_stride + 4 * (size_t)m;
+    d[0] = kUYVY ? cu : y0;
+    d[1] = kUYVY ? y0 : cu;
+    d[2] = kUYVY ? cv : y1;
+    d[3] = kUYVY ? y1 : cv;
+}
+
+int launch_pack422(Ctx* c, const MergeArgs& a) {
+    if (a.rows <= 0 || a.w <= 0) return SRCNN_OK;
+    const bool uyvy = a.order == SRCNN_ORDER_UYVY;
+    const bool wide = ((((uintptr_t)a.dst) | a.dst_stride | (uintptr_t)a.y | (uintptr_t)a.cr | (uintptr_t)a.cb | a.pitch) & 15) == 0 &&
+                      a.pitch >= align_up((size_t)a.w, 16);
+    c->merge_sel = -1;   // as for a merge: the whole-path caller says afterwards which Cr/Cb pair this launch reads
+    note_merge(c);
+    if (wide) {
+        const int groups16 = (a.w + 15) / 16;
+        const long long blocks = ((long long)groups16 * a.rows + 255) / 256;
+        (uyvy ? k_pack_yuv422_v16<true> : k_pack_yuv422_v16<false>)<<<(unsigned)blocks, 256, 0, c->stream>>>(a.y, a.cr, a.cb, a.pitch, a.w,
+                                                                                                            a.rows, a.dst, a.dst_stride, groups16);
+    } else {
+        const long long blocks = ((long long)(a.w / 2) * a.rows + 255) / 256;
+        (uyvy ? k_pack_yuv422<true> : k_pack_yuv422<false>)<<<(unsigned)blocks, 256, 0, c->stream>>>(a.y, a.cr, a.cb, a.pitch, a.w, a.rows,
+                                                                                                    a.dst, a.dst_stride);
+    }
+    c->launches++;
+    SRCNN_CUDA(c, cudaGetLastError());
+    return SRCNN_OK;
 }
 
 int launch_merge(Ctx* c, const MergeArgs& a) {

@@ -97,5 +97,7 @@ __device__ __forceinline__ unsigned long long f2_add_rn(unsigned long long a, un
 int launch_color_bicubic_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bool* done);
 // the same for a 4:2:0 frame (a.order NV12 / I420; p describes its Y plane as a grey call's): luma and chroma in one launch
 int launch_yuv420_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bool* done);
+// the same for a packed 4:2:2 frame (a.order YUY2 / UYVY; p describes its Y plane as a grey call's, a.ch its chroma): one launch
+int launch_yuv422_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bool* done);
 
 }  // namespace srcnn

@@ -455,9 +455,11 @@ __global__ void __launch_bounds__(96, S == 2 ? SRCNN_KA_MINB : SRCNN_KA_MINB4) k
     walk_tile<S, kGPitch>(p, t, &sP[0][w * (kITW / S)], 0, tid & 31, X0 + w * kITW, a, nit, fz);
 }
 
-// The grey kernel's tile as a device function, for k_yuv420_bicubic_int below.  k_gray_bicubic_int keeps its own copy of these
-// lines: calling this function from it compiles to different SASS.
-template <int S>
+// The grey kernel's tile as a device function, for k_yuv420_bicubic_int and k_yuv422_bicubic_int below.  k_gray_bicubic_int keeps
+// its own copy of these lines: calling this function from it compiles to different SASS.
+// kPacked: 0 = a plane of bytes; 1 / 2 = the Y bytes of packed 4:2:2 rows (YUY2: bytes 0, 2 of each macropixel; UYVY: 1, 3): a
+// four-pixel group is 8 source bytes (one 64-bit load when t.vec_ok == 2, two 32-bit loads when 1) and one byte permutation.
+template <int S, int kPacked = 0>
 __device__ __forceinline__ void gray_tile(const ResizeDev& p, const IntTaps& t, int tile, uint8_t (&sP)[kIRows][kGPitch]) {
     constexpr int GG = 3 * kITW / S / 4 + 2;       // four-byte groups per staged row
     static_assert(4 * GG + 4 <= kGPitch, "staged row too short");
@@ -482,11 +484,26 @@ __device__ __forceinline__ void gray_tile(const ResizeDev& p, const IntTaps& t, 
             const int r = g / GG, gx = F0 + 4 * (g - r * GG);
             const uint8_t* row = fsrc + (size_t)(clampi(a - 1 + r, 0, p.sh - 1) - p.src_row0) * p.src_stride;
             if (t.vec_ok && gx >= 0 && gx + 4 <= p.sw) {
-                raw[it] = *reinterpret_cast<const uint32_t*>(row + gx);
+                if (kPacked == 0) {
+                    raw[it] = *reinterpret_cast<const uint32_t*>(row + gx);
+                } else {
+                    const uint8_t* px = row + 2 * (size_t)gx;
+                    uint32_t w0, w1;
+                    if (t.vec_ok == 2) {
+                        const uint2 v = *reinterpret_cast<const uint2*>(px);
+                        w0 = v.x; w1 = v.y;
+                    } else {
+                        w0 = reinterpret_cast<const uint32_t*>(px)[0]; w1 = reinterpret_cast<const uint32_t*>(px)[1];
+                    }
+                    raw[it] = __byte_perm(w0, w1, kPacked == 2 ? 0x7531 : 0x6420);
+                }
             } else {
                 uint32_t v = 0;
 #pragma unroll
-                for (int j = 0; j < 4; j++) v |= (uint32_t)row[clampi(gx + j, 0, p.sw - 1)] << (8 * j);
+                for (int j = 0; j < 4; j++) {
+                    const int x = clampi(gx + j, 0, p.sw - 1);
+                    v |= (uint32_t)row[kPacked == 0 ? x : 2 * x + (kPacked == 2)] << (8 * j);
+                }
                 raw[it] = v;
             }
         }
@@ -622,7 +639,10 @@ __device__ __forceinline__ void walk_pair(const ChromaDev& q, const IntTaps& t, 
     }
 }
 
-template <int S, bool kNV12>
+// kPacked: 0 = the 4:2:0 chroma rows of kNV12; 1 / 2 = packed 4:2:2 rows (kNV12 false), U and V at bytes 1, 3 (YUY2) or 0, 2
+// (UYVY) of each macropixel: a four-column group is 16 source bytes (two 64-bit or four 32-bit loads, per t.vec_ok) and four
+// byte permutations for both planes.
+template <int S, bool kNV12, int kPacked = 0>
 __device__ __forceinline__ void chroma_tile(const ChromaDev& q, const IntTaps& t, unsigned long long nz, int tile, uint8_t* smem) {
     constexpr int G = CGeo<S>::G, kPitch = CGeo<S>::kPitch;
     uint8_t (*sU)[kPitch] = reinterpret_cast<uint8_t (*)[kPitch]>(smem);
@@ -648,7 +668,21 @@ __device__ __forceinline__ void chroma_tile(const ChromaDev& q, const IntTaps& t
             const int r = g / G, gx = F0 + 4 * (g - r * G);
             const uint8_t* row = fsrc + (size_t)clampi(a - 1 + r, 0, q.sh - 1) * q.src_pitch;
             if (t.vec_ok && gx >= 0 && gx + 4 <= q.sw) {
-                if (kNV12) {
+                if (kPacked) {
+                    const uint8_t* px = row + 4 * (size_t)gx;
+                    uint32_t w[4];
+                    if (t.vec_ok == 2) {
+                        const uint2 v0 = reinterpret_cast<const uint2*>(px)[0], v1 = reinterpret_cast<const uint2*>(px)[1];
+                        w[0] = v0.x; w[1] = v0.y; w[2] = v1.x; w[3] = v1.y;
+                    } else {
+#pragma unroll
+                        for (int k = 0; k < 4; k++) w[k] = reinterpret_cast<const uint32_t*>(px)[k];
+                    }
+                    constexpr unsigned kSel = kPacked == 2 ? 0x6240 : 0x7351;    // (U0 U1 V0 V1) of two macropixels
+                    const uint32_t lo = __byte_perm(w[0], w[1], kSel), hi = __byte_perm(w[2], w[3], kSel);
+                    ru[it] = __byte_perm(lo, hi, 0x5410);
+                    rv[it] = __byte_perm(lo, hi, 0x7632);
+                } else if (kNV12) {
                     const uint32_t* w = reinterpret_cast<const uint32_t*>(row + 2 * gx);
                     const uint32_t w0 = w[0], w1 = w[1];
                     ru[it] = __byte_perm(w0, w1, 0x6420);
@@ -662,8 +696,13 @@ __device__ __forceinline__ void chroma_tile(const ChromaDev& q, const IntTaps& t
 #pragma unroll
                 for (int j = 0; j < 4; j++) {
                     const int x = clampi(gx + j, 0, q.sw - 1);
-                    u |= (uint32_t)(kNV12 ? row[2 * x] : row[x]) << (8 * j);
-                    v |= (uint32_t)(kNV12 ? row[2 * x + 1] : row[q.src_v + x]) << (8 * j);
+                    if (kPacked) {
+                        u |= (uint32_t)row[4 * x + (kPacked == 1)] << (8 * j);
+                        v |= (uint32_t)row[4 * x + (kPacked == 1) + 2] << (8 * j);
+                    } else {
+                        u |= (uint32_t)(kNV12 ? row[2 * x] : row[x]) << (8 * j);
+                        v |= (uint32_t)(kNV12 ? row[2 * x + 1] : row[q.src_v + x]) << (8 * j);
+                    }
                 }
                 ru[it] = u;
                 rv[it] = v;
@@ -692,6 +731,35 @@ __global__ void __launch_bounds__(96, S == 2 ? SRCNN_KA420_MINB : SRCNN_KA420_MI
     __shared__ __align__(16) uint8_t sm[kLuma > kChroma ? kLuma : kChroma];
     if ((int)blockIdx.x < t.ntiles) gray_tile<S>(p, t, blockIdx.x, *reinterpret_cast<uint8_t (*)[kIRows][kGPitch]>(sm));
     else chroma_tile<S, kNV12>(q, tc, p.negzero2, (int)blockIdx.x - t.ntiles, sm);
+}
+
+// ------------------------------------------------------------------------------------------------
+// Packed 4:2:2 frames (SRCNN_ORDER_YUY2 / _UYVY): ONE launch for luma and chroma, like k_yuv420_bicubic_int.  CTAs [0, t.ntiles)
+// are the grey kernel's tiles of the Y plane (into the workspace plane the CNN reads), staged by de-interleaving the packed rows
+// (gray_tile, kPacked); the rest are chroma tiles: U and V staged as two shared-memory planes from the same packed rows, walked
+// as in a 4:2:0 chroma tile (a lane owns the same 4 columns of both), written as four bytes per lane and row into the workspace's
+// Cr (U') and Cb (V') planes, which the pack kernel (K-C) reads.  The chroma plane is w/2 x h -> ow/2 x oh: x S on both axes, so
+// its vertical taps are the luma ones.  Launch conditions: ow a multiple of 16 (luma and chroma widths multiples of 8), 8-byte
+// aligned luma stores and 4-byte aligned chroma stores (always true of the workspace).  Unlike a 4:2:0 call this call may start
+// beside the previous call's merge / pack kernel (api.cu, may_start_early): the last CTA waits for it, as in k_color_bicubic_int.
+// ------------------------------------------------------------------------------------------------
+#ifndef SRCNN_KA422_MINB
+#define SRCNN_KA422_MINB SRCNN_KA_MINB
+#endif
+#ifndef SRCNN_KA422_MINB4
+#define SRCNN_KA422_MINB4 SRCNN_KA_MINB4
+#endif
+
+template <int S, bool kUYVY>
+__global__ void __launch_bounds__(96, S == 2 ? SRCNN_KA422_MINB : SRCNN_KA422_MINB4) k_yuv422_bicubic_int(const ResizeDev p, const IntTaps t,
+                                                                                                        const ChromaDev q, const IntTaps tc) {
+    constexpr int kPacked = kUYVY ? 2 : 1;
+    constexpr int kLuma = kIRows * kGPitch, kChroma = 2 * kIRows * CGeo<S>::kPitch;
+    __shared__ __align__(16) uint8_t sm[kLuma > kChroma ? kLuma : kChroma];
+    const int b = (int)blockIdx.x;
+    if (b < t.ntiles) gray_tile<S, kPacked>(p, t, b, *reinterpret_cast<uint8_t (*)[kIRows][kGPitch]>(sm));
+    else chroma_tile<S, false, kPacked>(q, tc, p.negzero2, b - t.ntiles, sm);
+    if (b == t.ntiles + tc.ntiles - 1) asm volatile("griddepcontrol.wait;" ::: "memory");
 }
 
 inline int floordiv(int a, int b) { return a >= 0 ? a / b : -((-a + b - 1) / b); }
@@ -817,6 +885,60 @@ int launch_yuv420_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bool* don
     q.sw = ch.sw; q.sh = ch.sh; q.ow = ch.ow; q.row_begin = ch.row_begin; q.row_end = ch.row_end;
     // never early: a 4:2:0 call launches no merge (api.cu)
     const int rc = launch_ka(c, kern, t.ntiles + tc.ntiles, 96, false, p, t, q, tc);
+    if (rc) return rc;
+    *done = true;
+    return SRCNN_OK;
+}
+
+int launch_yuv422_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bool* done) {
+    *done = false;
+    const Chroma420& ch = a.ch;
+    const int S = a.tx->int_scale;
+    if (S == 0 || a.ty->int_scale != S || ch.tx->int_scale != S || ch.ty->int_scale != S) return SRCNN_OK;
+    if ((a.ow & 15) || a.row_end <= a.row_begin || ch.row_end <= ch.row_begin) return SRCNN_OK;
+    // stores: luma as in a grey call; chroma 4 bytes per plane, lane and row
+    if ((((uintptr_t)p.y | p.pitch | p.plane_frame) & 7) != 0) return SRCNN_OK;
+    if (p.y16 && (((uintptr_t)p.y16 | p.pitch16 | p.y16_frame) & 15) != 0) return SRCNN_OK;
+    if ((((uintptr_t)ch.dst | ch.dst_pitch | ch.dst_v | ch.dst_frame) & 3) != 0) return SRCNN_OK;
+    const bool uyvy = a.order == SRCNN_ORDER_UYVY;
+    const int nframes = std::max(1, a.nframes);
+
+    IntTaps t = {}, tc = {};
+    int_taps(a.tx, a.ty, S, a.row_begin, a.row_end, t);
+    int_taps(ch.tx, ch.ty, S, ch.row_begin, ch.row_end, tc);
+    // both tile kinds read the same packed rows: 64-bit group loads when they are 8-byte aligned, 32-bit when 4-byte aligned
+    const uintptr_t al = (uintptr_t)p.src | p.src_stride | p.src_frame | (uintptr_t)ch.src | ch.src_pitch;
+    t.vec_ok = tc.vec_ok = (al & 7) == 0 ? 2 : ((al & 3) == 0 ? 1 : 0);
+    t.ntx = ((a.ow + kITW - 1) / kITW + 2) / 3;    // a CTA per three adjacent tiles, as in a grey call
+    tc.ntx = (ch.ow + 3 * kCW - 1) / (3 * kCW);
+    auto kern = S == 2 ? (uyvy ? k_yuv422_bicubic_int<2, true> : k_yuv422_bicubic_int<2, false>)
+                       : (uyvy ? k_yuv422_bicubic_int<4, true> : k_yuv422_bicubic_int<4, false>);
+    static int ctas_per_sm[4][64] = {};            // per instance and device; a benign race: every writer stores the same value
+    int& per_sm = ctas_per_sm[(S == 4) * 2 + uyvy][c->device & 63];
+    if (per_sm == 0) {
+        int n = 0;
+        SRCNN_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kern, 96, 0));
+        per_sm = std::max(1, n);
+    }
+    // tile height: the rule of launch_variant over the launch's luma and chroma tiles together
+    const int resident = per_sm * std::max(1, c->sm_count);
+    const int nrows = t.i_last - t.a_first + 1, crows = tc.i_last - tc.a_first + 1;
+    auto tiles_for = [&](int isr) {
+        return ((long long)t.ntx * ((nrows + isr - 1) / isr) + (long long)tc.ntx * ((crows + isr - 1) / isr)) * nframes;
+    };
+    t.isr = tiles_for(kISRMax) > 2LL * resident ? kISRMax : 8;
+    if (c->ka_int_isr >= 4 && c->ka_int_isr <= kISRMax) t.isr = c->ka_int_isr;
+    tc.isr = t.isr;
+    if (tiles_for(t.isr) > 0x3fffffffLL) return SRCNN_OK;
+    t.nty = (nrows + t.isr - 1) / t.isr;
+    tc.nty = (crows + tc.isr - 1) / tc.isr;
+    t.ntiles = t.ntx * t.nty * nframes;
+    tc.ntiles = tc.ntx * tc.nty * nframes;
+    ChromaDev q;
+    q.src = ch.src; q.src_pitch = ch.src_pitch; q.src_v = 0; q.src_frame = p.src_frame;
+    q.dst = ch.dst; q.dst_pitch = ch.dst_pitch; q.dst_v = ch.dst_v; q.dst_frame = ch.dst_frame;
+    q.sw = ch.sw; q.sh = ch.sh; q.ow = ch.ow; q.row_begin = ch.row_begin; q.row_end = ch.row_end;
+    const int rc = launch_ka(c, kern, t.ntiles + tc.ntiles, 96, a.early, p, t, q, tc);
     if (rc) return rc;
     *done = true;
     return SRCNN_OK;
