@@ -909,6 +909,12 @@ extern "C" __attribute__((visibility("default"))) int srcnn_debug_tc2_partition(
     srcnn::tc2_partition(nstrips, hb, nworkers, ovh, bounds);
     return SRCNN_OK;
 }
+// the row-walking kernel's packed FP16 operand image (host code only, no device needed): `bytes` must be tc2_weight_bytes()
+extern "C" __attribute__((visibility("default"))) int srcnn_debug_tc2_weights(uint8_t* img, size_t bytes) {
+    if (!img || bytes != srcnn::tc2_weight_bytes()) return SRCNN_E_ARG;
+    srcnn::tc2_pack_weights((const float*)srcnn_weights_blob, img);
+    return SRCNN_OK;
+}
 extern "C" __attribute__((visibility("default"))) int srcnn_debug_set_tc2_seg_ovh(srcnn_ctx* c, int ovh) {
     if (!c || ovh < 0 || ovh > 64) return SRCNN_E_ARG;
     c->tc2_seg_ovh = ovh;

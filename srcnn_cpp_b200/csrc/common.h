@@ -292,6 +292,8 @@ void fraw_release(Ctx* c);   // frees the cached frawscale contribution tables
 int host_pipeline(Ctx* c, const uint8_t* src, int n, int w, int h, size_t src_stride, size_t src_frame_stride, int order,
                   float scale, int ow, int oh, int R0, int R1, uint8_t* dst, size_t dst_stride, size_t dst_frame_stride);
 int launch_cnn_tc2(Ctx* c, const CnnArgs& a);
+void tc2_pack_weights(const float* params, uint8_t* img);   // host only: img = tc2_weight_bytes() bytes
+size_t tc2_weight_bytes();
 int tc2_prepare_weights(Ctx* c, const float* params);
 void tc2_release(Ctx* c);
 void tc2_partition(int nstrips, int hb, int nworkers, int ovh, long long* bounds);

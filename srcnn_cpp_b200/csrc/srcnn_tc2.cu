@@ -865,10 +865,11 @@ static inline void put_h2(uint8_t* img, size_t byte_off, float v) {
 }
 
 // Packs the FP32 parameters into the FP16 operand images the kernel's UMMA descriptors expect
-// (SWIZZLE_NONE, K-major: element (n,k) of a [N][16] tile at (k/8)*(N*16) + n*16 + (k%8)*2 bytes).
-int tc2_prepare_weights(Ctx* c, const float* P) {
+// (SWIZZLE_NONE, K-major: element (n,k) of a [N][16] tile at (k/8)*(N*16) + n*16 + (k%8)*2 bytes).  Pure host code:
+// `img` (tc2_weight_bytes() bytes) is written in full; tests decode it through srcnn_debug_tc2_weights.
+void tc2_pack_weights(const float* P, uint8_t* img) {
     using namespace tc2;
-    std::vector<uint8_t> img(kWeightBytes, 0);
+    memset(img, 0, kWeightBytes);
     const float* w1 = P + kOffW1;
     const float* w2 = P + kOffW2;
     const float* w3 = P + kOffW3;
@@ -893,26 +894,34 @@ int tc2_prepare_weights(Ctx* c, const float* P) {
                     val = (k == 2 * kOnesCol) ? hi : lo;
                 }
                 const int ch = k / 16, kk = k % 16;
-                put_h2(img.data(), (size_t)v * kB1Var + (size_t)ch * kB1Chunk + (size_t)(kk / 8) * 1024 + (size_t)n * 16 + (kk % 8) * 2, val);
+                put_h2(img, (size_t)v * kB1Var + (size_t)ch * kB1Chunk + (size_t)(kk / 8) * 1024 + (size_t)n * 16 + (kk % 8) * 2, val);
             }
         }
     for (int ks = 0; ks < 4; ks++)  // conv2: B[n = out ch][k = in ch ks*16+k]
         for (int n = 0; n < 32; n++)
             for (int k = 0; k < 16; k++)
-                put_h2(img.data(), kImgB2 + (size_t)ks * 1024 + (size_t)(k / 8) * 512 + (size_t)n * 16 + (k % 8) * 2,
+                put_h2(img, kImgB2 + (size_t)ks * 1024 + (size_t)(k / 8) * 512 + (size_t)n * 16 + (k % 8) * 2,
                        w2[n * 64 + ks * 16 + k]);
     for (int n = 0; n < 32; n++) {  // conv2 bias step: A = ring columns 48..55, the ones column is K index 4,5 of it
         float hi, lo;
         hi_lo(P[kOffB2 + n], hi, lo);
         const int k0 = 2 * (kOnesCol - 48);
-        put_h2(img.data(), kImgB2 + 4 * 1024 + (size_t)(k0 / 8) * 512 + (size_t)n * 16 + (k0 % 8) * 2, hi);
-        put_h2(img.data(), kImgB2 + 4 * 1024 + (size_t)((k0 + 1) / 8) * 512 + (size_t)n * 16 + ((k0 + 1) % 8) * 2, lo);
+        put_h2(img, kImgB2 + 4 * 1024 + (size_t)(k0 / 8) * 512 + (size_t)n * 16 + (k0 % 8) * 2, hi);
+        put_h2(img, kImgB2 + 4 * 1024 + (size_t)((k0 + 1) / 8) * 512 + (size_t)n * 16 + ((k0 + 1) % 8) * 2, lo);
     }
     for (int ks = 0; ks < 2; ks++)  // conv3 tap GEMM: B[n = tap m*5+n][k = in ch]
         for (int n = 0; n < 32; n++)
             for (int k = 0; k < 16; k++)
-                put_h2(img.data(), kImgB3 + (size_t)ks * 1024 + (size_t)(k / 8) * 512 + (size_t)n * 16 + (k % 8) * 2,
+                put_h2(img, kImgB3 + (size_t)ks * 1024 + (size_t)(k / 8) * 512 + (size_t)n * 16 + (k % 8) * 2,
                        n < 25 ? w3[(ks * 16 + k) * 25 + n] : 0.f);
+}
+
+size_t tc2_weight_bytes() { return tc2::kWeightBytes; }
+
+int tc2_prepare_weights(Ctx* c, const float* P) {
+    using namespace tc2;
+    std::vector<uint8_t> img(kWeightBytes);
+    tc2_pack_weights(P, img.data());
     SRCNN_CUDA(c, cudaMalloc(&c->d_tc2_weights, kWeightBytes));
     // pageable source: the runtime has staged `img` when this returns; srcnn_create synchronises the device afterwards
     SRCNN_CUDA(c, cudaMemcpyAsync(c->d_tc2_weights, img.data(), kWeightBytes, cudaMemcpyHostToDevice, c->stream));
