@@ -915,6 +915,16 @@ extern "C" __attribute__((visibility("default"))) int srcnn_debug_tc2_weights(ui
     srcnn::tc2_pack_weights((const float*)srcnn_weights_blob, img);
     return SRCNN_OK;
 }
+// the colour+bicubic kernels' tap table for one axis (build_cubic_taps, host code only): ofs[dst], coef[4 * dst]
+extern "C" __attribute__((visibility("default"))) int srcnn_debug_cubic_taps(int src, int dst, int* ofs, int16_t* coef) {
+    if (src <= 0 || dst <= 0 || !ofs || !coef) return SRCNN_E_ARG;
+    std::vector<short4> c((size_t)dst);
+    srcnn::build_cubic_taps(src, dst, ofs, c.data());
+    for (int d = 0; d < dst; d++) {
+        coef[4 * d] = c[d].x; coef[4 * d + 1] = c[d].y; coef[4 * d + 2] = c[d].z; coef[4 * d + 3] = c[d].w;
+    }
+    return SRCNN_OK;
+}
 extern "C" __attribute__((visibility("default"))) int srcnn_debug_set_tc2_seg_ovh(srcnn_ctx* c, int ovh) {
     if (!c || ovh < 0 || ovh > 64) return SRCNN_E_ARG;
     c->tc2_seg_ovh = ovh;
