@@ -112,9 +112,7 @@ int get_taps(Ctx* c, int src, int dst, TapTable** out) {
 // geometry the tiled kernel's shared-memory footprint cannot hold (strong down-scales) and as the
 // in-library cross-check of the tiled kernel.
 // ------------------------------------------------------------------------------------------------
-// planes: 3 = Y, Cr, Cb of a colour source, 1 = the one plane of a grey source (no colour conversion), 4 = Y, Cr, Cb and the raw
-// alpha byte of a four-channel source (into pa); packed 4:2:2 rows: 5 = one plane of every second byte (Y, kOrderY422), 6 = two
-// planes at bytes 0 and 2 of each 4-byte macropixel (U, V, kOrderUV422) into p.y and p.cr
+// planes: 3 = Y, Cr, Cb of a colour source, 4 = Y, Cr, Cb and the raw alpha byte of a four-channel source (into pa)
 template <int NP>
 __global__ void __launch_bounds__(256) k_color_bicubic_direct(ResizeDev p, uint8_t* pa) {
     const int dx = blockIdx.x * 32 + (threadIdx.x & 31);
@@ -123,7 +121,6 @@ __global__ void __launch_bounds__(256) k_color_bicubic_direct(ResizeDev p, uint8
     const int sx = p.xofs[dx], sy = p.yofs[dy];
     const short4 cx = p.xcoef[dx], cy = p.ycoef[dy];
     const int cxs[4] = {cx.x, cx.y, cx.z, cx.w};
-    constexpr int NC = NP == 4 ? 4 : 3;   // bytes per colour pixel
     int hY[4], hCr[4], hCb[4], hA[4];
 #pragma unroll
     for (int r = 0; r < 4; r++) {
@@ -133,21 +130,8 @@ __global__ void __launch_bounds__(256) k_color_bicubic_direct(ResizeDev p, uint8
 #pragma unroll
         for (int k = 0; k < 4; k++) {
             const int gx = clampi(sx - 1 + k, 0, p.sw - 1);
-            if (NP == 1) {
-                aY += (int)row[gx] * cxs[k];
-                continue;
-            }
-            if (NP == 5) {
-                aY += (int)row[2 * gx] * cxs[k];
-                continue;
-            }
-            if (NP == 6) {
-                aY += (int)row[4 * gx] * cxs[k];
-                aCr += (int)row[4 * gx + 2] * cxs[k];
-                continue;
-            }
-            int c0 = row[NC * gx], c1 = row[NC * gx + 1], c2 = row[NC * gx + 2];
-            if (NP == 4) aA += (int)row[NC * gx + 3] * cxs[k];
+            int c0 = row[NP * gx], c1 = row[NP * gx + 1], c2 = row[NP * gx + 2];
+            if (NP == 4) aA += (int)row[NP * gx + 3] * cxs[k];
             int B = p.swapRB ? c2 : c0, R = p.swapRB ? c0 : c2;
             int Y, Cr, Cb;
             bgr_to_ycc(B, c1, R, Y, Cr, Cb);
@@ -160,41 +144,41 @@ __global__ void __launch_bounds__(256) k_color_bicubic_direct(ResizeDev p, uint8
     const bool fpath = dx < p.simd_w;
     const size_t o = (size_t)(dy - p.plane_row0) * p.pitch + dx;
     p.y[o] = (uint8_t)vertical_tap(hY[0], hY[1], hY[2], hY[3], cy, fpath);
-    if (NP == 1 || NP == 5) return;
     p.cr[o] = (uint8_t)vertical_tap(hCr[0], hCr[1], hCr[2], hCr[3], cy, fpath);
-    if (NP == 6) return;
     p.cb[o] = (uint8_t)vertical_tap(hCb[0], hCb[1], hCb[2], hCb[3], cy, fpath);
     if (NP == 4) pa[o] = (uint8_t)vertical_tap(hA[0], hA[1], hA[2], hA[3], cy, fpath);
 }
 
-// The two chroma planes of a 4:2:0 frame in one launch of the direct form (byte loads and stores: any alignment).  Plane k's
-// sample x of a row is byte k * vs + x * step past the row's start in the source (k * vd + x * step in the output): NV12's pairs
-// are vs = vd = 1, step = 2; I420's planes are vs / vd = the V plane's distance from U, step = 1.
-__global__ void __launch_bounds__(256) k_chroma420_direct(ResizeDev p, size_t vs, size_t vd, int step) {
+// The same for NPL planes of raw bytes (no colour conversion; byte loads and stores: any alignment).  Plane k's sample x of a
+// row is byte k * sv + x * sstep past the row's start in the source, k * dv + x * dstep past it in p.y.  A grey plane: one plane,
+// steps 1; the Y bytes of packed 4:2:2 rows: sstep 2; their U and V bytes: sv 2, sstep 4, dv the distance of the V output plane
+// from the U one; NV12's chroma pairs: sv = dv = 1, steps 2; I420's U and V planes: sv / dv = V's distance from U, steps 1.
+template <int NPL>
+__global__ void __launch_bounds__(256) k_planes_bicubic_direct(ResizeDev p, size_t sv, int sstep, size_t dv, int dstep) {
     const int dx = blockIdx.x * 32 + (threadIdx.x & 31);
     const int dy = p.row_begin + blockIdx.y * 8 + (threadIdx.x >> 5);
     if (dx >= p.ow || dy >= p.row_end) return;
     const int sx = p.xofs[dx], sy = p.yofs[dy];
     const short4 cx = p.xcoef[dx], cy = p.ycoef[dy];
     const int cxs[4] = {cx.x, cx.y, cx.z, cx.w};
-    int h[2][4];
+    int h[NPL][4];
 #pragma unroll
     for (int r = 0; r < 4; r++) {
-        const uint8_t* row = p.src + (size_t)clampi(sy - 1 + r, 0, p.sh - 1) * p.src_stride;
-        int a0 = 0, a1 = 0;
+        const uint8_t* row = p.src + (size_t)(clampi(sy - 1 + r, 0, p.sh - 1) - p.src_row0) * p.src_stride;
+        int acc[NPL] = {};
 #pragma unroll
         for (int k = 0; k < 4; k++) {
-            const size_t x = (size_t)clampi(sx - 1 + k, 0, p.sw - 1) * step;
-            a0 += (int)row[x] * cxs[k];
-            a1 += (int)row[vs + x] * cxs[k];
+            const size_t x = (size_t)clampi(sx - 1 + k, 0, p.sw - 1) * sstep;
+#pragma unroll
+            for (int pl = 0; pl < NPL; pl++) acc[pl] += (int)row[pl * sv + x] * cxs[k];
         }
-        h[0][r] = a0;
-        h[1][r] = a1;
+#pragma unroll
+        for (int pl = 0; pl < NPL; pl++) h[pl][r] = acc[pl];
     }
     const bool fpath = dx < p.simd_w;
-    uint8_t* d = p.y + (size_t)(dy - p.plane_row0) * p.pitch + (size_t)dx * step;
-    d[0] = (uint8_t)vertical_tap(h[0][0], h[0][1], h[0][2], h[0][3], cy, fpath);
-    d[vd] = (uint8_t)vertical_tap(h[1][0], h[1][1], h[1][2], h[1][3], cy, fpath);
+    uint8_t* d = p.y + (size_t)(dy - p.plane_row0) * p.pitch + (size_t)dx * dstep;
+#pragma unroll
+    for (int pl = 0; pl < NPL; pl++) d[pl * dv] = (uint8_t)vertical_tap(h[pl][0], h[pl][1], h[pl][2], h[pl][3], cy, fpath);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -211,7 +195,7 @@ __host__ __device__ constexpr int tiled_max_rows(int np) { return np == 4 ? kMax
 
 // NP = 4: the planes of a four-channel source, plane 3 (alpha, the raw byte 3 of each pixel) into pa.  NP = 2: the two bytes of an
 // interleaved pair (NV12 chroma) as two planes, written back interleaved into p.y (4-byte aligned rows).  NP = 5 / 6: packed 4:2:2
-// rows as in k_color_bicubic_direct (one / two planes, NPL below), written like a grey call's plane / into p.y and p.cr.
+// rows as in k_planes_bicubic_direct (one / two planes, NPL below), written like a grey call's plane / into p.y and p.cr.
 template <int kTH, int NP>
 __global__ void __launch_bounds__(256, 5) k_color_bicubic_tiled(ResizeDev p, uint8_t* pa) {   // 5 CTAs per SM: 48 registers (4 CTAs measured 6 % slower)
     constexpr int SR = tiled_max_rows(NP);
@@ -526,8 +510,16 @@ static int launch_yuv420(Ctx* c, const ResizeArgs& a);
 static int launch_yuv422(Ctx* c, const ResizeArgs& a);
 
 int launch_color_bicubic(Ctx* c, const ResizeArgs& a) {
-    if (yuv420(a.order)) return launch_yuv420(c, a);
-    if (yuv422(a.order)) return launch_yuv422(c, a);
+    if (yuv420(a.order) || yuv422(a.order)) {
+        if (c->ka_int) {   // x2 / x4: luma and chroma in one launch of the integer-scale kernel
+            ResizeArgs y = a;
+            y.order = SRCNN_ORDER_GRAY;
+            bool done = false;
+            const int rc = launch_yuv_int(c, resize_dev(y), a, &done);
+            if (rc || done) return rc;
+        }
+        return yuv420(a.order) ? launch_yuv420(c, a) : launch_yuv422(c, a);
+    }
     ResizeDev p = resize_dev(a);
     const int nframes = std::max(1, a.nframes);
     const int rows = a.row_end - a.row_begin;
@@ -574,13 +566,19 @@ int launch_color_bicubic(Ctx* c, const ResizeArgs& a) {
         ResizeDev q = p;
         q.src += (size_t)f * p.src_frame;
         q.y += (size_t)f * p.plane_frame;
-        if (!gray && !uv && !y422) q.cr += (size_t)f * p.plane_frame;
-        if (!gray && !uv && !y422 && !uv422) q.cb += (size_t)f * p.plane_frame;
-        uint8_t* const qa = four ? pa + (size_t)f * p.plane_frame : nullptr;
         dim3 grid((a.ow + 31) / 32, (rows + 7) / 8);
-        if (uv) k_chroma420_direct<<<grid, 256, 0, c->stream>>>(q, 1, 1, 2);
-        else (gray ? k_color_bicubic_direct<1> : four ? k_color_bicubic_direct<4> : y422 ? k_color_bicubic_direct<5> : uv422 ? k_color_bicubic_direct<6>
-              : k_color_bicubic_direct<3>)<<<grid, 256, 0, c->stream>>>(q, qa);
+        if (gray || y422) {
+            k_planes_bicubic_direct<1><<<grid, 256, 0, c->stream>>>(q, 0, y422 ? 2 : 1, 0, 1);
+        } else if (uv) {
+            k_planes_bicubic_direct<2><<<grid, 256, 0, c->stream>>>(q, 1, 2, 1, 2);
+        } else if (uv422) {
+            k_planes_bicubic_direct<2><<<grid, 256, 0, c->stream>>>(q, 2, 4, (size_t)(p.cr - p.y), 1);
+        } else {
+            q.cr += (size_t)f * p.plane_frame;
+            q.cb += (size_t)f * p.plane_frame;
+            uint8_t* const qa = four ? pa + (size_t)f * p.plane_frame : nullptr;
+            (four ? k_color_bicubic_direct<4> : k_color_bicubic_direct<3>)<<<grid, 256, 0, c->stream>>>(q, qa);
+        }
         c->launches++;
         SRCNN_CUDA(c, cudaGetLastError());
         if (a.pl.y16) {
@@ -595,15 +593,10 @@ int launch_color_bicubic(Ctx* c, const ResizeArgs& a) {
 // chroma (color_bicubic_int.cu).  Otherwise the Y plane takes the grey instances and the chroma planes the generic ones, resized as
 // an image of their own straight into the caller's output: NV12's pairs as two interleaved planes (NP = 2), I420's U and V planes
 // as two frames of a one-plane launch (one launch for a single frame, one per plane for a batch).  Chroma rows of the output that
-// are not 4-byte aligned (the tiled kernel stores words) take k_chroma420_direct, one launch per frame for both planes.
+// are not 4-byte aligned (the tiled kernel stores words) take k_planes_bicubic_direct, one launch per frame for both planes.
 static int launch_yuv420(Ctx* c, const ResizeArgs& a) {
     ResizeArgs y = a;
     y.order = SRCNN_ORDER_GRAY;
-    if (c->ka_int) {
-        bool done = false;
-        const int rc = launch_yuv420_int(c, resize_dev(y), a, &done);
-        if (rc || done) return rc;
-    }
     int rc = launch_color_bicubic(c, y);
     if (rc) return rc;
     const Chroma420& ch = a.ch;
@@ -625,7 +618,7 @@ static int launch_yuv420(Ctx* c, const ResizeArgs& a) {
             q.src += (size_t)f * a.src_frame_stride;
             q.y += (size_t)f * ch.dst_frame;
             dim3 grid((ch.ow + 31) / 32, (ch.row_end - ch.row_begin + 7) / 8);
-            k_chroma420_direct<<<grid, 256, 0, c->stream>>>(q, nv12 ? 1 : ch.src_v, nv12 ? 1 : ch.dst_v, nv12 ? 2 : 1);
+            k_planes_bicubic_direct<2><<<grid, 256, 0, c->stream>>>(q, nv12 ? 1 : ch.src_v, nv12 ? 2 : 1, nv12 ? 1 : ch.dst_v, nv12 ? 2 : 1);
             c->launches++;
             SRCNN_CUDA(c, cudaGetLastError());
         }
@@ -652,12 +645,6 @@ static int launch_yuv420(Ctx* c, const ResizeArgs& a) {
 static int launch_yuv422(Ctx* c, const ResizeArgs& a) {
     const bool uyvy = a.order == SRCNN_ORDER_UYVY;
     ResizeArgs y = a;
-    y.order = SRCNN_ORDER_GRAY;
-    if (c->ka_int) {
-        bool done = false;
-        const int rc = launch_yuv422_int(c, resize_dev(y), a, &done);
-        if (rc || done) return rc;
-    }
     y.order = kOrderY422;
     y.src = a.src + (uyvy ? 1 : 0);
     int rc = launch_color_bicubic(c, y);

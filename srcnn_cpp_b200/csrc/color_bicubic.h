@@ -91,13 +91,52 @@ __device__ __forceinline__ unsigned long long f2_add_rn(unsigned long long a, un
     asm("add.rn.f32x2 %0, %1, %2;" : "=l"(r) : "l"(a), "l"(b));
     return r;
 }
+// the vertical pass on a pair of columns: H0*b0 + (H1*b1 + (H2*b2 + H3*b3)), every product and sum rounded on its own
+__device__ __forceinline__ unsigned long long f2_vtap(unsigned long long h0, unsigned long long h1, unsigned long long h2, unsigned long long h3,
+                                                      unsigned long long b0, unsigned long long b1, unsigned long long b2, unsigned long long b3,
+                                                      unsigned long long negzero) {
+    unsigned long long v = f2_mul_rn(h3, b3, negzero);
+    v = f2_add_rn(f2_mul_rn(h2, b2, negzero), v);
+    v = f2_add_rn(f2_mul_rn(h1, b1, negzero), v);
+    return f2_add_rn(f2_mul_rn(h0, b0, negzero), v);
+}
+
+// two u8 values (the low bytes of `lo` and `hi`) -> an FP16 pair, exactly: 0x6400 | v is 1024 + v, minus 1024
+__device__ __forceinline__ uint32_t u8x2_to_h2(uint32_t lo, uint32_t hi) {
+    uint32_t u = __byte_perm(lo, hi, 0x5410) | 0x64006400u;
+    const __half2 h = __hsub2(*reinterpret_cast<__half2*>(&u), __float2half2_rn(1024.f));
+    return *reinterpret_cast<const uint32_t*>(&h);
+}
+
+// A walk down `nit` output-row groups with a window of four rows of horizontal sums in registers: hsum(r, h) fills h with the sums
+// of footprint row r, emit(h0, h1, h2, h3) produces the output rows of one window.  The window rotates by unrolling, not by
+// register moves.
+template <typename H, typename HSum, typename Emit>
+__device__ __forceinline__ void walk_window(int nit, HSum&& hsum, Emit&& emit) {
+    H hA, hB, hC, hD;
+    hsum(0, hA);
+    hsum(1, hB);
+    hsum(2, hC);
+    for (int tt = 0; tt < nit; tt += 4) {
+        hsum(tt + 3, hD);
+        emit(hA, hB, hC, hD);
+        if (tt + 1 >= nit) break;
+        hsum(tt + 4, hA);
+        emit(hB, hC, hD, hA);
+        if (tt + 2 >= nit) break;
+        hsum(tt + 5, hB);
+        emit(hC, hD, hA, hB);
+        if (tt + 3 >= nit) break;
+        hsum(tt + 6, hC);
+        emit(hD, hA, hB, hC);
+    }
+}
 
 
 // integer up-scales (color_bicubic_int.cu); returns SRCNN_OK with *done = false when the geometry is not eligible
 int launch_color_bicubic_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bool* done);
-// the same for a 4:2:0 frame (a.order NV12 / I420; p describes its Y plane as a grey call's): luma and chroma in one launch
-int launch_yuv420_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bool* done);
-// the same for a packed 4:2:2 frame (a.order YUY2 / UYVY; p describes its Y plane as a grey call's, a.ch its chroma): one launch
-int launch_yuv422_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bool* done);
+// the same for a 4:2:0 or packed 4:2:2 frame (a.order NV12 / I420 / YUY2 / UYVY; p describes its Y plane as a grey call's, a.ch
+// its chroma): luma and chroma in one launch
+int launch_yuv_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bool* done);
 
 }  // namespace srcnn

@@ -54,6 +54,28 @@ struct IntTaps {
     int ntx, nty, ntiles;               // tiles per row of tiles, rows of tiles per frame, tiles in the launch (frames included)
 };
 
+// where tile `tile` of a launch lies, for CTAs that cover `tw` output columns
+struct TilePos {
+    size_t fz;                          // frame
+    int X0;                             // first output column
+    int a;                              // source row index: footprint row r is source row a - 1 + r
+    int F0;                             // first footprint column (a multiple of 4: aligned groups)
+    int nit, nsr;                       // source rows the tile advances by; footprint rows
+};
+template <int S>
+__device__ __forceinline__ TilePos tile_pos(const IntTaps& t, int tile, int tw) {
+    TilePos r;
+    const int bx = tile % t.ntx, rest = tile / t.ntx;
+    const int by = rest % t.nty;
+    r.fz = (size_t)(rest / t.nty);
+    r.X0 = bx * tw;
+    r.a = t.a_first + by * t.isr;
+    r.F0 = r.X0 / S - 4;
+    r.nit = min(t.isr, t.i_last - r.a + 1);
+    r.nsr = r.nit + 3;
+    return r;
+}
+
 
 __device__ __forceinline__ int dp2a_lo_su(uint32_t k, uint32_t px, int c) {
     int d;
@@ -136,110 +158,83 @@ __device__ __forceinline__ void walk_tile(const ResizeDev& p, const IntTaps& t, 
     const bool y16 = pl == 0 && p.y16 != nullptr;
     const size_t ostep = y16 ? p.pitch16 : p.pitch;
 
-                auto hsum = [&](int r, unsigned long long (&h)[4]) {
-                    const uint32_t* w = reinterpret_cast<const uint32_t*>(srow + r * kPitch);
-                    const uint32_t w0 = w[0], w1 = w[1], w2 = w[2];
-                    uint32_t lo = 0, hi = 0;
-                    if (S != 2) { lo = __funnelshift_r(w0, w1, wsh); hi = __funnelshift_r(w1, w2, wsh); }
-                    float f[8];
-    #pragma unroll
-                    for (int c = 0; c < 8; c++) {
-                        const int o = win_ofs<S>(c);
-                        uint32_t px4;
-                        if (S == 2) {                  // bytes cb + o .. + 3 straight from the three words (cb & 3 == 2)
-                            const int sh = 16 + 8 * o;
-                            px4 = sh < 32 ? __funnelshift_r(w0, w1, sh) : (sh == 32 ? w1 : __funnelshift_r(w1, w2, sh - 32));
-                        } else {
-                            px4 = o == 0 ? lo : (o == 4 ? hi : __funnelshift_r(lo, hi, 8 * o));
-                        }
-                        const int acc = dp2a_hi_su(t.hk23[c % S], px4, dp2a_lo_su(t.hk01[c % S], px4, 0x4B400000));
-                        f[c] = __int_as_float(acc);    // = 12582912 + sum, exactly
-                    }
-    #pragma unroll
-                    for (int q = 0; q < 4; q++) h[q] = f2_add_rn(f2_pack(f[2 * q], f[2 * q + 1]), mm);   // = (float)sum, exactly
-                };
+    auto hsum = [&](int r, unsigned long long (&h)[4]) {
+        const uint32_t* w = reinterpret_cast<const uint32_t*>(srow + r * kPitch);
+        const uint32_t w0 = w[0], w1 = w[1], w2 = w[2];
+        uint32_t lo = 0, hi = 0;
+        if (S != 2) { lo = __funnelshift_r(w0, w1, wsh); hi = __funnelshift_r(w1, w2, wsh); }
+        float f[8];
+#pragma unroll
+        for (int c = 0; c < 8; c++) {
+            const int o = win_ofs<S>(c);
+            uint32_t px4;
+            if (S == 2) {                  // bytes cb + o .. + 3 straight from the three words (cb & 3 == 2)
+                const int sh = 16 + 8 * o;
+                px4 = sh < 32 ? __funnelshift_r(w0, w1, sh) : (sh == 32 ? w1 : __funnelshift_r(w1, w2, sh - 32));
+            } else {
+                px4 = o == 0 ? lo : (o == 4 ? hi : __funnelshift_r(lo, hi, 8 * o));
+            }
+            const int acc = dp2a_hi_su(t.hk23[c % S], px4, dp2a_lo_su(t.hk01[c % S], px4, 0x4B400000));
+            f[c] = __int_as_float(acc);    // = 12582912 + sum, exactly
+        }
+#pragma unroll
+        for (int q = 0; q < 4; q++) h[q] = f2_add_rn(f2_pack(f[2 * q], f[2 * q + 1]), mm);   // = (float)sum, exactly
+    };
 
-                // running output pointer: row S*a + S/2 first, one row further per emitted row (dereferenced only for wanted rows)
-                int dy = S * a + S / 2;
-                uint8_t* outp;
-                if (y16) outp = p.y16 + fz * p.y16_frame + ((long long)dy - p.plane_row0) * (long long)p.pitch16 + 2 * (size_t)(x0 + kY16Pad);
-                else outp = (pl == 0 ? p.y : (pl == 1 ? p.cr : (NPL == 4 && pl == 3 ? pa : p.cb))) + fz * p.plane_frame + ((long long)dy - p.plane_row0) * (long long)p.pitch + x0;
-                uint8_t* const outp0 = outp;
+    // running output pointer: row S*a + S/2 first, one row further per emitted row (dereferenced only for wanted rows)
+    int dy = S * a + S / 2;
+    uint8_t* outp;
+    if (y16) outp = p.y16 + fz * p.y16_frame + ((long long)dy - p.plane_row0) * (long long)p.pitch16 + 2 * (size_t)(x0 + kY16Pad);
+    else outp = (pl == 0 ? p.y : (pl == 1 ? p.cr : (NPL == 4 && pl == 3 ? pa : p.cb))) + fz * p.plane_frame + ((long long)dy - p.plane_row0) * (long long)p.pitch + x0;
+    uint8_t* const outp0 = outp;
 
-                auto emit = [&](const unsigned long long (&h0)[4], const unsigned long long (&h1)[4], const unsigned long long (&h2)[4],
-                                const unsigned long long (&h3)[4]) {
-    #pragma unroll
-                    for (int m = 0; m < S; m++) {
-                        const int ph = (S / 2 + m) % S;
-                        const bool wanted = dy >= p.row_begin && dy < p.row_end;     // uniform; only the first / last row of tiles has unwanted rows
-                        uint32_t r[8];
-    #pragma unroll
-                        for (int q = 0; q < 4; q++) {
-                            unsigned long long v = f2_mul_rn(h3[q], t.vb[ph][3], nz);
-                            v = f2_add_rn(f2_mul_rn(h2[q], t.vb[ph][2], nz), v);
-                            v = f2_add_rn(f2_mul_rn(h1[q], t.vb[ph][1], nz), v);
-                            v = f2_add_rn(f2_mul_rn(h0[q], t.vb[ph][0], nz), v);
-                            float va, vb;
-                            f2_unpack(v, va, vb);
-                            r[2 * q] = sat_u8_rn(va);
-                            r[2 * q + 1] = sat_u8_rn(vb);
-                        }
-                        if (y16) {   // exact u8 -> FP16: 0x6400 | v is 1024 + v, minus 1024
-                            const __half2 k1024 = __float2half2_rn(1024.f);
-                            uint32_t hw[4];
-    #pragma unroll
-                            for (int q = 0; q < 4; q++) {
-                                uint32_t u = __byte_perm(r[2 * q], r[2 * q + 1], 0x5410) | 0x64006400u;   // bytes (r0, 0x64, r1, 0x64)
-                                __half2 hh = __hsub2(*reinterpret_cast<__half2*>(&u), k1024);
-                                hw[q] = *reinterpret_cast<uint32_t*>(&hh);
-                            }
-                            if (wanted) *reinterpret_cast<uint4*>(outp) = make_uint4(hw[0], hw[1], hw[2], hw[3]);
-                        } else {
-                            const uint32_t lo4 = __byte_perm(__byte_perm(r[0], r[1], 0x0040), __byte_perm(r[2], r[3], 0x0040), 0x5410);
-                            const uint32_t hi4 = __byte_perm(__byte_perm(r[4], r[5], 0x0040), __byte_perm(r[6], r[7], 0x0040), 0x5410);
-                            if (wanted) *reinterpret_cast<uint2*>(outp) = make_uint2(lo4, hi4);
-                        }
-                        dy++;
-                        outp += ostep;
-                    }
-                };
+    auto emit = [&](const unsigned long long (&h0)[4], const unsigned long long (&h1)[4], const unsigned long long (&h2)[4],
+                    const unsigned long long (&h3)[4]) {
+#pragma unroll
+        for (int m = 0; m < S; m++) {
+            const int ph = (S / 2 + m) % S;
+            const bool wanted = dy >= p.row_begin && dy < p.row_end;     // uniform; only the first / last row of tiles has unwanted rows
+            uint32_t r[8];
+#pragma unroll
+            for (int q = 0; q < 4; q++) {
+                float va, vb;
+                f2_unpack(f2_vtap(h0[q], h1[q], h2[q], h3[q], t.vb[ph][0], t.vb[ph][1], t.vb[ph][2], t.vb[ph][3], nz), va, vb);
+                r[2 * q] = sat_u8_rn(va);
+                r[2 * q + 1] = sat_u8_rn(vb);
+            }
+            if (y16) {
+                const uint4 hw = make_uint4(u8x2_to_h2(r[0], r[1]), u8x2_to_h2(r[2], r[3]), u8x2_to_h2(r[4], r[5]), u8x2_to_h2(r[6], r[7]));
+                if (wanted) *reinterpret_cast<uint4*>(outp) = hw;
+            } else {
+                const uint32_t lo4 = __byte_perm(__byte_perm(r[0], r[1], 0x0040), __byte_perm(r[2], r[3], 0x0040), 0x5410);
+                const uint32_t hi4 = __byte_perm(__byte_perm(r[4], r[5], 0x0040), __byte_perm(r[6], r[7], 0x0040), 0x5410);
+                if (wanted) *reinterpret_cast<uint2*>(outp) = make_uint2(lo4, hi4);
+            }
+            dy++;
+            outp += ostep;
+        }
+    };
 
-                unsigned long long hA[4], hB[4], hC[4], hD[4];
-                hsum(0, hA);
-                hsum(1, hB);
-                hsum(2, hC);
-                for (int tt = 0; tt < nit; tt += 4) {  // window rotation by unrolling, not by register moves
-                    hsum(tt + 3, hD);
-                    emit(hA, hB, hC, hD);
-                    if (tt + 1 >= nit) break;
-                    hsum(tt + 4, hA);
-                    emit(hB, hC, hD, hA);
-                    if (tt + 2 >= nit) break;
-                    hsum(tt + 5, hB);
-                    emit(hC, hD, hA, hB);
-                    if (tt + 3 >= nit) break;
-                    hsum(tt + 6, hC);
-                    emit(hD, hA, hB, hC);
-                }
+    walk_window<unsigned long long[4]>(nit, hsum, emit);
 
-                // FP16 plane: the replicated columns -8..-1 and W..W+7 (conv1 reads Y[clamp(c-4)], src/srcnn.cpp:279) -- by the two
-                // lanes that own the first / last eight columns of the image, from what they have just stored
-                if (y16 && (x0 == 0 || x0 + 8 == p.ow)) {
-                    int d = S * a + S / 2;
-                    uint8_t* o = outp0;
-                    for (int j = 0; j < nit * S; j++, d++, o += ostep) {
-                        if (d < p.row_begin || d >= p.row_end) continue;
-                        const uint4 v = *reinterpret_cast<const uint4*>(o);
-                        if (x0 == 0) {
-                            const uint32_t e = __byte_perm(v.x, 0, 0x1010);
-                            *reinterpret_cast<uint4*>(o - 2 * kY16Pad) = make_uint4(e, e, e, e);
-                        }
-                        if (x0 + 8 == p.ow) {
-                            const uint32_t e = __byte_perm(v.w, 0, 0x3232);
-                            *reinterpret_cast<uint4*>(o + 16) = make_uint4(e, e, e, e);
-                        }
-                    }
-                }
+    // FP16 plane: the replicated columns -8..-1 and W..W+7 (conv1 reads Y[clamp(c-4)], src/srcnn.cpp:279) -- by the two
+    // lanes that own the first / last eight columns of the image, from what they have just stored
+    if (y16 && (x0 == 0 || x0 + 8 == p.ow)) {
+        int d = S * a + S / 2;
+        uint8_t* o = outp0;
+        for (int j = 0; j < nit * S; j++, d++, o += ostep) {
+            if (d < p.row_begin || d >= p.row_end) continue;
+            const uint4 v = *reinterpret_cast<const uint4*>(o);
+            if (x0 == 0) {
+                const uint32_t e = __byte_perm(v.x, 0, 0x1010);
+                *reinterpret_cast<uint4*>(o - 2 * kY16Pad) = make_uint4(e, e, e, e);
+            }
+            if (x0 + 8 == p.ow) {
+                const uint32_t e = __byte_perm(v.w, 0, 0x3232);
+                *reinterpret_cast<uint4*>(o + 16) = make_uint4(e, e, e, e);
+            }
+        }
+    }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -251,14 +246,7 @@ __global__ void __launch_bounds__(96, S == 2 ? SRCNN_KA_MINB : SRCNN_KA_MINB4) k
     __shared__ __align__(16) uint8_t sP[3][kIRows][kIPitch];
     const int tid = threadIdx.x;
     const int tile = blockIdx.x;
-    const int bx = tile % t.ntx, rest = tile / t.ntx;
-    const int by = rest % t.nty;
-    const size_t fz = (size_t)(rest / t.nty);
-    const int X0 = bx * kITW;
-    const int a = t.a_first + by * t.isr;          // footprint row r is source row a - 1 + r
-    const int F0 = X0 / S - 4;                     // first footprint column (a multiple of 4: aligned 12-byte groups)
-    const int nit = min(t.isr, t.i_last - a + 1);
-    const int nsr = nit + 3;
+    const auto [fz, X0, a, F0, nit, nsr] = tile_pos<S>(t, tile, kITW);
     const uint8_t* const fsrc = p.src + fz * p.src_frame;
 
     // (1) colour-convert the footprint; replicate border applied here
@@ -336,14 +324,7 @@ __global__ void __launch_bounds__(128, S == 2 ? SRCNN_KA4_MINB : SRCNN_KA4_MINB4
     __shared__ __align__(16) uint8_t sP[4][kIRows][kIPitch];
     const int tid = threadIdx.x;
     const int tile = blockIdx.x;
-    const int bx = tile % t.ntx, rest = tile / t.ntx;
-    const int by = rest % t.nty;
-    const size_t fz = (size_t)(rest / t.nty);
-    const int X0 = bx * kITW;
-    const int a = t.a_first + by * t.isr;          // footprint row r is source row a - 1 + r
-    const int F0 = X0 / S - 4;                     // first footprint column (a multiple of 4: 16-byte aligned groups)
-    const int nit = min(t.isr, t.i_last - a + 1);
-    const int nsr = nit + 3;
+    const auto [fz, X0, a, F0, nit, nsr] = tile_pos<S>(t, tile, kITW);
     const uint8_t* const fsrc = p.src + fz * p.src_frame;
     const bool swap = p.swapRB;
 
@@ -405,73 +386,16 @@ __global__ void __launch_bounds__(128, S == 2 ? SRCNN_KA4_MINB : SRCNN_KA4_MINB4
 // ------------------------------------------------------------------------------------------------
 constexpr int kGPitch = 400;       // bytes per staged row: 3 * 128 + 8 columns at x2 (98 words) + the spare word of the window read
 
-template <int S>
-__global__ void __launch_bounds__(96, S == 2 ? SRCNN_KA_MINB : SRCNN_KA_MINB4) k_gray_bicubic_int(const ResizeDev p, const IntTaps t) {
-    constexpr int GG = 3 * kITW / S / 4 + 2;       // four-byte groups per staged row
-    static_assert(4 * GG + 4 <= kGPitch, "staged row too short");
-    __shared__ __align__(16) uint8_t sP[kIRows][kGPitch];
-    const int tid = threadIdx.x;
-    const int tile = blockIdx.x;
-    const int bx = tile % t.ntx, rest = tile / t.ntx;
-    const int by = rest % t.nty;
-    const size_t fz = (size_t)(rest / t.nty);
-    const int X0 = 3 * kITW * bx;                  // first column of warp 0's tile
-    const int a = t.a_first + by * t.isr;          // staged row r is source row a - 1 + r
-    const int F0 = X0 / S - 4;                     // first staged column (a multiple of 4)
-    const int nit = min(t.isr, t.i_last - a + 1);
-    const int nsr = nit + 3;
-    const uint8_t* const fsrc = p.src + fz * p.src_frame;
-
-    // (1) stage the footprint: all of a thread's loads go out before its first shared store
-    constexpr int NG = (kIRows * GG + 95) / 96;
-    uint32_t raw[NG];
-#pragma unroll
-    for (int it = 0; it < NG; it++) {
-        const int g = tid + 96 * it;
-        if (g < nsr * GG) {
-            const int r = g / GG, gx = F0 + 4 * (g - r * GG);
-            const uint8_t* row = fsrc + (size_t)(clampi(a - 1 + r, 0, p.sh - 1) - p.src_row0) * p.src_stride;
-            if (t.vec_ok && gx >= 0 && gx + 4 <= p.sw) {
-                raw[it] = *reinterpret_cast<const uint32_t*>(row + gx);
-            } else {
-                uint32_t v = 0;
-#pragma unroll
-                for (int j = 0; j < 4; j++) v |= (uint32_t)row[clampi(gx + j, 0, p.sw - 1)] << (8 * j);
-                raw[it] = v;
-            }
-        }
-    }
-#pragma unroll
-    for (int it = 0; it < NG; it++) {
-        const int g = tid + 96 * it;
-        if (g < nsr * GG) {
-            const int r = g / GG;
-            *reinterpret_cast<uint32_t*>(&sP[r][4 * (g - r * GG)]) = raw[it];
-        }
-    }
-    __syncthreads();
-    // (2) the walk: warp w's tile starts w * kITW / S staged columns further
-    const int w = tid >> 5;
-    walk_tile<S, kGPitch>(p, t, &sP[0][w * (kITW / S)], 0, tid & 31, X0 + w * kITW, a, nit, fz);
-}
-
-// The grey kernel's tile as a device function, for k_yuv420_bicubic_int and k_yuv422_bicubic_int below.  k_gray_bicubic_int keeps
-// its own copy of these lines: calling this function from it compiles to different SASS.
-// kPacked: 0 = a plane of bytes; 1 / 2 = the Y bytes of packed 4:2:2 rows (YUY2: bytes 0, 2 of each macropixel; UYVY: 1, 3): a
-// four-pixel group is 8 source bytes (one 64-bit load when t.vec_ok == 2, two 32-bit loads when 1) and one byte permutation.
-template <int S, int kPacked = 0>
+// The grey kernel's tile `tile`, also the luma tile of k_yuv_bicubic_int.  L = SRCNN_ORDER_YUY2 / _UYVY: the Y bytes of packed
+// 4:2:2 rows (YUY2: bytes 0, 2 of each macropixel; UYVY: 1, 3): a four-pixel group is 8 source bytes (one 64-bit load when
+// t.vec_ok == 2, two 32-bit loads when 1) and one byte permutation.  Any other L: a plane of bytes.
+template <int S, int L>
 __device__ __forceinline__ void gray_tile(const ResizeDev& p, const IntTaps& t, int tile, uint8_t (&sP)[kIRows][kGPitch]) {
+    constexpr bool k422 = L == SRCNN_ORDER_YUY2 || L == SRCNN_ORDER_UYVY, kUYVY = L == SRCNN_ORDER_UYVY;
     constexpr int GG = 3 * kITW / S / 4 + 2;       // four-byte groups per staged row
     static_assert(4 * GG + 4 <= kGPitch, "staged row too short");
     const int tid = threadIdx.x;
-    const int bx = tile % t.ntx, rest = tile / t.ntx;
-    const int by = rest % t.nty;
-    const size_t fz = (size_t)(rest / t.nty);
-    const int X0 = 3 * kITW * bx;                  // first column of warp 0's tile
-    const int a = t.a_first + by * t.isr;          // staged row r is source row a - 1 + r
-    const int F0 = X0 / S - 4;                     // first staged column (a multiple of 4)
-    const int nit = min(t.isr, t.i_last - a + 1);
-    const int nsr = nit + 3;
+    const auto [fz, X0, a, F0, nit, nsr] = tile_pos<S>(t, tile, 3 * kITW);   // X0: first column of warp 0's tile
     const uint8_t* const fsrc = p.src + fz * p.src_frame;
 
     // (1) stage the footprint: all of a thread's loads go out before its first shared store
@@ -484,7 +408,7 @@ __device__ __forceinline__ void gray_tile(const ResizeDev& p, const IntTaps& t, 
             const int r = g / GG, gx = F0 + 4 * (g - r * GG);
             const uint8_t* row = fsrc + (size_t)(clampi(a - 1 + r, 0, p.sh - 1) - p.src_row0) * p.src_stride;
             if (t.vec_ok && gx >= 0 && gx + 4 <= p.sw) {
-                if (kPacked == 0) {
+                if (!k422) {
                     raw[it] = *reinterpret_cast<const uint32_t*>(row + gx);
                 } else {
                     const uint8_t* px = row + 2 * (size_t)gx;
@@ -495,14 +419,14 @@ __device__ __forceinline__ void gray_tile(const ResizeDev& p, const IntTaps& t, 
                     } else {
                         w0 = reinterpret_cast<const uint32_t*>(px)[0]; w1 = reinterpret_cast<const uint32_t*>(px)[1];
                     }
-                    raw[it] = __byte_perm(w0, w1, kPacked == 2 ? 0x7531 : 0x6420);
+                    raw[it] = __byte_perm(w0, w1, kUYVY ? 0x7531 : 0x6420);
                 }
             } else {
                 uint32_t v = 0;
 #pragma unroll
                 for (int j = 0; j < 4; j++) {
                     const int x = clampi(gx + j, 0, p.sw - 1);
-                    v |= (uint32_t)row[kPacked == 0 ? x : 2 * x + (kPacked == 2)] << (8 * j);
+                    v |= (uint32_t)row[!k422 ? x : 2 * x + kUYVY] << (8 * j);
                 }
                 raw[it] = v;
             }
@@ -522,25 +446,28 @@ __device__ __forceinline__ void gray_tile(const ResizeDev& p, const IntTaps& t, 
     walk_tile<S, kGPitch>(p, t, &sP[0][w * (kITW / S)], 0, tid & 31, X0 + w * kITW, a, nit, fz);
 }
 
-// ------------------------------------------------------------------------------------------------
-// 4:2:0 frames (SRCNN_ORDER_NV12 / _I420): ONE launch for luma and chroma.  CTAs [0, t.ntiles) are k_gray_bicubic_int's tiles
-// of the Y plane (into the workspace plane the CNN reads); the rest are chroma tiles, written straight into the caller's output
-// (no chroma workspace, no CNN).  A chroma CTA is three warps on three adjacent 128-column tiles whose footprints are staged
-// once, like the grey kernel's, as two shared-memory planes U and V: NV12's pairs are split with two byte permutations per
-// four columns, I420's planes are staged as they are.  A lane owns the SAME 4 columns of both planes, so the 8 horizontal
-// sums per footprint row, the four-row register window and the vertical pass are those of walk_tile (which gives a lane 8
-// columns of one plane); per output row it stores U0 V0 U1 V1 U2 V2 U3 V3 (NV12, one 8-byte store) or four bytes into each
-// plane (I420).  Launch conditions: ow/2 a multiple of 8, chroma rows of the output 8-byte aligned.
-// ------------------------------------------------------------------------------------------------
-#ifndef SRCNN_KA420_MINB
-#define SRCNN_KA420_MINB SRCNN_KA_MINB
-#endif
-#ifndef SRCNN_KA420_MINB4
-#define SRCNN_KA420_MINB4 SRCNN_KA_MINB4
-#endif
+template <int S>
+__global__ void __launch_bounds__(96, S == 2 ? SRCNN_KA_MINB : SRCNN_KA_MINB4) k_gray_bicubic_int(const ResizeDev p, const IntTaps t) {
+    __shared__ __align__(16) uint8_t sP[kIRows][kGPitch];
+    gray_tile<S, SRCNN_ORDER_GRAY>(p, t, blockIdx.x, sP);
+}
 
+// ------------------------------------------------------------------------------------------------
+// 4:2:0 and packed 4:2:2 frames (SRCNN_ORDER_NV12 / _I420 / _YUY2 / _UYVY, the layout L): ONE launch for luma and chroma.  CTAs
+// [0, t.ntiles) are the grey kernel's tiles of the Y plane (gray_tile, into the workspace plane the CNN reads); the rest are
+// chroma tiles.  A chroma CTA is three warps on three adjacent 128-column tiles whose footprints are staged once, like the grey
+// kernel's, as two shared-memory planes U and V: NV12's pairs are split with two byte permutations per four columns, I420's
+// planes are staged as they are, packed 4:2:2 rows give the U and V words of four columns with four byte permutations.  A lane
+// owns the SAME 4 columns of both planes, so the 8 horizontal sums per footprint row, the four-row register window and the
+// vertical pass are those of walk_tile (which gives a lane 8 columns of one plane); per output row it stores U0 V0 U1 V1 U2 V2
+// U3 V3 (NV12, one 8-byte store) or four bytes into each plane.  4:2:0 chroma goes straight into the caller's output (no chroma
+// workspace, no CNN); 4:2:2 chroma into the workspace's Cr (U') and Cb (V') planes, which the pack kernel (K-C) reads.  The 4:2:2
+// chroma plane is w/2 x h -> ow/2 x oh: x S on both axes, so its vertical taps are the luma ones.  Launch conditions: luma and
+// chroma widths multiples of 8, 8-byte aligned luma stores, chroma stores 8-byte (4:2:0) or 4-byte (4:2:2: always true of the
+// workspace) aligned.
+// ------------------------------------------------------------------------------------------------
 struct ChromaDev {
-    const uint8_t* src;               // chroma row 0 of frame 0 (NV12: pairs; I420: U)
+    const uint8_t* src;               // chroma row 0 of frame 0 (NV12: pairs; I420: U; 4:2:2: the packed rows)
     size_t src_pitch, src_v, src_frame;
     uint8_t* dst;
     size_t dst_pitch, dst_v, dst_frame;
@@ -553,9 +480,10 @@ struct CGeo {
     static constexpr int kPitch = (4 * G + 4 + 15) / 16 * 16;      // + the spare word of the window read
 };
 
-template <int S, bool kNV12>
+template <int S, int L>
 __device__ __forceinline__ void walk_pair(const ChromaDev& q, const IntTaps& t, unsigned long long nz, const uint8_t* su,
                                           const uint8_t* sv, int lane, int X0, int a, int nit, size_t fz) {
+    constexpr bool kNV12 = L == SRCNN_ORDER_NV12;
     constexpr int kPitch = CGeo<S>::kPitch;
     const int x0 = X0 + 4 * lane;
     if (x0 >= q.ow) return;                        // ow/2 is a multiple of 8 (launch condition)
@@ -594,12 +522,8 @@ __device__ __forceinline__ void walk_pair(const ChromaDev& q, const IntTaps& t, 
             uint32_t r[8];
 #pragma unroll
             for (int k = 0; k < 4; k++) {
-                unsigned long long v = f2_mul_rn(h3[k], t.vb[ph][3], nz);
-                v = f2_add_rn(f2_mul_rn(h2[k], t.vb[ph][2], nz), v);
-                v = f2_add_rn(f2_mul_rn(h1[k], t.vb[ph][1], nz), v);
-                v = f2_add_rn(f2_mul_rn(h0[k], t.vb[ph][0], nz), v);
                 float va, vb;
-                f2_unpack(v, va, vb);
+                f2_unpack(f2_vtap(h0[k], h1[k], h2[k], h3[k], t.vb[ph][0], t.vb[ph][1], t.vb[ph][2], t.vb[ph][3], nz), va, vb);
                 r[2 * k] = sat_u8_rn(va);
                 r[2 * k + 1] = sat_u8_rn(vb);
             }
@@ -620,42 +544,19 @@ __device__ __forceinline__ void walk_pair(const ChromaDev& q, const IntTaps& t, 
         }
     };
 
-    unsigned long long hA[4], hB[4], hC[4], hD[4];
-    hsum(0, hA);
-    hsum(1, hB);
-    hsum(2, hC);
-    for (int tt = 0; tt < nit; tt += 4) {
-        hsum(tt + 3, hD);
-        emit(hA, hB, hC, hD);
-        if (tt + 1 >= nit) break;
-        hsum(tt + 4, hA);
-        emit(hB, hC, hD, hA);
-        if (tt + 2 >= nit) break;
-        hsum(tt + 5, hB);
-        emit(hC, hD, hA, hB);
-        if (tt + 3 >= nit) break;
-        hsum(tt + 6, hC);
-        emit(hD, hA, hB, hC);
-    }
+    walk_window<unsigned long long[4]>(nit, hsum, emit);
 }
 
-// kPacked: 0 = the 4:2:0 chroma rows of kNV12; 1 / 2 = packed 4:2:2 rows (kNV12 false), U and V at bytes 1, 3 (YUY2) or 0, 2
-// (UYVY) of each macropixel: a four-column group is 16 source bytes (two 64-bit or four 32-bit loads, per t.vec_ok) and four
-// byte permutations for both planes.
-template <int S, bool kNV12, int kPacked = 0>
+// 4:2:2 rows (L = SRCNN_ORDER_YUY2 / _UYVY): U and V at bytes 1, 3 (YUY2) or 0, 2 (UYVY) of each macropixel, a four-column group
+// is 16 source bytes (two 64-bit or four 32-bit loads, per t.vec_ok) and four byte permutations for both planes.
+template <int S, int L>
 __device__ __forceinline__ void chroma_tile(const ChromaDev& q, const IntTaps& t, unsigned long long nz, int tile, uint8_t* smem) {
+    constexpr bool kNV12 = L == SRCNN_ORDER_NV12, k422 = L == SRCNN_ORDER_YUY2 || L == SRCNN_ORDER_UYVY, kUYVY = L == SRCNN_ORDER_UYVY;
     constexpr int G = CGeo<S>::G, kPitch = CGeo<S>::kPitch;
     uint8_t (*sU)[kPitch] = reinterpret_cast<uint8_t (*)[kPitch]>(smem);
     uint8_t (*sV)[kPitch] = sU + kIRows;
     const int tid = threadIdx.x;
-    const int bx = tile % t.ntx, rest = tile / t.ntx;
-    const int by = rest % t.nty;
-    const size_t fz = (size_t)(rest / t.nty);
-    const int X0 = 3 * kCW * bx;                   // first chroma column of warp 0's tile
-    const int a = t.a_first + by * t.isr;          // staged row r is chroma source row a - 1 + r
-    const int F0 = X0 / S - 4;                     // first staged column (a multiple of 4)
-    const int nit = min(t.isr, t.i_last - a + 1);
-    const int nsr = nit + 3;
+    const auto [fz, X0, a, F0, nit, nsr] = tile_pos<S>(t, tile, 3 * kCW);    // X0: first chroma column of warp 0's tile
     const uint8_t* const fsrc = q.src + fz * q.src_frame;
 
     // (1) stage both footprints: all of a thread's loads go out before its first shared store
@@ -668,7 +569,7 @@ __device__ __forceinline__ void chroma_tile(const ChromaDev& q, const IntTaps& t
             const int r = g / G, gx = F0 + 4 * (g - r * G);
             const uint8_t* row = fsrc + (size_t)clampi(a - 1 + r, 0, q.sh - 1) * q.src_pitch;
             if (t.vec_ok && gx >= 0 && gx + 4 <= q.sw) {
-                if (kPacked) {
+                if (k422) {
                     const uint8_t* px = row + 4 * (size_t)gx;
                     uint32_t w[4];
                     if (t.vec_ok == 2) {
@@ -678,7 +579,7 @@ __device__ __forceinline__ void chroma_tile(const ChromaDev& q, const IntTaps& t
 #pragma unroll
                         for (int k = 0; k < 4; k++) w[k] = reinterpret_cast<const uint32_t*>(px)[k];
                     }
-                    constexpr unsigned kSel = kPacked == 2 ? 0x6240 : 0x7351;    // (U0 U1 V0 V1) of two macropixels
+                    constexpr unsigned kSel = kUYVY ? 0x6240 : 0x7351;    // (U0 U1 V0 V1) of two macropixels
                     const uint32_t lo = __byte_perm(w[0], w[1], kSel), hi = __byte_perm(w[2], w[3], kSel);
                     ru[it] = __byte_perm(lo, hi, 0x5410);
                     rv[it] = __byte_perm(lo, hi, 0x7632);
@@ -696,9 +597,9 @@ __device__ __forceinline__ void chroma_tile(const ChromaDev& q, const IntTaps& t
 #pragma unroll
                 for (int j = 0; j < 4; j++) {
                     const int x = clampi(gx + j, 0, q.sw - 1);
-                    if (kPacked) {
-                        u |= (uint32_t)row[4 * x + (kPacked == 1)] << (8 * j);
-                        v |= (uint32_t)row[4 * x + (kPacked == 1) + 2] << (8 * j);
+                    if (k422) {
+                        u |= (uint32_t)row[4 * x + !kUYVY] << (8 * j);
+                        v |= (uint32_t)row[4 * x + !kUYVY + 2] << (8 * j);
                     } else {
                         u |= (uint32_t)(kNV12 ? row[2 * x] : row[x]) << (8 * j);
                         v |= (uint32_t)(kNV12 ? row[2 * x + 1] : row[q.src_v + x]) << (8 * j);
@@ -721,45 +622,21 @@ __device__ __forceinline__ void chroma_tile(const ChromaDev& q, const IntTaps& t
     __syncthreads();
     // (2) the walk: warp w's tile starts w * kCW / S staged columns further
     const int w = tid >> 5;
-    walk_pair<S, kNV12>(q, t, nz, &sU[0][w * (kCW / S)], &sV[0][w * (kCW / S)], tid & 31, X0 + w * kCW, a, nit, fz);
+    walk_pair<S, L>(q, t, nz, &sU[0][w * (kCW / S)], &sV[0][w * (kCW / S)], tid & 31, X0 + w * kCW, a, nit, fz);
 }
 
-template <int S, bool kNV12>
-__global__ void __launch_bounds__(96, S == 2 ? SRCNN_KA420_MINB : SRCNN_KA420_MINB4) k_yuv420_bicubic_int(const ResizeDev p, const IntTaps t,
-                                                                                                        const ChromaDev q, const IntTaps tc) {
-    constexpr int kLuma = kIRows * kGPitch, kChroma = 2 * kIRows * CGeo<S>::kPitch;
-    __shared__ __align__(16) uint8_t sm[kLuma > kChroma ? kLuma : kChroma];
-    if ((int)blockIdx.x < t.ntiles) gray_tile<S>(p, t, blockIdx.x, *reinterpret_cast<uint8_t (*)[kIRows][kGPitch]>(sm));
-    else chroma_tile<S, kNV12>(q, tc, p.negzero2, (int)blockIdx.x - t.ntiles, sm);
-}
-
-// ------------------------------------------------------------------------------------------------
-// Packed 4:2:2 frames (SRCNN_ORDER_YUY2 / _UYVY): ONE launch for luma and chroma, like k_yuv420_bicubic_int.  CTAs [0, t.ntiles)
-// are the grey kernel's tiles of the Y plane (into the workspace plane the CNN reads), staged by de-interleaving the packed rows
-// (gray_tile, kPacked); the rest are chroma tiles: U and V staged as two shared-memory planes from the same packed rows, walked
-// as in a 4:2:0 chroma tile (a lane owns the same 4 columns of both), written as four bytes per lane and row into the workspace's
-// Cr (U') and Cb (V') planes, which the pack kernel (K-C) reads.  The chroma plane is w/2 x h -> ow/2 x oh: x S on both axes, so
-// its vertical taps are the luma ones.  Launch conditions: ow a multiple of 16 (luma and chroma widths multiples of 8), 8-byte
-// aligned luma stores and 4-byte aligned chroma stores (always true of the workspace).  Unlike a 4:2:0 call this call may start
-// beside the previous call's merge / pack kernel (api.cu, may_start_early): the last CTA waits for it, as in k_color_bicubic_int.
-// ------------------------------------------------------------------------------------------------
-#ifndef SRCNN_KA422_MINB
-#define SRCNN_KA422_MINB SRCNN_KA_MINB
-#endif
-#ifndef SRCNN_KA422_MINB4
-#define SRCNN_KA422_MINB4 SRCNN_KA_MINB4
-#endif
-
-template <int S, bool kUYVY>
-__global__ void __launch_bounds__(96, S == 2 ? SRCNN_KA422_MINB : SRCNN_KA422_MINB4) k_yuv422_bicubic_int(const ResizeDev p, const IntTaps t,
-                                                                                                        const ChromaDev q, const IntTaps tc) {
-    constexpr int kPacked = kUYVY ? 2 : 1;
+template <int S, int L>
+__global__ void __launch_bounds__(96, S == 2 ? SRCNN_KA_MINB : SRCNN_KA_MINB4) k_yuv_bicubic_int(const ResizeDev p, const IntTaps t,
+                                                                                               const ChromaDev q, const IntTaps tc) {
     constexpr int kLuma = kIRows * kGPitch, kChroma = 2 * kIRows * CGeo<S>::kPitch;
     __shared__ __align__(16) uint8_t sm[kLuma > kChroma ? kLuma : kChroma];
     const int b = (int)blockIdx.x;
-    if (b < t.ntiles) gray_tile<S, kPacked>(p, t, b, *reinterpret_cast<uint8_t (*)[kIRows][kGPitch]>(sm));
-    else chroma_tile<S, false, kPacked>(q, tc, p.negzero2, b - t.ntiles, sm);
-    if (b == t.ntiles + tc.ntiles - 1) asm volatile("griddepcontrol.wait;" ::: "memory");
+    if (b < t.ntiles) gray_tile<S, L>(p, t, b, *reinterpret_cast<uint8_t (*)[kIRows][kGPitch]>(sm));
+    else chroma_tile<S, L>(q, tc, p.negzero2, b - t.ntiles, sm);
+    // A 4:2:2 call may start beside the previous call's merge / pack kernel (api.cu, may_start_early): the last CTA waits for it,
+    // as in k_color_bicubic_int.  A 4:2:0 call never starts early (it launches no merge), and leaves the wait out.
+    if constexpr (L == SRCNN_ORDER_YUY2 || L == SRCNN_ORDER_UYVY)
+        if (b == t.ntiles + tc.ntiles - 1) asm volatile("griddepcontrol.wait;" ::: "memory");
 }
 
 inline int floordiv(int a, int b) { return a >= 0 ? a / b : -((-a + b - 1) / b); }
@@ -787,33 +664,66 @@ int launch_ka(Ctx* c, K kern, int grid, int threads, bool early, const A&... arg
     return SRCNN_OK;
 }
 
-// NP = planes: 1 grey, 3 colour, 4 colour + alpha (pa)
-template <int S, int NP>
-int launch_variant(Ctx* c, const ResizeDev& p, IntTaps& t, uint8_t* pa, int nframes, bool early) {
-    constexpr int kThreads = NP == 4 ? 128 : 96;
-    static int ctas_per_sm[64] = {0};              // per device; a benign race: every writer stores the same value
+// The tiles of one launch of kernel K (kThreads threads per CTA): tile height, rows of tiles and tile count of t, and of tc when
+// the launch also has chroma tiles (the same height; their CTAs follow t's).  *ok = false when the launch would have more tiles
+// than the kernels index: the geometry is not eligible, and the caller falls back to the generic kernels.
+template <auto K, int kThreads>
+int plan_tiles(Ctx* c, int nframes, IntTaps& t, IntTaps* tc, bool* ok) {
+    static int ctas_per_sm[64] = {};               // per kernel instance and device; a benign race: every writer stores the same value
     int& per_sm = ctas_per_sm[c->device & 63];
     if (per_sm == 0) {
         int n = 0;
-        if (NP == 4) SRCNN_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, k_color4_bicubic_int<S>, kThreads, 0));
-        else SRCNN_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, NP == 1 ? k_gray_bicubic_int<S> : k_color_bicubic_int<S>, kThreads, 0));
+        SRCNN_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, K, kThreads, 0));
         per_sm = std::max(1, n);
     }
     // Tile height (same-box A/B, B200): a single 4K frame runs fastest as ~1.5 waves of 8-row tiles (23.6 us; 6 rows: 23.7,
     // 4 rows: 25.1, 12 rows: 25.5, 16 rows = one wave: 27.6 -- the CTAs of one wave wait for their source rows together, and the
     // last wave's tiles run at half occupancy for a whole tile life); launches of many waves (batches, 16K frames, gigapixel
-    // bands) take 16-row tiles for the smaller apron (7.5 vs 7.8 ms for 1024 720p frames).
+    // bands) take 16-row tiles for the smaller apron (7.5 vs 7.8 ms for 1024 720p frames).  Luma and chroma tiles count together.
     const int resident = per_sm * std::max(1, c->sm_count);
-    const int nrows = t.i_last - t.a_first + 1;
-    auto tiles_for = [&](int isr) { return (long long)t.ntx * ((nrows + isr - 1) / isr) * nframes; };
+    const int nrows = t.i_last - t.a_first + 1, crows = tc ? tc->i_last - tc->a_first + 1 : 0;
+    auto tiles_for = [&](int isr) {
+        return ((long long)t.ntx * ((nrows + isr - 1) / isr) + (tc ? (long long)tc->ntx * ((crows + isr - 1) / isr) : 0)) * nframes;
+    };
     t.isr = tiles_for(kISRMax) > 2LL * resident ? kISRMax : 8;
     if (c->ka_int_isr >= 4 && c->ka_int_isr <= kISRMax) t.isr = c->ka_int_isr;
-    const long long ntiles = tiles_for(t.isr);
-    if (ntiles > 0x3fffffffLL) return SRCNN_E_ARG;
+    *ok = tiles_for(t.isr) <= 0x3fffffffLL;
+    if (!*ok) return SRCNN_OK;
     t.nty = (nrows + t.isr - 1) / t.isr;
-    t.ntiles = (int)ntiles;
-    if (NP == 4) return launch_ka(c, k_color4_bicubic_int<S>, t.ntiles, kThreads, early, p, t, pa);
-    return launch_ka(c, NP == 1 ? k_gray_bicubic_int<S> : k_color_bicubic_int<S>, t.ntiles, kThreads, early, p, t);
+    t.ntiles = t.ntx * t.nty * nframes;
+    if (tc) {
+        tc->isr = t.isr;
+        tc->nty = (crows + tc->isr - 1) / tc->isr;
+        tc->ntiles = tc->ntx * tc->nty * nframes;
+    }
+    return SRCNN_OK;
+}
+
+// NP = planes: 1 grey, 3 colour, 4 colour + alpha (pa)
+template <int S, int NP>
+int launch_variant(Ctx* c, const ResizeDev& p, IntTaps& t, uint8_t* pa, int nframes, bool early, bool* done) {
+    bool ok = false;
+    int rc;
+    if constexpr (NP == 4) {
+        if ((rc = plan_tiles<k_color4_bicubic_int<S>, 128>(c, nframes, t, nullptr, &ok)) || !ok) return rc;
+        rc = launch_ka(c, k_color4_bicubic_int<S>, t.ntiles, 128, early, p, t, pa);
+    } else {
+        constexpr auto kern = NP == 1 ? k_gray_bicubic_int<S> : k_color_bicubic_int<S>;
+        if ((rc = plan_tiles<kern, 96>(c, nframes, t, nullptr, &ok)) || !ok) return rc;
+        rc = launch_ka(c, kern, t.ntiles, 96, early, p, t);
+    }
+    *done = rc == SRCNN_OK;
+    return rc;
+}
+
+template <int S, int L>
+int launch_yuv(Ctx* c, const ResizeDev& p, IntTaps& t, const ChromaDev& q, IntTaps& tc, int nframes, bool early, bool* done) {
+    bool ok = false;
+    int rc;
+    if ((rc = plan_tiles<k_yuv_bicubic_int<S, L>, 96>(c, nframes, t, &tc, &ok)) || !ok) return rc;
+    rc = launch_ka(c, k_yuv_bicubic_int<S, L>, t.ntiles + tc.ntiles, 96, early, p, t, q, tc);
+    *done = rc == SRCNN_OK;
+    return rc;
 }
 
 // the constant tap phases of an integer scale S and the source rows whose output rows [row_begin, row_end) are wanted
@@ -836,112 +746,43 @@ void int_taps(const TapTable* tx, const TapTable* ty, int S, int row_begin, int 
 
 }  // namespace
 
-int launch_yuv420_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bool* done) {
+int launch_yuv_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bool* done) {
     *done = false;
     const Chroma420& ch = a.ch;
+    const bool p422 = yuv422(a.order);
     const int S = a.tx->int_scale;
     if (S == 0 || a.ty->int_scale != S || ch.tx->int_scale != S || ch.ty->int_scale != S) return SRCNN_OK;
     if ((a.ow & 7) || (ch.ow & 7) || a.row_end <= a.row_begin || ch.row_end <= ch.row_begin) return SRCNN_OK;
-    // stores: luma as in a grey call; chroma 8 bytes (NV12) or 2 x 4 bytes (I420) per lane and row, 8-byte aligned chroma rows
+    // stores: luma as in a grey call; chroma 8 bytes (NV12) or 2 x 4 bytes per lane and row, 8-byte aligned chroma rows for 4:2:0
     if ((((uintptr_t)p.y | p.pitch | p.plane_frame) & 7) != 0) return SRCNN_OK;
     if (p.y16 && (((uintptr_t)p.y16 | p.pitch16 | p.y16_frame) & 15) != 0) return SRCNN_OK;
-    if ((((uintptr_t)ch.dst | ch.dst_pitch | ch.dst_v | ch.dst_frame) & 7) != 0) return SRCNN_OK;
-    const bool nv12 = a.order == SRCNN_ORDER_NV12;
-    const int nframes = std::max(1, a.nframes);
+    if ((((uintptr_t)ch.dst | ch.dst_pitch | ch.dst_v | ch.dst_frame) & (p422 ? 3 : 7)) != 0) return SRCNN_OK;
 
     IntTaps t = {}, tc = {};
     int_taps(a.tx, a.ty, S, a.row_begin, a.row_end, t);
     int_taps(ch.tx, ch.ty, S, ch.row_begin, ch.row_end, tc);
-    t.vec_ok = (((uintptr_t)p.src | p.src_stride | p.src_frame) & 3) == 0;
-    tc.vec_ok = (((uintptr_t)ch.src | ch.src_pitch | ch.src_v | p.src_frame) & 3) == 0;
+    if (p422) {   // both tile kinds read the same packed rows: 64-bit group loads when they are 8-byte aligned, 32-bit when 4-byte aligned
+        const uintptr_t al = (uintptr_t)p.src | p.src_stride | p.src_frame | (uintptr_t)ch.src | ch.src_pitch;
+        t.vec_ok = tc.vec_ok = (al & 7) == 0 ? 2 : ((al & 3) == 0 ? 1 : 0);
+    } else {
+        t.vec_ok = (((uintptr_t)p.src | p.src_stride | p.src_frame) & 3) == 0;
+        tc.vec_ok = (((uintptr_t)ch.src | ch.src_pitch | ch.src_v | p.src_frame) & 3) == 0;
+    }
     t.ntx = ((a.ow + kITW - 1) / kITW + 2) / 3;    // a CTA per three adjacent tiles, as in a grey call
     tc.ntx = (ch.ow + 3 * kCW - 1) / (3 * kCW);
-    auto kern = S == 2 ? (nv12 ? k_yuv420_bicubic_int<2, true> : k_yuv420_bicubic_int<2, false>)
-                       : (nv12 ? k_yuv420_bicubic_int<4, true> : k_yuv420_bicubic_int<4, false>);
-    static int ctas_per_sm[4][64] = {};            // per instance and device; a benign race: every writer stores the same value
-    int& per_sm = ctas_per_sm[(S == 4) * 2 + nv12][c->device & 63];
-    if (per_sm == 0) {
-        int n = 0;
-        SRCNN_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kern, 96, 0));
-        per_sm = std::max(1, n);
-    }
-    // tile height: the rule of launch_variant over the launch's luma and chroma tiles together
-    const int resident = per_sm * std::max(1, c->sm_count);
-    const int nrows = t.i_last - t.a_first + 1, crows = tc.i_last - tc.a_first + 1;
-    auto tiles_for = [&](int isr) {
-        return ((long long)t.ntx * ((nrows + isr - 1) / isr) + (long long)tc.ntx * ((crows + isr - 1) / isr)) * nframes;
-    };
-    t.isr = tiles_for(kISRMax) > 2LL * resident ? kISRMax : 8;
-    if (c->ka_int_isr >= 4 && c->ka_int_isr <= kISRMax) t.isr = c->ka_int_isr;
-    tc.isr = t.isr;
-    if (tiles_for(t.isr) > 0x3fffffffLL) return SRCNN_OK;
-    t.nty = (nrows + t.isr - 1) / t.isr;
-    tc.nty = (crows + tc.isr - 1) / tc.isr;
-    t.ntiles = t.ntx * t.nty * nframes;
-    tc.ntiles = tc.ntx * tc.nty * nframes;
     ChromaDev q;
     q.src = ch.src; q.src_pitch = ch.src_pitch; q.src_v = ch.src_v; q.src_frame = p.src_frame;
     q.dst = ch.dst; q.dst_pitch = ch.dst_pitch; q.dst_v = ch.dst_v; q.dst_frame = ch.dst_frame;
     q.sw = ch.sw; q.sh = ch.sh; q.ow = ch.ow; q.row_begin = ch.row_begin; q.row_end = ch.row_end;
-    // never early: a 4:2:0 call launches no merge (api.cu)
-    const int rc = launch_ka(c, kern, t.ntiles + tc.ntiles, 96, false, p, t, q, tc);
-    if (rc) return rc;
-    *done = true;
-    return SRCNN_OK;
-}
-
-int launch_yuv422_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bool* done) {
-    *done = false;
-    const Chroma420& ch = a.ch;
-    const int S = a.tx->int_scale;
-    if (S == 0 || a.ty->int_scale != S || ch.tx->int_scale != S || ch.ty->int_scale != S) return SRCNN_OK;
-    if ((a.ow & 15) || a.row_end <= a.row_begin || ch.row_end <= ch.row_begin) return SRCNN_OK;
-    // stores: luma as in a grey call; chroma 4 bytes per plane, lane and row
-    if ((((uintptr_t)p.y | p.pitch | p.plane_frame) & 7) != 0) return SRCNN_OK;
-    if (p.y16 && (((uintptr_t)p.y16 | p.pitch16 | p.y16_frame) & 15) != 0) return SRCNN_OK;
-    if ((((uintptr_t)ch.dst | ch.dst_pitch | ch.dst_v | ch.dst_frame) & 3) != 0) return SRCNN_OK;
-    const bool uyvy = a.order == SRCNN_ORDER_UYVY;
-    const int nframes = std::max(1, a.nframes);
-
-    IntTaps t = {}, tc = {};
-    int_taps(a.tx, a.ty, S, a.row_begin, a.row_end, t);
-    int_taps(ch.tx, ch.ty, S, ch.row_begin, ch.row_end, tc);
-    // both tile kinds read the same packed rows: 64-bit group loads when they are 8-byte aligned, 32-bit when 4-byte aligned
-    const uintptr_t al = (uintptr_t)p.src | p.src_stride | p.src_frame | (uintptr_t)ch.src | ch.src_pitch;
-    t.vec_ok = tc.vec_ok = (al & 7) == 0 ? 2 : ((al & 3) == 0 ? 1 : 0);
-    t.ntx = ((a.ow + kITW - 1) / kITW + 2) / 3;    // a CTA per three adjacent tiles, as in a grey call
-    tc.ntx = (ch.ow + 3 * kCW - 1) / (3 * kCW);
-    auto kern = S == 2 ? (uyvy ? k_yuv422_bicubic_int<2, true> : k_yuv422_bicubic_int<2, false>)
-                       : (uyvy ? k_yuv422_bicubic_int<4, true> : k_yuv422_bicubic_int<4, false>);
-    static int ctas_per_sm[4][64] = {};            // per instance and device; a benign race: every writer stores the same value
-    int& per_sm = ctas_per_sm[(S == 4) * 2 + uyvy][c->device & 63];
-    if (per_sm == 0) {
-        int n = 0;
-        SRCNN_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, kern, 96, 0));
-        per_sm = std::max(1, n);
-    }
-    // tile height: the rule of launch_variant over the launch's luma and chroma tiles together
-    const int resident = per_sm * std::max(1, c->sm_count);
-    const int nrows = t.i_last - t.a_first + 1, crows = tc.i_last - tc.a_first + 1;
-    auto tiles_for = [&](int isr) {
-        return ((long long)t.ntx * ((nrows + isr - 1) / isr) + (long long)tc.ntx * ((crows + isr - 1) / isr)) * nframes;
-    };
-    t.isr = tiles_for(kISRMax) > 2LL * resident ? kISRMax : 8;
-    if (c->ka_int_isr >= 4 && c->ka_int_isr <= kISRMax) t.isr = c->ka_int_isr;
-    tc.isr = t.isr;
-    if (tiles_for(t.isr) > 0x3fffffffLL) return SRCNN_OK;
-    t.nty = (nrows + t.isr - 1) / t.isr;
-    tc.nty = (crows + tc.isr - 1) / tc.isr;
-    t.ntiles = t.ntx * t.nty * nframes;
-    tc.ntiles = tc.ntx * tc.nty * nframes;
-    ChromaDev q;
-    q.src = ch.src; q.src_pitch = ch.src_pitch; q.src_v = 0; q.src_frame = p.src_frame;
-    q.dst = ch.dst; q.dst_pitch = ch.dst_pitch; q.dst_v = ch.dst_v; q.dst_frame = ch.dst_frame;
-    q.sw = ch.sw; q.sh = ch.sh; q.ow = ch.ow; q.row_begin = ch.row_begin; q.row_end = ch.row_end;
-    const int rc = launch_ka(c, kern, t.ntiles + tc.ntiles, 96, a.early, p, t, q, tc);
-    if (rc) return rc;
-    *done = true;
-    return SRCNN_OK;
+    // indexed by a.order - SRCNN_ORDER_NV12
+    static_assert(SRCNN_ORDER_I420 == SRCNN_ORDER_NV12 + 1 && SRCNN_ORDER_YUY2 == SRCNN_ORDER_NV12 + 2 &&
+                  SRCNN_ORDER_UYVY == SRCNN_ORDER_NV12 + 3, "kLaunch lists the YUV orders in enum order");
+    using Launch = int (*)(Ctx*, const ResizeDev&, IntTaps&, const ChromaDev&, IntTaps&, int, bool, bool*);
+    static constexpr Launch kLaunch[2][4] = {
+        {launch_yuv<2, SRCNN_ORDER_NV12>, launch_yuv<2, SRCNN_ORDER_I420>, launch_yuv<2, SRCNN_ORDER_YUY2>, launch_yuv<2, SRCNN_ORDER_UYVY>},
+        {launch_yuv<4, SRCNN_ORDER_NV12>, launch_yuv<4, SRCNN_ORDER_I420>, launch_yuv<4, SRCNN_ORDER_YUY2>, launch_yuv<4, SRCNN_ORDER_UYVY>}};
+    // a.early is false for every 4:2:0 call: it launches no merge (api.cu)
+    return kLaunch[S == 4][a.order - SRCNN_ORDER_NV12](c, p, t, q, tc, std::max(1, a.nframes), a.early, done);
 }
 
 int launch_color_bicubic_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bool* done) {
@@ -966,14 +807,9 @@ int launch_color_bicubic_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bo
     t.ntx = (a.ow + kITW - 1) / kITW;
     if (gray) t.ntx = (t.ntx + 2) / 3;             // a CTA per three adjacent tiles
     if ((long long)t.ntx * (t.i_last - t.a_first + 1) * nframes > 0x3fffffffLL) return SRCNN_OK;
-    int rc;
-    if (gray) rc = S == 2 ? launch_variant<2, 1>(c, p, t, pa, nframes, false) : launch_variant<4, 1>(c, p, t, pa, nframes, false);   // never early (api.cu)
-    else if (four) rc = S == 2 ? launch_variant<2, 4>(c, p, t, pa, nframes, a.early) : launch_variant<4, 4>(c, p, t, pa, nframes, a.early);
-    else rc = S == 2 ? launch_variant<2, 3>(c, p, t, pa, nframes, a.early) : launch_variant<4, 3>(c, p, t, pa, nframes, a.early);
-    if (rc) return rc;
-    *done = true;
-    return SRCNN_OK;
+    if (gray) return S == 2 ? launch_variant<2, 1>(c, p, t, pa, nframes, false, done) : launch_variant<4, 1>(c, p, t, pa, nframes, false, done);   // never early (api.cu)
+    if (four) return S == 2 ? launch_variant<2, 4>(c, p, t, pa, nframes, a.early, done) : launch_variant<4, 4>(c, p, t, pa, nframes, a.early, done);
+    return S == 2 ? launch_variant<2, 3>(c, p, t, pa, nframes, a.early, done) : launch_variant<4, 3>(c, p, t, pa, nframes, a.early, done);
 }
 
 }  // namespace srcnn
-

@@ -368,7 +368,7 @@ def test_alpha_plane_of_a_batch(engine, name):
 
 
 # 4:2:0 / 4:2:2 frames (even sizes, and an output whose chroma plane is half the luma plane): where the luma output is a
-# multiple of 16 wide, x2 / x4 take the one-launch integer kernels (k_yuv420_bicubic_int / k_yuv422_bicubic_int), the others
+# multiple of 16 wide, x2 / x4 take the one-launch integer kernels (k_yuv_bicubic_int), the others
 # the generic kernels per plane
 YUV_GEOMS = {"x2_int16": (96, 70, 2.0, 2), "x4_int16": (92, 40, 4.0, 4), "x2_tail4": (98, 70, 2.0, 2), "x1.5": (92, 72, 1.5, 0),
              "x2.7": (92, 60, 2.7, 0), "x0.5": (148, 120, 0.5, 0), "x0.3": (240, 160, 0.3, 0)}
