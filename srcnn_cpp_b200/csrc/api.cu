@@ -9,6 +9,7 @@
 #include <mutex>
 #include <new>
 #include <unordered_map>
+#include <utility>
 
 #include "common.h"
 
@@ -66,78 +67,128 @@ static int scaled_dim(int n, float scale) {
     return (int)((float)n * scale);
 }
 
-// bytes per pixel of a row (4:2:0: of a Y row; a chroma row of NV12 has as many, an I420 chroma row half as many; packed 4:2:2: 2)
-static size_t bytes_per_pixel(int order) {
-    return order == SRCNN_ORDER_GRAY || yuv420(order) ? 1 : (yuv422(order) ? 2 : (four_channel(order) ? 4 : 3));
-}
-// rows of one frame in memory (4:2:0: h rows of Y, then h/2 rows of NV12 pairs or of I420 U and V)
-static size_t frame_rows(int order, int h) { return yuv420(order) ? (size_t)h / 2 * 3 : (size_t)h; }
+// What the host path needs to know about a pixel order, from layout_of: no other function of the whole path asks for the order.
+struct Layout {
+    enum Finish { kCnnOut, kMerge, kPack };   // the last kernel: the CNN into the caller's frame, the merge, the 4:2:2 pack kernel
+    enum Chroma { kNone, k420, k422 };        // chroma resized without the CNN: none, w/2 x h/2, w/2 x h
+    int order = -1;                           // -1: not an order of the whole path
+    size_t bpp = 0;          // bytes per pixel of a row (4:2:0: of a Y row; NV12's chroma rows have as many, I420's half as many)
+    size_t row_align = 4;    // device staging rows (4:2:0: 16-byte multiples, so that I420's half-length rows stay 8-byte aligned)
+    Finish finish = kMerge;
+    Chroma chroma = kNone;
+    bool i420 = false;       // chroma rows half as long, stride/2 apart: even strides
+    bool alpha = false;      // four-channel: an A plane beside Cr / Cb
+    bool fuses = false;      // the fused merge takes it (a four-channel call needs the merge for alpha, a 4:2:2 call its pack kernel)
+    // 4:2:0: h rows of Y, then h/2 rows of NV12 pairs or of I420 U and V: even sizes, frames staged whole, no band calls
+    bool whole() const { return chroma == k420; }
+    bool cbcr() const { return finish != kCnnOut; }   // the workspace has Cr / Cb planes (4:2:2: U' / V'), so the call merges
+    int planes() const { return alpha ? 5 : 4; }    // u8 workspace planes per frame
+    size_t rows(int n) const { return whole() ? (size_t)n / 2 * 3 : (size_t)n; }   // rows in memory of a frame of n Y rows
+};
 
-static int check_image(Ctx* c, const void* src, int w, int h, size_t stride, int order, float scale, const void* dst,
-                       size_t dst_stride, int* ow, int* oh) {
+static Layout layout_of(int order) {
+    Layout L;
+    switch (order) {
+        case SRCNN_ORDER_BGR: case SRCNN_ORDER_RGB: L.bpp = 3; L.fuses = true; break;
+        case SRCNN_ORDER_BGRA: case SRCNN_ORDER_RGBA: L.bpp = 4; L.alpha = true; break;
+        case SRCNN_ORDER_GRAY: L.bpp = 1; L.finish = Layout::kCnnOut; break;
+        case SRCNN_ORDER_NV12: case SRCNN_ORDER_I420:
+            L.bpp = 1; L.row_align = 16; L.finish = Layout::kCnnOut; L.chroma = Layout::k420; L.i420 = order == SRCNN_ORDER_I420; break;
+        case SRCNN_ORDER_YUY2: case SRCNN_ORDER_UYVY: L.bpp = 2; L.finish = Layout::kPack; L.chroma = Layout::k422; break;
+        default: return L;
+    }
+    L.order = order;
+    return L;
+}
+
+// One whole-path call: frames of w x h -> ow x oh.  `src` / `dst` are at frame 0 (a band's: at its first source / output row),
+// the frames src_frame / dst_frame bytes apart; both are 0 for a single frame, whose kernels then take no frame strides.
+struct Image {
+    const uint8_t* src = nullptr;
+    size_t src_stride = 0, src_frame = 0;
+    uint8_t* dst = nullptr;
+    size_t dst_stride = 0, dst_frame = 0;
+    int w = 0, h = 0, ow = 0, oh = 0;
+    float scale = 0.f;
+    Layout L;
+    Image frame(int f) const {   // frame f as a call of its own
+        return Image{src + (size_t)f * src_frame, src_stride, 0, dst + (size_t)f * dst_frame, dst_stride, 0, w, h, ow, oh, scale, L};
+    }
+};
+
+static int check_image(Ctx* c, const uint8_t* src, int w, int h, size_t stride, int order, float scale, uint8_t* dst,
+                       size_t dst_stride, Image* im) {
     if (!c) return SRCNN_E_ARG;
     if (!src || !dst) return fail(c, SRCNN_E_ARG, "null image pointer");
     if (w <= 0 || h <= 0) return fail(c, SRCNN_E_ARG, "non-positive image size %dx%d", w, h);
-    if (order != SRCNN_ORDER_BGR && order != SRCNN_ORDER_RGB && order != SRCNN_ORDER_GRAY && !four_channel(order) && !yuv420(order) &&
-        !yuv422(order))
-        return fail(c, SRCNN_E_ARG, "unknown pixel order %d", order);
-    const size_t bpp = bytes_per_pixel(order);
-    if (stride < (size_t)w * bpp) return fail(c, SRCNN_E_ARG, "source stride %zu < %zu*w", stride, bpp);
-    if (yuv420(order) && ((w | h) & 1)) return fail(c, SRCNN_E_ARG, "4:2:0 frames need an even width and height, got %dx%d", w, h);
-    if (yuv422(order) && (w & 1)) return fail(c, SRCNN_E_ARG, "4:2:2 frames need an even width (whole macropixels), got %d", w);
-    if (order == SRCNN_ORDER_I420 && ((stride | dst_stride) & 1))
+    const Layout L = layout_of(order);
+    if (L.order < 0) return fail(c, SRCNN_E_ARG, "unknown pixel order %d", order);
+    if (stride < (size_t)w * L.bpp) return fail(c, SRCNN_E_ARG, "source stride %zu < %zu*w", stride, L.bpp);
+    if (L.whole() && ((w | h) & 1)) return fail(c, SRCNN_E_ARG, "4:2:0 frames need an even width and height, got %dx%d", w, h);
+    if (L.chroma == Layout::k422 && (w & 1)) return fail(c, SRCNN_E_ARG, "4:2:2 frames need an even width (whole macropixels), got %d", w);
+    if (L.i420 && ((stride | dst_stride) & 1))
         return fail(c, SRCNN_E_ARG, "I420 strides must be even (chroma rows are stride/2 apart), got %zu / %zu", stride, dst_stride);
-    // src/srcnn.cpp:485-495 "ratio too small"
-    if (!(((float)w * scale) > 0.f) || !(((float)h * scale) > 0.f)) return fail(c, SRCNN_E_RATIO, "scale %g gives an empty image", scale);
-    *ow = scaled_dim(w, scale);
-    *oh = scaled_dim(h, scale);
-    if (*ow <= 0 || *oh <= 0) return fail(c, SRCNN_E_RATIO, "scale %g gives an empty image", scale);
-    if (yuv420(order) && ((*ow | *oh) & 1))
-        return fail(c, SRCNN_E_ARG, "scale %g gives an odd 4:2:0 output size %dx%d (width and height must be even)", scale, *ow, *oh);
-    if (yuv422(order) && (*ow & 1))
-        return fail(c, SRCNN_E_ARG, "scale %g gives an odd 4:2:2 output width %d (whole macropixels: it must be even)", scale, *ow);
-    if (dst_stride < (size_t)*ow * bpp) return fail(c, SRCNN_E_ARG, "destination stride %zu < %zu*ow", dst_stride, bpp);
+    int ow, oh;   // src/srcnn.cpp:485-495 "ratio too small"
+    if (srcnn_out_dims(w, h, scale, &ow, &oh)) return fail(c, SRCNN_E_RATIO, "scale %g gives an empty image", scale);
+    if (L.whole() && ((ow | oh) & 1))
+        return fail(c, SRCNN_E_ARG, "scale %g gives an odd 4:2:0 output size %dx%d (width and height must be even)", scale, ow, oh);
+    if (L.chroma == Layout::k422 && (ow & 1))
+        return fail(c, SRCNN_E_ARG, "scale %g gives an odd 4:2:2 output width %d (whole macropixels: it must be even)", scale, ow);
+    if (dst_stride < (size_t)ow * L.bpp) return fail(c, SRCNN_E_ARG, "destination stride %zu < %zu*ow", dst_stride, L.bpp);
+    *im = Image{src, stride, 0, dst, dst_stride, 0, w, h, ow, oh, scale, L};
     return SRCNN_OK;
 }
 
-// The chroma planes of 4:2:0 frames whose Y rows start at `src` / `dst` (frame 0), for the luma output rows [r0, r1): chroma output
-// rows [r0/2, r1/2).  A chroma row is resized without the CNN, so it needs no halo.
-static int chroma_planes(Ctx* c, int order, const uint8_t* src, int w, int h, size_t src_stride, uint8_t* dst, int ow, int oh,
-                         size_t dst_stride, size_t dst_frame_stride, int r0, int r1, Chroma420* ch) {
-    TapTable *tx, *ty;
-    int rc = get_taps(c, w / 2, ow / 2, &tx);
+// check_image for a batch of n frames, and its frame strides.  n = 0 passes with nothing filled in.
+static int check_batch(Ctx* c, int n, const uint8_t* src, int w, int h, size_t stride, size_t src_frame, int order, float scale,
+                       uint8_t* dst, size_t dst_stride, size_t dst_frame, Image* im) {
+    if (n < 0) return fail(c, SRCNN_E_ARG, "negative frame count");
+    if (n == 0) return SRCNN_OK;
+    int rc = check_image(c, src, w, h, stride, order, scale, dst, dst_stride, im);
     if (rc) return rc;
-    if ((rc = get_taps(c, h / 2, oh / 2, &ty))) return rc;
-    const bool i420 = order == SRCNN_ORDER_I420;
-    ch->src = src + (size_t)h * src_stride;
-    ch->src_pitch = i420 ? src_stride / 2 : src_stride;
-    ch->src_v = i420 ? (size_t)(h / 2) * (src_stride / 2) : 0;
-    ch->dst = dst + (size_t)oh * dst_stride;
-    ch->dst_pitch = i420 ? dst_stride / 2 : dst_stride;
-    ch->dst_v = i420 ? (size_t)(oh / 2) * (dst_stride / 2) : 0;
-    ch->dst_frame = dst_frame_stride;
-    ch->sw = w / 2; ch->sh = h / 2; ch->ow = ow / 2; ch->oh = oh / 2;
-    ch->row_begin = r0 / 2; ch->row_end = r1 / 2;
-    ch->tx = tx; ch->ty = ty;
+    if (n > 1 && (src_frame < stride * im->L.rows(h) || dst_frame < dst_stride * im->L.rows(im->oh)))
+        return fail(c, SRCNN_E_ARG, "frame stride smaller than one frame");
+    im->src_frame = src_frame; im->dst_frame = dst_frame;
     return SRCNN_OK;
 }
 
-// The chroma planes of packed 4:2:2 frames whose row 0 is at `src` (frame 0), for the output rows [r0, r1): U' and V' go into the
-// Cr / Cb planes of `pl` (its first ow/2 columns), which the pack kernel reads for the same rows.  No halo: chroma has no CNN.
-static int chroma_planes422(Ctx* c, const uint8_t* src, int w, int h, size_t src_stride, const Planes& pl, int ow, int oh, int r0,
-                            int r1, Chroma420* ch) {
+constexpr int kHalo = 6;   // output rows the CNN reads around a band: 4 (conv1) + 2 (conv3)
+
+// The source rows that output rows [r0, r1) and `halo` output rows either side of them touch, from the tap table `ofs` (h -> oh)
+static std::pair<int, int> src_rows(const int* ofs, int h, int oh, int r0, int r1, int halo = kHalo) {
+    const int p0 = std::max(r0 - halo, 0), p1 = std::min(r1 + halo, oh);
+    return {std::min(std::max(ofs[p0] - 1, 0), h - 1), std::min(std::max(ofs[p1 - 1] + 2, 0), h - 1) + 1};
+}
+
+// The chroma descriptor of the luma output rows [r0, r1) of frames whose row 0 is at `src` / `dst` (frame 0).  No halo: a chroma
+// row is resized without the CNN.  4:2:0: the chroma rows after the Y rows, resized straight into the caller's frames (chroma
+// output rows [r0/2, r1/2)).  4:2:2: U' and V' of the packed rows go into the Cr / Cb planes of `pl` (their first ow/2 columns),
+// which the pack kernel reads for the same rows.
+static int chroma_planes(Ctx* c, const Image& im, const uint8_t* src, uint8_t* dst, const Planes& pl, int r0, int r1, Chroma420* ch) {
+    const int v = im.L.whole() ? 2 : 1;   // Y rows per chroma row
     TapTable *tx, *ty;
-    int rc = get_taps(c, w / 2, ow / 2, &tx);
+    int rc = get_taps(c, im.w / 2, im.ow / 2, &tx);
     if (rc) return rc;
-    if ((rc = get_taps(c, h, oh, &ty))) return rc;
-    ch->src = src; ch->src_pitch = src_stride; ch->src_v = 0;
-    ch->dst = pl.cr - (ptrdiff_t)pl.row0 * (ptrdiff_t)pl.pitch;   // chroma output row r at dst + r * pitch
-    ch->dst_pitch = pl.pitch;
-    ch->dst_v = (size_t)(pl.cb - pl.cr);
-    ch->dst_frame = pl.frame_stride;
-    ch->sw = w / 2; ch->sh = h; ch->ow = ow / 2; ch->oh = oh;
-    ch->row_begin = r0; ch->row_end = r1;
+    if ((rc = get_taps(c, im.h / v, im.oh / v, &ty))) return rc;
+    ch->sw = im.w / 2; ch->sh = im.h / v; ch->ow = im.ow / 2; ch->oh = im.oh / v;
+    ch->row_begin = r0 / v; ch->row_end = r1 / v;
     ch->tx = tx; ch->ty = ty;
+    if (!im.L.whole()) {
+        ch->src = src; ch->src_pitch = im.src_stride; ch->src_v = 0;
+        ch->dst = pl.cr - (ptrdiff_t)pl.row0 * (ptrdiff_t)pl.pitch;   // chroma output row r at dst + r * pitch
+        ch->dst_pitch = pl.pitch;
+        ch->dst_v = (size_t)(pl.cb - pl.cr);
+        ch->dst_frame = pl.frame_stride;
+        return SRCNN_OK;
+    }
+    const bool i420 = im.L.i420;
+    ch->src = src + (size_t)im.h * im.src_stride;
+    ch->src_pitch = i420 ? im.src_stride / 2 : im.src_stride;
+    ch->src_v = i420 ? (size_t)(im.h / 2) * (im.src_stride / 2) : 0;
+    ch->dst = dst + (size_t)im.oh * im.dst_stride;
+    ch->dst_pitch = i420 ? im.dst_stride / 2 : im.dst_stride;
+    ch->dst_v = i420 ? (size_t)(im.oh / 2) * (im.dst_stride / 2) : 0;
+    ch->dst_frame = im.dst_frame;
     return SRCNN_OK;
 }
 
@@ -152,8 +203,8 @@ static int chroma_planes422(Ctx* c, const uint8_t* src, int w, int h, size_t src
 // The host-buffer pipeline keeps to set 0 (its sub-bands are separated by copies and events anyway).  A grey or 4:2:0 call has no
 // Cr/Cb planes: it leaves the set selection alone (and ends the early-start chain, end_merge_chain).  A packed 4:2:2 call keeps its
 // U' / V' planes in the Cr / Cb slots and so takes part like a colour call.
-static int carve_planes(Ctx* c, int ow, int rows, int row0, Planes* pl, int nframes = 1, int order = SRCNN_ORDER_BGR) {
-    const bool gray = order == SRCNN_ORDER_GRAY || yuv420(order), four = four_channel(order);
+static int carve_planes(Ctx* c, int ow, int rows, int row0, Planes* pl, int nframes, const Layout& L) {
+    const bool gray = !L.cbcr(), four = L.alpha;
     const size_t pitch = align_up((size_t)ow, 128);
     const size_t plane = pitch * (size_t)rows;
     const size_t pitch16 = y16_pitch_bytes(ow);
@@ -237,190 +288,107 @@ static int run_cnn(Ctx* c, int variant, const CnnArgs& a) {
     return fail(c, SRCNN_E_ARG, "unknown variant %d", variant);
 }
 
-// rows [r0,r1) of the full output; d_src holds source rows [s0,s1); d_dst points at output row r0
-static int process_rows_impl(Ctx* c, const uint8_t* d_src, int w, int h, size_t src_stride, int s0, int s1, int order,
-                             float scale, int ow, int oh, int r0, int r1, uint8_t* d_dst, size_t dst_stride) {
+// The three stages over frames [f0, f0 + m) of `im`, output rows [r0, r1) from source rows [s0, s1) (im.src is at source row s0,
+// im.dst at output row r0).  A band or a single frame is m = 1.  A batch chunk is whole frames, ONE launch of each stage: the
+// colour+bicubic grid gets a frame dimension, the row-walking kernel sees the frames as more strips of one work list (no
+// per-frame pipeline fill / drain), the merge kernel sees the chunk's planes as one tall image.
+static int run_stages(Ctx* c, const Image& im, int f0, int m, int s0, int s1, int r0, int r1) {
+    const Layout& L = im.L;
+    const uint8_t* src = im.src + (size_t)f0 * im.src_frame;
+    uint8_t* dst = im.dst + (size_t)f0 * im.dst_frame;
     TapTable *tx, *ty;
     c->fail_stage = SRCNN_STAGE_COLOR_BICUBIC;
-    int rc = get_taps(c, w, ow, &tx);
+    int rc = get_taps(c, im.w, im.ow, &tx);
     if (rc) return rc;
-    rc = get_taps(c, h, oh, &ty);
-    if (rc) return rc;
-    const int p0 = std::max(r0 - 6, 0), p1 = std::min(r1 + 6, oh);  // 6-px halo: 4 (conv1) + 2 (conv3)
+    if ((rc = get_taps(c, im.h, im.oh, &ty))) return rc;
+    const int p0 = std::max(r0 - kHalo, 0), p1 = std::min(r1 + kHalo, im.oh);
     // grey: one-plane resize, then the CNN straight into the caller's rows; no chroma, no merge.  4:2:0: the same for Y, and the
-    // resize launch also writes the chroma rows [r0/2, r1/2) straight into the caller's frame (d_dst is its row r0)
-    const bool gray = order == SRCNN_ORDER_GRAY || yuv420(order);
-    if (gray) end_merge_chain(c);
+    // resize launch also writes the chroma rows [r0/2, r1/2) straight into the caller's frame
+    if (!L.cbcr()) end_merge_chain(c);
     Planes pl;
     c->fail_stage = SRCNN_STAGE_PLANES;
-    rc = carve_planes(c, ow, p1 - p0, p0, &pl, 1, order);
-    if (rc) return rc;
+    if ((rc = carve_planes(c, im.ow, p1 - p0, p0, &pl, m, L))) return rc;
     c->fail_stage = SRCNN_STAGE_COLOR_BICUBIC;
     // the band must bring every source row its taps touch
-    const int need0 = std::min(std::max(ty->h_ofs[p0] - 1, 0), h - 1);
-    const int need1 = std::min(std::max(ty->h_ofs[p1 - 1] + 2, 0), h - 1) + 1;
-    if (s0 > need0 || s1 < need1)
-        return fail(c, SRCNN_E_ARG, "band rows [%d,%d) need source rows [%d,%d), got [%d,%d)", r0, r1, need0, need1, s0, s1);
+    const auto need = src_rows(ty->h_ofs.data(), im.h, im.oh, r0, r1);
+    if (s0 > need.first || s1 < need.second)
+        return fail(c, SRCNN_E_ARG, "band rows [%d,%d) need source rows [%d,%d), got [%d,%d)", r0, r1, need.first, need.second, s0, s1);
 
     ResizeArgs ra;
-    ra.src = d_src; ra.src_stride = src_stride;
-    ra.sw = w; ra.sh = h; ra.src_row0 = s0; ra.src_row1 = s1;
-    ra.order = order;
-    ra.ow = ow; ra.oh = oh;
+    ra.src = src; ra.src_stride = im.src_stride;
+    ra.sw = im.w; ra.sh = im.h; ra.src_row0 = s0; ra.src_row1 = s1;
+    ra.order = L.order;
+    ra.ow = im.ow; ra.oh = im.oh;
     ra.row_begin = p0; ra.row_end = p1;
     ra.pl = pl; ra.tx = tx; ra.ty = ty;
-    if (yuv420(order) && (rc = chroma_planes(c, order, d_src - (size_t)s0 * src_stride, w, h, src_stride, d_dst - (size_t)r0 * dst_stride,
-                                             ow, oh, dst_stride, 0, r0, r1, &ra.ch)))
-        return rc;
-    // 4:2:2: chroma rows [r0, r1) only (the pack kernel's); the luma halo rows [p0, r0) and [r1, p1) are the CNN's
-    if (yuv422(order) && (rc = chroma_planes422(c, d_src - (size_t)s0 * src_stride, w, h, src_stride, pl, ow, oh, r0, r1, &ra.ch)))
+    ra.nframes = m; ra.src_frame_stride = im.src_frame;
+    // chroma for the rows [r0, r1) only: the luma halo rows [p0, r0) and [r1, p1) are the CNN's
+    if (L.chroma != Layout::kNone &&
+        (rc = chroma_planes(c, im, src - (size_t)s0 * im.src_stride, dst - (size_t)r0 * im.dst_stride, pl, r0, r1, &ra.ch)))
         return rc;
     if (c->variant != SRCNN_VARIANT_TC) ra.pl.y16 = nullptr;      // the strict FP32 kernels read the u8 plane
-    ra.early = !gray && may_start_early(c, d_src, (size_t)(s1 - s0) * src_stride);
+    ra.early = L.cbcr() && may_start_early(c, src, (size_t)(m - 1) * im.src_frame + (size_t)(s1 - s0) * im.src_stride);
     c->early_launches += ra.early;
     if ((rc = prof_mark(c, 0))) return rc;
-    rc = launch_color_bicubic(c, ra);
-    if (rc) return rc;
+    if ((rc = launch_color_bicubic(c, ra))) return rc;
     if ((rc = prof_mark(c, 1))) return rc;
 
     c->fail_stage = SRCNN_STAGE_CNN;
     CnnArgs ca;
     ca.y = pl.y; ca.pitch = pl.pitch;
     ca.y16 = pl.y16; ca.pitch16 = pl.pitch16;
-    ca.W = ow; ca.H = oh;
+    ca.W = im.ow; ca.H = im.oh;
     ca.row0 = p0; ca.rows = p1 - p0;
     ca.out_begin = r0; ca.out_end = r1;
-    if (gray) { ca.out = d_dst; ca.out_pitch = dst_stride; ca.out_row0 = r0; }
+    ca.nframes = m;
+    if (im.dst_frame) { ca.y16_frame_stride = pl.frame_stride16; ca.out_frame_stride = pl.frame_stride; }
+    if (!L.cbcr()) { ca.out = dst; ca.out_pitch = im.dst_stride; ca.out_row0 = r0; ca.out_frame_stride = im.dst_frame; }
     else { ca.out = pl.yout; ca.out_pitch = pl.pitch; ca.out_row0 = p0; }
     // optionally the row-walking tcgen05 kernel merges Cr/Cb and converts back to BGR in its last epilogue (no Y' plane, no
     // K-C launch); measured slower than the separate launch (byte stores from one-thread-per-column lanes), so off by default
-    // (colour orders only: a four-channel call takes the separate merge, which writes alpha too; a 4:2:2 call its pack kernel)
-    const bool fused = (order == SRCNN_ORDER_BGR || order == SRCNN_ORDER_RGB) && c->variant == SRCNN_VARIANT_TC && c->fuse_merge;
+    const bool fused = L.fuses && c->variant == SRCNN_VARIANT_TC && c->fuse_merge;
     if (fused) {
         ca.cr = pl.cr; ca.cb = pl.cb;
-        ca.bgr = d_dst; ca.bgr_stride = dst_stride; ca.order = order;
+        ca.bgr = dst; ca.bgr_stride = im.dst_stride; ca.order = L.order;
     }
-    rc = run_cnn(c, c->variant, ca);
-    if (rc) return rc;
+    if ((rc = run_cnn(c, c->variant, ca))) return rc;
     if ((rc = prof_mark(c, 2))) return rc;
-    if (fused || gray) return prof_mark(c, 3);
+    if (fused || !L.cbcr()) return prof_mark(c, 3);
 
     c->fail_stage = SRCNN_STAGE_MERGE;
     MergeArgs ma;
-    const size_t off = (size_t)(r0 - p0) * pl.pitch;
-    ma.y = pl.yout + off; ma.cr = pl.cr + off; ma.cb = pl.cb + off;
-    if (pl.a) ma.a = pl.a + off;
-    ma.pitch = pl.pitch; ma.w = ow; ma.rows = r1 - r0;
-    ma.order = order;
-    ma.dst = d_dst; ma.dst_stride = dst_stride;
-    rc = yuv422(order) ? launch_pack422(c, ma) : launch_merge(c, ma);
-    if (rc) return rc;
-    merged_into(c, d_dst, (size_t)(r1 - r0) * dst_stride);
+    ma.pitch = pl.pitch; ma.w = im.ow;
+    ma.order = L.order;
+    ma.dst_stride = im.dst_stride;
+    const bool tall = m == 1 || im.dst_frame == im.dst_stride * (size_t)im.oh;   // the chunk's results are one tall image
+    for (int f = 0; f < (tall ? 1 : m); f++) {
+        const size_t off = (size_t)(r0 - p0) * pl.pitch + (size_t)f * pl.frame_stride;
+        ma.y = pl.yout + off; ma.cr = pl.cr + off; ma.cb = pl.cb + off;
+        if (pl.a) ma.a = pl.a + off;
+        ma.rows = tall ? (r1 - r0) * m : r1 - r0;
+        ma.dst = dst + (size_t)f * im.dst_frame;
+        if ((rc = L.finish == Layout::kPack ? launch_pack422(c, ma) : launch_merge(c, ma))) return rc;
+    }
+    merged_into(c, dst, (size_t)(m - 1) * im.dst_frame + (size_t)(r1 - r0) * im.dst_stride);
     return prof_mark(c, 3);
 }
 
-static int process_rows(Ctx* c, const uint8_t* d_src, int w, int h, size_t src_stride, int s0, int s1, int order,
-                        float scale, int ow, int oh, int r0, int r1, uint8_t* d_dst, size_t dst_stride) {
-    const size_t ev0 = c->ev_used;
-    const int rc = process_rows_impl(c, d_src, w, h, src_stride, s0, s1, order, scale, ow, oh, r0, r1, d_dst, dst_stride);
-    if (rc) c->ev_used = ev0;        // a failed band leaves no half-recorded event group behind (srcnn_profile_read pairs by 4)
-    else c->fail_stage = SRCNN_STAGE_NONE;
-    return rc;
-}
-
-// `n` whole frames resident on the device, in chunks whose planes stay below ~1 GB: per chunk ONE launch of each stage -- the
-// colour+bicubic grid gets a frame dimension, the row-walking kernel sees the frames as more strips of one work list (no
-// per-frame pipeline fill / drain), the merge kernel sees the chunk's planes as one tall image.
-static int process_frames_impl(Ctx* c, const uint8_t* d_src, int n, int w, int h, size_t src_stride, size_t src_frame_stride, int order,
-                               float scale, int ow, int oh, uint8_t* d_dst, size_t dst_stride, size_t dst_frame_stride) {
-    TapTable *tx, *ty;
-    c->fail_stage = SRCNN_STAGE_COLOR_BICUBIC;
-    int rc = get_taps(c, w, ow, &tx);
-    if (rc) return rc;
-    if ((rc = get_taps(c, h, oh, &ty))) return rc;
-    const size_t per_frame = align_up((size_t)ow, 128) * (size_t)oh * (four_channel(order) ? 5 : 4) + y16_pitch_bytes(ow) * (size_t)oh;
-    const int chunk = (int)std::max<size_t>(1, std::min<size_t>((size_t)n, ((size_t)1 << 30) / per_frame));
-    const bool gray = order == SRCNN_ORDER_GRAY || yuv420(order);   // the CNN writes into the caller's frames, no merge
-    if (gray) end_merge_chain(c);
-    for (int f0 = 0; f0 < n; f0 += chunk) {
-        const int m = std::min(chunk, n - f0);
-        Planes pl;
-        c->fail_stage = SRCNN_STAGE_PLANES;
-        if ((rc = carve_planes(c, ow, oh, 0, &pl, m, order))) return rc;
-        c->fail_stage = SRCNN_STAGE_COLOR_BICUBIC;
-        ResizeArgs ra;
-        ra.src = d_src + (size_t)f0 * src_frame_stride; ra.src_stride = src_stride;
-        ra.sw = w; ra.sh = h; ra.src_row0 = 0; ra.src_row1 = h;
-        ra.order = order;
-        ra.ow = ow; ra.oh = oh;
-        ra.row_begin = 0; ra.row_end = oh;
-        ra.pl = pl; ra.tx = tx; ra.ty = ty;
-        ra.nframes = m; ra.src_frame_stride = src_frame_stride;
-        if (yuv420(order) && (rc = chroma_planes(c, order, ra.src, w, h, src_stride, d_dst + (size_t)f0 * dst_frame_stride, ow, oh, dst_stride,
-                                                 dst_frame_stride, 0, oh, &ra.ch)))
-            return rc;
-        if (yuv422(order) && (rc = chroma_planes422(c, ra.src, w, h, src_stride, pl, ow, oh, 0, oh, &ra.ch))) return rc;
-        ra.early = !gray && may_start_early(c, ra.src, (size_t)(m - 1) * src_frame_stride + (size_t)h * src_stride);
-        c->early_launches += ra.early;
-        if ((rc = prof_mark(c, 0))) return rc;
-        if ((rc = launch_color_bicubic(c, ra))) return rc;
-        if ((rc = prof_mark(c, 1))) return rc;
-        c->fail_stage = SRCNN_STAGE_CNN;
-        CnnArgs ca;
-        ca.y = pl.y; ca.pitch = pl.pitch;
-        ca.y16 = pl.y16; ca.pitch16 = pl.pitch16;
-        ca.W = ow; ca.H = oh;
-        ca.row0 = 0; ca.rows = oh;
-        ca.out_begin = 0; ca.out_end = oh;
-        ca.out = pl.yout; ca.out_pitch = pl.pitch;
-        ca.nframes = m; ca.y16_frame_stride = pl.frame_stride16; ca.out_frame_stride = pl.frame_stride;
-        uint8_t* dst0 = d_dst + (size_t)f0 * dst_frame_stride;
-        if (gray) { ca.out = dst0; ca.out_pitch = dst_stride; ca.out_frame_stride = dst_frame_stride; }
-        if ((rc = launch_cnn_tc2(c, ca))) return rc;
-        if ((rc = prof_mark(c, 2))) return rc;
-        if (gray) {
-            if ((rc = prof_mark(c, 3))) return rc;
-            continue;
-        }
-        c->fail_stage = SRCNN_STAGE_MERGE;
-        MergeArgs ma;
-        ma.y = pl.yout; ma.cr = pl.cr; ma.cb = pl.cb; ma.a = pl.a;
-        ma.pitch = pl.pitch; ma.w = ow;
-        ma.order = order;
-        auto merge = [&]() { return yuv422(order) ? launch_pack422(c, ma) : launch_merge(c, ma); };   // 4:2:2: the pack kernel
-        if (m == 1 || dst_frame_stride == dst_stride * (size_t)oh) {   // the chunk's results are one tall image too
-            ma.rows = oh * m; ma.dst = dst0; ma.dst_stride = dst_stride;
-            if ((rc = merge())) return rc;
-        } else {
-            for (int f = 0; f < m; f++) {
-                ma.y = pl.yout + (size_t)f * pl.frame_stride; ma.cr = pl.cr + (size_t)f * pl.frame_stride; ma.cb = pl.cb + (size_t)f * pl.frame_stride;
-                if (pl.a) ma.a = pl.a + (size_t)f * pl.frame_stride;
-                ma.rows = oh; ma.dst = dst0 + (size_t)f * dst_frame_stride; ma.dst_stride = dst_stride;
-                if ((rc = merge())) return rc;
-            }
-        }
-        merged_into(c, dst0, (size_t)(m - 1) * dst_frame_stride + (size_t)oh * dst_stride);
-        if ((rc = prof_mark(c, 3))) return rc;
-    }
-    return SRCNN_OK;
-}
-
-static int process_frames(Ctx* c, const uint8_t* d_src, int n, int w, int h, size_t src_stride, size_t src_frame_stride, int order,
-                          float scale, int ow, int oh, uint8_t* d_dst, size_t dst_stride, size_t dst_frame_stride) {
-    // one launch per stage and chunk needs the row-walking kernel with a separate merge; everything else goes frame by frame
-    // (the fused merge only takes the colour orders: grey and four-channel batches stay batched with it switched on)
-    const bool fuses = c->fuse_merge && (order == SRCNN_ORDER_BGR || order == SRCNN_ORDER_RGB);
-    if (n == 1 || c->variant != SRCNN_VARIANT_TC || fuses || !c->batch_launch) {
-        for (int f = 0; f < n; f++) {
-            int rc = process_rows(c, d_src + (size_t)f * src_frame_stride, w, h, src_stride, 0, h, order, scale, ow, oh, 0, oh,
-                                  d_dst + (size_t)f * dst_frame_stride, dst_stride);
-            if (rc) return rc;
-        }
+// n frames of `im` resident on the device (n > 1: whole frames).  A batch goes in chunks whose planes stay below ~1 GB, one
+// launch per stage and chunk; that needs the row-walking kernel with a separate merge, everything else goes frame by frame (the
+// fused merge only takes the colour orders: grey and four-channel batches stay batched with it switched on).
+static int process(Ctx* c, const Image& im, int n, int s0, int s1, int r0, int r1) {
+    if (n > 1 && (c->variant != SRCNN_VARIANT_TC || (c->fuse_merge && im.L.fuses) || !c->batch_launch)) {
+        for (int f = 0; f < n; f++)
+            if (int rc = process(c, im.frame(f), 1, s0, s1, r0, r1)) return rc;
         return SRCNN_OK;
     }
+    const Image frames = n == 1 ? im.frame(0) : im;
+    const size_t per_frame = align_up((size_t)im.ow, 128) * (size_t)im.oh * im.L.planes() + y16_pitch_bytes(im.ow) * (size_t)im.oh;
+    const int chunk = (int)std::max<size_t>(1, std::min<size_t>((size_t)n, ((size_t)1 << 30) / per_frame));
     const size_t ev0 = c->ev_used;
-    const int rc = process_frames_impl(c, d_src, n, w, h, src_stride, src_frame_stride, order, scale, ow, oh, d_dst, dst_stride, dst_frame_stride);
-    if (rc) c->ev_used = ev0;
+    int rc = SRCNN_OK;
+    for (int f0 = 0; f0 < n && !rc; f0 += chunk) rc = run_stages(c, frames, f0, std::min(chunk, n - f0), s0, s1, r0, r1);
+    if (rc) c->ev_used = ev0;        // a failed call leaves no half-recorded event group behind (srcnn_profile_read pairs by 4)
     else c->fail_stage = SRCNN_STAGE_NONE;
     return rc;
 }
@@ -463,203 +431,152 @@ void drop_graphs(Ctx* c) {
     c->graphs.clear();
 }
 
-// Luma rows [y0, y1) and chroma rows [c0, c1) of one 4:2:0 frame between two buffers whose Y rows are `ds` / `ss` bytes apart
-// (w x h: the frame's size).  NV12's chroma rows follow the Y rows with the same stride; I420's U and V rows are half as long.
-static int copy_420(Ctx* c, bool i420, uint8_t* dst, size_t ds, const uint8_t* src, size_t ss, int w, int h, int y0, int y1, int c0,
-                    int c1, cudaMemcpyKind kind, cudaStream_t st) {
+// What host_pipeline works out once for enqueue_chunk, which enqueues it live or under graph capture
+struct HostPlan {
+    int S0 = 0, S1 = 0;                      // source rows staged per frame (4:2:0: the whole frame)
+    std::vector<int> edges;                  // the sub-bands' output rows: R0, ..., R1
+    int group = 1;                           // frames of a batch per copy and launch
+    size_t s_row = 0, d_row = 0, s_frame = 0, d_frame = 0;   // device staging
+    TapTable *ty = nullptr, *cty = nullptr;  // vertical taps of Y and of 4:2:0 chroma
+};
+
+// Rows [y0, y1) of one w x h frame, and for 4:2:0 its chroma rows [c0, c1), between two buffers whose rows are `ds` / `ss`
+// bytes apart and which point at the same row (4:2:0: row 0).  NV12's chroma rows follow the Y rows with the same stride;
+// I420's U and V rows are half as long.
+static int copy_rows(Ctx* c, const Layout& L, uint8_t* dst, size_t ds, const uint8_t* src, size_t ss, int w, int h, int y0, int y1,
+                     int c0, int c1, cudaMemcpyKind kind, cudaStream_t st) {
     if (y1 > y0)
-        SRCNN_CUDA(c, cudaMemcpy2DAsync(dst + (size_t)y0 * ds, ds, src + (size_t)y0 * ss, ss, (size_t)w, y1 - y0, kind, st));
-    if (c1 <= c0) return SRCNN_OK;
+        SRCNN_CUDA(c, cudaMemcpy2DAsync(dst + (size_t)y0 * ds, ds, src + (size_t)y0 * ss, ss, (size_t)w * L.bpp, y1 - y0, kind, st));
+    if (!L.whole() || c1 <= c0) return SRCNN_OK;
     dst += (size_t)h * ds;
     src += (size_t)h * ss;
-    if (!i420) {
-        SRCNN_CUDA(c, cudaMemcpy2DAsync(dst + (size_t)c0 * ds, ds, src + (size_t)c0 * ss, ss, (size_t)w, c1 - c0, kind, st));
-        return SRCNN_OK;
-    }
-    ds /= 2;
-    ss /= 2;
-    for (int pl = 0; pl < 2; pl++) {   // U, then V h/2 rows further
+    const int np = L.i420 ? 2 : 1;   // NV12: one plane of pairs; I420: U, then V h/2 rows further
+    ds /= np;
+    ss /= np;
+    for (int pl = 0; pl < np; pl++) {
         const size_t r = (size_t)(pl * (h / 2) + c0);
-        SRCNN_CUDA(c, cudaMemcpy2DAsync(dst + r * ds, ds, src + r * ss, ss, (size_t)w / 2, c1 - c0, kind, st));
+        SRCNN_CUDA(c, cudaMemcpy2DAsync(dst + r * ds, ds, src + r * ss, ss, (size_t)w / np, c1 - c0, kind, st));
     }
     return SRCNN_OK;
 }
 
-// Enqueues the whole pipeline of one chunk of frames (f0 .. f0+m) on the three streams and joins the copy streams back
-// into the compute stream; does not wait.  Identical whether the streams are live or being captured into a CUDA graph.
-static int enqueue_chunk(Ctx* c, const uint8_t* src, int f0, int m, int w, int h, size_t src_stride, size_t src_frame_stride, int order,
-                         float scale, int ow, int oh, int R0, int R1, uint8_t* dst, size_t dst_stride, size_t dst_frame_stride,
-                         const TapTable* ty, const TapTable* cty, int S0, int S1, const std::vector<int>& edges, int group, size_t s_row, size_t d_row, size_t s_frame,
-                         size_t d_frame) {
-    const int bands = (int)edges.size() - 1;
-    const size_t bpp = bytes_per_pixel(order), w_bytes = (size_t)w * bpp, ow_bytes = (size_t)ow * bpp;
-    // 4:2:0: frames are staged whole (S0 = 0, R0 = 0), every row at its place in the frame; a sub-band copies the chroma rows its
-    // chroma output rows [r0/2, r1/2) read (chroma tap table cty) along with its Y rows
-    const bool yuv = yuv420(order), i420 = order == SRCNN_ORDER_I420;
-    const size_t in_rows = yuv ? frame_rows(order, h) : (size_t)(S1 - S0), out_rows = yuv ? frame_rows(order, oh) : (size_t)(R1 - R0);
+// Enqueues the whole pipeline of frames [f0, f0 + m) of `im` on the three streams and joins the copy streams back into the
+// compute stream; does not wait.  Identical whether the streams are live or being captured into a CUDA graph.
+static int enqueue_chunk(Ctx* c, const Image& im, int f0, int m, const HostPlan& p) {
+    const Layout& L = im.L;
+    const int R0 = p.edges.front(), R1 = p.edges.back(), bands = (int)p.edges.size() - 1;
+    const size_t w_bytes = (size_t)im.w * L.bpp, ow_bytes = (size_t)im.ow * L.bpp;
     int rc;
     uint8_t* ds = (uint8_t*)c->src_buf.p;
     uint8_t* dd = (uint8_t*)c->dst_buf.p;
-    auto event_at = [&](size_t i, cudaEvent_t* e) -> int {
-        while (c->pipe_events.size() <= i) {
+    auto staged = [&](int f) {   // the device staging from frame f on, as a call of its own
+        return Image{ds + (size_t)f * p.s_frame, p.s_row, p.s_frame, dd + (size_t)f * p.d_frame, p.d_row, p.d_frame,
+                     im.w, im.h, im.ow, im.oh, im.scale, L};
+    };
+    size_t ei = 0;
+    auto join = [&](cudaStream_t from, cudaStream_t to) -> int {   // `to` waits for what `from` has been given so far
+        if (ei == c->pipe_events.size()) {
             cudaEvent_t ev;
             SRCNN_CUDA(c, cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
             c->pipe_events.push_back(ev);
         }
-        *e = c->pipe_events[i];
+        SRCNN_CUDA(c, cudaEventRecord(c->pipe_events[ei], from));
+        SRCNN_CUDA(c, cudaStreamWaitEvent(to, c->pipe_events[ei++], 0));
         return SRCNN_OK;
     };
-    auto src_hi = [&](int r1) {   // one past the last source row output rows < r1 touch (6-px halo in the output)
-        const int p1 = std::min(r1 + 6, oh);
-        return std::min(std::max(ty->h_ofs[p1 - 1] + 2, 0), h - 1) + 1;
-    };
-    const int rows = R1 - R0;
-    cudaEvent_t ev_start;
-    if ((rc = event_at(0, &ev_start))) return rc;
-    size_t ei = 1;
     // everything queued earlier on the compute stream (previous calls, tap-table uploads) precedes the copies
-    SRCNN_CUDA(c, cudaEventRecord(ev_start, c->stream));
-    SRCNN_CUDA(c, cudaStreamWaitEvent(c->s_in, ev_start, 0));
-    SRCNN_CUDA(c, cudaStreamWaitEvent(c->s_out, ev_start, 0));
+    if ((rc = join(c->stream, c->s_in))) return rc;
+    SRCNN_CUDA(c, cudaStreamWaitEvent(c->s_out, c->pipe_events[0], 0));
     if (bands == 1 && m > 1) {
-        // A batch of whole frames: groups of frames travel together -- one copy in, ONE launch per stage (process_frames: no
+        // A batch of whole frames: groups of frames travel together -- one copy in, ONE launch per stage (process: no
         // per-frame pipeline fill / drain in the fused kernel), one copy out -- sized so that a group's result is >= 64 MB:
         // large copies keep the PCIe link busy, and the next group's kernels still hide behind this group's D2H.
-        const bool rows_tight_in = src_stride == w_bytes && s_row == w_bytes;      // a frame is one contiguous run of bytes
-        const bool rows_tight_out = dst_stride == ow_bytes && d_row == ow_bytes;
-        for (int g0 = 0; g0 < m; g0 += group) {
-            const int g = std::min(group, m - g0);
-            const uint8_t* hsrc = src + (size_t)(f0 + g0) * src_frame_stride;
-            uint8_t* hdst = dst + (size_t)(f0 + g0) * dst_frame_stride;
-            cudaEvent_t ev_in, ev_done;
-            if ((rc = event_at(ei++, &ev_in))) return rc;
-            if (rows_tight_in) {   // frames are the "rows" of one 2-D copy
-                SRCNN_CUDA(c, cudaMemcpy2DAsync(ds + (size_t)g0 * s_frame, s_frame, hsrc + (size_t)S0 * src_stride, src_frame_stride,
-                                                in_rows * s_row, g, cudaMemcpyHostToDevice, c->s_in));
-            } else if (yuv) {
+        const bool rows_tight_in = im.src_stride == w_bytes && p.s_row == w_bytes;      // a frame is one contiguous run of bytes
+        const bool rows_tight_out = im.dst_stride == ow_bytes && p.d_row == ow_bytes;
+        for (int g0 = 0; g0 < m; g0 += p.group) {
+            const int g = std::min(p.group, m - g0);
+            const uint8_t* hsrc = im.src + (size_t)(f0 + g0) * im.src_frame + (size_t)p.S0 * im.src_stride;
+            uint8_t* hdst = im.dst + (size_t)(f0 + g0) * im.dst_frame;
+            if (rows_tight_in)   // frames are the "rows" of one 2-D copy
+                SRCNN_CUDA(c, cudaMemcpy2DAsync(ds + (size_t)g0 * p.s_frame, p.s_frame, hsrc, im.src_frame, L.rows(p.S1 - p.S0) * p.s_row, g,
+                                                cudaMemcpyHostToDevice, c->s_in));
+            else
                 for (int f = 0; f < g; f++)
-                    if ((rc = copy_420(c, i420, ds + (size_t)(g0 + f) * s_frame, s_row, hsrc + (size_t)f * src_frame_stride, src_stride, w, h,
-                                       0, h, 0, h / 2, cudaMemcpyHostToDevice, c->s_in)))
+                    if ((rc = copy_rows(c, L, ds + (size_t)(g0 + f) * p.s_frame, p.s_row, hsrc + (size_t)f * im.src_frame, im.src_stride,
+                                        im.w, im.h, 0, p.S1 - p.S0, 0, im.h / 2, cudaMemcpyHostToDevice, c->s_in)))
                         return rc;
-            } else {
-                for (int f = 0; f < g; f++)
-                    SRCNN_CUDA(c, cudaMemcpy2DAsync(ds + (size_t)(g0 + f) * s_frame, s_row, hsrc + (size_t)f * src_frame_stride + (size_t)S0 * src_stride,
-                                                    src_stride, w_bytes, S1 - S0, cudaMemcpyHostToDevice, c->s_in));
-            }
-            SRCNN_CUDA(c, cudaEventRecord(ev_in, c->s_in));
-            SRCNN_CUDA(c, cudaStreamWaitEvent(c->stream, ev_in, 0));
-            if (R0 == 0 && R1 == oh) {
-                rc = process_frames(c, ds + (size_t)g0 * s_frame, g, w, h, s_row, s_frame, order, scale, ow, oh, dd + (size_t)g0 * d_frame, d_row, d_frame);
-                if (rc) return rc;
-            } else {
-                for (int f = 0; f < g; f++) {
-                    rc = process_rows(c, ds + (size_t)(g0 + f) * s_frame, w, h, s_row, S0, S1, order, scale, ow, oh, R0, R1, dd + (size_t)(g0 + f) * d_frame, d_row);
-                    if (rc) return rc;
-                }
-            }
-            if ((rc = event_at(ei++, &ev_done))) return rc;
-            SRCNN_CUDA(c, cudaEventRecord(ev_done, c->stream));
-            SRCNN_CUDA(c, cudaStreamWaitEvent(c->s_out, ev_done, 0));
-            if (rows_tight_out) {
-                SRCNN_CUDA(c, cudaMemcpy2DAsync(hdst, dst_frame_stride, dd + (size_t)g0 * d_frame, d_frame, out_rows * d_row, g,
+            if ((rc = join(c->s_in, c->stream))) return rc;
+            if ((rc = process(c, staged(g0), g, 0, im.h, 0, im.oh)) || (rc = join(c->stream, c->s_out))) return rc;   // whole frames
+            if (rows_tight_out)
+                SRCNN_CUDA(c, cudaMemcpy2DAsync(hdst, im.dst_frame, dd + (size_t)g0 * p.d_frame, p.d_frame, L.rows(R1 - R0) * p.d_row, g,
                                                 cudaMemcpyDeviceToHost, c->s_out));
-            } else if (yuv) {
+            else
                 for (int f = 0; f < g; f++)
-                    if ((rc = copy_420(c, i420, hdst + (size_t)f * dst_frame_stride, dst_stride, dd + (size_t)(g0 + f) * d_frame, d_row, ow, oh,
-                                       0, oh, 0, oh / 2, cudaMemcpyDeviceToHost, c->s_out)))
+                    if ((rc = copy_rows(c, L, hdst + (size_t)f * im.dst_frame, im.dst_stride, dd + (size_t)(g0 + f) * p.d_frame, p.d_row,
+                                        im.ow, im.oh, 0, R1 - R0, 0, im.oh / 2, cudaMemcpyDeviceToHost, c->s_out)))
                         return rc;
-            } else {
-                for (int f = 0; f < g; f++)
-                    SRCNN_CUDA(c, cudaMemcpy2DAsync(hdst + (size_t)f * dst_frame_stride, dst_stride, dd + (size_t)(g0 + f) * d_frame, d_row, ow_bytes, rows,
-                                                    cudaMemcpyDeviceToHost, c->s_out));
-            }
         }
     } else
     for (int f = 0; f < m; f++) {
-        const uint8_t* hsrc = src + (size_t)(f0 + f) * src_frame_stride;
-        uint8_t* hdst = dst + (size_t)(f0 + f) * dst_frame_stride;
-        int copied = S0;   // source rows [S0, copied) of this frame are on their way to the device
-        int c_copied = 0;  // 4:2:0: chroma source rows [0, c_copied) likewise
+        const uint8_t* hsrc = im.src + (size_t)(f0 + f) * im.src_frame + (size_t)p.S0 * im.src_stride;
+        uint8_t* hdst = im.dst + (size_t)(f0 + f) * im.dst_frame;
+        int copied = p.S0;   // source rows [S0, copied) of this frame are on their way to the device
+        int c_copied = 0;    // 4:2:0: chroma source rows [0, c_copied) likewise
         for (int bi = 0; bi < bands; bi++) {
-            const int r0 = edges[bi], r1 = edges[bi + 1];
-            const int s_hi = bi + 1 < bands ? src_hi(r1) : S1;
-            const int c_hi = !yuv ? 0 : bi + 1 < bands ? std::min(std::max(cty->h_ofs[r1 / 2 - 1] + 2, 0), h / 2 - 1) + 1 : h / 2;
+            const int r0 = p.edges[bi], r1 = p.edges[bi + 1];
+            const int s_hi = bi + 1 < bands ? src_rows(p.ty->h_ofs.data(), im.h, im.oh, r0, r1).second : p.S1;
+            // 4:2:0: a sub-band also copies the chroma rows its chroma output rows [r0/2, r1/2) read
+            const int c_hi = !L.whole() ? 0 : bi + 1 < bands ? src_rows(p.cty->h_ofs.data(), im.h / 2, im.oh / 2, r0 / 2, r1 / 2, 0).second
+                                                            : im.h / 2;
             if (s_hi > copied || c_hi > c_copied) {
-                cudaEvent_t ev_in;
-                if ((rc = event_at(ei++, &ev_in))) return rc;
-                if (yuv) {
-                    if ((rc = copy_420(c, i420, ds + f * s_frame, s_row, hsrc, src_stride, w, h, copied, s_hi, c_copied, c_hi,
-                                       cudaMemcpyHostToDevice, c->s_in)))
-                        return rc;
-                } else {
-                    SRCNN_CUDA(c, cudaMemcpy2DAsync(ds + f * s_frame + (size_t)(copied - S0) * s_row, s_row, hsrc + (size_t)copied * src_stride,
-                                                    src_stride, w_bytes, s_hi - copied, cudaMemcpyHostToDevice, c->s_in));
-                }
-                SRCNN_CUDA(c, cudaEventRecord(ev_in, c->s_in));
-                SRCNN_CUDA(c, cudaStreamWaitEvent(c->stream, ev_in, 0));
+                if ((rc = copy_rows(c, L, ds + (size_t)f * p.s_frame, p.s_row, hsrc, im.src_stride, im.w, im.h, copied - p.S0, s_hi - p.S0,
+                                    c_copied, c_hi, cudaMemcpyHostToDevice, c->s_in)))
+                    return rc;
+                if ((rc = join(c->s_in, c->stream))) return rc;
                 copied = std::max(copied, s_hi);
                 c_copied = std::max(c_copied, c_hi);
             }
-            rc = process_rows(c, ds + f * s_frame, w, h, s_row, S0, S1, order, scale, ow, oh, r0, r1,
-                              dd + f * d_frame + (size_t)(r0 - R0) * d_row, d_row);
-            if (rc) return rc;
-            cudaEvent_t ev_done;
-            if ((rc = event_at(ei++, &ev_done))) return rc;
-            SRCNN_CUDA(c, cudaEventRecord(ev_done, c->stream));
-            SRCNN_CUDA(c, cudaStreamWaitEvent(c->s_out, ev_done, 0));
-            if (yuv) {
-                if ((rc = copy_420(c, i420, hdst, dst_stride, dd + f * d_frame, d_row, ow, oh, r0, r1, r0 / 2, r1 / 2, cudaMemcpyDeviceToHost,
-                                   c->s_out)))
-                    return rc;
-                continue;
-            }
-            SRCNN_CUDA(c, cudaMemcpy2DAsync(hdst + (size_t)(r0 - R0) * dst_stride, dst_stride,
-                                            dd + f * d_frame + (size_t)(r0 - R0) * d_row, d_row, ow_bytes, r1 - r0,
-                                            cudaMemcpyDeviceToHost, c->s_out));
+            Image band = staged(f);
+            band.dst += (size_t)(r0 - R0) * p.d_row;
+            if ((rc = process(c, band, 1, p.S0, p.S1, r0, r1)) || (rc = join(c->stream, c->s_out))) return rc;
+            if ((rc = copy_rows(c, L, hdst, im.dst_stride, dd + (size_t)f * p.d_frame, p.d_row, im.ow, im.oh, r0 - R0, r1 - R0, r0 / 2, r1 / 2,
+                                cudaMemcpyDeviceToHost, c->s_out)))
+                return rc;
         }
     }
-    // join: the compute stream ends after the last copy in either direction
-    cudaEvent_t ev_j1, ev_j2;
-    if ((rc = event_at(ei++, &ev_j1))) return rc;
-    if ((rc = event_at(ei++, &ev_j2))) return rc;
-    SRCNN_CUDA(c, cudaEventRecord(ev_j1, c->s_in));
-    SRCNN_CUDA(c, cudaEventRecord(ev_j2, c->s_out));
-    SRCNN_CUDA(c, cudaStreamWaitEvent(c->stream, ev_j1, 0));
-    SRCNN_CUDA(c, cudaStreamWaitEvent(c->stream, ev_j2, 0));
-    return SRCNN_OK;
+    // the compute stream ends after the last copy in either direction
+    if ((rc = join(c->s_in, c->stream))) return rc;
+    return join(c->s_out, c->stream);
 }
 
-int host_pipeline(Ctx* c, const uint8_t* src, int n, int w, int h, size_t src_stride, size_t src_frame_stride, int order,
-                  float scale, int ow, int oh, int R0, int R1, uint8_t* dst, size_t dst_stride, size_t dst_frame_stride) {
+static int host_pipeline(Ctx* c, const Image& im, int n, int R0, int R1) {
+    const Layout& L = im.L;
     int rc;
     struct HostPath {   // the pipeline's sub-bands and groups share Cr/Cb pair 0 (carve_planes) and never start early
         Ctx* c;
         explicit HostPath(Ctx* c_) : c(c_) { c->host_path = true; c->merge_sel = -1; }
         ~HostPath() { c->host_path = false; c->merge_sel = -1; }
     } host_path{c};
-    TapTable *ty = nullptr, *tx = nullptr, *cty = nullptr, *ctx_ = nullptr;
-    if ((rc = get_taps(c, h, oh, &ty))) return rc;
-    if ((rc = get_taps(c, w, ow, &tx))) return rc;      // uploaded here, not inside a graph capture
-    const bool yuv = yuv420(order);
-    if (yuv && ((rc = get_taps(c, h / 2, oh / 2, &cty)) || (rc = get_taps(c, w / 2, ow / 2, &ctx_)))) return rc;   // chroma
-    if (yuv422(order) && (rc = get_taps(c, w / 2, ow / 2, &ctx_))) return rc;   // 4:2:2 chroma (its vertical table is ty)
-    auto src_hi = [&](int r1) {
-        const int p1 = std::min(r1 + 6, oh);
-        return std::min(std::max(ty->h_ofs[p1 - 1] + 2, 0), h - 1) + 1;
-    };
+    HostPlan p;
+    TapTable *tx, *ctx_;
+    if ((rc = get_taps(c, im.h, im.oh, &p.ty))) return rc;
+    if ((rc = get_taps(c, im.w, im.ow, &tx))) return rc;      // uploaded here, not inside a graph capture
+    if (L.whole() && (rc = get_taps(c, im.h / 2, im.oh / 2, &p.cty))) return rc;                      // chroma (4:2:2: its vertical
+    if (L.chroma != Layout::kNone && (rc = get_taps(c, im.w / 2, im.ow / 2, &ctx_))) return rc;       // table is ty)
     // 4:2:0 frames are staged whole (whole-frame calls only: R0 = 0, R1 = oh), every row at its place in the frame
-    const int S0 = yuv ? 0 : std::min(std::max(ty->h_ofs[std::max(R0 - 6, 0)] - 1, 0), h - 1), S1 = yuv ? h : src_hi(R1);
-    // device staging: tight rows (4:2:0: 16-byte multiples, so that I420's half-length chroma rows stay 8-byte aligned), 256-byte
-    // aligned frames; only the rows this call needs
-    const size_t bpp = bytes_per_pixel(order), row_align = yuv ? 16 : 4;
-    const size_t s_row = align_up((size_t)w * bpp, row_align), d_row = align_up((size_t)ow * bpp, row_align);
-    const size_t s_frame = align_up(s_row * (yuv ? frame_rows(order, h) : (size_t)(S1 - S0)), 256);
-    const size_t d_frame = align_up(d_row * (yuv ? frame_rows(order, oh) : (size_t)(R1 - R0)), 256);
+    const auto need = src_rows(p.ty->h_ofs.data(), im.h, im.oh, R0, R1);
+    p.S0 = L.whole() ? 0 : need.first;
+    p.S1 = L.whole() ? im.h : need.second;
+    // device staging: tight rows, 256-byte aligned frames; only the rows this call needs
+    p.s_row = align_up((size_t)im.w * L.bpp, L.row_align);
+    p.d_row = align_up((size_t)im.ow * L.bpp, L.row_align);
+    p.s_frame = align_up(p.s_row * L.rows(p.S1 - p.S0), 256);
+    p.d_frame = align_up(p.d_row * L.rows(R1 - R0), 256);
     // frames in flight are bounded so staging stays modest (<= 4 GiB of output; one frame may be larger).  Chunks are separated by
     // a full drain of the pipeline, so the bound is generous: 180 GB of HBM is not the scarce resource here.
-    const int chunk = (int)std::max<size_t>(1, std::min<size_t>((size_t)n, ((size_t)4 << 30) / d_frame));
-    if ((rc = ensure(c, c->src_buf, s_frame * chunk))) return rc;
-    if ((rc = ensure(c, c->dst_buf, d_frame * chunk))) return rc;
+    const int chunk = (int)std::max<size_t>(1, std::min<size_t>((size_t)n, ((size_t)4 << 30) / p.d_frame));
+    if ((rc = ensure(c, c->src_buf, p.s_frame * chunk))) return rc;
+    if ((rc = ensure(c, c->dst_buf, p.d_frame * chunk))) return rc;
     if (!c->s_in) {
         SRCNN_CUDA(c, cudaStreamCreateWithFlags(&c->s_in, cudaStreamNonBlocking));
         SRCNN_CUDA(c, cudaStreamCreateWithFlags(&c->s_out, cudaStreamNonBlocking));
@@ -670,34 +587,34 @@ int host_pipeline(Ctx* c, const uint8_t* src, int n, int w, int h, size_t src_st
     // the previous band's D2H (~0.21 us per row) does, so a short first band starts the D2H early and longer later bands
     // keep the per-band overhead of the persistent kernel small (equal bands: 8 x 47 us of fused kernel for a frame that takes
     // 147 us whole).  Very tall bands (a gigapixel image) are cut into equal pieces whose planes stay below ~256 MB.
-    const int rows = R1 - R0;
-    std::vector<int> edges{R0};
+    const int rows = R1 - R0, even = L.whole() ? ~1 : ~0;   // 4:2:0: even band edges
+    p.edges.push_back(R0);
     if (n == 1 && rows >= 1024) {
-        const long long by_mem = ((long long)rows * (long long)ow * (four_channel(order) ? 5 : 4) + (256ll << 20) - 1) / (256ll << 20);
+        const long long by_mem = ((long long)rows * (long long)im.ow * L.planes() + (256ll << 20) - 1) / (256ll << 20);
         if (by_mem > c->host_bands) {
             const int nb = (int)std::min<long long>(by_mem, rows / 64);
-            for (int bi = 1; bi < nb; bi++) edges.push_back((R0 + (int)((long long)rows * bi / nb)) & (yuv ? ~1 : ~0));   // 4:2:0: even
+            for (int bi = 1; bi < nb; bi++) p.edges.push_back((R0 + (int)((long long)rows * bi / nb)) & even);
         } else if (c->host_bands > 1) {
             double len = c->band_first > 0 ? (double)c->band_first : std::max(256.0, (double)rows / c->host_bands);
             int pos = R0;
-            while ((int)edges.size() < c->host_bands) {
-                const int take = (int)len & (yuv ? ~1 : ~0);
+            while ((int)p.edges.size() < c->host_bands) {
+                const int take = (int)len & even;
                 if (R1 - (pos + take) < take / 2) break;      // the rest joins the last band
                 pos += take;
-                edges.push_back(pos);
+                p.edges.push_back(pos);
                 len *= c->band_growth;
             }
         }
     }
-    edges.push_back(R1);
-    const int bands = (int)edges.size() - 1;
+    p.edges.push_back(R1);
+    const int bands = (int)p.edges.size() - 1;
     int tallest = 0;
-    for (int bi = 0; bi < bands; bi++) tallest = std::max(tallest, edges[bi + 1] - edges[bi]);
+    for (int bi = 0; bi < bands; bi++) tallest = std::max(tallest, p.edges[bi + 1] - p.edges[bi]);
     // frames of a batch travel in groups whose result is >= 64 MB (see enqueue_chunk)
-    const int group = (int)std::max<size_t>(1, std::min<size_t>(16, ((size_t)64 << 20) / std::max<size_t>(1, (size_t)ow * bpp * (size_t)rows) + 1));
+    p.group = (int)std::max<size_t>(1, std::min<size_t>(16, ((size_t)64 << 20) / std::max<size_t>(1, (size_t)im.ow * L.bpp * (size_t)rows) + 1));
     {   // the planes of the tallest sub-band / of a group of frames, allocated before anything is enqueued or captured
         Planes pl;
-        if ((rc = carve_planes(c, ow, std::min(tallest + 12, oh), 0, &pl, (bands == 1 && n > 1) ? std::min(group, n) : 1, order)))
+        if ((rc = carve_planes(c, im.ow, std::min(tallest + 12, im.oh), 0, &pl, (bands == 1 && n > 1) ? std::min(p.group, n) : 1, L)))
             return rc;
     }
 
@@ -707,8 +624,9 @@ int host_pipeline(Ctx* c, const uint8_t* src, int n, int w, int h, size_t src_st
     PipeGraph* hit = nullptr;
     const bool graphable = c->use_graphs && !c->profiling && chunk >= n && bands * n <= 256;
     if (graphable) {
-        PipeKey key{src, dst, n, w, h, src_stride, src_frame_stride, order, scale, R0, R1, dst_stride, dst_frame_stride, c->variant,
-                    (int)c->fuse_merge, c->host_bands * 4096 + c->band_first, c->tc2_seg_ovh + (int)(c->band_growth * 1000.0) * 256, (void*)c->stream};
+        PipeKey key{im.src, im.dst, n, im.w, im.h, im.src_stride, im.src_frame, L.order, im.scale, R0, R1, im.dst_stride, im.dst_frame,
+                    c->variant, (int)c->fuse_merge, c->host_bands * 4096 + c->band_first, c->tc2_seg_ovh + (int)(c->band_growth * 1000.0) * 256,
+                    (void*)c->stream};
         for (auto& g : c->graphs)
             if (g.key == key) hit = &g;
         if (!hit) {
@@ -727,15 +645,14 @@ int host_pipeline(Ctx* c, const uint8_t* src, int n, int w, int h, size_t src_st
             hit->stamp = ++c->graph_clock;
         }
     }
-    if (hit && !hit->exec && !hit->failed && is_pinned(src) && is_pinned(dst)) {
+    if (hit && !hit->exec && !hit->failed && is_pinned(im.src) && is_pinned(im.dst)) {
         // second sighting: capture.  Nothing below allocates, uploads or synchronises (tables, staging and planes exist).
         cudaGraph_t graph = nullptr;
         const long long launches_before = c->launches;   // capturing enqueues nothing: the launch counter must not move
         cudaError_t e = cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal);
         if (e == cudaSuccess) {
             c->capturing = true;
-            rc = enqueue_chunk(c, src, 0, n, w, h, src_stride, src_frame_stride, order, scale, ow, oh, R0, R1, dst, dst_stride,
-                               dst_frame_stride, ty, cty, S0, S1, edges, group, s_row, d_row, s_frame, d_frame);
+            rc = enqueue_chunk(c, im, 0, n, p);
             e = cudaStreamEndCapture(c->stream, &graph);
             c->capturing = false;
             if (rc == SRCNN_OK && e == cudaSuccess && graph && cudaGraphInstantiate(&hit->exec, graph, 0) != cudaSuccess) hit->exec = nullptr;
@@ -755,9 +672,7 @@ int host_pipeline(Ctx* c, const uint8_t* src, int n, int w, int h, size_t src_st
     for (int f0 = 0; f0 < n; f0 += chunk) {
         const int m = std::min(chunk, n - f0);
         const long long l0 = c->launches;
-        rc = enqueue_chunk(c, src, f0, m, w, h, src_stride, src_frame_stride, order, scale, ow, oh, R0, R1, dst, dst_stride,
-                           dst_frame_stride, ty, cty, S0, S1, edges, group, s_row, d_row, s_frame, d_frame);
-        if (rc) return rc;
+        if ((rc = enqueue_chunk(c, im, f0, m, p))) return rc;
         if (graphable && f0 == 0)
             for (auto& g : c->graphs)
                 if (!g.exec && g.kernel_launches == 0) g.kernel_launches = c->launches - l0;   // what a replay of this call launches
@@ -1060,39 +975,27 @@ int srcnn_host_unregister(void* p) {
 
 int srcnn_process_device(srcnn_ctx* c, const uint8_t* d_src, int w, int h, size_t src_stride, int order, float scale,
                          uint8_t* d_dst, size_t dst_stride) {
-    ENTER_PROCESS(c);
-    int ow, oh;
-    int rc = check_image(c, d_src, w, h, src_stride, order, scale, d_dst, dst_stride, &ow, &oh);
-    if (rc) return rc;
-    return process_rows(c, d_src, w, h, src_stride, 0, h, order, scale, ow, oh, 0, oh, d_dst, dst_stride);
+    return srcnn_process_batch_device(c, d_src, 1, w, h, src_stride, 0, order, scale, d_dst, dst_stride, 0);
 }
 
 int srcnn_process_batch_device(srcnn_ctx* c, const uint8_t* d_src, int n, int w, int h, size_t src_stride,
                                size_t src_frame_stride, int order, float scale, uint8_t* d_dst, size_t dst_stride,
                                size_t dst_frame_stride) {
     ENTER_PROCESS(c);
-    if (n < 0) return fail(c, SRCNN_E_ARG, "negative frame count");
-    if (n == 0) return SRCNN_OK;
-    int ow, oh;
-    int rc = check_image(c, d_src, w, h, src_stride, order, scale, d_dst, dst_stride, &ow, &oh);
-    if (rc) return rc;
-    if (n > 1 && (src_frame_stride < src_stride * frame_rows(order, h) || dst_frame_stride < dst_stride * frame_rows(order, oh)))
-        return fail(c, SRCNN_E_ARG, "frame stride smaller than one frame");
-    return process_frames(c, d_src, n, w, h, src_stride, src_frame_stride, order, scale, ow, oh, d_dst, dst_stride, dst_frame_stride);
+    Image im;
+    int rc = check_batch(c, n, d_src, w, h, src_stride, src_frame_stride, order, scale, d_dst, dst_stride, dst_frame_stride, &im);
+    if (rc || n == 0) return rc;
+    return process(c, im, n, 0, h, 0, im.oh);
 }
 
 int srcnn_process_batch_host(srcnn_ctx* c, const uint8_t* src, int n, int w, int h, size_t src_stride,
                              size_t src_frame_stride, int order, float scale, uint8_t* dst, size_t dst_stride,
                              size_t dst_frame_stride) {
     ENTER_PROCESS(c);
-    if (n < 0) return fail(c, SRCNN_E_ARG, "negative frame count");
-    if (n == 0) return SRCNN_OK;
-    int ow, oh;
-    int rc = check_image(c, src, w, h, src_stride, order, scale, dst, dst_stride, &ow, &oh);
-    if (rc) return rc;
-    if (n > 1 && (src_frame_stride < src_stride * frame_rows(order, h) || dst_frame_stride < dst_stride * frame_rows(order, oh)))
-        return fail(c, SRCNN_E_ARG, "frame stride smaller than one frame");
-    return host_pipeline(c, src, n, w, h, src_stride, src_frame_stride, order, scale, ow, oh, 0, oh, dst, dst_stride, dst_frame_stride);
+    Image im;
+    int rc = check_batch(c, n, src, w, h, src_stride, src_frame_stride, order, scale, dst, dst_stride, dst_frame_stride, &im);
+    if (rc || n == 0) return rc;
+    return host_pipeline(c, im, n, 0, im.oh);
 }
 
 int srcnn_process_host(srcnn_ctx* c, const uint8_t* src, int w, int h, size_t src_stride, int order, float scale,
@@ -1106,36 +1009,53 @@ int srcnn_band_src_rows(int h, float scale, int r0, int r1, int* s0, int* s1) {
     const int oh = scaled_dim(h, scale);
     if (oh <= 0) return SRCNN_E_RATIO;
     if (r0 < 0 || r1 > oh || r0 >= r1) return SRCNN_E_ARG;
-    const int p0 = std::max(r0 - 6, 0), p1 = std::min(r1 + 6, oh);
     std::vector<int> ofs(oh);
     std::vector<short4> coef(oh);
     build_cubic_taps(h, oh, ofs.data(), coef.data());
-    *s0 = std::min(std::max(ofs[p0] - 1, 0), h - 1);
-    *s1 = std::min(std::max(ofs[p1 - 1] + 2, 0), h - 1) + 1;
+    std::tie(*s0, *s1) = src_rows(ofs.data(), h, oh, r0, r1);
+    return SRCNN_OK;
+}
+
+// the output band of a band call, after check_image
+static int check_band(Ctx* c, const Image& im, int r0, int r1) {
+    if (im.L.whole()) return fail(c, SRCNN_E_ARG, "4:2:0 frames are whole-frame calls only (no band calls)");
+    if (r0 < 0 || r1 > im.oh || r0 >= r1) return fail(c, SRCNN_E_ARG, "bad output band [%d,%d) of %d rows", r0, r1, im.oh);
     return SRCNN_OK;
 }
 
 int srcnn_process_band_device(srcnn_ctx* c, const uint8_t* d_src, int w, int h, size_t src_stride, int s0, int s1,
                               int order, float scale, int r0, int r1, uint8_t* d_dst, size_t dst_stride) {
     ENTER_PROCESS(c);
-    int ow, oh;
-    int rc = check_image(c, d_src, w, h, src_stride, order, scale, d_dst, dst_stride, &ow, &oh);
-    if (rc) return rc;
-    if (yuv420(order)) return fail(c, SRCNN_E_ARG, "4:2:0 frames are whole-frame calls only (no band calls)");
-    if (r0 < 0 || r1 > oh || r0 >= r1) return fail(c, SRCNN_E_ARG, "bad output band [%d,%d) of %d rows", r0, r1, oh);
+    Image im;
+    int rc = check_image(c, d_src, w, h, src_stride, order, scale, d_dst, dst_stride, &im);
+    if (rc || (rc = check_band(c, im, r0, r1))) return rc;
     if (s0 < 0 || s1 > h || s0 >= s1) return fail(c, SRCNN_E_ARG, "bad source band [%d,%d) of %d rows", s0, s1, h);
-    return process_rows(c, d_src, w, h, src_stride, s0, s1, order, scale, ow, oh, r0, r1, d_dst, dst_stride);
+    return process(c, im, 1, s0, s1, r0, r1);
 }
 
 int srcnn_process_band_host(srcnn_ctx* c, const uint8_t* src, int w, int h, size_t src_stride, int order, float scale,
                             int r0, int r1, uint8_t* dst_rows, size_t dst_stride) {
     ENTER_PROCESS(c);
-    int ow, oh;
-    int rc = check_image(c, src, w, h, src_stride, order, scale, dst_rows, dst_stride, &ow, &oh);
+    Image im;
+    int rc = check_image(c, src, w, h, src_stride, order, scale, dst_rows, dst_stride, &im);
+    if (rc || (rc = check_band(c, im, r0, r1))) return rc;
+    return host_pipeline(c, im, 1, r0, r1);
+}
+
+// Rows [0, oh) of a whole image through the colour+bicubic kernels into `pl` (the stage entry points)
+static int resize_image(Ctx* c, const uint8_t* d_src, int w, int h, size_t src_stride, int order, int ow, int oh, const Planes& pl) {
+    TapTable *tx, *ty;
+    int rc = get_taps(c, w, ow, &tx);
     if (rc) return rc;
-    if (yuv420(order)) return fail(c, SRCNN_E_ARG, "4:2:0 frames are whole-frame calls only (no band calls)");
-    if (r0 < 0 || r1 > oh || r0 >= r1) return fail(c, SRCNN_E_ARG, "bad output band [%d,%d) of %d rows", r0, r1, oh);
-    return host_pipeline(c, src, 1, w, h, src_stride, 0, order, scale, ow, oh, r0, r1, dst_rows, dst_stride, 0);
+    if ((rc = get_taps(c, h, oh, &ty))) return rc;
+    ResizeArgs ra;
+    ra.src = d_src; ra.src_stride = src_stride;
+    ra.sw = w; ra.sh = h; ra.src_row0 = 0; ra.src_row1 = h;
+    ra.order = order; ra.ow = ow; ra.oh = oh;
+    ra.row_begin = 0; ra.row_end = oh;
+    ra.pl = pl; ra.pl.row0 = 0; ra.pl.rows = oh;
+    ra.tx = tx; ra.ty = ty;
+    return launch_color_bicubic(c, ra);
 }
 
 int srcnn_stage_color_bicubic_device(srcnn_ctx* c, const uint8_t* d_src, int w, int h, size_t src_stride, int order,
@@ -1149,38 +1069,18 @@ int srcnn_stage_color_bicubic_device(srcnn_ctx* c, const uint8_t* d_src, int w, 
     if (ow <= 0 || oh <= 0) return fail(c, SRCNN_E_RATIO, "ratio too small");
     if (plane_pitch < align_up((size_t)ow, 4) || (plane_pitch & 3) || (((uintptr_t)d_y | (uintptr_t)d_cr | (uintptr_t)d_cb) & 3))
         return fail(c, SRCNN_E_ARG, "planes must be 4-byte aligned with pitch a multiple of 4 and >= ow rounded up to 4");
-    TapTable *tx, *ty;
-    int rc = get_taps(c, w, ow, &tx);
-    if (rc) return rc;
-    rc = get_taps(c, h, oh, &ty);
-    if (rc) return rc;
-    ResizeArgs ra;
-    ra.src = d_src; ra.src_stride = src_stride;
-    ra.sw = w; ra.sh = h; ra.src_row0 = 0; ra.src_row1 = h;
-    ra.order = order; ra.ow = ow; ra.oh = oh;
-    ra.row_begin = 0; ra.row_end = oh;
-    ra.pl.y = d_y; ra.pl.cr = d_cr; ra.pl.cb = d_cb; ra.pl.yout = nullptr; ra.pl.y16 = nullptr;
-    ra.pl.pitch = plane_pitch; ra.pl.row0 = 0; ra.pl.rows = oh;
-    ra.tx = tx; ra.ty = ty;
-    return launch_color_bicubic(c, ra);
+    Planes pl;
+    pl.y = d_y; pl.cr = d_cr; pl.cb = d_cb; pl.pitch = plane_pitch;
+    return resize_image(c, d_src, w, h, src_stride, order, ow, oh, pl);
 }
 
 // One 8-bit plane through cv::resize(..., INTER_CUBIC) (src/srcnn.cpp:577-582): the one-plane resize kernels.  Device buffers,
 // enqueued; d_dst must be 4-byte aligned with a pitch that is a multiple of 4 (the tiled kernel's word stores).
 static int resize_plane(Ctx* c, const uint8_t* d_src, int w, int h, size_t src_stride, int ow, int oh, uint8_t* d_dst,
                         size_t dst_stride) {
-    TapTable *tx, *ty;
-    int rc = get_taps(c, w, ow, &tx);
-    if (rc) return rc;
-    if ((rc = get_taps(c, h, oh, &ty))) return rc;
-    ResizeArgs ra;
-    ra.src = d_src; ra.src_stride = src_stride;
-    ra.sw = w; ra.sh = h; ra.src_row0 = 0; ra.src_row1 = h;
-    ra.order = SRCNN_ORDER_GRAY; ra.ow = ow; ra.oh = oh;
-    ra.row_begin = 0; ra.row_end = oh;
-    ra.pl.y = d_dst; ra.pl.pitch = dst_stride; ra.pl.row0 = 0; ra.pl.rows = oh;
-    ra.tx = tx; ra.ty = ty;
-    return launch_color_bicubic(c, ra);
+    Planes pl;
+    pl.y = d_dst; pl.pitch = dst_stride;
+    return resize_image(c, d_src, w, h, src_stride, SRCNN_ORDER_GRAY, ow, oh, pl);
 }
 
 static int check_plane(Ctx* c, const void* src, int w, int h, size_t src_stride, float scale, const void* dst, size_t dst_stride,

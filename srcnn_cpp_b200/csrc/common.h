@@ -289,8 +289,6 @@ struct CnnArgs {
 int launch_cnn_fp32(Ctx* c, const CnnArgs& a, float* act2_out /* optional full act2 dump, may be null */);
 int fp32_prepare(Ctx* c);    // uploads the parameters to the device's constant bank (once per device and process)
 void fraw_release(Ctx* c);   // frees the cached frawscale contribution tables
-int host_pipeline(Ctx* c, const uint8_t* src, int n, int w, int h, size_t src_stride, size_t src_frame_stride, int order,
-                  float scale, int ow, int oh, int R0, int R1, uint8_t* dst, size_t dst_stride, size_t dst_frame_stride);
 int launch_cnn_tc2(Ctx* c, const CnnArgs& a);
 void tc2_pack_weights(const float* params, uint8_t* img);   // host only: img = tc2_weight_bytes() bytes
 size_t tc2_weight_bytes();
