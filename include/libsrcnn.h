@@ -4,8 +4,8 @@
 // srcnn_b200.h, implemented in srcnn_cpp_b200/cli/libsrcnn.cpp and exported by libsrcnn_b200.so.
 //
 //   refbuff   packed 8-bit pixels, `d` bytes per pixel: 3 = RGB, 4 = RGBA (one SRCNN_ORDER_RGBA call: colour goes through the
-//             SRCNN path, straight alpha takes the path's plain bicubic resize, no CNN), 1 = grey, 2 = grey+alpha (grey: the
-//             one-plane path, SRCNN_ORDER_GRAY; its alpha through srcnn_resize_plane_host) -- the inputs
+//             SRCNN path, straight alpha takes the path's plain bicubic resize, no CNN), 1 = grey (SRCNN_ORDER_GRAY), 2 =
+//             grey+alpha (one SRCNN_ORDER_GRAYA call: grey through the one-plane path, alpha as for d = 4) -- the inputs
 //             src/test.cpp:34-134 (convImage) can produce
 //   w, h, d   geometry
 //   muliply   scale ratio (sic, the reference's spelling)

@@ -53,6 +53,14 @@
  * with the even luma samples, so it gets the quarter-pixel horizontal shift any centre-aligned resize gives -- not compensated.
  * The planes are treated independently, so YVYU and VYUY (V before U) are the same two orders.  Chroma has the full vertical
  * resolution, so every whole-path call takes these orders, the band calls and srcnn_mgpu_process_banded_* included.
+ * SRCNN_ORDER_GRAYA: grey + alpha, 2 interleaved bytes per pixel in and out -- PNG colour type 4, FFmpeg's ya8, two-channel
+ * luminance-alpha textures, ProcessSRCNN's d = 2.  Grey in byte 0, straight (not premultiplied) alpha in byte 1.  stride >= 2*w,
+ * dst_stride >= 2*ow, batch frame strides >= stride*h (dst_stride*oh); any w, h and scale (no evenness rule) and any alignment
+ * (unaligned buffers may take slower kernels).  Byte for byte: byte 0 of every output pixel is the SRCNN_ORDER_GRAY call on the
+ * source's grey plane (alpha has no influence on it); byte 1 is the alpha plane through the one-plane resize
+ * (srcnn_stage_resize_plane_device: resize(alpha, INTER_CUBIC), no CNN).  It is NOT always channel 1 of cv::resize on a CV_8UC2
+ * image, whose float body / integer tail split differs (see the four-channel orders above).  Alpha has the full vertical
+ * resolution, so every whole-path call takes this order, the band calls and srcnn_mgpu_process_banded_* included.
  * Output size is ow=(int)((float)w*scale), oh=(int)((float)h*scale) -- the reference's truncation (src/srcnn.cpp:573-575,
  * src/test.cpp:357-358).
  */
@@ -82,7 +90,7 @@ enum {
 
 /* 5 is not assigned: it has been rejected as an unknown order since the four-channel orders were added, and stays so. */
 enum { SRCNN_ORDER_BGR = 0, SRCNN_ORDER_RGB = 1, SRCNN_ORDER_GRAY = 2, SRCNN_ORDER_BGRA = 3, SRCNN_ORDER_RGBA = 4,
-       SRCNN_ORDER_NV12 = 6, SRCNN_ORDER_I420 = 7, SRCNN_ORDER_YUY2 = 8, SRCNN_ORDER_UYVY = 9 };
+       SRCNN_ORDER_NV12 = 6, SRCNN_ORDER_I420 = 7, SRCNN_ORDER_YUY2 = 8, SRCNN_ORDER_UYVY = 9, SRCNN_ORDER_GRAYA = 10 };
 
 /* Status codes.  -1 / -2 / -3 / -10 keep the reference CLI's meanings (src/srcnn.cpp:479,493,526,555,684). */
 enum {
@@ -234,11 +242,12 @@ void srcnn_jpeg_free(uint8_t* p);
 
 /* ---- stages (device pointers; enqueued on the context stream) ------------------------------------ */
 /* cvtColor + split + 3x resize (src/srcnn.cpp:509,540,570-583): BGR8 -> three u8 planes of ow x oh.  Colour orders only
- * (SRCNN_ORDER_GRAY, _BGRA, _RGBA, the 4:2:0 and 4:2:2 orders: SRCNN_E_ARG; srcnn_stage_resize_plane_device is the one-plane stage). */
+ * (SRCNN_ORDER_GRAY, _BGRA, _RGBA, _GRAYA, the 4:2:0 and 4:2:2 orders: SRCNN_E_ARG; srcnn_stage_resize_plane_device is the
+ * one-plane stage). */
 int srcnn_stage_color_bicubic_device(srcnn_ctx* ctx, const uint8_t* d_src, int w, int h, size_t src_stride,
                                      int order, float scale, uint8_t* d_y, uint8_t* d_cr, uint8_t* d_cb,
                                      size_t plane_pitch);
-/* One 8-bit plane through resize(..., CV_INTER_CUBIC) (src/srcnn.cpp:577-582), host buffers (ProcessSRCNN's alpha). */
+/* One 8-bit plane through resize(..., CV_INTER_CUBIC) (src/srcnn.cpp:577-582), host buffers. */
 int srcnn_resize_plane_host(srcnn_ctx* ctx, const uint8_t* src, int w, int h, size_t src_stride, float scale,
                             uint8_t* dst, size_t dst_stride);
 /* The same on device buffers, enqueued on the context stream: one u8 plane through resize(..., CV_INTER_CUBIC).  Any

@@ -27,6 +27,8 @@ ORDER_NV12 = 6   # packed 4:2:0 video frames: (H*3/2)xW ((N)x(H*3/2)xW) arrays a
 ORDER_I420 = 7   # chroma planes = the one-plane cubic resize of the source's (no CNN).  yuv420_planes() splits a frame
 ORDER_YUY2 = 8   # packed 4:2:2 (bytes Y0 U Y1 V / U Y0 V Y1): HxWx2 (NxHxWx2) arrays and tensors in and out, OpenCV's CV_8UC2 shape;
 ORDER_UYVY = 9   # Y plane = the grey call's, U / V = the one-plane cubic resize of the source's.  yuv422_planes() splits a frame
+ORDER_GRAYA = 10   # grey + straight alpha (bytes G A): HxWx2 (NxHxWx2) arrays and tensors in and out; byte 0 = the grey call's,
+                   # byte 1 = the one-plane cubic resize of the alpha plane (no CNN).  img[..., 0] / img[..., 1] are the planes
 
 OK = 0
 E_RATIO = -1
@@ -186,10 +188,10 @@ class PinnedBuffer:
 
 def _pixel_shape(order):
     """trailing shape of one pixel: () for ORDER_GRAY and the 4:2:0 orders, (4,) for ORDER_BGRA / ORDER_RGBA, (2,) for the 4:2:2
-    orders, (3,) for the colour orders"""
+    orders and ORDER_GRAYA, (3,) for the colour orders"""
     if order in (ORDER_GRAY, ORDER_NV12, ORDER_I420):
         return ()
-    if order in (ORDER_YUY2, ORDER_UYVY):
+    if order in (ORDER_YUY2, ORDER_UYVY, ORDER_GRAYA):
         return (2,)
     return (4,) if order in (ORDER_BGRA, ORDER_RGBA) else (3,)
 
@@ -323,7 +325,8 @@ class Engine:
     # -- whole path, host buffers (numpy) ----------------------------------------------------------
     def process(self, img, scale, order=ORDER_BGR, out=None):
         """img: HxWx3 uint8 numpy array (BGR by default, like cv::imread), HxW with order=ORDER_GRAY, HxWx4 with
-        order=ORDER_BGRA / ORDER_RGBA, an (H*3/2)xW frame with ORDER_NV12 / ORDER_I420, or HxWx2 with ORDER_YUY2 / ORDER_UYVY.
+        order=ORDER_BGRA / ORDER_RGBA, an (H*3/2)xW frame with ORDER_NV12 / ORDER_I420, or HxWx2 with ORDER_YUY2 / ORDER_UYVY /
+        ORDER_GRAYA.
         Returns OHxOWx3 (OHxOW, OHxOWx4, (OH*3/2)xOW, OHxOWx2) uint8."""
         img = np.asarray(img)
         _check_host_image(img, order, 1)
@@ -338,8 +341,8 @@ class Engine:
         return out
 
     def process_batch(self, frames, scale, order=ORDER_BGR, out=None):
-        """frames: NxHxWx3 (NxHxW with order=ORDER_GRAY, NxHxWx4 with ORDER_BGRA / ORDER_RGBA) uint8 numpy array -> NxOHxOWx3
-        (NxOHxOW, NxOHxOWx4)."""
+        """frames: NxHxWx3 (NxHxW with order=ORDER_GRAY, NxHxWx4 with ORDER_BGRA / ORDER_RGBA, NxHxWx2 with ORDER_YUY2 /
+        ORDER_UYVY / ORDER_GRAYA) uint8 numpy array -> NxOHxOWx3 (NxOHxOW, NxOHxOWx4, NxOHxOWx2)."""
         frames = np.ascontiguousarray(frames)
         _check_host_image(frames, order, 2)
         n, h, w = frames.shape[0], _frame_h(order, frames.shape[1]), frames.shape[2]
@@ -355,7 +358,7 @@ class Engine:
     def process_device(self, src, scale, dst, order=ORDER_BGR):
         """src: HxWx3 (HxW with order=ORDER_GRAY, HxWx4 with ORDER_BGRA / ORDER_RGBA) uint8 device tensor; dst: OHxOWx3
         (OHxOW, OHxOWx4); (H*3/2)xW and (OH*3/2)xOW frames with ORDER_NV12 / ORDER_I420; HxWx2 and OHxOWx2 with ORDER_YUY2 /
-        ORDER_UYVY."""
+        ORDER_UYVY / ORDER_GRAYA."""
         h, w = _frame_h(order, src.shape[0]), src.shape[1]
         self._check(self.L.srcnn_process_device(self.ctx, _dptr(src), w, h, src.stride(0), order, C.c_float(scale),
                                                 _dptr(dst), dst.stride(0)))
@@ -369,7 +372,7 @@ class Engine:
 
     def process_band_device(self, src_rows, w, h, s0, s1, scale, r0, r1, dst_rows, order=ORDER_BGR):
         """src_rows: (s1-s0)xWx3 device tensor holding source rows [s0,s1); dst_rows: (r1-r0)xOWx3 (no x3 with ORDER_GRAY, x4
-        with ORDER_BGRA / ORDER_RGBA)."""
+        with ORDER_BGRA / ORDER_RGBA, x2 with ORDER_YUY2 / ORDER_UYVY / ORDER_GRAYA)."""
         self._check(self.L.srcnn_process_band_device(self.ctx, _dptr(src_rows), w, h, src_rows.stride(0), s0, s1, order,
                                                      C.c_float(scale), r0, r1, _dptr(dst_rows), dst_rows.stride(0)))
         return dst_rows
@@ -399,8 +402,8 @@ class Engine:
         self._check(self.L.srcnn_debug_set_host_bands(self.ctx, int(bands)))
 
     def process_band_host(self, img, scale, r0, r1, out_rows=None, order=ORDER_BGR):
-        """img: the WHOLE HxWx3 (HxW, HxWx4) source image; returns output rows [r0, r1) as an (r1-r0)xOWx3 ((r1-r0)xOW,
-        (r1-r0)xOWx4) array."""
+        """img: the WHOLE HxWx3 (HxW, HxWx4, HxWx2) source image; returns output rows [r0, r1) as an (r1-r0)xOWx3 ((r1-r0)xOW,
+        (r1-r0)xOWx4, (r1-r0)xOWx2) array."""
         img = np.ascontiguousarray(img)
         _check_host_image(img, order, 1)
         h, w = img.shape[:2]
@@ -536,7 +539,8 @@ class MultiEngine:
 
     # -- device-resident shares (torch CUDA tensors, one per worker, each on that worker's device) -----
     def process_batch_device(self, srcs, scale, dsts, order=ORDER_BGR):
-        """srcs[i]: n_i x H x W x 3 (no x 3 with ORDER_GRAY, x 4 with ORDER_BGRA / ORDER_RGBA) on worker i's device (n_i may be
+        """srcs[i]: n_i x H x W x 3 (no x 3 with ORDER_GRAY, x 4 with ORDER_BGRA / ORDER_RGBA, x 2 with ORDER_YUY2 / ORDER_UYVY /
+        ORDER_GRAYA) on worker i's device (n_i may be
         0 -> pass None); dsts[i]: n_i x OH x OW x 3 (likewise)."""
         ref = next(t for t in srcs if t is not None)
         h, w = _frame_h(order, ref.shape[1]), ref.shape[2]
@@ -548,7 +552,7 @@ class MultiEngine:
                                                            pd, dref.stride(1), dref.stride(0)))
 
     def process_banded_device(self, src_bands, w, h, scale, dst_bands, order=ORDER_BGR):
-        """src_bands[i]: (s1_i-s0_i) x W x 3 (x 4, or no channel dim, per `order`) holding the source rows of band_plan()[i];
+        """src_bands[i]: (s1_i-s0_i) x W x 3 (x 4, x 2, or no channel dim, per `order`) holding the source rows of band_plan()[i];
         dst_bands[i]: (r1_i-r0_i) x OW x 3 (likewise)."""
         ps = (C.c_void_p * self.n)(*[t.data_ptr() if t is not None else None for t in src_bands])
         pd = (C.c_void_p * self.n)(*[t.data_ptr() if t is not None else None for t in dst_bands])

@@ -69,8 +69,9 @@ static int scaled_dim(int n, float scale) {
 
 // What the host path needs to know about a pixel order, from layout_of: no other function of the whole path asks for the order.
 struct Layout {
-    enum Finish { kCnnOut, kMerge, kPack };   // the last kernel: the CNN into the caller's frame, the merge, the 4:2:2 pack kernel
-    enum Chroma { kNone, k420, k422 };        // chroma resized without the CNN: none, w/2 x h/2, w/2 x h
+    enum Finish { kCnnOut, kMerge, kPack };   // the last kernel: the CNN into the caller's frame, the merge, the pack kernel
+                                              // (4:2:2, grey + alpha)
+    enum Chroma { kNone, k420, k422, kAlpha };   // planes resized without the CNN: none, chroma w/2 x h/2, w/2 x h, alpha w x h
     int order = -1;                           // -1: not an order of the whole path
     size_t bpp = 0;          // bytes per pixel of a row (4:2:0: of a Y row; NV12's chroma rows have as many, I420's half as many)
     size_t row_align = 4;    // device staging rows (4:2:0: 16-byte multiples, so that I420's half-length rows stay 8-byte aligned)
@@ -78,10 +79,12 @@ struct Layout {
     Chroma chroma = kNone;
     bool i420 = false;       // chroma rows half as long, stride/2 apart: even strides
     bool alpha = false;      // four-channel: an A plane beside Cr / Cb
-    bool fuses = false;      // the fused merge takes it (a four-channel call needs the merge for alpha, a 4:2:2 call its pack kernel)
+    bool fuses = false;      // the fused merge takes it (a four-channel call needs the merge for alpha, 4:2:2 and GRAYA their pack kernel)
     // 4:2:0: h rows of Y, then h/2 rows of NV12 pairs or of I420 U and V: even sizes, frames staged whole, no band calls
     bool whole() const { return chroma == k420; }
-    bool cbcr() const { return finish != kCnnOut; }   // the workspace has Cr / Cb planes (4:2:2: U' / V'), so the call merges
+    int csub() const { return chroma == kAlpha ? 1 : 2; }   // Y columns per column of the planes resized without the CNN
+    // the workspace has Cr / Cb planes (4:2:2: U' / V'; GRAYA: A' in the Cr slot, Cb unused), so the call merges
+    bool cbcr() const { return finish != kCnnOut; }
     int planes() const { return alpha ? 5 : 4; }    // u8 workspace planes per frame
     size_t rows(int n) const { return whole() ? (size_t)n / 2 * 3 : (size_t)n; }   // rows in memory of a frame of n Y rows
 };
@@ -95,6 +98,7 @@ static Layout layout_of(int order) {
         case SRCNN_ORDER_NV12: case SRCNN_ORDER_I420:
             L.bpp = 1; L.row_align = 16; L.finish = Layout::kCnnOut; L.chroma = Layout::k420; L.i420 = order == SRCNN_ORDER_I420; break;
         case SRCNN_ORDER_YUY2: case SRCNN_ORDER_UYVY: L.bpp = 2; L.finish = Layout::kPack; L.chroma = Layout::k422; break;
+        case SRCNN_ORDER_GRAYA: L.bpp = 2; L.finish = Layout::kPack; L.chroma = Layout::kAlpha; break;
         default: return L;
     }
     L.order = order;
@@ -163,14 +167,14 @@ static std::pair<int, int> src_rows(const int* ofs, int h, int oh, int r0, int r
 // The chroma descriptor of the luma output rows [r0, r1) of frames whose row 0 is at `src` / `dst` (frame 0).  No halo: a chroma
 // row is resized without the CNN.  4:2:0: the chroma rows after the Y rows, resized straight into the caller's frames (chroma
 // output rows [r0/2, r1/2)).  4:2:2: U' and V' of the packed rows go into the Cr / Cb planes of `pl` (their first ow/2 columns),
-// which the pack kernel reads for the same rows.
+// which the pack kernel reads for the same rows.  GRAYA: the alpha plane (w x h -> ow x oh) likewise, into the Cr plane.
 static int chroma_planes(Ctx* c, const Image& im, const uint8_t* src, uint8_t* dst, const Planes& pl, int r0, int r1, Chroma420* ch) {
-    const int v = im.L.whole() ? 2 : 1;   // Y rows per chroma row
+    const int v = im.L.whole() ? 2 : 1, u = im.L.csub();   // Y rows per chroma row, Y columns per chroma column
     TapTable *tx, *ty;
-    int rc = get_taps(c, im.w / 2, im.ow / 2, &tx);
+    int rc = get_taps(c, im.w / u, im.ow / u, &tx);
     if (rc) return rc;
     if ((rc = get_taps(c, im.h / v, im.oh / v, &ty))) return rc;
-    ch->sw = im.w / 2; ch->sh = im.h / v; ch->ow = im.ow / 2; ch->oh = im.oh / v;
+    ch->sw = im.w / u; ch->sh = im.h / v; ch->ow = im.ow / u; ch->oh = im.oh / v;
     ch->row_begin = r0 / v; ch->row_end = r1 / v;
     ch->tx = tx; ch->ty = ty;
     if (!im.L.whole()) {
@@ -202,7 +206,7 @@ static int chroma_planes(Ctx* c, const Image& im, const uint8_t* src, uint8_t* d
 // at 4K) measured 3 us slower in the colour+bicubic kernel.
 // The host-buffer pipeline keeps to set 0 (its sub-bands are separated by copies and events anyway).  A grey or 4:2:0 call has no
 // Cr/Cb planes: it leaves the set selection alone (and ends the early-start chain, end_merge_chain).  A packed 4:2:2 call keeps its
-// U' / V' planes in the Cr / Cb slots and so takes part like a colour call.
+// U' / V' planes in the Cr / Cb slots, a GRAYA call its A' plane in the Cr slot, and so they take part like a colour call.
 static int carve_planes(Ctx* c, int ow, int rows, int row0, Planes* pl, int nframes, const Layout& L) {
     const bool gray = !L.cbcr(), four = L.alpha;
     const size_t pitch = align_up((size_t)ow, 128);
@@ -367,7 +371,7 @@ static int run_stages(Ctx* c, const Image& im, int f0, int m, int s0, int s1, in
         if (pl.a) ma.a = pl.a + off;
         ma.rows = tall ? (r1 - r0) * m : r1 - r0;
         ma.dst = dst + (size_t)f * im.dst_frame;
-        if ((rc = L.finish == Layout::kPack ? launch_pack422(c, ma) : launch_merge(c, ma))) return rc;
+        if ((rc = L.finish == Layout::kPack ? launch_pack(c, ma) : launch_merge(c, ma))) return rc;
     }
     merged_into(c, dst, (size_t)(m - 1) * im.dst_frame + (size_t)(r1 - r0) * im.dst_stride);
     return prof_mark(c, 3);
@@ -562,7 +566,7 @@ static int host_pipeline(Ctx* c, const Image& im, int n, int R0, int R1) {
     if ((rc = get_taps(c, im.h, im.oh, &p.ty))) return rc;
     if ((rc = get_taps(c, im.w, im.ow, &tx))) return rc;      // uploaded here, not inside a graph capture
     if (L.whole() && (rc = get_taps(c, im.h / 2, im.oh / 2, &p.cty))) return rc;                      // chroma (4:2:2: its vertical
-    if (L.chroma != Layout::kNone && (rc = get_taps(c, im.w / 2, im.ow / 2, &ctx_))) return rc;       // table is ty)
+    if (L.chroma != Layout::kNone && (rc = get_taps(c, im.w / L.csub(), im.ow / L.csub(), &ctx_))) return rc;   // table is ty)
     // 4:2:0 frames are staged whole (whole-frame calls only: R0 = 0, R1 = oh), every row at its place in the frame
     const auto need = src_rows(p.ty->h_ofs.data(), im.h, im.oh, R0, R1);
     p.S0 = L.whole() ? 0 : need.first;
@@ -1110,7 +1114,7 @@ int srcnn_stage_resize_plane_device(srcnn_ctx* c, const uint8_t* d_src, int w, i
     return SRCNN_OK;
 }
 
-// Host buffers (ProcessSRCNN's alpha): copy the plane in, resize, copy the result out.
+// Host buffers: copy the plane in, resize, copy the result out.
 int srcnn_resize_plane_host(srcnn_ctx* c, const uint8_t* src, int w, int h, size_t src_stride, float scale, uint8_t* dst,
                             size_t dst_stride) {
     ENTER(c);

@@ -508,8 +508,10 @@ static ResizeDev resize_dev(const ResizeArgs& a) {
 
 static int launch_yuv420(Ctx* c, const ResizeArgs& a);
 static int launch_yuv422(Ctx* c, const ResizeArgs& a);
+static int launch_graya(Ctx* c, const ResizeArgs& a);
 
 int launch_color_bicubic(Ctx* c, const ResizeArgs& a) {
+    if (a.order == SRCNN_ORDER_GRAYA) return launch_graya(c, a);
     if (yuv420(a.order) || yuv422(a.order)) {
         if (c->ka_int) {   // x2 / x4: luma and chroma in one launch of the integer-scale kernel
             ResizeArgs y = a;
@@ -661,6 +663,34 @@ static int launch_yuv422(Ctx* c, const ResizeArgs& a) {
     u.tx = ch.tx; u.ty = ch.ty;
     u.nframes = a.nframes; u.src_frame_stride = a.src_frame_stride;
     return launch_color_bicubic(c, u);
+}
+
+// A grey + alpha frame (SRCNN_ORDER_GRAYA).  x2 / x4 with ow % 8 == 0: one launch for grey and alpha (color_bicubic_int.cu).
+// Otherwise two launches of the generic kernels, both on every second byte of the rows (kOrderY422, as a YUY2 / UYVY Y plane):
+// grey from byte 0 into pl.y / pl.y16 as a grey call's, then alpha from byte 1 into the workspace's Cr plane, for the output rows
+// [r0, r1) of `ch` only (the halo rows around them are the CNN's).  (The direct kernels, for strong down-scales, go frame by frame.)
+static int launch_graya(Ctx* c, const ResizeArgs& a) {
+    ResizeArgs y = a;
+    if (c->ka_int) {
+        y.order = SRCNN_ORDER_GRAY;
+        bool done = false;
+        const int rc = launch_graya_int(c, resize_dev(y), a, &done);
+        if (rc || done) return rc;
+    }
+    y.order = kOrderY422;
+    int rc = launch_color_bicubic(c, y);
+    if (rc) return rc;
+    const Chroma420& ch = a.ch;
+    ResizeArgs al;
+    al.order = kOrderY422;
+    al.src = ch.src + 1; al.src_stride = ch.src_pitch;
+    al.sw = ch.sw; al.sh = ch.sh; al.src_row0 = 0; al.src_row1 = ch.sh;
+    al.ow = ch.ow; al.oh = ch.oh;
+    al.row_begin = ch.row_begin; al.row_end = ch.row_end;
+    al.pl.y = ch.dst; al.pl.pitch = ch.dst_pitch; al.pl.row0 = 0; al.pl.rows = ch.oh; al.pl.frame_stride = ch.dst_frame;
+    al.tx = ch.tx; al.ty = ch.ty;
+    al.nframes = a.nframes; al.src_frame_stride = a.src_frame_stride;
+    return launch_color_bicubic(c, al);
 }
 
 // u8 Y plane -> padded FP16 plane (Planes::y16): 8 pixels per thread; the first / last group of a row also writes the
@@ -918,9 +948,52 @@ __global__ void __launch_bounds__(256) k_pack_yuv422(const uint8_t* __restrict__
     d[3] = kUYVY ? y1 : cv;
 }
 
-int launch_pack422(Ctx* c, const MergeArgs& a) {
+// ------------------------------------------------------------------------------------------------
+// K-C for grey + alpha (SRCNN_ORDER_GRAYA): Y' and the resized A' plane (the Cr slot) interleaved into byte pairs.  16 pixels per
+// thread: one 128-bit load of each plane, eight byte permutations, two 128-bit stores (needs 16-byte aligned rows).  Releases its
+// dependents on entry like k_pack_yuv422_v16.
+// ------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) k_pack_ya_v16(const uint8_t* __restrict__ y, const uint8_t* __restrict__ a, size_t pitch, int w,
+                                                     int rows, uint8_t* __restrict__ dst, size_t dst_stride, int groups_per_row) {
+    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+    const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const int row = (int)(gid / groups_per_row), x = 16 * (int)(gid - (long long)row * groups_per_row);
+    if (row >= rows) return;
+    const size_t o = (size_t)row * pitch + x;
+    const uint4 vy = *reinterpret_cast<const uint4*>(y + o), va = *reinterpret_cast<const uint4*>(a + o);
+    const uint32_t wy[4] = {vy.x, vy.y, vy.z, vy.w}, wa[4] = {va.x, va.y, va.z, va.w};
+    uint32_t out[8];
+#pragma unroll
+    for (int k = 0; k < 4; k++) {   // Y0 A0 Y1 A1 | Y2 A2 Y3 A3
+        out[2 * k] = __byte_perm(wy[k], wa[k], 0x5140);
+        out[2 * k + 1] = __byte_perm(wy[k], wa[k], 0x7362);
+    }
+    uint8_t* d = dst + (size_t)row * dst_stride + 2 * (size_t)x;
+    if (x + 15 < w) {
+        reinterpret_cast<uint4*>(d)[0] = make_uint4(out[0], out[1], out[2], out[3]);
+        reinterpret_cast<uint4*>(d)[1] = make_uint4(out[4], out[5], out[6], out[7]);
+    } else {   // the row's last, partial group: one aligned 16-bit store per pixel (static indices keep out in registers)
+#pragma unroll
+        for (int j = 0; j < 16; j++)
+            if (x + j < w) reinterpret_cast<uint16_t*>(d)[j] = (uint16_t)(out[j >> 1] >> (16 * (j & 1)));
+    }
+}
+
+// The same for destinations the 128-bit stores cannot take: one pixel per thread, byte stores.
+__global__ void __launch_bounds__(256) k_pack_ya(const uint8_t* __restrict__ y, const uint8_t* __restrict__ a, size_t pitch, int w, int rows,
+                                                 uint8_t* __restrict__ dst, size_t dst_stride) {
+    const long long gid = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const int row = (int)(gid / w), x = (int)(gid - (long long)row * w);
+    if (row >= rows) return;
+    const size_t o = (size_t)row * pitch + x;
+    uint8_t* d = dst + (size_t)row * dst_stride + 2 * (size_t)x;
+    d[0] = y[o];
+    d[1] = a[o];
+}
+
+int launch_pack(Ctx* c, const MergeArgs& a) {
     if (a.rows <= 0 || a.w <= 0) return SRCNN_OK;
-    const bool uyvy = a.order == SRCNN_ORDER_UYVY;
+    const bool ya = a.order == SRCNN_ORDER_GRAYA, uyvy = a.order == SRCNN_ORDER_UYVY;
     const bool wide = ((((uintptr_t)a.dst) | a.dst_stride | (uintptr_t)a.y | (uintptr_t)a.cr | (uintptr_t)a.cb | a.pitch) & 15) == 0 &&
                       a.pitch >= align_up((size_t)a.w, 16);
     c->merge_sel = -1;   // as for a merge: the whole-path caller says afterwards which Cr/Cb pair this launch reads
@@ -928,8 +1001,14 @@ int launch_pack422(Ctx* c, const MergeArgs& a) {
     if (wide) {
         const int groups16 = (a.w + 15) / 16;
         const long long blocks = ((long long)groups16 * a.rows + 255) / 256;
-        (uyvy ? k_pack_yuv422_v16<true> : k_pack_yuv422_v16<false>)<<<(unsigned)blocks, 256, 0, c->stream>>>(a.y, a.cr, a.cb, a.pitch, a.w,
-                                                                                                            a.rows, a.dst, a.dst_stride, groups16);
+        if (ya)
+            k_pack_ya_v16<<<(unsigned)blocks, 256, 0, c->stream>>>(a.y, a.cr, a.pitch, a.w, a.rows, a.dst, a.dst_stride, groups16);
+        else
+            (uyvy ? k_pack_yuv422_v16<true> : k_pack_yuv422_v16<false>)<<<(unsigned)blocks, 256, 0, c->stream>>>(a.y, a.cr, a.cb, a.pitch, a.w,
+                                                                                                                a.rows, a.dst, a.dst_stride, groups16);
+    } else if (ya) {
+        const long long blocks = ((long long)a.w * a.rows + 255) / 256;
+        k_pack_ya<<<(unsigned)blocks, 256, 0, c->stream>>>(a.y, a.cr, a.pitch, a.w, a.rows, a.dst, a.dst_stride);
     } else {
         const long long blocks = ((long long)(a.w / 2) * a.rows + 255) / 256;
         (uyvy ? k_pack_yuv422<true> : k_pack_yuv422<false>)<<<(unsigned)blocks, 256, 0, c->stream>>>(a.y, a.cr, a.cb, a.pitch, a.w, a.rows,

@@ -138,5 +138,7 @@ int launch_color_bicubic_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bo
 // the same for a 4:2:0 or packed 4:2:2 frame (a.order NV12 / I420 / YUY2 / UYVY; p describes its Y plane as a grey call's, a.ch
 // its chroma): luma and chroma in one launch
 int launch_yuv_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bool* done);
+// the same for a grey + alpha frame (a.order SRCNN_ORDER_GRAYA; p describes its grey plane as a grey call's, a.ch its alpha plane)
+int launch_graya_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bool* done);
 
 }  // namespace srcnn

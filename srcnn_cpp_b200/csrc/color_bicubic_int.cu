@@ -639,6 +639,26 @@ __global__ void __launch_bounds__(96, S == 2 ? SRCNN_KA_MINB : SRCNN_KA_MINB4) k
         if (b == t.ntiles + tc.ntiles - 1) asm volatile("griddepcontrol.wait;" ::: "memory");
 }
 
+// ------------------------------------------------------------------------------------------------
+// Grey + alpha frames (SRCNN_ORDER_GRAYA): ONE launch for both planes.  A row of byte pairs (G A G A ...) keeps grey where a YUY2 row
+// keeps its Y bytes (the even bytes) and alpha where a UYVY row keeps them (the odd bytes), so both tile kinds are gray_tile's 4:2:2
+// luma staging as it is -- group loads of 64 bits when the rows are 8-byte aligned, 32 bits when 4-byte aligned, clamped bytes
+// otherwise -- and its walk.  CTAs [0, t.ntiles) stage the even bytes into the plane the CNN reads (p: the FP16 plane or the u8
+// Y plane); the rest stage the odd bytes into the workspace's Cr plane (pa: the same source rows, the u8 output plane A' and the
+// output rows [r0, r1) -- the halo rows around them are the CNN's).  The source is staged twice, once per tile kind.
+// ------------------------------------------------------------------------------------------------
+template <int S>
+__global__ void __launch_bounds__(96, S == 2 ? SRCNN_KA_MINB : SRCNN_KA_MINB4) k_graya_bicubic_int(const ResizeDev p, const IntTaps t,
+                                                                                                 const ResizeDev pa, const IntTaps ta) {
+    __shared__ __align__(16) uint8_t sP[kIRows][kGPitch];
+    const int b = (int)blockIdx.x;
+    if (b < t.ntiles) gray_tile<S, SRCNN_ORDER_YUY2>(p, t, b, sP);
+    else gray_tile<S, SRCNN_ORDER_UYVY>(pa, ta, b - t.ntiles, sP);
+    // may start beside the previous call's merge / pack kernel (api.cu, may_start_early): the last CTA waits for it, as in
+    // k_color_bicubic_int
+    if (b == t.ntiles + ta.ntiles - 1) asm volatile("griddepcontrol.wait;" ::: "memory");
+}
+
 inline int floordiv(int a, int b) { return a >= 0 ? a / b : -((-a + b - 1) / b); }
 
 // one launch of an integer-scale kernel, ordinary or with programmatic stream serialisation
@@ -726,6 +746,16 @@ int launch_yuv(Ctx* c, const ResizeDev& p, IntTaps& t, const ChromaDev& q, IntTa
     return rc;
 }
 
+template <int S>
+int launch_ga(Ctx* c, const ResizeDev& p, IntTaps& t, const ResizeDev& pa, IntTaps& ta, int nframes, bool early, bool* done) {
+    bool ok = false;
+    int rc;
+    if ((rc = plan_tiles<k_graya_bicubic_int<S>, 96>(c, nframes, t, &ta, &ok)) || !ok) return rc;
+    rc = launch_ka(c, k_graya_bicubic_int<S>, t.ntiles + ta.ntiles, 96, early, p, t, pa, ta);
+    *done = rc == SRCNN_OK;
+    return rc;
+}
+
 // the constant tap phases of an integer scale S and the source rows whose output rows [row_begin, row_end) are wanted
 void int_taps(const TapTable* tx, const TapTable* ty, int S, int row_begin, int row_end, IntTaps& t) {
     const float sc = 1.0f / 4194304.0f;   // 2^-22, exact
@@ -783,6 +813,29 @@ int launch_yuv_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bool* done) 
         {launch_yuv<4, SRCNN_ORDER_NV12>, launch_yuv<4, SRCNN_ORDER_I420>, launch_yuv<4, SRCNN_ORDER_YUY2>, launch_yuv<4, SRCNN_ORDER_UYVY>}};
     // a.early is false for every 4:2:0 call: it launches no merge (api.cu)
     return kLaunch[S == 4][a.order - SRCNN_ORDER_NV12](c, p, t, q, tc, std::max(1, a.nframes), a.early, done);
+}
+
+int launch_graya_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bool* done) {
+    *done = false;
+    const Chroma420& ch = a.ch;
+    const int S = a.tx->int_scale;
+    if (S == 0 || a.ty->int_scale != S || (a.ow & 7) || a.row_end <= a.row_begin || ch.row_end <= ch.row_begin) return SRCNN_OK;
+    ResizeDev pa = p;   // alpha: the same source rows, into the Cr plane (output row r at ch.dst + r * ch.dst_pitch), no FP16 copy
+    pa.y = ch.dst; pa.pitch = ch.dst_pitch; pa.plane_frame = ch.dst_frame; pa.plane_row0 = 0; pa.y16 = nullptr;
+    pa.row_begin = ch.row_begin; pa.row_end = ch.row_end;
+    // stores: 8 bytes per lane and row into the u8 planes, 16 into the FP16 plane
+    if ((((uintptr_t)p.y | p.pitch | p.plane_frame | (uintptr_t)pa.y | pa.pitch | pa.plane_frame) & 7) != 0) return SRCNN_OK;
+    if (p.y16 && (((uintptr_t)p.y16 | p.pitch16 | p.y16_frame) & 15) != 0) return SRCNN_OK;
+
+    IntTaps t = {}, ta = {};
+    int_taps(a.tx, a.ty, S, a.row_begin, a.row_end, t);
+    int_taps(a.tx, a.ty, S, ch.row_begin, ch.row_end, ta);
+    // both tile kinds read the same rows of byte pairs: 64-bit group loads when they are 8-byte aligned, 32-bit when 4-byte aligned
+    const uintptr_t al = (uintptr_t)p.src | p.src_stride | p.src_frame;
+    t.vec_ok = ta.vec_ok = (al & 7) == 0 ? 2 : ((al & 3) == 0 ? 1 : 0);
+    t.ntx = ta.ntx = ((a.ow + kITW - 1) / kITW + 2) / 3;   // a CTA per three adjacent tiles, as in a grey call
+    const int nframes = std::max(1, a.nframes);
+    return S == 2 ? launch_ga<2>(c, p, t, pa, ta, nframes, a.early, done) : launch_ga<4>(c, p, t, pa, ta, nframes, a.early, done);
 }
 
 int launch_color_bicubic_int(Ctx* c, const ResizeDev& p, const ResizeArgs& a, bool* done) {

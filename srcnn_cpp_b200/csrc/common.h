@@ -206,6 +206,8 @@ constexpr int kOrderY422 = 101, kOrderUV422 = 102;
 // Packed 4:2:2 frames (SRCNN_ORDER_YUY2 / _UYVY) use the same description: `src` is row 0 of the packed frame (src_pitch its
 // stride, src_v = 0: the order says where U and V sit in a macropixel), `dst` / `dst + dst_v` are the workspace's Cr / Cb planes
 // (U', V'), `dst` shifted so that chroma output row r is at dst + r * dst_pitch; sizes w/2 x h -> ow/2 x oh, rows [r0, r1).
+// Grey + alpha frames (SRCNN_ORDER_GRAYA) describe their alpha plane the same way: `src` is row 0 of the frame (alpha is byte 1 of
+// each pixel), `dst` the workspace's Cr plane (A'); sizes w x h -> ow x oh, rows [r0, r1).
 struct Chroma420 {
     const uint8_t* src = nullptr;   // chroma row 0 of frame 0 (NV12: the interleaved pairs, I420: the U plane)
     size_t src_pitch = 0;           // bytes between chroma rows
@@ -233,12 +235,13 @@ struct ResizeArgs {
     int nframes = 1;      // same-sized frames in one launch, src_frame_stride / pl.frame_stride apart
     size_t src_frame_stride = 0;
     bool early = false;   // may start while the previous kernel of the stream (a merge kernel of ours) is still running
-    Chroma420 ch;         // SRCNN_ORDER_NV12 / _I420 / _YUY2 / _UYVY: the chroma planes (the Y plane is `src`, as for a grey call)
+    Chroma420 ch;         // SRCNN_ORDER_NV12 / _I420 / _YUY2 / _UYVY: the chroma planes (the Y plane is `src`, as for a grey call);
+                          // SRCNN_ORDER_GRAYA: the alpha plane
 };
 int launch_color_bicubic(Ctx* c, const ResizeArgs& a);   // order SRCNN_ORDER_GRAY: the one plane, into pl.y / pl.y16;
                                                          // SRCNN_ORDER_BGRA / _RGBA: pl.a as well;
-                                                         // SRCNN_ORDER_NV12 / _I420 / _YUY2 / _UYVY: Y into pl.y / pl.y16,
-                                                         // chroma per `ch`
+                                                         // SRCNN_ORDER_NV12 / _I420 / _YUY2 / _UYVY / _GRAYA: Y into pl.y /
+                                                         // pl.y16, chroma or alpha per `ch`
 inline bool four_channel(int order) { return order == SRCNN_ORDER_BGRA || order == SRCNN_ORDER_RGBA; }
 
 struct MergeArgs {
@@ -254,8 +257,9 @@ struct MergeArgs {
 };
 int launch_merge(Ctx* c, const MergeArgs& a);
 // packed 4:2:2 (a.order SRCNN_ORDER_YUY2 / _UYVY): Y' (a.y) and U', V' (a.cr, a.cb: a.w/2 columns, same pitch) interleaved into
-// macropixels; in place of the merge, and like it the last kernel of the call (releases its dependents on entry)
-int launch_pack422(Ctx* c, const MergeArgs& a);
+// macropixels; grey + alpha (SRCNN_ORDER_GRAYA): Y' (a.y) and A' (a.cr) interleaved into byte pairs.  In place of the merge, and
+// like it the last kernel of the call (releases its dependents on entry)
+int launch_pack(Ctx* c, const MergeArgs& a);
 void note_merge(Ctx* c);   // api.cu: this context has just put a merge kernel (which releases its dependents early) on its stream
 // u8 Y plane -> FP16 plane in the Planes::y16 layout (replicated edge columns included)
 int launch_y8_to_y16(Ctx* c, const uint8_t* y, size_t pitch, int w, int rows, uint8_t* y16, size_t pitch16);

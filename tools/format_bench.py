@@ -17,12 +17,17 @@ host-buffer end-to-end call, and a few format-specific lines.  One context, seed
           srcnn_stage_resize_plane_device calls on already de-interleaved U / V planes (the de-interleave not timed); the host
           call NV12 / YUY2 against BGR.  The frames, the Y planes and the U / V planes of one buffer set hold the same content,
           and every line says whether both orders gave the composition's bytes.
+  graya   grey + alpha (SRCNN_ORDER_GRAYA) against the grey call on the grey plane alone, the colour (BGR) call on a frame of the
+          same size, and the composition a caller has without the path -- the grey call plus srcnn_stage_resize_plane_device on an
+          already de-interleaved alpha plane (the de-interleave and re-interleave not timed); the host call GRAYA against grey and
+          BGR; every line checks that the GRAYA bytes equal the composition's.  Also ProcessSRCNN with d = 2 before and after it
+          became one GRAYA call, as for d = 4 above.
 
 Timing: CUDA events on the context stream around blocks of back-to-back calls (so the colour path keeps its cross-call overlap),
 the forms of a line alternating, median of the blocks.  Every call of a block reads and writes its own buffer set, and the sets
 of one block together are larger than the 126 MB L2.  The host-side lines take a host clock around calls that end in a
 synchronise.  Every line carries the GPU name and its power limit.
-usage: format_bench.py [--format gray|rgba|yuv420|yuv422|all] [--quick]"""
+usage: format_bench.py [--format gray|rgba|yuv420|yuv422|graya|all] [--quick]"""
 import argparse
 import ctypes as C
 import json
@@ -37,7 +42,7 @@ import torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import srcnn_cpp_b200 as S
 
-FORMATS = ("gray", "rgba", "yuv420", "yuv422")
+FORMATS = ("gray", "rgba", "yuv420", "yuv422", "graya")
 ap = argparse.ArgumentParser()
 ap.add_argument("--format", choices=FORMATS + ("all",), default="all")
 ap.add_argument("--quick", action="store_true")
@@ -205,7 +210,35 @@ def yuv_forms(fmt, w, h, ow, oh, scale, n):
     return nb, forms, fields
 
 
-FORMS = dict(gray=gray_forms, rgba=rgba_forms, yuv420=lambda *a: yuv_forms("yuv420", *a), yuv422=lambda *a: yuv_forms("yuv422", *a))
+def graya_forms(w, h, ow, oh, scale, n):
+    nb = sets_for(n * (w * h + ow * oh) * 2)
+    g = torch.Generator(device="cuda").manual_seed(0)
+    rnd = lambda *shape: torch.randint(0, 256, shape, dtype=torch.uint8, device="cuda", generator=g)
+    sets = []
+    for _ in range(nb):
+        y, a = rnd(n, h, w), rnd(n, h, w)
+        sets.append(dict(y=y, a=a, ga=torch.stack([y, a], dim=-1).contiguous(), bgr=rnd(n, h, w, 3), o_ga=zeros(n, oh, ow, 2),
+                         o_y=zeros(n, oh, ow), o_a=zeros(n, oh, ow), o_bgr=zeros(n, oh, ow, 3)))
+
+    def composition(s):
+        (eng.process_device(s["y"][0], scale, s["o_y"][0], order=S.ORDER_GRAY) if n == 1 else
+         eng.process_batch_device(s["y"], scale, s["o_y"], order=S.ORDER_GRAY))
+        for f in range(n):
+            eng.stage_resize_plane(s["a"][f], scale, s["o_a"][f])
+
+    forms = dict(graya=whole(sets, "ga", "o_ga", S.ORDER_GRAYA, scale, n), grey=whole(sets, "y", "o_y", S.ORDER_GRAY, scale, n),
+                 bgr=whole(sets, "bgr", "o_bgr", S.ORDER_BGR, scale, n), composition=[lambda s=s: composition(s) for s in sets])
+
+    def fields(t):
+        same = all(torch.equal(s["o_ga"][..., 0], s["o_y"]) and torch.equal(s["o_ga"][..., 1], s["o_a"]) for s in sets)
+        return {**{k + "_ms_per_frame": round(v, 4) for k, v in t.items()}, "graya_over_grey": round(t["graya"] / t["grey"], 3),
+                "graya_over_bgr": round(t["graya"] / t["bgr"], 3), "graya_over_composition": round(t["graya"] / t["composition"], 3),
+                "bytes_equal_composition": bool(same)}
+    return nb, forms, fields
+
+
+FORMS = dict(gray=gray_forms, rgba=rgba_forms, yuv420=lambda *a: yuv_forms("yuv420", *a), yuv422=lambda *a: yuv_forms("yuv422", *a),
+             graya=graya_forms)
 
 
 def device_line(fmt, name, w, h, scale, n, rounds):
@@ -255,6 +288,14 @@ def host_line(fmt, w, h, scale, reps):
         q, qb = host_ms(img.reshape(-1), w, h, w * 4, S.ORDER_BGRA, scale, ow * oh * 4, ow * 4, reps)
         emit(**head, bgr_ms=round(c, 4), bgra_ms=round(q, 4), bgra_over_bgr=round(q / c, 3),
              bgra_colour_bytes_equal_bgr=bool(np.array_equal(qb.reshape(oh, ow, 4)[..., :3], cb.reshape(oh, ow, 3))))
+    elif fmt == "graya":
+        rng = np.random.default_rng(2)
+        ga = rng.integers(0, 256, (h, w, 2), dtype=np.uint8)
+        c, _ = host_ms(rng.integers(0, 256, w * h * 3, dtype=np.uint8), w, h, w * 3, S.ORDER_BGR, scale, ow * oh * 3, ow * 3, reps)
+        y, yb = host_ms(np.ascontiguousarray(ga[..., 0]).reshape(-1), w, h, w, S.ORDER_GRAY, scale, ow * oh, ow, reps)
+        q, qb = host_ms(ga.reshape(-1), w, h, w * 2, S.ORDER_GRAYA, scale, ow * oh * 2, ow * 2, reps)
+        emit(**head, bgr_ms=round(c, 4), grey_ms=round(y, 4), graya_ms=round(q, 4), graya_over_bgr=round(q / c, 3),
+             graya_over_grey=round(q / y, 3), graya_grey_bytes_equal_grey=bool(np.array_equal(qb.reshape(oh, ow, 2)[..., 0], yb.reshape(oh, ow))))
     else:   # 4:2:0: h * 3/2 rows of w bytes; 4:2:2: h rows of 2w bytes
         if fmt == "yuv420":
             name, order, src_bytes, stride, dst_bytes, dstride = "nv12", S.ORDER_NV12, w * h * 3 // 2, w, ow * oh * 3 // 2, ow
@@ -280,27 +321,32 @@ def stage_line(w, h, scale, rounds):
          bytes=nbytes, TBps=round(nbytes / (ms * 1e-3) / 1e12, 3), share_of_hbm_peak=round(nbytes / (ms * 1e-3) / HBM_PEAK, 3))
 
 
-def process_srcnn_line(w, h, scale, reps):
+def process_srcnn_line(w, h, scale, reps, d=4):
     fn = S.load_library()._Z12ProcessSRCNNPKhjjjfRPhRj
     fn.restype = C.c_int
     fn.argtypes = [C.c_void_p, C.c_uint, C.c_uint, C.c_uint, C.c_float, C.POINTER(C.c_void_p), C.POINTER(C.c_uint)]
     ow, oh = S.out_dims(w, h, scale)
     rgba = rgba_seeded(101, (1, h, w))[0].cpu().numpy()
+    if d == 2:   # grey + alpha: the G and alpha bytes of the same image
+        rgba = np.ascontiguousarray(rgba[..., 1::2])
 
-    def before():   # the old d = 4 composition, step by step
-        rgb = np.ascontiguousarray(rgba[..., :3])
-        alpha = np.ascontiguousarray(rgba[..., 3])
-        out = np.empty((oh, ow, 4), np.uint8)
-        out[..., :3] = eng.process(rgb, scale, order=S.ORDER_RGB)
-        out[..., 3] = eng.resize_plane(alpha, scale)
+    def before():   # the old composition, step by step
+        col = np.ascontiguousarray(rgba[..., :d - 1]) if d == 4 else np.ascontiguousarray(rgba[..., 0])
+        alpha = np.ascontiguousarray(rgba[..., d - 1])
+        out = np.empty((oh, ow, d), np.uint8)
+        if d == 4:
+            out[..., :3] = eng.process(col, scale, order=S.ORDER_RGB)
+        else:
+            out[..., 0] = eng.process(col, scale, order=S.ORDER_GRAY)
+        out[..., d - 1] = eng.resize_plane(alpha, scale)
         return out
 
     def after():
         out, sz = C.c_void_p(), C.c_uint()
-        if fn(rgba.ctypes.data, w, h, 4, C.c_float(scale), C.byref(out), C.byref(sz)) != 0:
+        if fn(rgba.ctypes.data, w, h, d, C.c_float(scale), C.byref(out), C.byref(sz)) != 0:
             raise RuntimeError("ProcessSRCNN failed")
         # the caller delete[]s the buffer in C++; here it is copied out and left to the process (a few calls of a benchmark)
-        return np.ctypeslib.as_array((C.c_uint8 * sz.value).from_address(out.value)).reshape(oh, ow, 4).copy()
+        return np.ctypeslib.as_array((C.c_uint8 * sz.value).from_address(out.value)).reshape(oh, ow, d).copy()
 
     times = {before: [], after: []}
     for fn_ in (before, after):
@@ -312,10 +358,12 @@ def process_srcnn_line(w, h, scale, reps):
             fn_()
             times[fn_].append(time.perf_counter() - t0)
     b, a = float(np.median(times[before])) * 1e3, float(np.median(times[after])) * 1e3
-    emit(line="ProcessSRCNN_d4", src="%dx%d" % (w, h), dst="%dx%d" % (ow, oh), scale=scale, before_ms=round(b, 3), after_ms=round(a, 3),
-         after_over_before=round(a / b, 3), bytes_equal=bool(np.array_equal(before(), after())),
-         colour_bytes_equal_bgr_path=bool(np.array_equal(after()[..., :3], eng.process(np.ascontiguousarray(rgba[..., :3]), scale,
-                                                                                          order=S.ORDER_RGB))))
+    extra = {}
+    if d == 4:
+        extra["colour_bytes_equal_bgr_path"] = bool(np.array_equal(after()[..., :3], eng.process(np.ascontiguousarray(rgba[..., :3]),
+                                                                                                 scale, order=S.ORDER_RGB)))
+    emit(line="ProcessSRCNN_d%d" % d, src="%dx%d" % (w, h), dst="%dx%d" % (ow, oh), scale=scale, before_ms=round(b, 3), after_ms=round(a, 3),
+         after_over_before=round(a / b, 3), bytes_equal=bool(np.array_equal(before(), after())), **extra)
 
 
 R = 3 if ARGS.quick else 7
@@ -329,6 +377,6 @@ for fmt in FORMATS if ARGS.format == "all" else (ARGS.format,):
         stage_line(3840, 2160, 4.0, R)
         stage_line(1920, 1080, 1.5, R)
     host_line(fmt, 1920, 1080, 2.0, 10 if ARGS.quick else 30)
-    if fmt == "rgba":
-        process_srcnn_line(1920, 1080, 2.0, 5 if ARGS.quick else 15)
+    if fmt in ("rgba", "graya"):
+        process_srcnn_line(1920, 1080, 2.0, 5 if ARGS.quick else 15, d=4 if fmt == "rgba" else 2)
 eng.close()
