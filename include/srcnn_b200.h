@@ -267,7 +267,14 @@ int srcnn_stage_merge_device(srcnn_ctx* ctx, const uint8_t* d_y, const uint8_t* 
 /* ---- optional: frawscale-compatible float-plane resize (SURVEY 8f, N3) --------------------------- */
 /* FRAWResizeEngine::scale (src/frawscale.h:160-161, src/frawscale.cpp:162-286) on device float planes (tight
  * rows).  filter: 0 = Box, 1 = Bilinear, 2 = Bicubic (Mitchell B = C = 1/3, the reference default).  Not used by
- * the bin/srcnn path (the reference never calls frawscale either); bit-identical to the compiled reference. */
+ * the bin/srcnn path (the reference never calls frawscale either); bit-identical to the compiled reference: every
+ * non-NaN output has the reference's bits, and NaN appears where it does.  Only NaN-ness is promised: on a B200 a NaN
+ * input kept its sign and payload and Inf - Inf gave x86's NaN in every case measured, but which payload survives a sum
+ * of several NaNs is the hardware's choice.  The claim rests on the golden vectors and on a float64 restatement
+ * (oracle/fraw.py) that equals them, checked against the stage on planes built to show FMA contraction, another tap
+ * order, a float accumulator and off-by-an-ulp table weights (tests/test_fraw_precision.py).  A plane of equal size is
+ * copied whole.  Source and destination must not overlap (SRCNN_E_ARG): a one-axis resize reads the source while it
+ * writes the destination.  At most 65535 rows on either side. */
 enum { SRCNN_FRAW_BOX = 0, SRCNN_FRAW_BILINEAR = 1, SRCNN_FRAW_BICUBIC = 2 };
 int srcnn_fraw_scale_device(srcnn_ctx* ctx, const float* d_src, unsigned src_w, unsigned src_h, unsigned dst_w,
                             unsigned dst_h, float* d_dst, int filter);

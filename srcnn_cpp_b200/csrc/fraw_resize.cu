@@ -13,10 +13,11 @@
 //     vertical (src/frawscale.cpp:195-278);
 //   * every output sample = (float) of a double sum accumulated in tap order with separate multiply and
 //     add (__dmul_rn/__dadd_rn), as the -O0 x86-64 reference objects do (src/frawscale.cpp:316-325, 369-378).
-// Bit-identical to the compiled reference (tests/test_fraw.py).  HBM-bound: 4 B read + 4 B written per
-// sample and pass.  One documented deviation: for equal source and destination size the reference copies
-// only sizeof(unsigned short) bytes per sample (src/frawscale.cpp:189) and leaves the rest uninitialised;
-// this stage copies the whole plane.
+// Bit-identical to the compiled reference (tests/test_fraw.py) and to a float64 restatement of it on planes built to
+// expose FMA, tap order and last-bit table changes (tests/test_fraw_precision.py); NaN only as NaN.  HBM-bound: 4 B
+// read + 4 B written per sample and pass.  One documented deviation: for equal source and destination size the
+// reference copies only sizeof(unsigned short) bytes per sample (src/frawscale.cpp:189) and leaves the rest
+// uninitialised; this stage copies the whole plane.
 #include <cmath>
 
 #include "common.h"
@@ -206,6 +207,22 @@ void fraw_release(Ctx* c) {
 
 using namespace srcnn;
 
+// FrawTable of one axis (host code only, no device needed).  With left, count and w all null only *window is written;
+// otherwise left[dst], count[dst] and w[dst * (window + 1)] receive the table as the passes read it.
+extern "C" __attribute__((visibility("default"))) int srcnn_debug_fraw_table(int filter, unsigned dst, unsigned src, int* left,
+                                                                             int* count, double* w, int* window) {
+    if (filter < 0 || filter > 2 || dst == 0 || src == 0 || !window) return SRCNN_E_ARG;
+    const bool query = !left && !count && !w;
+    if (!query && (!left || !count || !w)) return SRCNN_E_ARG;
+    const FrawTable t(FrawFilter(filter), dst, src);
+    *window = t.window;
+    if (query) return SRCNN_OK;
+    std::copy(t.left.begin(), t.left.end(), left);
+    std::copy(t.count.begin(), t.count.end(), count);
+    std::copy(t.w.begin(), t.w.end(), w);
+    return SRCNN_OK;
+}
+
 extern "C" int srcnn_fraw_scale_device(srcnn_ctx* c, const float* d_src, unsigned sw, unsigned sh, unsigned dw, unsigned dh,
                                        float* d_dst, int filter) {
     if (!c) return SRCNN_E_ARG;
@@ -215,6 +232,10 @@ extern "C" int srcnn_fraw_scale_device(srcnn_ctx* c, const float* d_src, unsigne
     if (sw == 0 || sh == 0 || dw == 0 || dh == 0) return fail(c, SRCNN_E_ARG, "empty plane");      // :168-169
     if (filter < 0 || filter > 2) return fail(c, SRCNN_E_ARG, "unknown filter %d", filter);
     if (dh > 65535u || sh > 65535u) return fail(c, SRCNN_E_ARG, "plane taller than 65535 rows: split it into bands");
+    // a one-pass resize reads d_src while it writes d_dst (and a copy of overlapping ranges is undefined): no overlap
+    const uintptr_t s0 = (uintptr_t)d_src, s1 = s0 + sizeof(float) * (size_t)sw * sh;
+    const uintptr_t d0 = (uintptr_t)d_dst, d1 = d0 + sizeof(float) * (size_t)dw * dh;
+    if (s0 < d1 && d0 < s1) return fail(c, SRCNN_E_ARG, "source and destination planes overlap");
     const FrawFilter f(filter);
     if (sw == dw && sh == dh) {
         SRCNN_CUDA(c, cudaMemcpyAsync(d_dst, d_src, sizeof(float) * (size_t)sw * sh, cudaMemcpyDeviceToDevice, c->stream));
