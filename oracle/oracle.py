@@ -63,6 +63,12 @@ class Oracle:
         L.orc_pipeline.restype = C.c_int
         L.orc_pipeline.argtypes = [_f32p, _u8p, C.c_size_t, C.c_int, C.c_int, C.c_float, _u8p, C.c_size_t,
                                    _u8p, _u8p, _u8p, _u8p]
+        vp = C.c_void_p
+        L.orc_at_modes.restype = C.c_int
+        L.orc_cnn_at.restype = C.c_int
+        L.orc_cnn_at.argtypes = [vp, vp, C.c_int, C.c_int, vp, vp, C.c_int, C.c_int, vp, vp]
+        L.orc_act2_at.restype = C.c_int
+        L.orc_act2_at.argtypes = [vp, vp, C.c_int, C.c_int, vp, vp, C.c_int, C.c_int, vp]
         self.params = load_params()
 
     def threads(self):
@@ -118,6 +124,38 @@ class Oracle:
         out = np.empty((h, w), np.uint8)
         rc = self.lib.orc_cnn(_ptr(self.params, _f32p), _ptr(y, _u8p), w, h, _ptr(out, _u8p), None)
         assert rc == 0
+        return out
+
+    # orc_cnn_at modes (oracle/srcnn_oracle.c): 0 is orc_cnn, the others near misses of its arithmetic
+    AT_EXACT, AT_TEMP_DOUBLE, AT_INNER_FLOAT, AT_EXACT_PRODUCTS, AT_CHANNELS_REVERSED, AT_FMA_DOUBLE, AT_TAPS_NM, \
+        AT_B3_DOUBLE, AT_CONV1_FMA, AT_CONV1_BIAS_FIRST, AT_CONV1_JI, AT_CONV2_FMA, AT_CONV2_REVERSED = range(13)
+
+    def _at_args(self, y, rows, cols):
+        y = np.ascontiguousarray(y, dtype=np.uint8)
+        rows = np.ascontiguousarray(rows, dtype=np.int32).ravel()
+        cols = np.ascontiguousarray(cols, dtype=np.int32).ravel()
+        assert rows.shape == cols.shape
+        return y, rows, cols
+
+    def cnn_at(self, y, rows, cols, mode=0):
+        """The CNN at pixels (rows[p], cols[p]) of the u8 plane y -> (temp + b3 as float32, the byte), both [n]"""
+        y, rows, cols = self._at_args(y, rows, cols)
+        h, w = y.shape
+        v = np.empty(rows.size, np.float32)
+        b = np.empty(rows.size, np.uint8)
+        rc = self.lib.orc_cnn_at(self.params.ctypes.data, y.ctypes.data, w, h, rows.ctypes.data, cols.ctypes.data,
+                                 rows.size, int(mode), v.ctypes.data, b.ctypes.data)
+        assert rc == 0, (rc, mode)
+        return v, b
+
+    def act2_at(self, y, rows, cols, mode=0):
+        """conv2's activations at the listed pixels, [n][32] float32 (mode 0 or a conv1 / conv2 near miss)"""
+        y, rows, cols = self._at_args(y, rows, cols)
+        h, w = y.shape
+        out = np.empty((rows.size, 32), np.float32)
+        rc = self.lib.orc_act2_at(self.params.ctypes.data, y.ctypes.data, w, h, rows.ctypes.data, cols.ctypes.data,
+                                  rows.size, int(mode), out.ctypes.data)
+        assert rc == 0, (rc, mode)
         return out
 
     def pipeline(self, bgr, scale, stages=False):

@@ -13,6 +13,7 @@
  *   orc_conv55      Convolution55,    src/srcnn.cpp:189-243
  *   orc_ycrcb2bgr   cv::cvtColor(YCrCb->BGR) call at src/srcnn.cpp:657
  *   orc_pipeline    the timed region of pthreadcall, src/srcnn.cpp:505-659
+ *   orc_cnn_at      orc_cnn at listed pixels, exactly or with one near miss of its arithmetic (tests only)
  *
  * The OpenCV arithmetic lives in a third-party dependency that is NOT vendored in the reference
  * (Makefile:8-9, pkg-config opencv4, no version pin).  It is restated from OpenCV's published
@@ -299,6 +300,125 @@ ORC_API int orc_cnn(const float* params, const uint8_t* y, int w, int h, uint8_t
     orc_conv99x11(params, y, w, h, tmp);
     orc_conv55(params, tmp, w, h, out);
     if (!act2) free(tmp);
+    return 0;
+}
+
+/* ------------------------------------------------------------------------------------------------
+ * The CNN at listed pixels only, exactly (mode 0) or with one near miss of its arithmetic (modes 1-12).
+ * Mode 0 is orc_conv99x11 + orc_conv55 restricted to the pixels asked for: the same clamped 13x13 field,
+ * the same roundings in the same order.  The near misses are what a kernel that claims bit-identity
+ * could plausibly do instead; tests/test_fp32_cnn_witnesses.py builds planes on which they show.
+ * fma / fmaf round once (C99 7.12.13.1); nothing else here contracts (SAFE_FP in the Makefile).
+ * ---------------------------------------------------------------------------------------------- */
+enum {
+    ORC_AT_EXACT = 0,
+    ORC_AT_TEMP_DOUBLE = 1,        /* M1 conv3: `temp` accumulated in double, one float rounding at the end */
+    ORC_AT_INNER_FLOAT = 2,        /* M2 conv3: the inner 25-term sum in float */
+    ORC_AT_EXACT_PRODUCTS = 3,     /* M3 conv3: products formed exactly in double (no float rounding) */
+    ORC_AT_CHANNELS_REVERSED = 4,  /* M4 conv3: channels summed 31 .. 0 */
+    ORC_AT_FMA_DOUBLE = 5,         /* M5 conv3: fma(w, a, tp) into the double sum */
+    ORC_AT_TAPS_NM = 6,            /* conv3: (n,m) tap order instead of (m,n) */
+    ORC_AT_B3_DOUBLE = 7,          /* conv3: b3 added in double, then rounded to float */
+    ORC_AT_CONV1_FMA = 8,          /* conv1: acc = fmaf(w, y, acc) */
+    ORC_AT_CONV1_BIAS_FIRST = 9,   /* conv1: accumulator starts at b1 instead of adding it last */
+    ORC_AT_CONV1_JI = 10,          /* conv1: (j,i) tap order */
+    ORC_AT_CONV2_FMA = 11,         /* conv2: res = fmaf(act1, w, res) */
+    ORC_AT_CONV2_REVERSED = 12,    /* conv2: inputs summed 63 .. 0 */
+    ORC_AT_NMODES = 13
+};
+
+ORC_API int orc_at_modes(void) { return ORC_AT_NMODES; }
+
+/* conv1 + ReLU + conv2 + ReLU at image pixel (row, col) (src/srcnn.cpp:283-321), modes 0 and 8-12 */
+static void act2_px(const float* params, const uint8_t* y, int w, int h, int row, int col, int mode, float out[32]) {
+    const float* w1 = params + ORC_W1;
+    const float* b1 = params + ORC_B1;
+    const float* w2 = params + ORC_W2;
+    const float* b2 = params + ORC_B2;
+    float temp[64];
+    for (int k = 0; k < 64; k++) {
+        float acc = mode == ORC_AT_CONV1_BIAS_FIRST ? b1[k] : 0.0f;
+        for (int a = 0; a < 9; a++)
+            for (int b = 0; b < 9; b++) {
+                const int i = mode == ORC_AT_CONV1_JI ? b : a, j = mode == ORC_AT_CONV1_JI ? a : b;
+                const float wv = w1[(k * 9 + i) * 9 + j];
+                const float x = (float)(int)y[(size_t)int_trim(0, h - 1, row + i - 4) * w + int_trim(0, w - 1, col + j - 4)];
+                if (mode == ORC_AT_CONV1_FMA) acc = fmaf(wv, x, acc);
+                else { float p = wv * x; acc = acc + p; }
+            }
+        if (mode != ORC_AT_CONV1_BIAS_FIRST) acc = acc + b1[k];
+        temp[k] = (acc < 0) ? 0 : acc;
+    }
+    for (int k = 0; k < 32; k++) {
+        float res = 0.0f;
+        for (int t = 0; t < 64; t++) {
+            const int i = mode == ORC_AT_CONV2_REVERSED ? 63 - t : t;
+            if (mode == ORC_AT_CONV2_FMA) res = fmaf(temp[i], w2[k * 64 + i], res);
+            else { float p = temp[i] * w2[k * 64 + i]; res = res + p; }
+        }
+        res = res + b2[k];
+        out[k] = (res < 0) ? 0 : res;
+    }
+}
+
+/* conv3 at (row, col) over the 25 clamped act2 positions (src/srcnn.cpp:213-240), modes 0-7; returns temp + b3 */
+static float conv55_px(const float* params, const float a2[25][32], int mode) {
+    const float* w3 = params + ORC_W3;
+    const float b3 = params[ORC_B3];
+    float temp = 0;
+    double td = 0;
+    for (int t = 0; t < 32; t++) {
+        const int i = mode == ORC_AT_CHANNELS_REVERSED ? 31 - t : t;
+        double tp = 0;
+        float tf = 0;
+        for (int a = 0; a < 5; a++)
+            for (int b = 0; b < 5; b++) {
+                const int m = mode == ORC_AT_TAPS_NM ? b : a, n = mode == ORC_AT_TAPS_NM ? a : b;
+                const float wv = w3[(i * 5 + m) * 5 + n], sv = a2[m * 5 + n][i];
+                if (mode == ORC_AT_INNER_FLOAT) { float p = wv * sv; tf = tf + p; }
+                else if (mode == ORC_AT_EXACT_PRODUCTS) tp = tp + (double)wv * (double)sv;
+                else if (mode == ORC_AT_FMA_DOUBLE) tp = fma((double)wv, (double)sv, tp);
+                else { float p = wv * sv; tp = tp + (double)p; }
+            }
+        if (mode == ORC_AT_INNER_FLOAT) tp = (double)tf;
+        if (mode == ORC_AT_TEMP_DOUBLE) td = td + tp;
+        else temp = (float)((double)temp + tp);
+    }
+    if (mode == ORC_AT_TEMP_DOUBLE) temp = (float)td;
+    return mode == ORC_AT_B3_DOUBLE ? (float)((double)temp + (double)b3) : temp + b3;
+}
+
+/* pixels (rows[p], cols[p]), p < n: out_v[p] = temp + b3 (float, before truncation), out_byte[p] = the byte.
+ * Returns -1 for a bad mode or a pixel outside the plane. */
+ORC_API int orc_cnn_at(const float* params, const uint8_t* y, int w, int h, const int* rows, const int* cols, int n,
+                       int mode, float* out_v, uint8_t* out_byte) {
+    if (mode < 0 || mode >= ORC_AT_NMODES) return -1;
+    for (int p = 0; p < n; p++)
+        if (rows[p] < 0 || rows[p] >= h || cols[p] < 0 || cols[p] >= w) return -1;
+    const int mode12 = mode >= ORC_AT_CONV1_FMA ? mode : ORC_AT_EXACT;
+    const int mode3 = mode >= ORC_AT_CONV1_FMA ? ORC_AT_EXACT : mode;
+#pragma omp parallel for schedule(dynamic, 16)
+    for (int p = 0; p < n; p++) {
+        float a2[25][32];
+        for (int m = 0; m < 5; m++)
+            for (int q = 0; q < 5; q++)
+                act2_px(params, y, w, h, int_trim(0, h - 1, rows[p] + m - 2), int_trim(0, w - 1, cols[p] + q - 2), mode12,
+                        a2[m * 5 + q]);
+        const float v = conv55_px(params, (const float(*)[32])a2, mode3);
+        if (out_v) out_v[p] = v;
+        if (out_byte) out_byte[p] = (uint8_t)int_trim(0, 255, (int)v);
+    }
+    return 0;
+}
+
+/* conv2's 32 activations at the listed pixels (out: [n][32]), exactly (mode 0) or under a conv1 / conv2 near miss (8-12) */
+ORC_API int orc_act2_at(const float* params, const uint8_t* y, int w, int h, const int* rows, const int* cols, int n,
+                        int mode, float* out) {
+    if (mode != ORC_AT_EXACT && (mode < ORC_AT_CONV1_FMA || mode >= ORC_AT_NMODES)) return -1;
+    for (int p = 0; p < n; p++)
+        if (rows[p] < 0 || rows[p] >= h || cols[p] < 0 || cols[p] >= w) return -1;
+#pragma omp parallel for schedule(static)
+    for (int p = 0; p < n; p++) act2_px(params, y, w, h, rows[p], cols[p], mode, out + (size_t)p * 32);
     return 0;
 }
 
